@@ -237,6 +237,34 @@ def config_legs(ctx, stream, torch, peak, peaks):
     return out
 
 
+DUMP_SAMPLES = 1 << 16     # per realization and polarization: 2 x 16 x 2^16 x 16 B = 32 MiB for the default batch
+DUMP_FIELD_BYTES = 48 << 20   # larger batches get fewer samples so that a dump stays below 64 MB
+DUMP_SEED = 20240601
+
+
+def dump_outputs(d, work, link):
+    """What the timed step hands its caller, from the last timed step: the received field of every realization and
+    the number of SSFM steps each span took.  The field (32 MiB per realization) is sampled at DUMP_SAMPLES indices
+    drawn once from a fixed seed, the same in every run, so that two builds can be compared output for output:
+      field_x.npy, field_y.npy  float64 [batch, S, 2]  (real, imaginary) at the S sampled indices
+      sample_index.npy          float64 [S]            the indices into the 2^20 samples of a realization
+      ncycle.npy                float64 [spans, batch] steps per span and realization"""
+    os.makedirs(d, exist_ok=True)
+    n = work.nfft
+    ns = min(DUMP_SAMPLES, n, DUMP_FIELD_BYTES // (32 * work.batch))
+    idx = np.sort(np.random.Generator(np.random.PCG64(DUMP_SEED)).choice(n, ns, replace=False))
+    fx = np.empty((work.batch, idx.size, 2))
+    fy = np.empty_like(fx)
+    for b in range(work.batch):                    # one realization at a time keeps the host copy at 32 MiB
+        x, y = work.download(b0=b, nb=1)
+        for out, f in ((fx, x), (fy, y)):
+            out[b, :, 0], out[b, :, 1] = f[0, 0, idx].real, f[0, 0, idx].imag
+    np.save(os.path.join(d, 'field_x.npy'), fx)
+    np.save(os.path.join(d, 'field_y.npy'), fy)
+    np.save(os.path.join(d, 'sample_index.npy'), idx.astype(np.float64))
+    np.save(os.path.join(d, 'ncycle.npy'), np.array(link.ncycles, dtype=np.float64))
+
+
 def _claim_stdout():
     """Keep stdout for the one JSON line: libraries (NCCL's version banner, torchrun notices) that write to
     file descriptor 1 are redirected to stderr; returns a writer bound to the original stdout."""
@@ -261,6 +289,8 @@ def main():
     ap.add_argument('--mc-realizations', type=int, default=1024,
                     help='Monte-Carlo leg (C5): realizations in TOTAL over all ranks (strong scaling)')
     ap.add_argument('--no-configs', action='store_true', help='skip the per-configuration legs (C1, C3, C4)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help="write rank 0's output of the last timed step to DIR/*.npy (see dump_outputs)")
     args = ap.parse_args()
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
@@ -328,6 +358,8 @@ def main():
     barrier()
     ms = e0.elapsed_time(e1)
     gpu_launches = ctx.launches - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, work, link)
     sampler.stop_flag = True
     t = torch.tensor([ms, float(total)], dtype=torch.float64, device='cuda')
     if world > 1:

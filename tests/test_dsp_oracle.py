@@ -1,6 +1,6 @@
 """The DSP oracle (oracle/dsp_oracle.py) pinned against the reference's own M source, executed by the mini interpreter:
 cmaadaptivefilter.m, samp2pat.m, pat_decoder.m (+ pat2stars.m, stars2pat.m, fastshift.m, nmod.m) and the sub-functions
-vitvit / cmapolardemux of dsp4cohdec.m.  CPU only; needs the reference tree (skipped on the GPU box)."""
+vitvit / cmapolardemux of dsp4cohdec.m.  CPU only; the pins need the toolbox's M source and skip without it."""
 import os
 
 import numpy as np
@@ -10,7 +10,7 @@ import oracle.dsp_oracle as dsp
 from oracle.mini_m.interp import Interp, MStruct, to_m
 
 REF = '/root/reference'
-pytestmark = pytest.mark.skipif(not os.path.exists(os.path.join(REF, 'dsp4cohdec.m')), reason='reference tree not present')
+needs_ref = pytest.mark.skipif(not os.path.exists(os.path.join(REF, 'dsp4cohdec.m')), reason='reference tree not present')
 
 
 def _signals(L, seed, rot=0.3, noise=0.05, dphi=2e-3):
@@ -22,6 +22,7 @@ def _signals(L, seed, rot=0.3, noise=0.05, dphi=2e-3):
     return x * np.exp(1j * (0.2 + dphi * np.arange(L)))[:, None], sym
 
 
+@needs_ref
 def test_cmaadaptivefilter_matches_reference_source():
     x, _ = _signals(200, 1)
     ext = np.concatenate([x[-3:], x, x[:3]])
@@ -42,6 +43,7 @@ def _local(it, name, args, nargout=1):
     return it.call(name, args, nargout, local_funcs=table)
 
 
+@needs_ref
 @pytest.mark.parametrize('P,M,k,unwrap', [(4, 4, 20, False), (2, 4, 3, True), (4, 4, 0, True), (2, 4, 300, True)])
 def test_vitvit_matches_reference_source(P, M, k, unwrap):
     x, _ = _signals(256, 2)
@@ -51,6 +53,7 @@ def test_vitvit_matches_reference_source(P, M, k, unwrap):
     np.testing.assert_allclose(got, ref, rtol=0, atol=2e-12)
 
 
+@needs_ref
 def test_cmapolardemux_matches_reference_source():
     x, _ = _signals(300, 3, rot=0.25)
     it = Interp(REF)
@@ -61,6 +64,7 @@ def test_cmapolardemux_matches_reference_source():
     np.testing.assert_allclose(got, ref, rtol=0, atol=1e-11)
 
 
+@needs_ref
 def test_easiadaptivefilter_matches_reference_source():
     x, _ = _signals(200, 5, rot=0.5)
     h1 = np.array([[1.0, 0.2j]])
@@ -73,6 +77,7 @@ def test_easiadaptivefilter_matches_reference_source():
     np.testing.assert_allclose(bo, b, rtol=0, atol=1e-13)
 
 
+@needs_ref
 def test_easipolardemux_matches_reference_source():
     x, _ = _signals(300, 6, rot=0.6)
     it = Interp(REF)
@@ -83,6 +88,7 @@ def test_easipolardemux_matches_reference_source():
     np.testing.assert_allclose(got, ref, rtol=0, atol=1e-11)
 
 
+@needs_ref
 def test_dispcompfilter_matches_reference_source():
     it = Interp(REF)
     beta2l = -800.0 * 1550.0 ** 2 / 2 / np.pi / 299792458.0 * 1e-21
@@ -93,6 +99,7 @@ def test_dispcompfilter_matches_reference_source():
         assert abs(np.abs(got).mean() - 1) < 0.2          # close to an all-pass response
 
 
+@needs_ref
 def test_nlrotation_matches_reference_source():
     x, _ = _signals(128, 7)
     x = x * (1 + 0.3 * np.random.Generator(np.random.PCG64(8)).standard_normal((128, 1)))
@@ -101,6 +108,7 @@ def test_nlrotation_matches_reference_source():
     np.testing.assert_allclose(dsp.nl_rotation(x, 0.37), ref, rtol=0, atol=1e-14)
 
 
+@needs_ref
 def test_adc_emulation_matches_reference_source():
     """the ADC lines of dsp4cohdec.m sit in its main body: they are cut out of the file as text and executed"""
     import re
@@ -119,6 +127,7 @@ def test_adc_emulation_matches_reference_source():
         assert len(np.unique(np.round(got, 12))) <= 2 ** bits + 1
 
 
+@needs_ref
 def test_decision_and_differential_decoding_match_reference_source():
     g = np.random.Generator(np.random.PCG64(4))
     phase = g.uniform(-np.pi, np.pi, (64, 2))

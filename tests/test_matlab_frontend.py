@@ -1,10 +1,12 @@
 """matlab/fiber.m and matlab/ampliflat.m -- the thin M front-ends that replace the toolbox's fiber.m on the path --
 executed by the mini M interpreter (oracle/mini_m).
 
-CPU (here, where /root/reference exists): the front-end with an oracle-backed ssfm_mex reproduces the goldens the
-interpreted ORIGINAL fiber.m produced (same plate draws from the same rand stream, same DELAY / DISP, same brf, same
-simul_out text), with create_field.m / reset_all.m taken from the reference tree -- i.e. the scripts' calls run
-unchanged with matlab/ first on the path.
+CPU: the front-end with an oracle-backed ssfm_mex reproduces the goldens the interpreted ORIGINAL fiber.m produced
+(same plate draws from the same rand stream, same DELAY / DISP, same brf, same simul_out text), starting from the Tx
+field the interpreted reset_all.m / create_field.m left in GSTATE (stored with each golden).  The toolbox functions the
+front-ends call (avg_power.m, myfilter.m, fastexp.m) are stood in for by the oracle's restatements, pinned on the
+interpreted originals by test_golden and test_receiver_oracle.  Where the toolbox's own M source is at hand, the
+scripts' calls also run unchanged with matlab/ first on the path against it.
 GPU: the same front-end with the real gateway (mexFunction of mex/ssfm_mex.c through the mex.h stand-in) against the
 goldens, including C1 at its full size, the resident span loop fiber(); ampliflat(); and the FP32 option."""
 import glob
@@ -47,29 +49,36 @@ def globals_from_python(it, nsymb, nt, nch, rate, pavg, fx, fy, lams=None):
     it.globals['PMXOPT'] = np.zeros((0, 0))
 
 
-def tx_through_reference(it, m, z):
-    it.call('reset_all', [to_m(m['nsymb']), to_m(m['nt']), to_m(m['nch'])], 0)
-    G = it.globals['GSTATE'].copy()
-    G['SYMBOLRATE'] = to_m(m['rate'])
-    G['LAMBDA'] = to_m(synth.wdm_lambdas(m['nch']).reshape(1, -1))
-    G['POWER'] = to_m(np.full((1, m['nch']), float(m['pavg'])))
-    it.globals['GSTATE'] = G
-    it.globals['PMXOPT'] = np.zeros((0, 0))
-    args = [m['ftype'], to_m(z['in_ex']), to_m(z['in_ey']) if m['two_pol'] else np.zeros((0, 0)), MStruct({'power': 'average'})]
-    it.call('create_field', args, 0)
+def tx_from_golden(it, m, z):
+    """GSTATE as the interpreted reset_all.m + create_field.m left it: the golden's stored Tx field and power"""
+    globals_from_python(it, m['nsymb'], m['nt'], m['nch'], m['rate'], m['pavg'], z['tx_FIELDX'],
+                        z['tx_FIELDY'] if m['two_pol'] else None)
+    it.globals['GSTATE']['POWER'] = np.array(z['tx_POWER'], dtype=np.float64).reshape(1, -1)
 
 
-@needs_ref
+def avg_power_stand_in(m):
+    """the toolbox's avg_power.m (called by matlab/ampliflat.m for 'fixpower') as the oracle's restatement, pinned on
+    the interpreted avg_power.m by test_golden"""
+    def avg_power(it_, a, nargout):
+        Gm = it_.globals['GSTATE']
+        gs = orc.reset_all(m['nsymb'], m['nt'], m['nch'])
+        gs.FIELDX, fy = np.asarray(Gm['FIELDX']), np.asarray(Gm['FIELDY'])
+        gs.FIELDY = fy if fy.size else None
+        assert a[1] == 'abs'
+        return [to_m(orc.avg_power_abs(gs, int(np.asarray(a[0]).ravel()[0])))]
+    return avg_power
+
+
 @pytest.mark.parametrize('scalmode', [0, 1])
 @pytest.mark.parametrize('name', CASES)
 def test_front_end_reproduces_the_interpreted_original(name, scalmode):
-    """matlab/fiber.m (first on the path) + the reference's reset_all.m / create_field.m + an oracle-backed ssfm_mex
+    """matlab/fiber.m + the Tx field of the interpreted create_field.m + an oracle-backed ssfm_mex
     == the interpreted original fiber.m: fields <= 1e-13, DELAY / DISP, the brf struct and its plate draws"""
     z, m = load(name)
     calls = []
-    it = Interp([MDIR, REF], rng=np.random.Generator(np.random.PCG64(m['seed'])))
+    it = Interp([MDIR], rng=np.random.Generator(np.random.PCG64(m['seed'])))
     it.builtins['ssfm_mex'] = mex_bridge.oracle_gateway(calls)
-    tx_through_reference(it, m, z)
+    tx_from_golden(it, m, z)
     it.globals['PMXOPT'] = MStruct({'scalar': to_m(float(scalmode))})
     want_brf = 'brf_theta' in z.files
     res = it.call('fiber', [to_m(m['fiber']), m['flag']], 1 if want_brf else 0)
@@ -92,22 +101,26 @@ def test_front_end_reproduces_the_interpreted_original(name, scalmode):
         assert float(np.asarray(brf['lcorr']).ravel()[0]) == float(z['brf_lcorr'][0])
     if 'amp_FIELDX' in z.files:    # matlab/ampliflat.m ('gain' and 'fixpower', the latter through the toolbox's avg_power.m)
         a = m['amp']
+        it.builtins['avg_power'] = avg_power_stand_in(m)
         opt = MStruct({'f': to_m(a['f']), 'noise': to_m(z['amp_noise'])})
         it.call('ampliflat', [to_m(a['gain']), a.get('atype', 'gain'), opt], 0)
         G = it.globals['GSTATE']
         assert orc.rel_l2(G['FIELDX'], G['FIELDY'], z['amp_FIELDX'], z['amp_FIELDY']) < 1e-13
 
 
-@needs_ref
 @pytest.mark.parametrize('name', sorted(os.path.basename(p)[len('simul_out_'):-5] for p in
                                         glob.glob(os.path.join(GOLD, 'simul_out_*.json'))))
 def test_front_end_prints_the_same_summary(name):
-    """GSTATE.PRINT: the block matlab/fiber.m appends to simul_out is character-identical to the original's"""
+    """GSTATE.PRINT: the block matlab/fiber.m appends to simul_out is character-identical to the original's (Tx field
+    from the oracle's create_field, pinned on the interpreted create_field.m by test_golden)"""
     m = json.load(open(os.path.join(GOLD, 'simul_out_%s.json' % name)))
     ex, ey, _, _ = synth.pdm_qpsk(m['nsymb'], m['nt'], m['nch'])
-    it = Interp([MDIR, REF], rng=np.random.Generator(np.random.PCG64(m['seed'])))
+    gs = orc.reset_all(m['nsymb'], m['nt'], m['nch'])
+    gs.SYMBOLRATE, gs.POWER, gs.LAMBDA = m['rate'], np.full(m['nch'], float(m['pavg'])), synth.wdm_lambdas(m['nch'])
+    orc.create_field(gs, m['ftype'], ex, ey if m['two_pol'] else None, power_average=True)
+    it = Interp([MDIR], rng=np.random.Generator(np.random.PCG64(m['seed'])))
     it.builtins['ssfm_mex'] = mex_bridge.oracle_gateway()
-    tx_through_reference(it, m, {'in_ex': ex, 'in_ey': ey})
+    tx_from_golden(it, m, {'tx_FIELDX': gs.FIELDX, 'tx_FIELDY': gs.FIELDY, 'tx_POWER': gs.POWER})
     G = it.globals['GSTATE'].copy()
     G['PRINT'] = to_m(True)
     G['DIR'] = 'sim'
@@ -117,12 +130,11 @@ def test_front_end_prints_the_same_summary(name):
     assert ''.join(it.printed) == m['text']
 
 
-@needs_ref
 def test_front_end_errors_like_the_original():
-    it = Interp([MDIR, REF])
+    it = Interp([MDIR])
     it.builtins['ssfm_mex'] = mex_bridge.oracle_gateway()
     z, m = load('scalar_gs')
-    tx_through_reference(it, m, z)
+    tx_from_golden(it, m, z)
     with pytest.raises(MError, match='wrong flag'):
         it.call('fiber', [to_m(m['fiber']), 'abcd'], 0)
     with pytest.raises(MError, match='only for channels separated'):
@@ -132,12 +144,12 @@ def test_front_end_errors_like_the_original():
     with pytest.raises(MError, match='wrong string atype'):
         it.call('ampliflat', [to_m(3.0), 'boost'], 0)
     z3, m3 = load('wdm3_unique_manakov')         # three channels in one 'unique' field
-    tx_through_reference(it, m3, z3)
+    tx_from_golden(it, m3, z3)
     with pytest.raises(MError, match='only for channels separated'):
         it.call('ampliflat', [to_m(1.0), 'fixpower'], 0)
-    tx_through_reference(it, m, z)
+    tx_from_golden(it, m, z)
     z, m = load('cnlse_nopmd')
-    tx_through_reference(it, m, z)
+    tx_from_golden(it, m, z)
     with pytest.raises(MError, match='absence of polarization'):
         it.call('fiber', [to_m(dict(m['fiber'], ltol=1e-6)), 'g-s-'], 0)
 
@@ -212,6 +224,14 @@ def _rx_case(name):
     return z, m, MStruct({k: (v if isinstance(v, str) else to_m(v)) for k, v in x.items()})
 
 
+def _rx_toolbox_stand_ins(it):
+    """myfilter.m / fastexp.m belong to the toolbox: the oracle's restatement (pinned by test_receiver_oracle)"""
+    import oracle.receiver_oracle as rxo
+    it.builtins['myfilter'] = lambda it_, a, nargout: [rxo.myfilter(a[0], np.asarray(a[1]), float(np.asarray(a[2]).ravel()[0]),
+                                                                   float(np.asarray(a[3]).ravel()[0]) if len(a) > 3 else 0).reshape(-1, 1)]
+    it.builtins['fastexp'] = lambda it_, a, nargout: [np.cos(np.asarray(a[0])) + 1j * np.sin(np.asarray(a[0]))]
+
+
 def _rx_globals(it, z, m):
     globals_from_python(it, m['nsymb'], m['nt'], m['nch'], m['rate'], m['pavg'], z['FIELDX'],
                         z['FIELDY'] if z['FIELDY'].size else None)
@@ -236,14 +256,14 @@ def _rx_check(it, z, m, x, tol):
     assert np.array_equal(np.asarray(one), np.asarray(iric))
 
 
-@needs_ref
 @pytest.mark.parametrize('name', RXCASES)
 def test_receiver_front_end_reproduces_the_interpreted_original(name):
-    """matlab/receiver_cohmix.m (first on the path) + the toolbox's myfilter.m / fastexp.m + an oracle-backed ssfm_mex
+    """matlab/receiver_cohmix.m + the oracle's myfilter / fastexp + an oracle-backed ssfm_mex
     == the interpreted original receiver_cohmix.m: currents, avgebx / avgeby, post_delay"""
     z, m, x = _rx_case(name)
-    it = Interp([MDIR, REF])
+    it = Interp([MDIR])
     it.builtins['ssfm_mex'] = mex_bridge.oracle_gateway()
+    _rx_toolbox_stand_ins(it)
     _rx_globals(it, z, m)
     _rx_check(it, z, m, x, 1e-13)
 
@@ -276,11 +296,10 @@ def _inv_check(z, tag, uinv, u, G, tol):
     np.testing.assert_array_equal(np.asarray(G['DISP']), np.zeros((2, 1)) if applied else np.ones((2, 1)))
 
 
-@needs_ref
 @pytest.mark.parametrize('tag', list(INVVARIANTS))
 def test_inverse_pmd_front_end_reproduces_the_interpreted_original(tag):
     """matlab/inverse_pmd.m + an oracle-backed ssfm_mex('invpmd', ...) == the interpreted original inverse_pmd.m with every option"""
-    it = Interp([MDIR, REF])
+    it = Interp([MDIR])
     it.builtins['ssfm_mex'] = mex_bridge.oracle_gateway()
     z, uinv, u, G = _inv_run(it, tag)
     _inv_check(z, tag, uinv, u, G, 1e-12)
@@ -317,16 +336,8 @@ def test_interpreted_front_end_on_the_device(name):
     np.testing.assert_allclose(G['DELAY'], z['out_DELAY'], rtol=1e-13, atol=1e-13)
     np.testing.assert_allclose(G['DISP'], z['out_DISP'], rtol=1e-13, atol=1e-13)
     if 'amp' in m:
-        # matlab/ampliflat.m, 'fixpower' included.  It calls the toolbox's avg_power.m, which is not on the GPU box: the
-        # test stands in for it with the oracle's restatement (pinned on the interpreted avg_power.m by test_golden)
-        def avg_power(it_, a, nargout):
-            Gm = it_.globals['GSTATE']
-            gs = orc.reset_all(m['nsymb'], m['nt'], m['nch'])
-            gs.FIELDX, fy = np.asarray(Gm['FIELDX']), np.asarray(Gm['FIELDY'])
-            gs.FIELDY = fy if fy.size else None
-            assert a[1] == 'abs'
-            return [to_m(orc.avg_power_abs(gs, int(np.asarray(a[0]).ravel()[0])))]
-        it.builtins['avg_power'] = avg_power
+        # matlab/ampliflat.m, 'fixpower' included (its avg_power.m call answered by the oracle's restatement)
+        it.builtins['avg_power'] = avg_power_stand_in(m)
         opt = MStruct({'f': to_m(m['amp']['f']), 'noise': to_m(z['amp_noise'])})
         it.call('ampliflat', [to_m(m['amp']['gain']), m['amp'].get('atype', 'gain'), opt], 0)
         G = it.globals['GSTATE']
@@ -337,14 +348,10 @@ def test_interpreted_front_end_on_the_device(name):
 @pytest.mark.parametrize('name', RXCASES)
 def test_interpreted_receiver_front_end_on_the_device(name):
     """matlab/receiver_cohmix.m interpreted, its ssfm_mex('cohmix', ...) the compiled gateway on the GPU (pmx_cohmix_run),
-    against the interpreted original's goldens, FP64 <= 1e-10.  myfilter.m / fastexp.m belong to the toolbox, which is
-    not on the GPU box: the test stands in for them with the oracle's restatement (pinned by test_receiver_oracle)."""
-    import oracle.receiver_oracle as rxo
+    against the interpreted original's goldens, FP64 <= 1e-10 (myfilter / fastexp as the oracle's restatement)."""
     z, m, x = _rx_case(name)
     it, gw = _gpu_interp(0)
-    it.builtins['myfilter'] = lambda it_, a, nargout: [rxo.myfilter(a[0], np.asarray(a[1]), float(np.asarray(a[2]).ravel()[0]),
-                                                                   float(np.asarray(a[3]).ravel()[0]) if len(a) > 3 else 0).reshape(-1, 1)]
-    it.builtins['fastexp'] = lambda it_, a, nargout: [np.cos(np.asarray(a[0])) + 1j * np.sin(np.asarray(a[0]))]
+    _rx_toolbox_stand_ins(it)
     _rx_globals(it, z, m)
     _rx_check(it, z, m, x, 1e-10)
 
