@@ -241,6 +241,37 @@ int pmx_link_exec(pmx_plan* plan, pmx_devfield* f, const pmx_link_desc* link, pm
 int pmx_link_run(pmx_ctx* ctx, const pmx_fiber_desc* desc, const pmx_link_desc* link, pmx_field* io,
                  pmx_fiber_result* out);
 
+/* ---- digital backpropagation: the link run backwards on the receive side ----------------------------------------------
+ * An extension (the reference has no DBP).  The field is propagated through a virtual copy of the link with dispersion,
+ * nonlinearity and loss negated, spans last first.  With u the field of one realization, for span k = nspan..1:
+ *   u <- u / sqrt(gain)                                          (when a gain is given: the amplifier after the span)
+ *   for the span's steps h = h_M .. h_1 (reverse of their forward order):
+ *     u <- exp(+alpha*h/2) * u
+ *     u <- ifft( fft(u) .* exp(+i*betat*h) )                     per column
+ *     u <- N(-xi*gam, h) u                                       matrix_nl_step (fiber.m:827-851) with gam -> -xi*gam and
+ *                                                                the forward leff(h) = (1 - exp(-alpha*h))/alpha
+ * With xi = 1 and the forward run's own steps (pmx_fiber_result.trace_dz), DBP inverts a noise-free fiber without PMD up
+ * to rounding.  DBP ignores the 'p' flag, the plates and dgdrms; the 'x' flag fails with PMX_ERR_XPM_VECTOR as in fiber.
+ * Two-polarization fields (scalar_field = 0), nfc <= 64, nfft from 2^12 to 2^24, FP64 or FP32; other fields fail with
+ * PMX_ERR_UNSUPPORTED.  Every step is the three HBM passes of a forward step; the step packages of the whole schedule
+ * are built when the plan is created, so pmx_dbp_exec enqueues every step without reading anything back. */
+typedef struct pmx_dbp_desc {
+    int32_t nspan;
+    int32_t steps_per_span;    /* > 0: uniform steps of length/steps_per_span; 0: the explicit schedule below           */
+    const int32_t* span_steps; /* [nspan] steps of each span (explicit schedule), or NULL (uniform steps)               */
+    const double* step_len;    /* all spans' steps concatenated, each span in FORWARD order (e.g. trace_dz)             */
+    double xi;                 /* fraction of gamma backpropagated; 1 = all                                              */
+    double gain;               /* linear amplifier gain after every span, undone first; 0 = none                         */
+} pmx_dbp_desc;
+/* fiber: the link's fiber (length, alphalin, gam, manakov, fls, dispersion as for pmx_plan_create; batch and precision of
+ * the fields the plan will run on).  Validates dbp: PMX_ERR_INVALID for nspan < 1, a non-finite xi, gain < 0, a
+ * negative or non-finite step, or a span whose steps do not sum to fiber->length within 1e-9 relative.  The explicit
+ * schedule (steps_per_span = 0) needs span_steps and step_len, span_steps[k] >= 1. */
+int pmx_dbp_create(pmx_ctx* ctx, const pmx_fiber_desc* fiber, const pmx_dbp_desc* dbp, pmx_plan** plan);
+/* In place on a resident field; returns when the field is backpropagated.  The field may belong to another context of
+ * the same device (as for pmx_fiber_exec).  Destroy the plan with pmx_plan_destroy. */
+int pmx_dbp_exec(pmx_plan* plan, pmx_devfield* f);
+
 /* ---- create_field('unique'): the WDM multiplex on the device (create_field.m:113-149,180-199) ----------------
  * The reference builds the single field as
  *   FIELDX = ifft( sum_ch fastshift( fft(sigx(:,ch)), -ndfn(ch) ) ),   ndfn = round(deltafn/SYMBOLRATE/minfreq)
@@ -349,7 +380,7 @@ int pmx_dsp_phases(pmx_ctx* ctx, pmx_devfield* f, const pmx_dsp_desc* dsp, doubl
  * The caller replays ber_estimate's recursion (ber_estimate.m:121-127) over counts[] in realization order. */
 /* The reference's receive chain behind the link of a Monte-Carlo job (ex20_coherent_polmux.m:151-176): receiver_cohmix's
  * front-end, the sampler and the DSP core, per resident batch.  hf_opt already carries whatever all-pass compensation the
- * receiver applies (x.dpost, receiver_cohmix.m:139-166, or p.applydcf).  Single-column ('unique') FP64 fields.  The chain of
+ * receiver applies (x.dpost, receiver_cohmix.m:139-166, or p.applydcf), unless dbp is set.  Single-column ('unique') FP64 fields.  The chain of
  * a group runs on a context (stream) and host thread of its own beside the propagation of the next group. */
 typedef struct pmx_mc_receiver {
     const double* hf_opt;      /* [nfft] complex: post fiber .* optical filter                              */
@@ -360,6 +391,9 @@ typedef struct pmx_mc_receiver {
     int32_t reserved;
     pmx_dsp_desc dsp;          /* sampler (sample_shift, peak), demultiplexer, carrier recovery             */
     const uint8_t* ref_patmat; /* [nsymb][4] decoded transmitted pattern (pmx_dsp_count)                    */
+    const pmx_dbp_desc* dbp;   /* NULL: hf_opt carries the all-pass compensation; else digital backpropagation of the  */
+                               /* link (pmx_dbp_exec) on every received batch before the front-end, hf_opt then     */
+                               /* carrying the optical filter only                                                  */
 } pmx_mc_receiver;
 
 typedef struct pmx_mc_desc {

@@ -9,6 +9,7 @@ from .fiber import fiber, fiber_setup, LAST as FIBER_LAST  # noqa: F401
 from .ampliflat import ampliflat  # noqa: F401
 from .inverse_pmd import inverse_pmd  # noqa: F401
 from .link import link  # noqa: F401
+from .dbp import dbp  # noqa: F401
 from .receiver import receiver_cohmix, myfilter, evaldelay  # noqa: F401
 from .dsp import dsp4cohdec  # noqa: F401
 from ._lib import PolmuxError, Context, DeviceField, Plan  # noqa: F401

@@ -34,6 +34,7 @@ EXPORTS = [
     'pmx_host_is_pinned', 'pmx_scalar_adaptive_run', 'pmx_mc_run', 'pmx_mc_nccl_available',
     'pmx_ampliflat_exec_at', 'pmx_dsp_count', 'pmx_field_mean_power', 'pmx_pmd_matrix', 'pmx_field_jones', 'pmx_filter_create', 'pmx_field_copy_cols', 'pmx_field_modulate',
     'pmx_cohmix_exec', 'pmx_field_mean_power_xy', 'pmx_cohmix_run', 'pmx_dsp_phases', 'pmx_field_quantize', 'pmx_inverse_pmd_run',
+    'pmx_dbp_create', 'pmx_dbp_exec',
 ]
 
 
@@ -78,9 +79,15 @@ class DspDesc(C.Structure):
                 ('easi_phizero', C.c_double), ('easi_passes', C.POINTER(C.c_int32)), ('nlr_alpha', C.c_double), ('dcf_h', _dp), ('decim_ntaps', C.c_int32), ('reserved2', C.c_int32), ('decim_taps', _dp)]
 
 
+class DbpDesc(C.Structure):
+    _fields_ = [('nspan', C.c_int32), ('steps_per_span', C.c_int32), ('span_steps', _ip), ('step_len', _dp),
+                ('xi', C.c_double), ('gain', C.c_double)]
+
+
 class McReceiver(C.Structure):
     _fields_ = [('hf_opt', _dp), ('hf_el', _dp), ('lo_ecw', C.c_double), ('lo_detune', C.c_double), ('lo_phase', _dp),
-                ('balanced', C.c_int32), ('reserved', C.c_int32), ('dsp', DspDesc), ('ref_patmat', C.POINTER(C.c_uint8))]
+                ('balanced', C.c_int32), ('reserved', C.c_int32), ('dsp', DspDesc), ('ref_patmat', C.POINTER(C.c_uint8)),
+                ('dbp', C.POINTER(DbpDesc))]
 
 
 class McDesc(C.Structure):
@@ -171,6 +178,8 @@ def load():
                                   C.POINTER(C.c_int64)]
     lib.pmx_link_exec.argtypes = [vp, vp, C.POINTER(LinkDesc), C.POINTER(FiberResult)]
     lib.pmx_link_run.argtypes = [vp, C.POINTER(FiberDesc), C.POINTER(LinkDesc), C.POINTER(Field), C.POINTER(FiberResult)]
+    lib.pmx_dbp_create.argtypes = [vp, C.POINTER(FiberDesc), C.POINTER(DbpDesc), C.POINTER(vp)]
+    lib.pmx_dbp_exec.argtypes = [vp, vp]
     _lib = lib
     return lib
 
@@ -508,6 +517,45 @@ class Plan:
             self.close()
         except Exception:
             pass
+
+
+class DbpPlan(Plan):
+    """Digital backpropagation of a link (pmx_dbp_create): execute(field) runs it in place on a resident field."""
+
+    def __init__(self, ctx: Context, desc: FiberDesc, keep, dbp: DbpDesc, dbp_keep):
+        self.ctx, self.desc, self.keep, self.dbp, self.dbp_keep = ctx, desc, keep, dbp, dbp_keep
+        h = C.c_void_p()
+        ctx.check(ctx.lib.pmx_dbp_create(ctx.h, C.byref(desc), C.byref(dbp), C.byref(h)))
+        self.h = h
+
+    def execute(self, field: DeviceField, trace_cap=0):
+        self.ctx.check(self.ctx.lib.pmx_dbp_exec(self.h, field.h))
+
+
+def make_dbp(nspan, gain=0.0, steps_per_span=None, step_len=None, span_steps=None, xi=1.0):
+    """-> (DbpDesc, keep-alive dict).  Either steps_per_span (uniform steps) or step_len: the steps of one span in forward
+    order (every span gets them), or with span_steps [nspan] the steps of all spans concatenated."""
+    keep = {}
+    d = DbpDesc()
+    d.nspan, d.xi, d.gain = int(nspan), float(xi), float(gain)
+    if step_len is None:
+        d.steps_per_span = int(1 if steps_per_span is None else steps_per_span)
+        return d, keep
+    if steps_per_span is not None:
+        raise ValueError('give steps_per_span or step_len, not both')
+    keep['step_len'] = _f64(np.asarray(step_len, dtype=np.float64).reshape(-1))
+    if span_steps is None:
+        keep['step_len'] = np.ascontiguousarray(np.tile(keep['step_len'], int(nspan)))
+        span_steps = [keep['step_len'].size // int(nspan)] * int(nspan)
+    keep['span_steps'] = np.ascontiguousarray(np.asarray(span_steps, dtype=np.int32).reshape(-1))
+    if keep['span_steps'].size != int(nspan):
+        raise ValueError('span_steps must give the steps of every span')
+    if int(keep['span_steps'].astype(np.int64).sum()) != keep['step_len'].size:
+        raise ValueError('step_len must hold sum(span_steps) steps')
+    d.steps_per_span = 0
+    d.step_len = _ptr(keep['step_len'])
+    d.span_steps = keep['span_steps'].ctypes.data_as(_ip)
+    return d, keep
 
 
 class Filter(Plan):

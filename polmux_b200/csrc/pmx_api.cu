@@ -84,7 +84,7 @@ struct pmx_ctx {
     std::string error;
     std::map<int, StageTw> stage_tw;          // by L
     std::map<long long, FourStepTw> four_tw;  // by N
-    struct Occ { int a = 0, b = 0, c = 0; };
+    struct Occ { int a = 0, b = 0, c = 0, cnl = 0; };   // cnl: pmx_k_passC_nl (digital backpropagation), set on first use
     std::map<int, Occ> setup_done;  // by L: resident CTAs per SM of passes A, B, C
     int sm_count = 148;
     PFN_cuTensorMapEncodeTiled_v12000 encode = nullptr;
@@ -230,6 +230,12 @@ struct pmx_plan {
     int trace_cap = 0;
     bool single_step;
     bool onchip = false;   // nfft <= 4096: the single-launch kernel of small fields (pmx_onchip.cuh)
+    // digital-backpropagation plans (pmx_dbp_create): the constants of passes A (no NL step) and B / C' (gam = -xi*gam), the
+    // distinct step packages [npkg][batch] and the package of every step in execution order
+    bool dbp = false;
+    FiberConst fc_a, fc_c;
+    StepPkg* sched = nullptr;
+    std::vector<int> sched_idx;
 };
 
 static int set_err(pmx_ctx* ctx, int code, const char* fmt, ...) {
@@ -736,10 +742,12 @@ extern "C" void pmx_plan_destroy(pmx_plan* p) {
     if (p->pkg) cudaFreeAsync(p->pkg, st);
     if (p->trace_dz) cudaFreeAsync(p->trace_dz, st);
     if (p->trace_ntrunk) cudaFreeAsync(p->trace_ntrunk, st);
+    if (p->sched) cudaFreeAsync(p->sched, st);
     delete p;
 }
 
-extern "C" int pmx_plan_create(pmx_ctx* c, const pmx_fiber_desc* d, pmx_plan** out) {
+// passes_only: 2^12 fields run on the three passes instead of the single-launch kernel (digital backpropagation)
+static int plan_create(pmx_ctx* c, const pmx_fiber_desc* d, pmx_plan** out, bool passes_only) {
     if (!c || !d || !out) return set_err(c, PMX_ERR_INVALID, "pmx_plan_create: null argument");
     *out = nullptr;
     if (d->precision != PMX_F64 && d->precision != PMX_F32)
@@ -751,7 +759,7 @@ extern "C" int pmx_plan_create(pmx_ctx* c, const pmx_fiber_desc* d, pmx_plan** o
     // Fields of up to 4096 samples run in the single-launch on-chip kernel (one CTA per column, the columns of a
     // realization in one thread-block cluster): at most 8 columns.  PMX_NO_ONCHIP=1 sends 2^12 through the three passes.
     const bool no_onchip = getenv("PMX_NO_ONCHIP") && atoi(getenv("PMX_NO_ONCHIP"));
-    const bool onchip = lg <= 12 && d->nfc <= 8 && !(no_onchip && lg == 12);
+    const bool onchip = lg <= 12 && d->nfc <= 8 && !(no_onchip && lg == 12) && !passes_only;
     if (lg < 12 && !onchip)
         return set_err(c, PMX_ERR_UNSUPPORTED, "nfft=%lld (< 2^12) with nfc=%d: small fields take at most 8 columns",
                        (long long)d->nfft, d->nfc);
@@ -932,6 +940,8 @@ extern "C" int pmx_plan_create(pmx_ctx* c, const pmx_fiber_desc* d, pmx_plan** o
     return PMX_OK;
 }
 
+extern "C" int pmx_plan_create(pmx_ctx* c, const pmx_fiber_desc* d, pmx_plan** out) { return plan_create(c, d, out, false); }
+
 // ---------------------------------------------------------------------------
 // A linear filter as a plan: one step of a fiber without dispersion, birefringence, nonlinearity or loss whose per-bin
 // factor is the caller's H instead of exp(-i*betat*dz).  pmx_fiber_exec on it is u <- ifft(fft(u) .* H).
@@ -1019,6 +1029,7 @@ extern "C" int pmx_fiber_exec(pmx_plan* p, pmx_devfield* fld, pmx_fiber_result* 
     if (fld->nfft != p->d.nfft || fld->nfc != p->d.nfc || fld->batch != p->d.batch)
         return set_err(c, PMX_ERR_INVALID, "field shape (%lld,%d,%d) does not match the plan (%lld,%d,%d)",
                        (long long)fld->nfft, fld->nfc, fld->batch, (long long)p->d.nfft, p->d.nfc, p->d.batch);
+    if (p->dbp) return set_err(c, PMX_ERR_INVALID, "pmx_fiber_exec: a digital-backpropagation plan runs with pmx_dbp_exec");
     CK(c, cudaSetDevice(c->device));
     const int batch = p->d.batch, nfc = p->d.nfc;
     int rc = ensure_hctl(c, batch);
@@ -3299,5 +3310,254 @@ extern "C" int pmx_scalar_adaptive_run(pmx_ctx* c, const pmx_fiber_desc* d, doub
         if (out->ntot) out->ntot[0] = 0;
         if (out->status) out->status[0] = PMX_OK;
     }
+    return PMX_OK;
+}
+
+// ---------------------------------------------------------------------------
+// Digital backpropagation (polmux_ssfm.h, pmx_dbp_desc): a step of length h is the three passes of a forward step --
+// pass A without the nonlinear step, pass B with the dispersion negated, pass C' (pmx_k_passC_nl) with the scale
+// exp(+alpha*h/2)/N and the nonlinear step with gam -> -xi*gam -- in the order N(-xi*gam) L(-h) A(-h), the inverse of the
+// forward A(h) L(h) N(h).  The schedule is known when the plan is made: every step's package is built here and the host
+// enqueues the whole link without reading anything back.
+extern "C" int pmx_dbp_create(pmx_ctx* c, const pmx_fiber_desc* fd, const pmx_dbp_desc* g, pmx_plan** out) {
+    // (the descriptors are checked before the context, so that the checks run without a device)
+    if (!fd || !g || !out) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: null argument");
+    *out = nullptr;
+    if (fd->scalar_field)
+        return set_err(c, PMX_ERR_UNSUPPORTED, "digital backpropagation is built for two-polarization fields, not the scalar path");
+    if (fd->fls[3]) return set_err(c, PMX_ERR_XPM_VECTOR, "The CNLSE with separate fields is not yet implemented");
+    const int lg = ilog2_exact(fd->nfft);
+    if (lg < 12 || lg > 24)
+        return set_err(c, PMX_ERR_UNSUPPORTED, "digital backpropagation: nfft=%lld, built for powers of two from 2^12 to 2^24",
+                       (long long)fd->nfft);
+    if (g->nspan < 1) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: nspan must be >= 1");
+    if (!std::isfinite(g->xi)) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: xi must be finite");
+    if (!(g->gain >= 0) || !std::isfinite(g->gain)) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: gain must be >= 0 (0: none)");
+    if (!(fd->length > 0) || !std::isfinite(fd->length)) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: length must be > 0");
+    // the steps of every span, forward order
+    std::vector<double> h;
+    std::vector<int> nstep(g->nspan);
+    if (g->steps_per_span > 0) {
+        if ((long long)g->steps_per_span * g->nspan > 10000000)
+            return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: more than 10^7 steps in all");
+        for (int k = 0; k < g->nspan; ++k) {
+            nstep[k] = g->steps_per_span;
+            for (int j = 0; j < g->steps_per_span; ++j) h.push_back(fd->length / g->steps_per_span);
+        }
+    } else if (g->steps_per_span < 0) {
+        return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: steps_per_span must be >= 0");
+    } else {
+        if (!g->span_steps || !g->step_len)
+            return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: an explicit schedule needs span_steps and step_len");
+        size_t o = 0;
+        for (int k = 0; k < g->nspan; ++k) {
+            const int n = g->span_steps[k];
+            if (n < 1 || (long long)o + n > 10000000)
+                return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: span %d has %d steps (at least one, at most 10^7 in all)", k, n);
+            double sum = 0;
+            for (int j = 0; j < n; ++j, ++o) {
+                const double v = g->step_len[o];
+                if (!(v >= 0) || !std::isfinite(v))
+                    return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: step %d of span %d is negative or not finite (%g)", j, k, v);
+                sum += v;
+                h.push_back(v);
+            }
+            if (std::fabs(sum - fd->length) > 1e-9 * fd->length)
+                return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: the steps of span %d sum to %.17g, not the fiber length %.17g", k,
+                               sum, fd->length);
+            nstep[k] = n;
+        }
+    }
+    if (!c) return set_err(nullptr, PMX_ERR_INVALID, "pmx_dbp_create: null context");
+    // the virtual fiber: no PMD, no XPM, dispersion negated, one step at a time
+    const double zero1 = 0.0;
+    std::vector<double> nb1, nb2, nbt;
+    pmx_fiber_desc e = *fd;
+    e.fls[1] = 0;
+    e.nplates = e.plate_sets = 1;
+    e.db0 = e.theta = e.epsilon = &zero1;
+    e.db1 = nullptr;
+    e.dgdrms = 0.0;
+    e.dphimaxt = INFINITY;
+    e.dzmaxt = fd->length;
+    e.z_start = e.dz_first = 0.0;
+    if (fd->disp_mode == PMX_DISP_SCALAR) {
+        if (!fd->beta1 || !fd->beta2) return set_err(c, PMX_ERR_INVALID, "scalar dispersion mode needs beta1 and beta2");
+        for (int k = 0; k < std::max(fd->nfc, 0) && k < PMX_MAX_NFC; ++k) {
+            nb1.push_back(-fd->beta1[k]);
+            nb2.push_back(-fd->beta2[k]);
+        }
+        e.beta1 = nb1.data();
+        e.beta2 = nb2.data();
+        e.b30 = -fd->b30;
+    } else if (fd->betat && fd->nfc >= 1 && fd->nfc <= PMX_MAX_NFC) {
+        nbt.assign(fd->betat, fd->betat + (size_t)fd->nfc * fd->nfft);
+        for (auto& v : nbt) v = -v;
+        e.betat = nbt.data();
+    }
+    pmx_plan* p = nullptr;
+    int rc = plan_create(c, &e, &p, true);
+    if (rc) return rc;
+    p->dbp = true;
+    p->fc_a = p->fc;
+    p->fc_a.spm = 0;                            // pass A: the transform only
+    p->fc_c = p->fc;
+    for (int k = 0; k < p->fc.nfc; ++k) p->fc_c.gam[k] = -g->xi * p->fc.gam[k];   // (gam carries the Manakov 8/9)
+    const int key = p->tA->L + 65536 * p->tA->precision;
+    if (c->setup_done[key].cnl < 1) {
+        int n = 0;
+        cudaError_t err = p->tA->passC_nl_setup(&n);
+        if (err != cudaSuccess || n < 1) {
+            pmx_plan_destroy(p);
+            return set_err(c, PMX_ERR_CUDA, "kernel setup (pass C', L=%d) failed: %s", p->tA->L, cudaGetErrorString(err));
+        }
+        c->setup_done[key].cnl = n;
+    }
+    // step packages in execution order: spans last first, each span's steps reversed; the amplifier's 1/sqrt(G) joins the
+    // scale of a span's first step.  Equal packages are stored once.
+    const FiberConst& f = p->fc;
+    const double ig = g->gain > 0 ? 1.0 / std::sqrt(g->gain) : 1.0;
+    std::vector<StepPkg> uniq;
+    std::map<std::pair<double, double>, int> seen;
+    std::vector<size_t> span0(g->nspan, 0);
+    for (int k = 1; k < g->nspan; ++k) span0[k] = span0[k - 1] + nstep[k - 1];
+    for (int k = g->nspan - 1; k >= 0; --k)
+        for (int j = nstep[k] - 1; j >= 0; --j) {
+            const double hh = h[span0[k] + j];
+            const double scale = std::exp(f.halfalpha * hh) * f.invN * (j == nstep[k] - 1 ? ig : 1.0);
+            auto it = seen.find({hh, scale});
+            if (it == seen.end()) {
+                StepPkg s;
+                memset(&s, 0, sizeof s);
+                s.dz_cur = s.dzb_first = s.dzb_last = hh;
+                s.leff = (f.alphalin == 0.0) ? hh : (1.0 - std::exp(-f.alphalin * hh)) / f.alphalin;   // fiber.m:827-831
+                s.scale = scale;
+                s.ntrunk = 1;
+                s.state = PMX_ST_RUN;
+                if (f.disp_scalar && f.gvd_any) {   // third difference of the common phase (pmx_ctl_step)
+                    const double a3 = -(hh * (6.0 * f.b30_6) * f.domega * f.domega * f.domega);
+                    s.gd3_r = std::cos(a3);
+                    s.gd3_i = std::sin(a3);
+                }
+                it = seen.emplace(std::make_pair(hh, scale), (int)uniq.size()).first;
+                uniq.push_back(s);
+            }
+            p->sched_idx.push_back(it->second);
+        }
+    const int batch = p->d.batch;
+    std::vector<StepPkg> tab(uniq.size() * (size_t)batch);
+    for (size_t u = 0; u < uniq.size(); ++u)
+        for (int b = 0; b < batch; ++b) tab[u * batch + b] = uniq[u];
+    cudaError_t err = cudaMallocAsync(&p->sched, tab.size() * sizeof(StepPkg), c->stream);
+    if (err == cudaSuccess) err = cudaMemcpyAsync(p->sched, tab.data(), tab.size() * sizeof(StepPkg), cudaMemcpyHostToDevice, c->stream);
+    if (err == cudaSuccess) err = cudaStreamSynchronize(c->stream);
+    if (err != cudaSuccess) {
+        pmx_plan_destroy(p);
+        return set_err(c, PMX_ERR_CUDA, "pmx_dbp_create: step table: %s", cudaGetErrorString(err));
+    }
+    *out = p;
+    return PMX_OK;
+}
+
+extern "C" int pmx_dbp_exec(pmx_plan* p, pmx_devfield* fld) {
+    if (!p || !fld) return set_err(nullptr, PMX_ERR_INVALID, "pmx_dbp_exec: null argument");
+    pmx_ctx* c = p->ctx;
+    if (!p->dbp) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_exec: the plan was not made by pmx_dbp_create");
+    if (fld->ctx != c && fld->ctx->device != c->device)
+        return set_err(c, PMX_ERR_INVALID, "field and plan belong to contexts on different devices");
+    if (fld->precision != p->d.precision)
+        return set_err(c, PMX_ERR_INVALID, "field precision %d does not match the plan's %d", fld->precision, p->d.precision);
+    if (fld->nfft != p->d.nfft || fld->nfc != p->d.nfc || fld->batch != p->d.batch)
+        return set_err(c, PMX_ERR_INVALID, "field shape (%lld,%d,%d) does not match the plan (%lld,%d,%d)",
+                       (long long)fld->nfft, fld->nfc, fld->batch, (long long)p->d.nfft, p->d.nfc, p->d.batch);
+    if (!fld->has_maps) return set_err(c, PMX_ERR_INVALID, "field has no tensor maps (unsupported nfft)");
+    CK(c, cudaSetDevice(c->device));
+    const int batch = p->d.batch, nfc = p->d.nfc;
+    const void *tw4A = nullptr, *tw4B = nullptr, *twA = nullptr, *twB = nullptr;
+    int rc = get_four_tw(c, p->d.nfft, p->tA, p->N2, &tw4A);
+    if (!rc) rc = get_four_tw(c, p->d.nfft, p->tB, p->N1, &tw4B);
+    if (!rc) rc = get_stage_tw(c, p->tA, &twA);
+    if (!rc) rc = get_stage_tw(c, p->tB, &twB);
+    if (rc) return rc;
+    PassParams pa;
+    memset(&pa, 0, sizeof pa);
+    pa.field = fld->data;
+    pa.ctl = p->ctl;
+    pa.betat_p = p->betat_p;
+    pa.plates = p->plates;
+    pa.N1 = p->N1;
+    pa.N2 = p->N2;
+    pa.log2N1 = p->log2N1;
+    pa.log2N2 = p->log2N2;
+    pa.dbg = g_dbg;
+    PassParams pA = pa, pB = pa;
+    pA.tw_stage = twA;
+    pA.tw4 = tw4A;
+    pB.tw_stage = twB;
+    pB.tw4 = tw4B;
+    const pmx_ctx::Occ oA = c->setup_done[p->N1 + 65536 * p->d.precision], oB = c->setup_done[p->N2 + 65536 * p->d.precision];
+    // realization groups and dependent launches as in pmx_fiber_exec: two groups on two streams once a pass has more
+    // than about two rounds of tiles, else one group with programmatic dependent launch
+    const long tiles_all = (long)(p->N2 / p->tA->gAC) * batch * nfc;
+    const int ngroups = std::min(tiles_all > 2L * c->sm_count * oA.a ? 2 : 1, batch);
+    for (int gi = 1; gi < ngroups; ++gi)
+        if (!c->gstream[gi - 1]) {
+            CK(c, cudaStreamCreateWithFlags(&c->gstream[gi - 1], cudaStreamNonBlocking));
+            CK(c, cudaEventCreateWithFlags(&c->ev_join[gi - 1], cudaEventDisableTiming));
+            if (!c->ev_fork) CK(c, cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming));
+        }
+    struct Grp {
+        cudaStream_t st;
+        PassParams pA, pB;
+        int b0, gA, gB, gC;
+    } grp[2];
+    const size_t N = (size_t)p->d.nfft;
+    auto grid_of = [&](int tiles, int ctas_per_sm) {   // one CTA per tile between one and two rounds, else persistent
+        const int slots = ctas_per_sm * c->sm_count;
+        if (tiles > slots && tiles <= 2 * slots) return tiles;
+        return std::min(tiles, slots);
+    };
+    for (int gi = 0; gi < ngroups; ++gi) {
+        Grp& G = grp[gi];
+        G.b0 = (int)((long long)gi * batch / ngroups);
+        const int nb = (int)((long long)(gi + 1) * batch / ngroups) - G.b0;
+        G.st = gi == 0 ? c->stream : c->gstream[gi - 1];
+        for (PassParams* q : {&G.pA, &G.pB}) {
+            *q = (q == &G.pA) ? pA : pB;
+            q->field = (char*)pa.field + (size_t)G.b0 * nfc * N * 2 * fld->cbytes();
+            q->batch = nb;
+            q->bc0 = G.b0 * nfc;
+            q->pdl = ngroups == 1 ? 1 : 0;
+        }
+        const int tilesAC = (p->N2 / p->tA->gAC) * nb * nfc, tilesB = (p->N1 / p->tB->gB) * nb * nfc;
+        G.gA = grid_of(tilesAC, oA.a);
+        G.gB = grid_of(tilesB, oB.b);
+        G.gC = grid_of(tilesAC, c->setup_done[p->N1 + 65536 * p->d.precision].cnl);
+    }
+    if (ngroups > 1) {   // the other stream starts after everything queued on the first one so far
+        CK(c, cudaEventRecord(c->ev_fork, c->stream));
+        for (int gi = 1; gi < ngroups; ++gi) CK(c, cudaStreamWaitEvent(c->gstream[gi - 1], c->ev_fork, 0));
+    }
+    int rev[2] = {1, 1};
+    for (size_t s = 0; s < p->sched_idx.size(); ++s) {
+        StepPkg* pk = p->sched + (size_t)p->sched_idx[s] * batch;
+        for (int gi = 0; gi < ngroups; ++gi) {
+            Grp& G = grp[gi];
+            G.pA.pkg = G.pB.pkg = pk + G.b0;
+            G.pA.reverse = (rev[gi] ^= 1);   // serpentine tile order, as in pmx_fiber_exec
+            CK(c, p->tA->passA(G.gA, G.st, G.pA, p->fc_a, fld->map_rows));
+            G.pB.reverse = (rev[gi] ^= 1);
+            CK(c, p->tB->passB(G.gB, G.st, G.pB, p->fc_c, fld->map_cols));
+            G.pA.reverse = (rev[gi] ^= 1);
+            CK(c, p->tA->passC_nl(G.gC, G.st, G.pA, p->fc_c, fld->map_rows));
+            c->launches += 3;
+        }
+    }
+    CK(c, cudaGetLastError());
+    for (int gi = 1; gi < ngroups; ++gi) {
+        CK(c, cudaEventRecord(c->ev_join[gi - 1], c->gstream[gi - 1]));
+        CK(c, cudaStreamWaitEvent(c->stream, c->ev_join[gi - 1], 0));
+    }
+    CK(c, cudaStreamSynchronize(c->stream));
     return PMX_OK;
 }

@@ -9,6 +9,8 @@
 //   pass C  rows    : W_N^(-n2*k1) -> IFFT over k1 -> 1/N * exp(-alpha/2 dz) (:531-532) ->
 //                     max |u|^2 (warp shuffle + one atomicMax per CTA and realization)
 //   ctl     one CTA per realization: nextstep + checkstep for the next step, step package for the passes
+//   pass C' rows    : (digital backpropagation, pmx_k_passC_nl) as pass C, scale exp(+alpha/2 h)/N, then the nonlinear
+//                     step with -xi*gam; A without the NL step and B with the dispersion negated complete the step
 #pragma once
 #include "pmx_fft.cuh"
 #include "pmx_tma.cuh"
@@ -1332,4 +1334,156 @@ __global__ void __launch_bounds__(G*(L / 8), PMX_MINB_C(G*(L / 8), PF))
         PMX_T_MARK(6)
     }
     PMX_T_FLUSH(2)
+}
+
+// ---------------------------------------------------------------------------
+// pass C of a digital-backpropagation step (pmx_dbp_exec): the same tile walk, twiddle and inverse transform over k1 as
+// pmx_k_passC, then the scale exp(+alpha/2*h)/N of the step package (times 1/sqrt(G) on the first step of a span), then
+// the nonlinear step N(-xi*gam) of pmx_nl_step on the rows the CTA holds, in time, before the store.  The caller hands
+// in a FiberConst whose gam is -xi*gam and a package whose bmode has no PMX_BM_NL_SMALL.  The schedule is known before
+// the first launch, so there is no max reduction and no step control.  (A kernel of its own: pmx_k_passC stays as it is.)
+template <typename R, int L, int G, bool PF>
+__global__ void __launch_bounds__(G*(L / 8), PMX_MINB_C(G*(L / 8), PF))
+    pmx_k_passC_nl(PassParams p, FiberConst f, const __grid_constant__ CUtensorMap tmap) {
+    using S = PassSmem<L, G, PF, 2>;
+    using W = PmxTw4<L>;
+    constexpr int T = L / 8;
+    constexpr int LINES = G * L * PMX_SA_BYTES / 128;
+    extern __shared__ __align__(1024) unsigned char smraw[];
+    unsigned char* sm = pmx_checked1024(smraw);
+    unsigned char* in = sm;
+    cpx* work = reinterpret_cast<cpx*>(sm + S::WORK_OFF);
+    cpx* stw = reinterpret_cast<cpx*>(sm + S::TW_OFF);
+    unsigned char* aux0 = sm + S::AUX_OFF;
+    unsigned char* sdone = sm + S::LIVE_OFF;
+    uint64_t* mbar = reinterpret_cast<uint64_t*>(sm + S::MBAR_OFF);
+    const int rl = threadIdx.x / T, t = threadIdx.x % T;
+    const size_t N = (size_t)p.N1 * p.N2;
+    PmxWalk wk;
+    wk.ltpb = p.log2N2 - pmx_ilog2(G);
+    wk.tpb_mask = (1 << wk.ltpb) - 1;
+    wk.total = (p.batch * f.nfc) << wk.ltpb;
+    wk.reverse = p.reverse;
+    const int total = wk.total;
+
+    auto live = [&](int tl) {
+        while (tl < total) {
+            int b_, col_;
+            pmx_split_bc(wk.phys(tl) >> wk.ltpb, f, b_, col_);
+            if (!pmx_is_done(sdone, p, b_)) break;
+            tl += gridDim.x;
+        }
+        return tl;
+    };
+    // a tile = G adjacent rows of the [N2][N1] time-domain matrix = G*L contiguous Sa
+    auto issue = [&](int tl, int buf) {  // one thread
+        pmx_fence_proxy_async();
+        const int tt = wk.phys(tl), bc = tt >> wk.ltpb, row0 = (tt & wk.tpb_mask) * G;
+#ifdef PMX_AC_LDG
+        pmx_mbar_expect_tx(mbar, S::AUX_BYTES);
+#else
+        pmx_mbar_expect_tx(mbar, S::LOAD_BYTES);
+        for (int l0 = 0; l0 < LINES; l0 += 256)
+            pmx_tma_load_3d(in + l0 * 128, &tmap, 0, (tt & wk.tpb_mask) * LINES + l0, p.bc0 + bc, mbar);
+#endif
+        int b_, col_;
+        pmx_split_bc(bc, f, b_, col_);
+        unsigned char* a = aux0 + buf * S::AUX_BYTES;
+        pmx_bulk_load(a, &p.pkg[b_], S::PKG_BYTES, mbar);
+        pmx_bulk_load(a + S::PKG_BYTES, reinterpret_cast<const cpx*>(p.tw4) + (size_t)row0 * W::PER, S::TAB_BYTES, mbar);
+    };
+    if (threadIdx.x == 0) {
+        pmx_mbar_init(mbar, 1);
+        pmx_fence_mbar_init();
+    }
+    pmx_load_stage_tw<L>(stw, p.tw_stage);
+    if (p.pdl) {  // everything above is independent of the previous kernel of the stream
+        pmx_pdl_launch_dependents();
+        pmx_pdl_wait();
+    }
+    pmx_cache_live(sdone, p);
+    __syncthreads();
+    int tile = live(blockIdx.x), it = 0;
+    if (threadIdx.x == 0 && tile < total) issue(tile, 0);
+    pmx_stagger(p);
+    uint32_t phase = 0;
+    PMX_T_DECL
+    while (tile < total) {
+        const int tt = wk.phys(tile), bc = tt >> wk.ltpb, row0 = (tt & wk.tpb_mask) * G;
+        int b, col;
+        pmx_split_bc(bc, f, b, col);
+        PMX_ASSERT(tt >= 0 && tt < total && bc < p.batch * f.nfc && b < p.batch && col < f.nfc && b * f.nfc + col == bc);
+        PMX_ASSERT(row0 + G <= p.N2 && L == p.N1);
+        const unsigned char* aux = aux0 + (it & 1) * S::AUX_BYTES;
+        const StepPkg* st = reinterpret_cast<const StepPkg*>(aux);
+        const cpx* gtab = reinterpret_cast<const cpx*>(aux + S::PKG_BYTES);
+        const int next = live(tile + gridDim.x);
+        cpx x[8], y[8];
+        PMX_T_MARK(0)
+#ifdef PMX_AC_LDG
+        {
+            const cpx* src = reinterpret_cast<const cpx*>(p.field) + ((size_t)bc * N + (size_t)(row0 + rl) * L) * 2;
+#pragma unroll
+            for (int q = 0; q < 8; ++q) ld_sa(src + (size_t)(t + q * T) * 2, x[q], y[q]);
+        }
+#endif
+        pmx_mbar_wait(mbar, phase);
+        phase ^= 1u;
+        PMX_T_MARK(1)
+#ifndef PMX_AC_LDG
+#pragma unroll
+        for (int q = 0; q < 8; ++q) lds_sa(in, pmx_swz<7>((uint32_t)((rl * L + t + q * T) * PMX_SA_BYTES)), x[q], y[q]);
+#endif
+        {   // Pass B left v = conj(z), z = its transform output before the four-step twiddle W_N^(-n2*k1), k1 = t + q*T.
+            // The inverse transform over k1 = conj o forward o conj applied to conj(z)*conj(W): its input is z*W.
+            const cpx* tb = gtab + rl * W::PER;
+            const cpx wl = tb[t & (W::NLO - 1)];
+#pragma unroll
+            for (int q = 0; q < 8; ++q) {
+                const cpx w = cmul(wl, tb[W::NLO + ((t + q * T) >> W::LO)]);
+                x[q] = cmul(cconj(x[q]), w);
+                y[q] = cmul(cconj(y[q]), w);
+            }
+        }
+        const real sc = (real)st->scale, nsc = -sc;
+        __syncthreads();  // every thread has seen this phase complete before the barrier is armed again
+#ifdef PMX_AC_LDG
+        if (threadIdx.x == 0 && next < total) issue(next, (it + 1) & 1);
+#else
+        if (PF && threadIdx.x == 0 && next < total) issue(next, (it + 1) & 1);
+#endif
+        PMX_T_MARK(2)
+        cpx* sx = work + rl * PmxSmem<L, G>::STRIDE;
+        cpx* sy = sx + L;
+        PMX_T_MARK(3)
+#if defined(PMX_AC_LDG) || defined(PMX_AC_LATE_ISSUE)
+        CtaFFT<R, L>::run(x, y, sx, sy, t, stw);
+        PMX_T_MARK(4)
+#ifndef PMX_AC_LDG
+        if (!PF && threadIdx.x == 0 && next < total) issue(next, (it + 1) & 1);
+#endif
+#else
+        CtaFFT<R, L>::run(x, y, sx, sy, t, stw, [&] {
+            if (!PF && threadIdx.x == 0 && next < total) issue(next, (it + 1) & 1);
+        });
+        PMX_T_MARK(4)
+#endif
+        {
+            cpx* base = reinterpret_cast<cpx*>(p.field) + ((size_t)bc * N + (size_t)(row0 + rl) * L) * 2;
+#pragma unroll
+            for (int q = 0; q < 8; ++q) {
+                x[q] = mkc(x[q].x * sc, x[q].y * nsc);
+                y[q] = mkc(y[q].x * sc, y[q].y * nsc);
+            }
+            pmx_nl_step(x, y, st, f, col);   // ---- N(-xi*gam): the gam of f is the backpropagated one
+#pragma unroll
+            for (int q = 0; q < 8; ++q) st_sa(base + (size_t)(t + q * T) * 2, x[q], y[q]);
+        }
+        PMX_T_MARK(5)
+        tile = next;
+        ++it;
+        __syncthreads();  // everyone is done with this tile's auxiliary buffer
+        PMX_T_MARK(6)
+    }
+    PMX_T_FLUSH(3)
 }

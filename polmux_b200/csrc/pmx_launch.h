@@ -33,6 +33,10 @@ struct PmxLaunchTable {
     size_t smemOnchip;
     cudaError_t (*onchip_setup)();
     cudaError_t (*onchip)(int nfc, int batch, cudaStream_t s, const PassParams& p, const FiberConst& f);
+    // digital backpropagation: pass C with the nonlinear step after the scale and no max reduction (pmx_k_passC_nl);
+    // the setup opts in to the shared memory and reports its resident CTAs per SM
+    cudaError_t (*passC_nl_setup)(int* ctas);
+    cudaError_t (*passC_nl)(int grid_x, cudaStream_t s, const PassParams& p, const FiberConst& f, const CUtensorMap& cols);
 };
 
 const PmxLaunchTable* pmx_get_table(int L, int precision = 0);  // nullptr if L is not built

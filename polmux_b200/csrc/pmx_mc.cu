@@ -67,7 +67,7 @@ struct Worker {
 // realizations [r0, r1) on one device
 void run_shard(Worker& w, int dev, int r0, int r1, const pmx_fiber_desc& fd, const pmx_mc_desc& m, const pmx_field& tx) {
     pmx_devfield *ftx = nullptr, *work = nullptr, *work2 = nullptr;
-    pmx_plan *plan = nullptr, *inv = nullptr, *fo = nullptr, *fe = nullptr;
+    pmx_plan *plan = nullptr, *inv = nullptr, *fo = nullptr, *fe = nullptr, *dbp = nullptr;
     pmx_ctx* rxctx = nullptr;   // the receive chain's own context (stream): it runs beside the next group's propagation
     int64_t *tmp = nullptr, *tmp2 = nullptr;
     std::future<int> pending;
@@ -183,6 +183,14 @@ void run_shard(Worker& w, int dev, int r0, int r1, const pmx_fiber_desc& fd, con
                 w.err = std::string("pmx_filter_create: ") + pmx_last_error(rxctx);
                 goto done;
             }
+            if (m.rx->dbp) {   // digital backpropagation of the link, first thing of the receive chain
+                const int rc = pmx_dbp_create(rxctx, &d, m.rx->dbp, &dbp);
+                if (rc != PMX_OK) {
+                    w.rc = rc;
+                    w.err = std::string("pmx_dbp_create: ") + pmx_last_error(rxctx);
+                    goto done;
+                }
+            }
         }
         for (int g0 = r0, gi = 0; g0 < r1; g0 += B, ++gi) {
             const int nb = std::min(B, r1 - g0);
@@ -232,7 +240,8 @@ void run_shard(Worker& w, int dev, int r0, int r1, const pmx_fiber_desc& fd, con
                 }
                 int64_t* const dst = w.counts_dev + g0;
                 pending = std::async(std::launch::async, [=, &m, &rxerr]() -> int {
-                    int rc = pmx_fiber_exec(fo, cur, nullptr);
+                    int rc = dbp ? pmx_dbp_exec(dbp, cur) : PMX_OK;
+                    if (rc == PMX_OK) rc = pmx_fiber_exec(fo, cur, nullptr);
                     if (rc == PMX_OK) rc = pmx_cohmix_exec(rxctx, cur, m.rx->lo_ecw, m.rx->lo_detune, m.rx->lo_phase, m.rx->balanced);
                     if (rc == PMX_OK) rc = pmx_fiber_exec(fe, cur, nullptr);
                     if (rc == PMX_OK) rc = pmx_dsp_count(rxctx, cur, &m.rx->dsp, m.rx->ref_patmat, ctmp, nullptr);
@@ -271,6 +280,7 @@ done:
     if (tmp2) cudaFree(tmp2);
     pmx_plan_destroy(fo);
     pmx_plan_destroy(fe);
+    pmx_plan_destroy(dbp);
     pmx_plan_destroy(inv);
     pmx_plan_destroy(plan);
     pmx_field_destroy(work);

@@ -94,6 +94,15 @@ cudaError_t passB(int gx, cudaStream_t s, const PassParams& p, const FiberConst&
 cudaError_t passC(int gx, cudaStream_t s, const PassParams& p, const FiberConst& f, const CUtensorMap& m) {
     return launch(pmx_k_passC<real, L, GAC, PFAC>, gx, SC::THREADS, SC::TOTAL, s, p, f, m);
 }
+cudaError_t passC_nl_setup(int* ctas) {
+    cudaError_t e = cudaFuncSetAttribute(pmx_k_passC_nl<real, L, GAC, PFAC>, cudaFuncAttributeMaxDynamicSharedMemorySize, SC::TOTAL);
+    if (e != cudaSuccess) return e;
+    cudaFuncSetAttribute(pmx_k_passC_nl<real, L, GAC, PFAC>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas, pmx_k_passC_nl<real, L, GAC, PFAC>, SC::THREADS, SC::TOTAL);
+}
+cudaError_t passC_nl(int gx, cudaStream_t s, const PassParams& p, const FiberConst& f, const CUtensorMap& m) {
+    return launch(pmx_k_passC_nl<real, L, GAC, PFAC>, gx, SC::THREADS, SC::TOTAL, s, p, f, m);
+}
 // precision-dependent helpers that do not depend on L (every table carries them)
 void init_max(dim3 grid, cudaStream_t s, const PassParams& p, const FiberConst& f) {
     pmx_k_init<<<grid, 256, 256, s>>>(p, f);
@@ -141,4 +150,5 @@ cudaError_t onchip(int nfc, int batch, cudaStream_t s, const PassParams& p, cons
 extern const PmxLaunchTable PMX_TABLE_NAME = {
     L, GAC, GB, PFAC ? 1 : 0, PFB ? 1 : 0, SA::THREADS, SB::THREADS, (size_t)SA::TOTAL, (size_t)SB::TOTAL,
     pmx_tw_total(L), pmx_tw_layout(L), PmxTw4<L>::LO, PmxTw4<L>::PER, PMX_PRECISION, (int)sizeof(cpx),
-    setup, passA, passB, passC, init_max, fill_tw4, xpm_sum, (size_t)SO::TOTAL, onchip_setup, onchip};
+    setup, passA, passB, passC, init_max, fill_tw4, xpm_sum, (size_t)SO::TOTAL, onchip_setup, onchip, passC_nl_setup,
+    passC_nl};

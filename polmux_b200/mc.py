@@ -206,7 +206,8 @@ class McRunner:
 
     def __init__(self, ctx: _lib.Context, setup: FiberSetup, tx_x, tx_y, sym, nsymb: int, nt: int, nspan: int,
                  gain_db: float, nf_db: float, nreal: int, batch: int, rank: int = 0, world: int = 1,
-                 receiver: str = 'genie', dsp_params=None, rx_params=None, ich: int = 1, pipeline: bool = True):
+                 receiver: str = 'genie', dsp_params=None, rx_params=None, ich: int = 1, pipeline: bool = True,
+                 compensation: str = 'cd', dbp_params=None):
         """receiver: 'genie' -- ideal linear equaliser from the known plates + data-aided decision (pmx_qpsk_count);
         'blind' -- chromatic dispersion compensated, then the DSP core of dsp4cohdec (CMA polarization demultiplexer,
         Viterbi & Viterbi carrier recovery, differential decision: pmx_dsp_count, polmux_b200/dsp.py);
@@ -214,12 +215,19 @@ class McRunner:
         filter, LO mixing, photodiodes, low-pass filter; rx_params = its x struct, polmux_b200/receiver.py), the
         currents sampled at the symbol centres delayed by the filters' 'theory' delay (dsp4cohdec.m:490-503) and
         divided by 4*sqrt(POWER(ich)) (dsp4cohdec.m:226-227), then the same DSP core.
-        pipeline: run the receive chain of a group beside the propagation of the next one (same counts either way)"""
+        pipeline: run the receive chain of a group beside the propagation of the next one (same counts either way)
+        compensation ('blind' and 'cohmix'): 'cd' -- the all-pass step that undoes the link's dispersion; 'dbp' -- digital
+        backpropagation of the link (polmux_b200/dbp.py) with dbp_params (steps_per_span, step_len, span_steps, xi; default
+        one step per span, xi = 1), the amplifier gain undone before each span"""
         import torch
         from . import dsp as _dsp
         self.receiver, self.dsp_params = receiver, dict(dsp_params or {})
         if receiver not in ('genie', 'blind', 'cohmix'):
             raise ValueError("receiver must be 'genie', 'blind' or 'cohmix'")
+        if compensation not in ('cd', 'dbp'):
+            raise ValueError("compensation must be 'cd' or 'dbp'")
+        if compensation == 'dbp' and receiver == 'genie':
+            raise ValueError("the genie receiver undoes the link with the known plates: compensation='dbp' needs 'blind' or 'cohmix'")
         self.ref_patmat = _dsp.reference_pattern(np.asarray(sym)[0], np.asarray(sym)[1]) if receiver != 'genie' else None
         self.passes = []
         self.ctx, self.setup, self.sym, self.nsymb, self.nt = ctx, setup, sym, nsymb, nt
@@ -241,7 +249,12 @@ class McRunner:
         self.rx = None
         if receiver != 'genie':
             self.rxctx = _lib.Context(ctx.device) if self.pipelined else ctx
-            self.rx = dict(cd=self.link.cd_plan(self.rxctx), S=None)
+            if compensation == 'dbp':
+                from .dbp import dbp_plan
+                comp = dbp_plan(self.rxctx, setup, nspan, gain_db, batch=batch, precision='f64', **dict(dbp_params or {}))
+            else:
+                comp = self.link.cd_plan(self.rxctx)
+            self.rx = dict(cd=comp, S=None)
             if receiver == 'cohmix':
                 from . import receiver as _rx
                 from .gstate import GSTATE
@@ -324,7 +337,7 @@ class McRunner:
             for k in ('fo', 'fe', 'col'):
                 if self.rx.get(k) is not None:
                     self.rx[k].close()
-            if self.pipelined:
+            if self.pipelined or isinstance(self.rx['cd'], _lib.DbpPlan):
                 self.rx['cd'].close()
 
 
@@ -340,12 +353,13 @@ def run_mc(ctx: _lib.Context, setup: FiberSetup, tx_x, tx_y, sym, nsymb: int, nt
 
 def run_mc_native(setup: FiberSetup, tx_x, tx_y, sym, nsymb: int, nt: int, nspan: int, gain_db: float, nf_db: float,
                   nreal: int, batch: int, devices=(0,), ase_seed: int = 1, equalize: bool = True, receiver=None,
-                  dsp_params=None, ich: int = 1):
+                  dsp_params=None, ich: int = 1, dbp_params=None):
     """The same Monte-Carlo job through pmx_mc_run: one process, one host thread and one context per GPU of `devices`,
     the integer all-reduce done with NCCL inside the library (no torch.distributed).  Plate draws as run_mc's.
     receiver: None -- the data-aided counter (with `equalize`); a dict = the x struct of receiver_cohmix -- the reference's
     receive chain (front-end, sampler, DSP core with dsp_params) behind the link, its optical response carrying the
-    compensation of the link's chromatic dispersion (as x.dpost / p.applydcf would).
+    compensation of the link's chromatic dispersion (as x.dpost / p.applydcf would), or with dbp_params (a dict as
+    McRunner's) the digital backpropagation of the link ahead of the front-end and the optical filter alone.
     -> (counts [nreal] int64, Sa*steps over all realizations)"""
     import ctypes as C
     lib = _lib.load()
@@ -376,8 +390,11 @@ def run_mc_native(setup: FiberSetup, tx_x, tx_y, sym, nsymb: int, nt: int, nspan
         delay = _rx.evaldelay(x['oftype'], x['obw'] * 0.5) + _rx.evaldelay(x['eftype'], x['ebw']) + x['post_delay']
         p = dict(dsp_params or {})
         p.update(sample_shift=int(round(delay * nt)), peak=4.0 * math.sqrt(float(np.asarray(GSTATE.POWER).ravel()[ich - 1])))
-        ph = np.asarray(setup.betat, dtype=np.float64)[:, 0] * (setup.length * nspan)      # the link's all-pass phase, undone
-        hopt = np.ascontiguousarray(S.hf_opt * (np.cos(ph) + 1j * np.sin(ph)))
+        if dbp_params is None:
+            ph = np.asarray(setup.betat, dtype=np.float64)[:, 0] * (setup.length * nspan)      # the link's all-pass phase, undone
+            hopt = np.ascontiguousarray(S.hf_opt * (np.cos(ph) + 1j * np.sin(ph)))
+        else:
+            hopt = np.ascontiguousarray(np.asarray(S.hf_opt, dtype=np.complex128))
         hel = np.ascontiguousarray(np.asarray(S.hf_el, dtype=np.complex128))
         ref = np.ascontiguousarray(_dsp.reference_pattern(np.asarray(sym)[0], np.asarray(sym)[1]), dtype=np.uint8)
         lop = None if S.lophase is None else np.ascontiguousarray(S.lophase, dtype=np.float64)
@@ -387,7 +404,15 @@ def run_mc_native(setup: FiberSetup, tx_x, tx_y, sym, nsymb: int, nt: int, nspan
         rx.lo_phase = None if lop is None else lop.ctypes.data_as(_lib._dp)
         rx.dsp = _dsp._desc(nsymb, nt, p)
         rx.ref_patmat = ref.ctypes.data_as(C.POINTER(C.c_uint8))
-        rxkeep = (hopt, hel, ref, lop, rx)
+        if dbp_params is not None:
+            pd = dict(dbp_params)
+            if pd.get('step_len') is None and pd.get('steps_per_span') is None:
+                pd['steps_per_span'] = 1
+            dd, dkeep = _lib.make_dbp(nspan, gain, **pd)
+            rx.dbp = C.pointer(dd)
+            rxkeep = (hopt, hel, ref, lop, rx, dd, dkeep)
+        else:
+            rxkeep = (hopt, hel, ref, lop, rx)
         m.rx = C.pointer(rx)
         m.equalize = 0
     fx = np.ascontiguousarray(np.asarray(tx_x, dtype=np.complex128).T)[None]
