@@ -251,7 +251,15 @@ int pmx_link_run(pmx_ctx* ctx, const pmx_fiber_desc* desc, const pmx_link_desc* 
  *     u <- N(-xi*gam, h) u                                       matrix_nl_step (fiber.m:827-851) with gam -> -xi*gam and
  *                                                                the forward leff(h) = (1 - exp(-alpha*h))/alpha
  * With xi = 1 and the forward run's own steps (pmx_fiber_result.trace_dz), DBP inverts a noise-free fiber without PMD up
- * to rounding.  DBP ignores the 'p' flag, the plates and dgdrms; the 'x' flag fails with PMX_ERR_XPM_VECTOR as in fiber.
+ * to rounding.  With pmd = 0, DBP ignores the 'p' flag, the plates and dgdrms; the 'x' flag fails with
+ * PMX_ERR_XPM_VECTOR as in fiber.
+ * PMD-aware DBP (pmd = 1, the fiber's 'p' flag, plates from pmx_dbp_set_plates): the linear operator of a step is the
+ * inverse of the forward step's trunk product (matrix_step, fiber.m:904-935): the same trunk pieces in reverse order,
+ * the plates last to first, db0, db1 (dgdrms) and betat negated, from and back to the laboratory basis.  The trunk
+ * pieces of every step are the forward run's: checkstep (fiber.m:739-758) replayed on the span's forward steps, with
+ * zprop accumulated step by step and the last step ending at the fiber length, so that trace_dz reproduces the forward
+ * run's partition exactly.  Steps that would index past the last plate fail with PMX_ERR_PLATE_INDEX as fiber would.
+ * With xi = 1 and trace_dz, PMD-aware DBP inverts a noise-free 'gps-' link up to rounding.
  * Two-polarization fields (scalar_field = 0), nfc <= 64, nfft from 2^12 to 2^24, FP64 or FP32; other fields fail with
  * PMX_ERR_UNSUPPORTED.  Every step is the three HBM passes of a forward step; the step packages of the whole schedule
  * are built when the plan is created, so pmx_dbp_exec enqueues every step without reading anything back. */
@@ -262,14 +270,24 @@ typedef struct pmx_dbp_desc {
     const double* step_len;    /* all spans' steps concatenated, each span in FORWARD order (e.g. trace_dz)             */
     double xi;                 /* fraction of gamma backpropagated; 1 = all                                              */
     double gain;               /* linear amplifier gain after every span, undone first; 0 = none                         */
+    int32_t pmd;               /* 1: PMD-aware (the fiber's 'p' flag, plates from pmx_dbp_set_plates); 0: PMD ignored    */
+    int32_t reserved;
 } pmx_dbp_desc;
 /* fiber: the link's fiber (length, alphalin, gam, manakov, fls, dispersion as for pmx_plan_create; batch and precision of
- * the fields the plan will run on).  Validates dbp: PMX_ERR_INVALID for nspan < 1, a non-finite xi, gain < 0, a
- * negative or non-finite step, or a span whose steps do not sum to fiber->length within 1e-9 relative.  The explicit
- * schedule (steps_per_span = 0) needs span_steps and step_len, span_steps[k] >= 1. */
+ * the fields the plan will run on; with pmd, nplates, dgdrms or db1 as well).  Validates dbp: PMX_ERR_INVALID for
+ * nspan < 1, a non-finite xi, gain < 0, a negative or non-finite step, or a span whose steps do not sum to fiber->length
+ * within 1e-9 relative.  The explicit schedule (steps_per_span = 0) needs span_steps and step_len, span_steps[k] >= 1.
+ * pmd = 1 needs the 'p' flag and nplates >= 1 (PMX_ERR_INVALID) and a step package table of at most 1 GiB
+ * (steps * batch * 2800 bytes, PMX_ERR_INVALID); a schedule that indexes past the last plate fails with
+ * PMX_ERR_PLATE_INDEX. */
 int pmx_dbp_create(pmx_ctx* ctx, const pmx_fiber_desc* fiber, const pmx_dbp_desc* dbp, pmx_plan** plan);
+/* The waveplates of a PMD-aware plan: db0, theta, epsilon [nspan][plate_sets][nplates] in FORWARD span and plate order
+ * and sign, as pmx_link_desc takes them; plate_sets is 1 (shared by the batch) or batch.  The library reverses and
+ * negates them and rebuilds the step packages on the device; calling it again swaps in a new draw. */
+int pmx_dbp_set_plates(pmx_plan* plan, int32_t plate_sets, const double* db0, const double* theta, const double* epsilon);
 /* In place on a resident field; returns when the field is backpropagated.  The field may belong to another context of
- * the same device (as for pmx_fiber_exec).  Destroy the plan with pmx_plan_destroy. */
+ * the same device (as for pmx_fiber_exec).  A PMD-aware plan needs its plates first (PMX_ERR_INVALID).  Destroy the
+ * plan with pmx_plan_destroy. */
 int pmx_dbp_exec(pmx_plan* plan, pmx_devfield* f);
 
 /* ---- create_field('unique'): the WDM multiplex on the device (create_field.m:113-149,180-199) ----------------
@@ -413,6 +431,9 @@ typedef struct pmx_mc_desc {
     const uint8_t* sym;          /* [2][nsymb] transmitted QPSK symbol indices (pmx_qpsk_count)               */
     int32_t nsymb, nt;
     const pmx_mc_receiver* rx;   /* NULL: the data-aided counter above; else the reference's receive chain     */
+    const pmx_dbp_desc* dbp;     /* without rx: NULL, or PMD-aware DBP (pmd = 1) with every group's own plates in place */
+                                 /* of the equaliser ahead of the data-aided counter; pmd = 0 is PMX_ERR_INVALID       */
+                                 /* there.  With rx, rx->dbp with pmd = 1 gets the group's plates the same way.       */
 } pmx_mc_desc;
 /* fiber: the span's fiber (batch / plate_sets / plates are taken from mc); tx: HOST Tx field of one realization;
  * counts: [nreal] bit errors per realization; sa_steps (may be NULL): sum over all realizations of nfft*nfc*ncycle;

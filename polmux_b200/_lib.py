@@ -34,7 +34,7 @@ EXPORTS = [
     'pmx_host_is_pinned', 'pmx_scalar_adaptive_run', 'pmx_mc_run', 'pmx_mc_nccl_available',
     'pmx_ampliflat_exec_at', 'pmx_dsp_count', 'pmx_field_mean_power', 'pmx_pmd_matrix', 'pmx_field_jones', 'pmx_filter_create', 'pmx_field_copy_cols', 'pmx_field_modulate',
     'pmx_cohmix_exec', 'pmx_field_mean_power_xy', 'pmx_cohmix_run', 'pmx_dsp_phases', 'pmx_field_quantize', 'pmx_inverse_pmd_run',
-    'pmx_dbp_create', 'pmx_dbp_exec',
+    'pmx_dbp_create', 'pmx_dbp_exec', 'pmx_dbp_set_plates',
 ]
 
 
@@ -81,7 +81,7 @@ class DspDesc(C.Structure):
 
 class DbpDesc(C.Structure):
     _fields_ = [('nspan', C.c_int32), ('steps_per_span', C.c_int32), ('span_steps', _ip), ('step_len', _dp),
-                ('xi', C.c_double), ('gain', C.c_double)]
+                ('xi', C.c_double), ('gain', C.c_double), ('pmd', C.c_int32), ('reserved', C.c_int32)]
 
 
 class McReceiver(C.Structure):
@@ -94,7 +94,7 @@ class McDesc(C.Structure):
     _fields_ = [('ndev', C.c_int32), ('device_ids', C.POINTER(C.c_int32)), ('nreal', C.c_int32), ('batch', C.c_int32),
                 ('nspan', C.c_int32), ('equalize', C.c_int32), ('db0', _dp), ('theta', _dp), ('epsilon', _dp),
                 ('gain', C.c_double), ('sigma', _dp), ('ase_seed', C.c_uint64), ('sym', C.POINTER(C.c_uint8)),
-                ('nsymb', C.c_int32), ('nt', C.c_int32), ('rx', C.POINTER(McReceiver))]
+                ('nsymb', C.c_int32), ('nt', C.c_int32), ('rx', C.POINTER(McReceiver)), ('dbp', C.POINTER(DbpDesc))]
 
 
 class BrfDesc(C.Structure):
@@ -180,6 +180,7 @@ def load():
     lib.pmx_link_run.argtypes = [vp, C.POINTER(FiberDesc), C.POINTER(LinkDesc), C.POINTER(Field), C.POINTER(FiberResult)]
     lib.pmx_dbp_create.argtypes = [vp, C.POINTER(FiberDesc), C.POINTER(DbpDesc), C.POINTER(vp)]
     lib.pmx_dbp_exec.argtypes = [vp, vp]
+    lib.pmx_dbp_set_plates.argtypes = [vp, C.c_int32, _dp, _dp, _dp]
     _lib = lib
     return lib
 
@@ -531,13 +532,23 @@ class DbpPlan(Plan):
     def execute(self, field: DeviceField, trace_cap=0):
         self.ctx.check(self.ctx.lib.pmx_dbp_exec(self.h, field.h))
 
+    def set_plates(self, db0, theta, epsilon, plate_sets=1):
+        """the waveplates of a PMD-aware plan (pmx_dbp_set_plates): each [nspan][plate_sets][nplates] in forward span and
+        plate order and sign, as the link took them; plate_sets is 1 or the batch"""
+        a, b, c = _f64(db0).reshape(-1), _f64(theta).reshape(-1), _f64(epsilon).reshape(-1)
+        n = int(self.dbp.nspan) * int(plate_sets) * int(self.desc.nplates)
+        if not (a.size == b.size == c.size == n):
+            raise ValueError('plates must be [nspan][plate_sets][nplates] = %d values each' % n)
+        self.ctx.check(self.ctx.lib.pmx_dbp_set_plates(self.h, int(plate_sets), _ptr(a), _ptr(b), _ptr(c)))
 
-def make_dbp(nspan, gain=0.0, steps_per_span=None, step_len=None, span_steps=None, xi=1.0):
+
+def make_dbp(nspan, gain=0.0, steps_per_span=None, step_len=None, span_steps=None, xi=1.0, pmd=False):
     """-> (DbpDesc, keep-alive dict).  Either steps_per_span (uniform steps) or step_len: the steps of one span in forward
-    order (every span gets them), or with span_steps [nspan] the steps of all spans concatenated."""
+    order (every span gets them), or with span_steps [nspan] the steps of all spans concatenated.  pmd: PMD-aware DBP
+    (the plates follow with DbpPlan.set_plates)."""
     keep = {}
     d = DbpDesc()
-    d.nspan, d.xi, d.gain = int(nspan), float(xi), float(gain)
+    d.nspan, d.xi, d.gain, d.pmd = int(nspan), float(xi), float(gain), int(bool(pmd))
     if step_len is None:
         d.steps_per_span = int(1 if steps_per_span is None else steps_per_span)
         return d, keep

@@ -211,6 +211,13 @@ static int build_maps(pmx_ctx* c, pmx_devfield* f) {
     return PMX_OK;
 }
 
+// One step of a PMD-aware DBP plan (pmx_dbp_create), in execution order: what the step control would have left in
+// StepCtl, mirrored onto the span's reversed plate table, and the span whose plates the step reads.
+struct DbpGeo {
+    double dz, leff, scale, dzb_first, dzb_last;
+    int ntrunk, n_first, span, bmode;
+};
+
 struct pmx_plan {
     pmx_ctx* ctx;
     pmx_fiber_desc d;  // scalar copy (pointers not kept)
@@ -236,6 +243,12 @@ struct pmx_plan {
     FiberConst fc_a, fc_c;
     StepPkg* sched = nullptr;
     std::vector<int> sched_idx;
+    // PMD-aware DBP: the geometry of every step in execution order (device), each step's span, and whether
+    // pmx_dbp_set_plates has filled plates ([nspan][plate_sets][nplates], reversed and negated) and packages
+    bool dbp_pmd = false, dbp_plates_set = false;
+    int dbp_nspan = 0;
+    DbpGeo* geo_d = nullptr;
+    std::vector<int> sched_span;
 };
 
 static int set_err(pmx_ctx* ctx, int code, const char* fmt, ...) {
@@ -743,6 +756,7 @@ extern "C" void pmx_plan_destroy(pmx_plan* p) {
     if (p->trace_dz) cudaFreeAsync(p->trace_dz, st);
     if (p->trace_ntrunk) cudaFreeAsync(p->trace_ntrunk, st);
     if (p->sched) cudaFreeAsync(p->sched, st);
+    if (p->geo_d) cudaFreeAsync(p->geo_d, st);
     delete p;
 }
 
@@ -3319,6 +3333,150 @@ extern "C" int pmx_scalar_adaptive_run(pmx_ctx* c, const pmx_fiber_desc* d, doub
 // exp(+alpha*h/2)/N and the nonlinear step with gam -> -xi*gam -- in the order N(-xi*gam) L(-h) A(-h), the inverse of the
 // forward A(h) L(h) N(h).  The schedule is known when the plan is made: every step's package is built here and the host
 // enqueues the whole link without reading anything back.
+//
+// PMD-aware DBP (pmd = 1): pass B of step j applies the inverse of the forward step's trunk product.  The forward step
+// covers plates n_first .. n_first+ntrunk-1 with pieces dzb_first, lcorr, ..., dzb_last (checkstep); its inverse is the
+// same product on the table with the plates reversed (n' = nplates-1-n) and db0, db1, betat negated, over the pieces in
+// reverse order -- a forward matrix_step of the reversed fiber with n_first' = nplates - n_first - ntrunk and the first
+// and last piece swapped.  The partition is the forward run's own, replayed here from the forward steps: a fresh
+// checkstep on the reversed coordinate would round differently at the plate boundaries.
+
+// pmx_ctl_next's checkstep on each span's forward steps, same operation order (zprop accumulated step by step, the last
+// step ending at the fiber length; the host compiles this without FMA contraction), mirrored; execution order.
+static int dbp_geometry(pmx_ctx* c, const pmx_fiber_desc& fd, const pmx_dbp_desc* g, const std::vector<double>& h,
+                        const std::vector<int>& nstep, std::vector<DbpGeo>& geo) {
+    const int np = fd.nplates;
+    const double Lf = fd.length, lcorr = fd.length / np, alpha = fd.alphalin, halfalpha = 0.5 * fd.alphalin;
+    const double invN = 1.0 / (double)fd.nfft, ig = g->gain > 0 ? 1.0 / std::sqrt(g->gain) : 1.0;
+    size_t total = 0;
+    for (int k = 0; k < g->nspan; ++k) total += (size_t)nstep[k];
+    if (fd.batch < 1 || fd.batch > 65535)
+        return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: PMD-aware DBP takes batches of 1 to 65535, got %d", fd.batch);
+    const double bytes = (double)total * fd.batch * sizeof(StepPkg);
+    if (bytes > (double)(1u << 30))
+        return set_err(c, PMX_ERR_INVALID,
+                       "pmx_dbp_create: the step package table of PMD-aware DBP (%zu steps x batch %d x %zu B) exceeds 1 GiB", total,
+                       fd.batch, sizeof(StepPkg));
+    std::vector<size_t> span0(g->nspan, 0);
+    for (int k = 1; k < g->nspan; ++k) span0[k] = span0[k - 1] + nstep[k - 1];
+    geo.clear();
+    geo.reserve(total);
+    std::vector<DbpGeo> fw;
+    for (int k = g->nspan - 1; k >= 0; --k) {
+        fw.assign(nstep[k], DbpGeo());
+        double zprop = 0.0, dz_miss = 0.0;
+        int ntot = 0;
+        for (int j = 0; j < nstep[k]; ++j) {
+            const double dz = h[span0[k] + j];
+            zprop = zprop + dz;
+            const double zend = (j == nstep[k] - 1) ? Lf : zprop;
+            const int nzc = (int)std::ceil(zend / lcorr);
+            int ntrunk, nmem;
+            double dzb_first, dzb_last;
+            if (dz_miss == 0.0) {
+                nmem = 0;
+                ntrunk = nzc - ntot;
+                const double dzlast = dz - lcorr * (double)(ntrunk - 1);
+                dzb_first = (ntrunk > 1) ? lcorr : dzlast;
+                dzb_last = dzlast;
+                dz_miss = lcorr - dzlast;
+            } else {
+                nmem = 1;
+                ntrunk = nzc - ntot + 1;
+                if (ntrunk == 1) {
+                    dzb_first = dzb_last = dz;
+                    dz_miss = dz_miss - dz;
+                } else {
+                    const double dzlast = (dz - dz_miss) - lcorr * (double)(ntrunk - 2);
+                    dzb_first = dz_miss;
+                    dzb_last = dzlast;
+                    dz_miss = lcorr - dzlast;
+                }
+            }
+            const int n_first = ntot - nmem;
+            if (ntrunk > 0 && (ntot + ntrunk - nmem > np || n_first < 0))   // brf.theta(n) index error (fiber.m:910)
+                return set_err(c, PMX_ERR_PLATE_INDEX, "pmx_dbp_create: step %d of span %d reaches plate %d of %d", j, k,
+                               ntot + ntrunk - nmem, np);
+            DbpGeo& G = fw[j];
+            G.dz = dz;
+            G.leff = (alpha == 0.0) ? dz : (1.0 - std::exp(-alpha * dz)) / alpha;   // fiber.m:827-831
+            G.scale = std::exp(halfalpha * dz) * invN * (j == nstep[k] - 1 ? ig : 1.0);
+            G.ntrunk = std::max(ntrunk, 0);
+            G.n_first = np - n_first - ntrunk;   // mirrored
+            G.dzb_first = dzb_last;
+            G.dzb_last = dzb_first;
+            G.span = k;
+            G.bmode = ntrunk > 0 ? (PMX_BM_ENTRY_R | PMX_BM_EXIT_R) : 0;   // laboratory basis between the steps
+            ntot += ntrunk - nmem;
+        }
+        for (int j = nstep[k] - 1; j >= 0; --j) geo.push_back(fw[j]);
+    }
+    return PMX_OK;
+}
+
+// The step packages of a PMD-aware DBP plan, one CTA per (step, realization): the geometry goes into a step control
+// block in shared memory and pmx_pkg_fill builds the package from it as the step control does for a forward step.
+__global__ void __launch_bounds__(128) pmx_k_dbp_pkg(const DbpGeo* __restrict__ geo, const PlateConst* plates, StepPkg* out,
+                                                     FiberConst f, int batch) {
+    const int s = blockIdx.x, b = blockIdx.y;
+    __shared__ StepCtl c;
+    const DbpGeo& G = geo[s];
+    StepPkg* g = out + (size_t)s * batch + b;
+    if (threadIdx.x == 0) {
+        c.dz_cur = G.dz;
+        c.leff = G.leff;
+        c.scale = G.scale;
+        c.dzb_first = G.dzb_first;
+        c.dzb_last = G.dzb_last;
+        c.ntrunk = G.ntrunk;
+        c.n_first = G.n_first;
+        c.bmode = G.bmode;
+        g->state = PMX_ST_RUN;
+    }
+    __syncthreads();
+    pmx_pkg_fill(&c, g, f, plates + ((size_t)G.span * f.plate_sets + (f.plate_sets > 1 ? b : 0)) * f.nplates);
+}
+
+extern "C" int pmx_dbp_set_plates(pmx_plan* p, int32_t sets, const double* db0, const double* theta, const double* epsilon) {
+    if (!p) return set_err(nullptr, PMX_ERR_INVALID, "pmx_dbp_set_plates: null plan");
+    pmx_ctx* c = p->ctx;
+    if (!p->dbp_pmd) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_set_plates: not a PMD-aware DBP plan (pmx_dbp_create with pmd = 1)");
+    if (sets != 1 && sets != p->d.batch)
+        return set_err(c, PMX_ERR_INVALID, "pmx_dbp_set_plates: plate_sets must be 1 or batch (%d), got %d", p->d.batch, sets);
+    if (!db0 || !theta || !epsilon) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_set_plates: db0, theta and epsilon are required");
+    const int np = p->d.nplates;
+    const size_t per = (size_t)sets * np;
+    std::vector<double> r[3];
+    for (auto& v : r) v.resize(per);
+    std::vector<PlateConst> all, one;
+    all.reserve((size_t)p->dbp_nspan * per);
+    for (int k = 0; k < p->dbp_nspan; ++k) {   // reversed plate order, db0 negated (inverse_pmd)
+        for (int s = 0; s < sets; ++s)
+            for (int n = 0; n < np; ++n) {
+                const size_t src = (size_t)k * per + (size_t)s * np + (np - 1 - n), dst = (size_t)s * np + n;
+                r[0][dst] = -db0[src];
+                r[1][dst] = theta[src];
+                r[2][dst] = epsilon[src];
+            }
+        fill_plates(p->d, sets, r[0].data(), r[1].data(), r[2].data(), one);
+        all.insert(all.end(), one.begin(), one.end());
+    }
+    CK(c, cudaSetDevice(c->device));
+    if (p->plates) CK(c, cudaFreeAsync(p->plates, c->stream));
+    p->plates = nullptr;
+    p->dbp_plates_set = false;
+    CK(c, cudaMallocAsync(&p->plates, all.size() * sizeof(PlateConst), c->stream));
+    CK(c, cudaMemcpyAsync(p->plates, all.data(), all.size() * sizeof(PlateConst), cudaMemcpyHostToDevice, c->stream));
+    p->fc.plate_sets = p->fc_a.plate_sets = p->fc_c.plate_sets = sets;
+    pmx_k_dbp_pkg<<<dim3((unsigned)p->sched_idx.size(), (unsigned)p->d.batch), 128, 0, c->stream>>>(p->geo_d, p->plates, p->sched,
+                                                                                                     p->fc, p->d.batch);
+    c->launches++;
+    CK(c, cudaGetLastError());
+    CK(c, cudaStreamSynchronize(c->stream));   // the host vectors go away
+    p->dbp_plates_set = true;
+    return PMX_OK;
+}
+
 extern "C" int pmx_dbp_create(pmx_ctx* c, const pmx_fiber_desc* fd, const pmx_dbp_desc* g, pmx_plan** out) {
     // (the descriptors are checked before the context, so that the checks run without a device)
     if (!fd || !g || !out) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: null argument");
@@ -3334,6 +3492,12 @@ extern "C" int pmx_dbp_create(pmx_ctx* c, const pmx_fiber_desc* fd, const pmx_db
     if (!std::isfinite(g->xi)) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: xi must be finite");
     if (!(g->gain >= 0) || !std::isfinite(g->gain)) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: gain must be >= 0 (0: none)");
     if (!(fd->length > 0) || !std::isfinite(fd->length)) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: length must be > 0");
+    if (g->pmd != 0 && g->pmd != 1) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: pmd must be 0 or 1");
+    const bool pmd = g->pmd != 0;
+    if (pmd && !fd->fls[1])
+        return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: PMD-aware DBP (pmd = 1) needs the fiber's 'p' flag");
+    if (pmd && fd->nplates < 1)
+        return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: PMD-aware DBP (pmd = 1) needs nplates >= 1");
     // the steps of every span, forward order
     std::vector<double> h;
     std::vector<int> nstep(g->nspan);
@@ -3368,16 +3532,28 @@ extern "C" int pmx_dbp_create(pmx_ctx* c, const pmx_fiber_desc* fd, const pmx_db
             nstep[k] = n;
         }
     }
+    std::vector<DbpGeo> geo;
+    if (pmd) {
+        const int rc = dbp_geometry(c, *fd, g, h, nstep, geo);
+        if (rc) return rc;
+    }
     if (!c) return set_err(nullptr, PMX_ERR_INVALID, "pmx_dbp_create: null context");
-    // the virtual fiber: no PMD, no XPM, dispersion negated, one step at a time
+    // the virtual fiber: no XPM, dispersion negated, one step at a time; without pmd no PMD either, with pmd the plates
+    // come from pmx_dbp_set_plates and db1 (dgdrms) is negated
     const double zero1 = 0.0;
-    std::vector<double> nb1, nb2, nbt;
+    std::vector<double> nb1, nb2, nbt, ndb1;
     pmx_fiber_desc e = *fd;
-    e.fls[1] = 0;
-    e.nplates = e.plate_sets = 1;
-    e.db0 = e.theta = e.epsilon = &zero1;
+    e.fls[1] = pmd ? 1 : 0;
+    e.nplates = pmd ? fd->nplates : 1;
+    e.plate_sets = 1;
+    e.db0 = e.theta = e.epsilon = pmd ? nullptr : &zero1;
     e.db1 = nullptr;
-    e.dgdrms = 0.0;
+    e.dgdrms = pmd ? -fd->dgdrms : 0.0;
+    if (pmd && fd->disp_mode != PMX_DISP_SCALAR && fd->db1 && fd->nfc >= 1 && fd->nfc <= PMX_MAX_NFC) {
+        ndb1.assign(fd->db1, fd->db1 + (size_t)fd->nfc * fd->nfft);
+        for (auto& v : ndb1) v = -v;
+        e.db1 = ndb1.data();
+    }
     e.dphimaxt = INFINITY;
     e.dzmaxt = fd->length;
     e.z_start = e.dz_first = 0.0;
@@ -3412,6 +3588,27 @@ extern "C" int pmx_dbp_create(pmx_ctx* c, const pmx_fiber_desc* fd, const pmx_db
             return set_err(c, PMX_ERR_CUDA, "kernel setup (pass C', L=%d) failed: %s", p->tA->L, cudaGetErrorString(err));
         }
         c->setup_done[key].cnl = n;
+    }
+    if (pmd) {   // one package per step and realization, built by pmx_dbp_set_plates from the geometry table
+        const size_t bytes = geo.size() * (size_t)p->d.batch * sizeof(StepPkg);
+        cudaError_t err = cudaMallocAsync(&p->sched, bytes, c->stream);
+        if (err == cudaSuccess) err = cudaMemsetAsync(p->sched, 0, bytes, c->stream);
+        if (err == cudaSuccess) err = cudaMallocAsync(&p->geo_d, geo.size() * sizeof(DbpGeo), c->stream);
+        if (err == cudaSuccess)
+            err = cudaMemcpyAsync(p->geo_d, geo.data(), geo.size() * sizeof(DbpGeo), cudaMemcpyHostToDevice, c->stream);
+        if (err == cudaSuccess) err = cudaStreamSynchronize(c->stream);
+        if (err != cudaSuccess) {
+            pmx_plan_destroy(p);
+            return set_err(c, PMX_ERR_CUDA, "pmx_dbp_create: step table: %s", cudaGetErrorString(err));
+        }
+        p->dbp_pmd = true;
+        p->dbp_nspan = g->nspan;
+        for (size_t s = 0; s < geo.size(); ++s) {
+            p->sched_idx.push_back((int)s);
+            p->sched_span.push_back(geo[s].span);
+        }
+        *out = p;
+        return PMX_OK;
     }
     // step packages in execution order: spans last first, each span's steps reversed; the amplifier's 1/sqrt(G) joins the
     // scale of a span's first step.  Equal packages are stored once.
@@ -3463,6 +3660,8 @@ extern "C" int pmx_dbp_exec(pmx_plan* p, pmx_devfield* fld) {
     if (!p || !fld) return set_err(nullptr, PMX_ERR_INVALID, "pmx_dbp_exec: null argument");
     pmx_ctx* c = p->ctx;
     if (!p->dbp) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_exec: the plan was not made by pmx_dbp_create");
+    if (p->dbp_pmd && !p->dbp_plates_set)
+        return set_err(c, PMX_ERR_INVALID, "pmx_dbp_exec: a PMD-aware plan needs its plates (pmx_dbp_set_plates) first");
     if (fld->ctx != c && fld->ctx->device != c->device)
         return set_err(c, PMX_ERR_INVALID, "field and plan belong to contexts on different devices");
     if (fld->precision != p->d.precision)
@@ -3544,6 +3743,9 @@ extern "C" int pmx_dbp_exec(pmx_plan* p, pmx_devfield* fld) {
         for (int gi = 0; gi < ngroups; ++gi) {
             Grp& G = grp[gi];
             G.pA.pkg = G.pB.pkg = pk + G.b0;
+            if (p->dbp_pmd)   // the step's span: trunks beyond the package's PMX_PKG_PLATES are read from its table
+                G.pB.plates = p->plates + ((size_t)p->sched_span[s] * p->fc.plate_sets + (p->fc.plate_sets > 1 ? G.b0 : 0)) *
+                                              p->fc.nplates;
             G.pA.reverse = (rev[gi] ^= 1);   // serpentine tile order, as in pmx_fiber_exec
             CK(c, p->tA->passA(G.gA, G.st, G.pA, p->fc_a, fld->map_rows));
             G.pB.reverse = (rev[gi] ^= 1);

@@ -158,22 +158,12 @@ __device__ __forceinline__ void pmx_block_max(unsigned long long key, void* scra
     }
 }
 
-// nextstep + checkstep for the step about to run and the step package of the realization, by all threads of a CTA
-// (thread 0 runs the scalar logic, everybody copies).  c, g: the realization's control block and package (global
-// memory for the pass kernels, shared memory in the single-CTA kernel of small fields).  -> false when the realization
-// has no further step.
-__device__ __forceinline__ bool pmx_ctl_step(StepCtl* c, StepPkg* g, const PassParams& p, const FiberConst& f, int first, int b,
-                                             int* s_go) {
-    if (threadIdx.x == 0) {
-        const int go = first || c->state < PMX_ST_DONE;
-        if (go) pmx_ctl_next(c, f, first != 0, b, p.trace_dz, p.trace_ntrunk);
-        g->state = c->state;
-        *s_go = go && c->state < PMX_ST_DONE;
-    }
-    __syncthreads();
-    if (!*s_go) return false;
+// The step package of a realization (all but its state) from the step's schedule in c, by all threads of a CTA: the
+// header, the scalar-mode phasors, the entry / exit matrices and the first plates of the step.  plates: the
+// realization's plate table [nplates].  Shared by the step control and the PMD-aware DBP packages (pmx_k_dbp_pkg).
+__device__ __forceinline__ void pmx_pkg_fill(const StepCtl* c, StepPkg* g, const FiberConst& f, const PlateConst* plates) {
     const int ntrunk = c->ntrunk, n_first = c->n_first;
-    const PlateConst* plg = p.plates + (f.plate_sets > 1 ? (size_t)b * f.nplates : 0) + n_first;
+    const PlateConst* plg = plates + n_first;
     // Scalar dispersion mode: the step's phasors, one thread each (seven independent evaluations instead of a serial
     // chain on thread 0): per-bin-step factors exp(-i*0.5*dgdrms*domega*dzb/lcorr) of the first / last (partial) trunk
     // with their squares and fourth powers, and exp(-i*dz*b30*domega^3), the third difference of the common phase.
@@ -202,7 +192,7 @@ __device__ __forceinline__ bool pmx_ctl_step(StepCtl* c, StepPkg* g, const PassP
         g->n_first = n_first;
         g->bmode = f.pmd ? c->bmode : (c->bmode & PMX_BM_NL_SMALL);
     }
-    if (!f.pmd || ntrunk <= 0) return true;
+    if (!f.pmd || ntrunk <= 0) return;
     for (int i = threadIdx.x; i < 16; i += blockDim.x) {
         if (i < 8) {  // entry matrix
             double v = (i == 0 || i == 6) ? 1.0 : 0.0;
@@ -223,6 +213,23 @@ __device__ __forceinline__ bool pmx_ctl_step(StepCtl* c, StepPkg* g, const PassP
     const double* src = reinterpret_cast<const double*>(plg);
     double* dst = reinterpret_cast<double*>(g->plates);
     for (int i = threadIdx.x; i < n; i += blockDim.x) dst[i] = src[i];
+}
+
+// nextstep + checkstep for the step about to run and the step package of the realization, by all threads of a CTA
+// (thread 0 runs the scalar logic, everybody copies).  c, g: the realization's control block and package (global
+// memory for the pass kernels, shared memory in the single-CTA kernel of small fields).  -> false when the realization
+// has no further step.
+__device__ __forceinline__ bool pmx_ctl_step(StepCtl* c, StepPkg* g, const PassParams& p, const FiberConst& f, int first, int b,
+                                             int* s_go) {
+    if (threadIdx.x == 0) {
+        const int go = first || c->state < PMX_ST_DONE;
+        if (go) pmx_ctl_next(c, f, first != 0, b, p.trace_dz, p.trace_ntrunk);
+        g->state = c->state;
+        *s_go = go && c->state < PMX_ST_DONE;
+    }
+    __syncthreads();
+    if (!*s_go) return false;
+    pmx_pkg_fill(c, g, f, p.plates + (f.plate_sets > 1 ? (size_t)b * f.nplates : 0));
     return true;
 }
 

@@ -67,7 +67,7 @@ struct Worker {
 // realizations [r0, r1) on one device
 void run_shard(Worker& w, int dev, int r0, int r1, const pmx_fiber_desc& fd, const pmx_mc_desc& m, const pmx_field& tx) {
     pmx_devfield *ftx = nullptr, *work = nullptr, *work2 = nullptr;
-    pmx_plan *plan = nullptr, *inv = nullptr, *fo = nullptr, *fe = nullptr, *dbp = nullptr;
+    pmx_plan *plan = nullptr, *inv = nullptr, *fo = nullptr, *fe = nullptr, *dbp = nullptr, *dbpl = nullptr;
     pmx_ctx* rxctx = nullptr;   // the receive chain's own context (stream): it runs beside the next group's propagation
     int64_t *tmp = nullptr, *tmp2 = nullptr;
     std::future<int> pending;
@@ -115,7 +115,14 @@ void run_shard(Worker& w, int dev, int r0, int r1, const pmx_fiber_desc& fd, con
         d.theta = pl[1].data();
         d.epsilon = pl[2].data();
         MC_CK(pmx_plan_create(w.ctx, &d, &plan));
-        if (m.equalize) {   // one linear single-step fiber per span with the plate order reversed and every phase negated
+        if (m.dbp && !m.rx) {   // PMD-aware DBP with the group's plates in place of the equaliser
+            const int rc = pmx_dbp_create(w.ctx, &d, m.dbp, &dbpl);
+            if (rc != PMX_OK) {
+                w.rc = rc;
+                w.err = std::string("pmx_dbp_create: ") + pmx_last_error(w.ctx);
+                goto done;
+            }
+        } else if (m.equalize) {   // one linear single-step fiber per span with the plate order reversed and every phase negated
             pmx_fiber_desc e = d;
             e.fls[2] = e.fls[3] = 0;
             e.dphimaxt = INFINITY;
@@ -217,6 +224,10 @@ void run_shard(Worker& w, int dev, int r0, int r1, const pmx_fiber_desc& fd, con
             MC_CK(pmx_link_exec(plan, cur, &l, &res));
             for (int k = 0; k < nspan; ++k)
                 for (int b = 0; b < nb; ++b) w.sa_steps += (long long)ncyc[(size_t)k * B + b] * fd.nfft * nfc;
+            if (dbpl) {
+                MC_CK(pmx_dbp_set_plates(dbpl, B, pl[0].data(), pl[1].data(), pl[2].data()));
+                MC_CK(pmx_dbp_exec(dbpl, cur));
+            }
             if (inv) {
                 for (int k = nspan - 1; k >= 0; --k) {
                     for (int b = 0; b < B; ++b)
@@ -237,6 +248,14 @@ void run_shard(Worker& w, int dev, int r0, int r1, const pmx_fiber_desc& fd, con
                     w.rc = PMX_ERR_CUDA;
                     w.err = rxerr;
                     goto done;
+                }
+                if (dbp && m.rx->dbp->pmd) {   // this group's plates, before the next gather() overwrites pl
+                    const int rc = pmx_dbp_set_plates(dbp, B, pl[0].data(), pl[1].data(), pl[2].data());
+                    if (rc != PMX_OK) {
+                        w.rc = rc;
+                        w.err = std::string("pmx_dbp_set_plates: ") + pmx_last_error(rxctx);
+                        goto done;
+                    }
                 }
                 int64_t* const dst = w.counts_dev + g0;
                 pending = std::async(std::launch::async, [=, &m, &rxerr]() -> int {
@@ -281,6 +300,7 @@ done:
     pmx_plan_destroy(fo);
     pmx_plan_destroy(fe);
     pmx_plan_destroy(dbp);
+    pmx_plan_destroy(dbpl);
     pmx_plan_destroy(inv);
     pmx_plan_destroy(plan);
     pmx_field_destroy(work);
@@ -304,6 +324,11 @@ extern "C" int pmx_mc_run(const pmx_fiber_desc* fiber, const pmx_mc_desc* mc, co
         return fail(PMX_ERR_INVALID, "pmx_mc_run: ndev, nreal, batch, nspan must be >= 1; device_ids and sym are required");
     if (fiber->fls[1] && (!mc->db0 || !mc->theta || !mc->epsilon))
         return fail(PMX_ERR_INVALID, "pmx_mc_run: plate draws [nspan][nreal][nplates] are required with the 'p' flag");
+    if (mc->dbp && !mc->rx && !mc->dbp->pmd)
+        return fail(PMX_ERR_INVALID, "pmx_mc_run: dbp without a receive chain must be PMD-aware (pmd = 1): the data-aided "
+                                     "decision needs the PMD undone");
+    if ((mc->dbp && mc->dbp->pmd && !mc->rx) || (mc->rx && mc->rx->dbp && mc->rx->dbp->pmd))
+        if (!fiber->fls[1]) return fail(PMX_ERR_INVALID, "pmx_mc_run: PMD-aware DBP needs the fiber's 'p' flag");
     const int ndev = mc->ndev;
     const bool have_nccl = g_nccl.load();
     if (ndev > 1 && !have_nccl) return fail(PMX_ERR_UNSUPPORTED, "pmx_mc_run: libnccl.so.2 not found (needed for more than one GPU)");

@@ -5,11 +5,15 @@ nonlinearity and loss negated, spans last first, the amplifier gain undone befor
 kernels as fiber() (pmx_dbp_create / pmx_dbp_exec, include/polmux_ssfm.h).  With xi = 1 and the forward run's own
 steps (fiber(..., trace=True) leaves them in FIBER_LAST['trace_dz']) it inverts a noise-free link without PMD up to
 rounding; with fewer steps or xi < 1 it is the receiver-side nonlinear compensation a Monte-Carlo run can count errors
-behind (McRunner(compensation='dbp')).  There is no CPU fallback.
+behind (McRunner(compensation='dbp')).  Given the link's waveplates (dbp_plan(plates=...), dbp(brf=...)) it is PMD-aware:
+every step undoes the forward step's own trunk product as well, so that it inverts a 'gps-' link too
+(McRunner(compensation='dbp_pmd')).  There is no CPU fallback.
 """
 from __future__ import annotations
 
 from typing import Optional
+
+import numpy as np
 
 from . import _lib
 from .fiber import FiberSetup, _get, fiber_setup, setup_to_desc
@@ -18,30 +22,60 @@ from .gstate import GSTATE
 
 def dbp_plan(ctx: _lib.Context, setup: FiberSetup, nspan: int = 1, gain_db: Optional[float] = None,
              steps_per_span: Optional[int] = None, step_len=None, span_steps=None, xi: float = 1.0, batch: int = 1,
-             precision: Optional[str] = None, disp_mode: Optional[str] = None) -> _lib.DbpPlan:
-    """The DBP of nspan spans of the fiber `setup` describes (its 'p' flag, plates and dgdrms are ignored), for resident
-    fields of `batch` realizations.  Schedule: steps_per_span uniform steps per span (default 1), or step_len -- one
-    span's steps in forward order for every span, or with span_steps [nspan] all spans' steps concatenated."""
+             precision: Optional[str] = None, disp_mode: Optional[str] = None, plates=None) -> _lib.DbpPlan:
+    """The DBP of nspan spans of the fiber `setup` describes, for resident fields of `batch` realizations.  Schedule:
+    steps_per_span uniform steps per span (default 1), or step_len -- one span's steps in forward order for every span,
+    or with span_steps [nspan] all spans' steps concatenated.  plates: None -- the 'p' flag, plates and dgdrms are
+    ignored; (db0, theta, epsilon), each [nspan][plate_sets][nplates] in forward order (plate_sets 1 or batch) -- PMD-aware
+    DBP through those waveplates (setup must carry the 'p' flag; DbpPlan.set_plates swaps in another draw)."""
+    if plates is not None and not setup.fls[1]:
+        raise ValueError("PMD-aware DBP (plates given) needs a fiber with the 'p' flag")
     desc, keep = setup_to_desc(setup, batch=batch, disp_mode=disp_mode, precision=precision)
     gain = 0.0 if gain_db is None else 10 ** (gain_db * 0.1)
     if step_len is None and steps_per_span is None:
         steps_per_span = 1
-    d, dkeep = _lib.make_dbp(nspan, gain, steps_per_span=steps_per_span, step_len=step_len, span_steps=span_steps, xi=xi)
-    return _lib.DbpPlan(ctx, desc, keep, d, dkeep)
+    d, dkeep = _lib.make_dbp(nspan, gain, steps_per_span=steps_per_span, step_len=step_len, span_steps=span_steps, xi=xi,
+                             pmd=plates is not None)
+    plan = _lib.DbpPlan(ctx, desc, keep, d, dkeep)
+    if plates is not None:
+        try:
+            arrs = [np.asarray(a, dtype=np.float64).reshape(int(nspan), -1, setup.nplates) for a in plates]
+            plan.set_plates(*arrs, plate_sets=arrs[0].shape[1])
+        except Exception:
+            plan.close()
+            raise
+    return plan
 
 
 def dbp(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, steps_per_span: Optional[int] = None, step_len=None,
-        span_steps=None, xi: float = 1.0, ctx: Optional[_lib.Context] = None, precision: Optional[str] = None):
+        span_steps=None, xi: float = 1.0, ctx: Optional[_lib.Context] = None, precision: Optional[str] = None, brf=None):
     """Backpropagates GSTATE.FIELDX / FIELDY in place through nspan spans of the fiber x, the amplifier of gain_db [dB]
-    after each (None: no amplifier).  x and flag are what fiber() takes; the flag's 'p' is dropped (no plates are drawn,
-    nothing is taken from the global random stream) but the fiber's nonlinear model stays the one fiber() used: Manakov
-    when x.manakov is 'yes' and the flag has 'p', else the CNLSE.  xi: fraction of gamma backpropagated.
-    The field stays resident on the device like fiber() and ampliflat() leave it."""
+    after each (None: no amplifier).  x and flag are what fiber() takes.  Without brf the flag's 'p' is dropped (no plates
+    are drawn, nothing is taken from the global random stream) but the fiber's nonlinear model stays the one fiber() used:
+    Manakov when x.manakov is 'yes' and the flag has 'p', else the CNLSE.  brf: the struct fiber() returned (every span
+    the same plates) or a list of nspan of them in forward span order, with 'p' in the flag: PMD-aware DBP through those
+    plates.  xi: fraction of gamma backpropagated.  The field stays resident on the device like fiber() and ampliflat()
+    leave it."""
     G = GSTATE
     f = str(flag).lower()
     if len(f) != 4:
         raise ValueError("wrong flag. E.g. flag can be 'g---','gp--','-s--', etc")
-    s = fiber_setup(x, f[0] + '-' + f[2:])
+    plates = None
+    if brf is None:
+        s = fiber_setup(x, f[0] + '-' + f[2:])
+    else:
+        if f[1] != 'p':
+            raise ValueError("dbp: brf (PMD-aware DBP) needs the 'p' flag")
+        # (a private stream: the plates come from brf, nothing is drawn from the global one)
+        s = fiber_setup(x, f, rng=np.random.Generator(np.random.PCG64(0)))
+        brfs = [brf] * int(nspan) if isinstance(brf, dict) else list(brf)
+        if len(brfs) != int(nspan):
+            raise ValueError('dbp: brf must be one struct or a list of nspan of them')
+        for b in brfs:
+            if np.asarray(b['theta']).size != s.nplates:
+                raise ValueError('dbp: brf has %d plates, the fiber %d' % (np.asarray(b['theta']).size, s.nplates))
+        plates = tuple(np.stack([np.asarray(b[k], dtype=np.float64).reshape(1, -1) for b in brfs])
+                       for k in ('db0', 'theta', 'epsilon'))
     if not (s.isv and G.has_y()):
         raise NotImplementedError('dbp: two-polarization fields only (the scalar path has no DBP)')
     if s.fls[3]:
@@ -52,7 +86,7 @@ def dbp(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, steps_per
     prec = {'f64': _lib.PMX_F64, 'f32': _lib.PMX_F32}[precision or PRECISION]
     fld, hx, hy = G.take_device(ctx, prec)
     try:
-        plan = dbp_plan(ctx, s, nspan, gain_db, steps_per_span, step_len, span_steps, xi, precision=precision)
+        plan = dbp_plan(ctx, s, nspan, gain_db, steps_per_span, step_len, span_steps, xi, precision=precision, plates=plates)
     except Exception:
         G.restore_host(fld, hx, hy)     # nothing ran: the caller's field is as it was
         raise

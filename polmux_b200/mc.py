@@ -218,14 +218,15 @@ class McRunner:
         pipeline: run the receive chain of a group beside the propagation of the next one (same counts either way)
         compensation ('blind' and 'cohmix'): 'cd' -- the all-pass step that undoes the link's dispersion; 'dbp' -- digital
         backpropagation of the link (polmux_b200/dbp.py) with dbp_params (steps_per_span, step_len, span_steps, xi; default
-        one step per span, xi = 1), the amplifier gain undone before each span"""
+        one step per span, xi = 1), the amplifier gain undone before each span.  'dbp_pmd' (every receiver) -- PMD-aware
+        DBP through each group's own plate draws (Link.plates); with 'genie' it replaces the linear equaliser"""
         import torch
         from . import dsp as _dsp
         self.receiver, self.dsp_params = receiver, dict(dsp_params or {})
         if receiver not in ('genie', 'blind', 'cohmix'):
             raise ValueError("receiver must be 'genie', 'blind' or 'cohmix'")
-        if compensation not in ('cd', 'dbp'):
-            raise ValueError("compensation must be 'cd' or 'dbp'")
+        if compensation not in ('cd', 'dbp', 'dbp_pmd'):
+            raise ValueError("compensation must be 'cd', 'dbp' or 'dbp_pmd'")
         if compensation == 'dbp' and receiver == 'genie':
             raise ValueError("the genie receiver undoes the link with the known plates: compensation='dbp' needs 'blind' or 'cohmix'")
         self.ref_patmat = _dsp.reference_pattern(np.asarray(sym)[0], np.asarray(sym)[1]) if receiver != 'genie' else None
@@ -247,11 +248,17 @@ class McRunner:
         self.bufs = [torch.zeros(batch, dtype=torch.int64, device=self.dev) for _ in range(nslot)]
         self.work, self.buf = self.works[0], self.bufs[0]
         self.rx = None
+        self.dbp_genie = None
+        if compensation == 'dbp_pmd' and receiver == 'genie':
+            from .dbp import dbp_plan
+            self.dbp_genie = dbp_plan(ctx, setup, nspan, gain_db, batch=batch, precision='f64', plates=self._link_plates(),
+                                      **dict(dbp_params or {}))
         if receiver != 'genie':
             self.rxctx = _lib.Context(ctx.device) if self.pipelined else ctx
-            if compensation == 'dbp':
+            if compensation in ('dbp', 'dbp_pmd'):
                 from .dbp import dbp_plan
-                comp = dbp_plan(self.rxctx, setup, nspan, gain_db, batch=batch, precision='f64', **dict(dbp_params or {}))
+                comp = dbp_plan(self.rxctx, setup, nspan, gain_db, batch=batch, precision='f64',
+                                plates=self._link_plates() if compensation == 'dbp_pmd' else None, **dict(dbp_params or {}))
             else:
                 comp = self.link.cd_plan(self.rxctx)
             self.rx = dict(cd=comp, S=None)
@@ -266,6 +273,10 @@ class McRunner:
                                fo=_lib.Filter(self.rxctx, setup.nfft, 1, S.hf_opt, batch=batch),
                                fe=_lib.Filter(self.rxctx, setup.nfft, 1, _rx.hermitian_part(S.hf_el), batch=batch),
                                col=_lib.DeviceField(self.rxctx, setup.nfft, 1, batch) if setup.nfc > 1 else None)
+
+    def _link_plates(self):
+        """the current group's plates as DbpPlan.set_plates takes them: (db0, theta, epsilon), each [nspan][batch][nplates]"""
+        return tuple(np.stack([pl[i] for pl in self.link.plates]) for i in range(3))
 
     def _receive(self, work, buf, g0, nb):
         """the receive chain of one propagated group, on the receiver's context; -> the group's counts land in self.local"""
@@ -311,15 +322,21 @@ class McRunner:
                 work.broadcast_from(self.tx)
                 sa_steps += self.link.run(work, ase_seed)            # (returns when the group is propagated)
                 if self.receiver == 'genie':
-                    self.link.equalize(work)
+                    if self.dbp_genie is not None:
+                        self.dbp_genie.set_plates(*self._link_plates(), plate_sets=self.batch)
+                        self.dbp_genie.execute(work)
+                    else:
+                        self.link.equalize(work)
                     _lib.qpsk_count(self.ctx, work, self.sym, self.nsymb, self.nt, buf.data_ptr())   # writes the send buffer
                     self.ctx.sync()
                     self.local[g0 - self.r0:g0 - self.r0 + nb] = buf[:nb]
                 elif pool is None:
+                    self._set_rx_plates()
                     self.passes.append(self._receive(work, buf, g0, nb))
                 else:
                     if pending is not None:                          # the other slot's receive chain ran beside this link
                         self.passes.append(pending.result())
+                    self._set_rx_plates()                            # (before the next retarget draws new plates)
                     pending = pool.submit(self._receive, work, buf, g0, nb)
             if pending is not None:
                 self.passes.append(pending.result())
@@ -330,7 +347,15 @@ class McRunner:
         counts = allreduce_counts(self.local, self.r0, self.nreal)
         return counts.cpu().numpy(), sa_steps
 
+    def _set_rx_plates(self):
+        """PMD-aware DBP in the receive chain: this group's plates, while no chain uses the plan"""
+        c = self.rx['cd']
+        if isinstance(c, _lib.DbpPlan) and c.dbp.pmd:
+            c.set_plates(*self._link_plates(), plate_sets=self.batch)
+
     def close(self):
+        if self.dbp_genie is not None:
+            self.dbp_genie.close()
         for f in self.works + [self.tx]:
             f.close()
         if self.rx:
@@ -360,6 +385,9 @@ def run_mc_native(setup: FiberSetup, tx_x, tx_y, sym, nsymb: int, nt: int, nspan
     receive chain (front-end, sampler, DSP core with dsp_params) behind the link, its optical response carrying the
     compensation of the link's chromatic dispersion (as x.dpost / p.applydcf would), or with dbp_params (a dict as
     McRunner's) the digital backpropagation of the link ahead of the front-end and the optical filter alone.
+    dbp_params with 'pmd': True -- PMD-aware DBP through every group's own plates: with a receive chain in its place,
+    without one (receiver None) in place of the linear equaliser ahead of the data-aided counter; without 'pmd' and
+    without a receive chain, dbp_params is ignored.
     -> (counts [nreal] int64, Sa*steps over all realizations)"""
     import ctypes as C
     lib = _lib.load()
@@ -381,6 +409,18 @@ def run_mc_native(setup: FiberSetup, tx_x, tx_y, sym, nsymb: int, nt: int, nspan
     m.gain, m.sigma, m.ase_seed = gain, sigma.ctypes.data_as(_lib._dp), int(ase_seed)
     m.sym, m.nsymb, m.nt = symb.ctypes.data_as(C.POINTER(C.c_uint8)), int(nsymb), int(nt)
     rxkeep = None
+    dbp_pmd = bool(dict(dbp_params or {}).get('pmd', False))
+
+    def _dbp_desc():
+        pd = dict(dbp_params)
+        pmd = bool(pd.pop('pmd', False))
+        if pd.get('step_len') is None and pd.get('steps_per_span') is None:
+            pd['steps_per_span'] = 1
+        return _lib.make_dbp(nspan, gain, pmd=pmd, **pd)
+    if receiver is None and dbp_pmd:
+        dd, dkeep = _dbp_desc()
+        m.dbp = C.pointer(dd)
+        rxkeep = (dd, dkeep)
     if receiver is not None:
         from . import dsp as _dsp
         from . import receiver as _rx
@@ -405,10 +445,7 @@ def run_mc_native(setup: FiberSetup, tx_x, tx_y, sym, nsymb: int, nt: int, nspan
         rx.dsp = _dsp._desc(nsymb, nt, p)
         rx.ref_patmat = ref.ctypes.data_as(C.POINTER(C.c_uint8))
         if dbp_params is not None:
-            pd = dict(dbp_params)
-            if pd.get('step_len') is None and pd.get('steps_per_span') is None:
-                pd['steps_per_span'] = 1
-            dd, dkeep = _lib.make_dbp(nspan, gain, **pd)
+            dd, dkeep = _dbp_desc()
             rx.dbp = C.pointer(dd)
             rxkeep = (hopt, hel, ref, lop, rx, dd, dkeep)
         else:

@@ -1,13 +1,16 @@
 """Times digital backpropagation (pmx_dbp_exec) against the forward link on one resident C2 batch.
 
-    python tools/dbp_time.py [--batch 16] [--nsymb 65536] [--reps 3] [--out DIR]
+    python tools/dbp_time.py [--batch 16] [--nsymb 65536] [--reps 3] [--pmd] [--out DIR]
 
 C2 (BASELINE.md): 10 x 80 km Manakov spans, 16 dB amplifiers, 2^16 symbols x 16 samples = 2^20 samples.  In one process:
 the forward link (pmx_link_exec, noise-free, 'g-s-' with the Manakov model: the nonlinear-phase step control) and DBP of
 the same 10 spans with M = 1, 4 and 16 uniform steps per span.  Reported per run: wall time of the call (it returns
 synchronised), GSa*steps/s = batch*nfft*steps/time and the share of the HBM roofline for the 192 algorithmic bytes a
 step moves per Sa in FP64 (3 passes x read + write x 32 B), against the same peak bench.py uses (MEASURED_PEAKS.json
-hbm_gbs, else 6650 GB/s).  The card's name and power limit are printed with the numbers."""
+hbm_gbs, else 6650 GB/s).  The card's name and power limit are printed with the numbers.
+--pmd: the 'gps-' C2 link with 100 plates per span and a plate draw per span and realization; timed are the forward link,
+PMD-blind DBP and PMD-aware DBP (each at M = 1, 4, 16) and the genie equaliser (Link.equalize, one 100-trunk step per
+span)."""
 import argparse
 import json
 import os
@@ -44,6 +47,7 @@ def main():
     ap.add_argument('--nt', type=int, default=16)
     ap.add_argument('--nspan', type=int, default=10)
     ap.add_argument('--reps', type=int, default=3)
+    ap.add_argument('--pmd', action='store_true', help="the 'gps-' link with 100 plates; PMD-aware DBP and the equaliser too")
     ap.add_argument('--out', default=None, help='directory for dbp_time.json')
     a = ap.parse_args()
     try:
@@ -57,7 +61,11 @@ def main():
     pmx.create_field('unique', ex, ey, {'power': 'average'})
     fib = dict(synth.SMF)
     fib['length'] = 8e4
-    s = fiber_setup(fib, 'g-s-')
+    if a.pmd:
+        fib.update(dgd=0.3, nplates=100, manakov='yes')
+        s = fiber_setup(fib, 'gps-', rng=np.random.Generator(np.random.PCG64(0)))
+    else:
+        s = fiber_setup(fib, 'g-s-')
     s.manakov = True
     ctx = _lib.default_context(0)
     B, n = a.batch, s.nfft
@@ -86,11 +94,24 @@ def main():
             print('%-14s rep %d  %8.2f ms  %6d steps/realization  %7.2f GSa*steps/s  %5.1f %% of %.0f GB/s x 192 B'
                   % (name, rep, dt * 1e3, steps / B, rows[-1]['gsa_steps_per_s'], 100 * rows[-1]['roofline_share'], peak))
 
-    timed('forward', lambda: fwd.link_exec(fld, link, lkeep), lambda r: int(r.ncycle.sum()))
+    if a.pmd:
+        fwd.close()
+        from polmux_b200 import mc
+        lk = mc.Link(ctx, s, a.nspan, B, 16.0, None)        # noise-free, a plate draw per span and realization
+        plates = tuple(np.stack([pl[i] for pl in lk.plates]) for i in range(3))
+        timed('forward', lambda: lk.run(fld, 1), lambda r: r // n)
+    else:
+        timed('forward', lambda: fwd.link_exec(fld, link, lkeep), lambda r: int(r.ncycle.sum()))
     for m in (1, 4, 16):
         plan = dbp_plan(ctx, s, a.nspan, 16.0, steps_per_span=m, batch=B)
         timed('dbp M=%d' % m, lambda: plan.execute(fld), lambda _r, m=m: m * a.nspan * B)
         plan.close()
+    if a.pmd:
+        for m in (1, 4, 16):
+            plan = dbp_plan(ctx, s, a.nspan, 16.0, steps_per_span=m, batch=B, plates=plates)
+            timed('dbp_pmd M=%d' % m, lambda: plan.execute(fld), lambda _r, m=m: m * a.nspan * B)
+            plan.close()
+        timed('equalize', lambda: lk.equalize(fld), lambda _r: a.nspan * B)
     info = card()
     print('card: %s' % info)
     summary = {}
@@ -103,7 +124,7 @@ def main():
         print('%-14s median %7.2f GSa*steps/s  (%.3f x forward)' % (name, v['gsa_steps_per_s_median'], v['vs_forward']))
     if a.out:
         os.makedirs(a.out, exist_ok=True)
-        json.dump(dict(card=info, peak_gbs=peak, batch=B, nfft=n, nspan=a.nspan, runs=rows, summary=summary),
+        json.dump(dict(card=info, peak_gbs=peak, batch=B, nfft=n, nspan=a.nspan, pmd=a.pmd, runs=rows, summary=summary),
                   open(os.path.join(a.out, 'dbp_time.json'), 'w'), indent=1)
 
 
