@@ -13,7 +13,7 @@ import os
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# POLMUX_SSFM_LIB: another build of the same CUDA library (kernel-tuning variants, tools/build_variant.sh)
+# POLMUX_SSFM_LIB: another build of the same CUDA library (e.g. the index-assert build of `make -C polmux_b200/csrc debug`)
 LIB_PATH = os.environ.get('POLMUX_SSFM_LIB') or os.path.join(_HERE, 'lib', 'libpolmux_ssfm.so')
 
 PMX_OK = 0

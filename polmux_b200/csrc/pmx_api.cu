@@ -84,8 +84,8 @@ struct pmx_ctx {
     std::string error;
     std::map<int, StageTw> stage_tw;          // by L
     std::map<long long, FourStepTw> four_tw;  // by N
-    struct Occ { int a = 0, b = 0, c = 0, cnl = 0; };   // cnl: pmx_k_passC_nl (digital backpropagation), set on first use
-    std::map<int, Occ> setup_done;  // by L: resident CTAs per SM of passes A, B, C
+    struct Occ { int a = 0, b = 0, c = 0, cnl = 0; };
+    std::map<int, Occ> setup_done;  // by L: resident CTAs per SM of passes A, B, C and C' (digital backpropagation)
     int sm_count = 148;
     PFN_cuTensorMapEncodeTiled_v12000 encode = nullptr;
     StepCtl* h_ctl = nullptr;  // pinned readback buffer
@@ -155,14 +155,8 @@ static int ilog2_exact(int64_t v) {
     return ((1ll << l) == v) ? l : -1;
 }
 
-// Four-step split N = N1*N2: log2(N1).  PMX_SPLIT_SHIFT (tuning knob) moves it off the balanced choice.
-static int split_log2N1(int lg) {
-    int l1 = lg / 2;
-    if (const char* e = getenv("PMX_SPLIT_SHIFT")) l1 += atoi(e);
-    if (l1 < 6) l1 = 6;
-    if (lg - l1 < 6) l1 = lg - 6;
-    return l1;
-}
+// Four-step split N = N1*N2: log2(N1), the balanced split (measured against the unbalanced ones in DESIGN.md §7).
+static int split_log2N1(int lg) { return lg / 2; }
 
 // Tensor maps over a resident field for the four-step split N = N1*N2 (see pmx_tma.cuh).
 static int build_maps(pmx_ctx* c, pmx_devfield* f) {
@@ -834,11 +828,11 @@ static int plan_create(pmx_ctx* c, const pmx_fiber_desc* d, pmx_plan** out, bool
         if (onchip) break;
         if (!c->setup_done.count(t->L + 65536 * t->precision)) {
             pmx_ctx::Occ o;
-            cudaError_t e = t->setup(&o.a, &o.b, &o.c);
-            if (e != cudaSuccess || o.a < 1 || o.b < 1 || o.c < 1) {
+            cudaError_t e = t->setup(&o.a, &o.b, &o.c, &o.cnl);
+            if (e != cudaSuccess || o.a < 1 || o.b < 1 || o.c < 1 || o.cnl < 1) {
                 delete p;
-                return set_err(c, PMX_ERR_CUDA, "kernel setup (L=%d) failed: %s (resident CTAs %d/%d/%d)", t->L,
-                               cudaGetErrorString(e), o.a, o.b, o.c);
+                return set_err(c, PMX_ERR_CUDA, "kernel setup (L=%d) failed: %s (resident CTAs %d/%d/%d/%d)", t->L,
+                               cudaGetErrorString(e), o.a, o.b, o.c, o.cnl);
             }
             c->setup_done[t->L + 65536 * t->precision] = o;
             if (getenv("PMX_VERBOSE"))
@@ -1031,8 +1025,11 @@ static int ensure_hctl(pmx_ctx* c, int batch) {
     return PMX_OK;
 }
 
-extern "C" int pmx_fiber_exec(pmx_plan* p, pmx_devfield* fld, pmx_fiber_result* out) {
-    if (!p || !fld) return set_err(nullptr, PMX_ERR_INVALID, "pmx_fiber_exec: null argument");
+// ---------------------------------------------------------------------------
+// Launch scaffold of the three passes, shared by pmx_fiber_exec and pmx_dbp_exec.
+
+// A field runs with a plan of the same device, precision and shape.
+static int check_field(pmx_plan* p, const pmx_devfield* fld) {
     pmx_ctx* c = p->ctx;
     // a field may be worked on by a plan of another context of the SAME device (a second stream, e.g. a receive chain running
     // beside the next group's propagation): the caller orders the two streams (every call here returns synchronised)
@@ -1043,10 +1040,139 @@ extern "C" int pmx_fiber_exec(pmx_plan* p, pmx_devfield* fld, pmx_fiber_result* 
     if (fld->nfft != p->d.nfft || fld->nfc != p->d.nfc || fld->batch != p->d.batch)
         return set_err(c, PMX_ERR_INVALID, "field shape (%lld,%d,%d) does not match the plan (%lld,%d,%d)",
                        (long long)fld->nfft, fld->nfc, fld->batch, (long long)p->d.nfft, p->d.nfc, p->d.batch);
+    if (!p->onchip && !fld->has_maps) return set_err(c, PMX_ERR_INVALID, "field has no tensor maps (unsupported nfft)");
+    return PMX_OK;
+}
+
+// The launch parameters of plan p on field fld: pa for every kernel, pA and pB for passes A (and C) and B with their
+// stage and four-step twiddles (an on-chip plan runs no passes: pA and pB are pa).
+static int pass_params(pmx_plan* p, const pmx_devfield* fld, PassParams& pa, PassParams& pA, PassParams& pB) {
+    pmx_ctx* c = p->ctx;
+    memset(&pa, 0, sizeof pa);
+    pa.field = fld->data;
+    pa.ctl = p->ctl;
+    pa.betat_p = p->betat_p;
+    pa.db1_p = p->db1_p;
+    pa.hfilt = p->hfilt;
+    pa.hfilt_stride = p->hfilt_stride;
+    pa.plates = p->plates;
+    pa.trace_dz = p->trace_dz;
+    pa.trace_ntrunk = p->trace_ntrunk;
+    pa.N1 = p->N1;
+    pa.N2 = p->N2;
+    pa.log2N1 = p->log2N1;
+    pa.log2N2 = p->log2N2;
+    pa.batch = p->d.batch;
+    pa.dbg = g_dbg;
+    pa.pkg = p->pkg;
+    pA = pB = pa;
+    if (p->onchip) return PMX_OK;
+    int rc = get_four_tw(c, p->d.nfft, p->tA, p->N2, &pA.tw4);       // pass A: one row per column n2, W_N^(n2*k1), k1 < N1
+    if (!rc) rc = get_four_tw(c, p->d.nfft, p->tB, p->N1, &pB.tw4);  // pass B: one row per k1, W_N^(k1*n2), n2 < N2
+    if (!rc) rc = get_stage_tw(c, p->tA, &pA.tw_stage);
+    if (!rc) rc = get_stage_tw(c, p->tB, &pB.tw_stage);
+    return rc;
+}
+
+// Realization groups.  The batch is split into groups that run on their own streams with full-size persistent
+// grids: while the last CTAs of one group's pass drain (tile-count quantisation, stragglers, the launch gap and
+// the one-CTA-per-realization step control), the other group's pass already fills the freed SM slots.
+struct PassGroup {
+    cudaStream_t st;
+    int b0, nb;             // realizations b0 .. b0 + nb - 1
+    int gA, gB, gC;         // grids of passes A, B and C
+    PassParams pA, pB, pc;  // pass A (and C), pass B, the other kernels: pa, pA, pB of pass_params on the group's realizations
+};
+struct PassGroups {
+    int n;
+    int pdl;  // launch with programmatic stream serialization
+    PassGroup g[4];
+};
+
+// occC: resident CTAs per SM of the pass-C kernel the caller launches; allow_pdl: programmatic dependent launch with a
+// single group.
+static int plan_groups(pmx_plan* p, const pmx_devfield* fld, const PassParams& pa, const PassParams& pA,
+                       const PassParams& pB, int occC, bool allow_pdl, PassGroups& gs) {
+    pmx_ctx* c = p->ctx;
+    const int batch = p->d.batch, nfc = p->d.nfc;
+    const pmx_ctx::Occ oA = c->setup_done[p->N1 + 65536 * p->d.precision], oB = c->setup_done[p->N2 + 65536 * p->d.precision];
+    static const int env_groups = getenv("PMX_GROUPS") ? atoi(getenv("PMX_GROUPS")) : 0;
+    // two groups pay once a pass has more than about two rounds of tiles; below that a single group with
+    // programmatic dependent launches (prologue of the next kernel under the tail of the current one) is faster
+    const long tiles_all = (long)(p->N2 / p->tA->gAC) * batch * nfc;
+    const int want_groups = env_groups ? env_groups : (tiles_all > 2L * c->sm_count * oA.a ? 2 : 1);
+    gs.n = c->profile ? 1 : std::max(1, std::min(std::min(want_groups, 4), batch));
+    // programmatic dependent launch pays when nothing else fills the gap between two kernels of a stream, i.e. with a
+    // single realization group (a batch of one: the reference-style fiber() call)
+    gs.pdl = (gs.n == 1 && allow_pdl) ? 1 : 0;
+    for (int g = 1; g < gs.n; ++g)
+        if (!c->gstream[g - 1]) {
+            CK(c, cudaStreamCreateWithFlags(&c->gstream[g - 1], cudaStreamNonBlocking));
+            CK(c, cudaEventCreateWithFlags(&c->ev_join[g - 1], cudaEventDisableTiming));
+            if (!c->ev_fork) CK(c, cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming));
+        }
+    // Persistent grids of one CTA per resident slot -- except when a pass has between one and two rounds of
+    // tiles (a batch of one at N = 2^20: 1024 tiles on 592 slots): then one CTA per tile, so that the hardware
+    // hands the tiles of the partial second round to whichever slot frees first (measured +8 % at batch 1, N = 2^20;
+    // with more rounds the persistent grid is the faster one, grid sizing in DESIGN.md)
+    auto grid_of = [&](int tiles, int ctas_per_sm) {
+        const int slots = ctas_per_sm * c->sm_count;
+        if (tiles > slots && tiles <= 2 * slots) return tiles;
+        return std::min(tiles, slots);
+    };
+    const size_t N = (size_t)p->d.nfft;
+    for (int g = 0; g < gs.n; ++g) {
+        PassGroup& G = gs.g[g];
+        G.b0 = (int)((long long)g * batch / gs.n);
+        G.nb = (int)((long long)(g + 1) * batch / gs.n) - G.b0;
+        G.st = g == 0 ? c->stream : c->gstream[g - 1];
+        for (PassParams* q : {&G.pA, &G.pB, &G.pc}) {
+            *q = (q == &G.pA) ? pA : (q == &G.pB ? pB : pa);
+            q->field = (char*)pa.field + (size_t)G.b0 * nfc * N * 2 * fld->cbytes();
+            q->ctl = pa.ctl + G.b0;
+            q->pkg = pa.pkg + G.b0;
+            if (p->fc.plate_sets > 1) q->plates = pa.plates + (size_t)G.b0 * p->fc.nplates;
+            if (pa.trace_dz) {
+                q->trace_dz = pa.trace_dz + (size_t)G.b0 * p->trace_cap;
+                q->trace_ntrunk = pa.trace_ntrunk + (size_t)G.b0 * p->trace_cap;
+            }
+            q->batch = G.nb;
+            q->bc0 = G.b0 * nfc;
+            q->pdl = gs.pdl;
+        }
+        const int tilesAC = (p->N2 / p->tA->gAC) * G.nb * nfc, tilesB = (p->N1 / p->tB->gB) * G.nb * nfc;
+        G.gA = grid_of(tilesAC, oA.a);
+        G.gB = grid_of(tilesB, oB.b);
+        G.gC = grid_of(tilesAC, occC);
+    }
+    return PMX_OK;
+}
+
+// The streams of the other groups start after everything queued on the first one so far.
+static int fork_groups(pmx_ctx* c, int ngroups) {
+    if (ngroups < 2) return PMX_OK;
+    CK(c, cudaEventRecord(c->ev_fork, c->stream));
+    for (int g = 1; g < ngroups; ++g) CK(c, cudaStreamWaitEvent(c->gstream[g - 1], c->ev_fork, 0));
+    return PMX_OK;
+}
+// The first stream waits for what the other groups have queued.
+static int join_groups(pmx_ctx* c, int ngroups) {
+    for (int g = 1; g < ngroups; ++g) {
+        CK(c, cudaEventRecord(c->ev_join[g - 1], c->gstream[g - 1]));
+        CK(c, cudaStreamWaitEvent(c->stream, c->ev_join[g - 1], 0));
+    }
+    return PMX_OK;
+}
+
+extern "C" int pmx_fiber_exec(pmx_plan* p, pmx_devfield* fld, pmx_fiber_result* out) {
+    if (!p || !fld) return set_err(nullptr, PMX_ERR_INVALID, "pmx_fiber_exec: null argument");
+    pmx_ctx* c = p->ctx;
+    int rc = check_field(p, fld);
+    if (rc) return rc;
     if (p->dbp) return set_err(c, PMX_ERR_INVALID, "pmx_fiber_exec: a digital-backpropagation plan runs with pmx_dbp_exec");
     CK(c, cudaSetDevice(c->device));
     const int batch = p->d.batch, nfc = p->d.nfc;
-    int rc = ensure_hctl(c, batch);
+    rc = ensure_hctl(c, batch);
     if (rc) return rc;
 
     // optional schedule trace
@@ -1069,41 +1195,9 @@ extern "C" int pmx_fiber_exec(pmx_plan* p, pmx_devfield* fld, pmx_fiber_result* 
     }
     p->fc.trace_cap = p->trace_cap;
 
-    PassParams pa;
-    memset(&pa, 0, sizeof pa);
-    pa.field = fld->data;
-    pa.ctl = p->ctl;
-    pa.betat_p = p->betat_p;
-    pa.db1_p = p->db1_p;
-    pa.hfilt = p->hfilt;
-    pa.hfilt_stride = p->hfilt_stride;
-    pa.plates = p->plates;
-    pa.trace_dz = p->trace_dz;
-    pa.trace_ntrunk = p->trace_ntrunk;
-    pa.N1 = p->N1;
-    pa.N2 = p->N2;
-    pa.log2N1 = p->log2N1;
-    pa.log2N2 = p->log2N2;
-    pa.batch = batch;
-    pa.dbg = g_dbg;
-    pa.pkg = p->pkg;
-    const void *tw4A = nullptr, *tw4B = nullptr, *twA = nullptr, *twB = nullptr;
-    if (!p->onchip) {
-        rc = get_four_tw(c, p->d.nfft, p->tA, p->N2, &tw4A);  // pass A: one row per column n2, W_N^(n2*k1), k1 < N1
-        if (rc) return rc;
-        rc = get_four_tw(c, p->d.nfft, p->tB, p->N1, &tw4B);  // pass B: one row per k1, W_N^(k1*n2), n2 < N2
-        if (rc) return rc;
-        rc = get_stage_tw(c, p->tA, &twA);
-        if (rc) return rc;
-        rc = get_stage_tw(c, p->tB, &twB);
-        if (rc) return rc;
-    }
-    PassParams pA = pa, pB = pa;
-    pA.tw_stage = twA;
-    pB.tw_stage = twB;
-    pA.tw4 = tw4A;
-    pB.tw4 = tw4B;
-
+    PassParams pa, pA, pB;
+    rc = pass_params(p, fld, pa, pA, pB);
+    if (rc) return rc;
     CK(c, cudaMemsetAsync(p->ctl, 0, 2 * (size_t)batch * sizeof(StepCtl), c->stream));   // ([1]: the second block of the fused control)
     CK(c, cudaMemsetAsync(p->pkg, 0, (size_t)batch * sizeof(StepPkg), c->stream));
     // what the caller gets back, from the control blocks read into h_ctl
@@ -1148,8 +1242,7 @@ extern "C" int pmx_fiber_exec(pmx_plan* p, pmx_devfield* fld, pmx_fiber_result* 
     // runs the control itself (pmx_k_passA<..., FUSED>), three dependent launches per step instead of four.
     // Every CTA of that pass A repeats the (scalar, 2-3 us) control, so it pays while the pass is a single round of CTAs --
     // fields of up to 2^19 samples; measured at 2^16: 31.9 -> 27.9 us per step, at 2^20 (1024 CTAs in two rounds) -3 %.
-    static const int fused_env = getenv("PMX_FUSED_CTL") ? atoi(getenv("PMX_FUSED_CTL")) : 1;
-    const bool fused = fused_env && batch == 1 && !p->fc.xpm && !c->profile &&
+    const bool fused = batch == 1 && !p->fc.xpm && !c->profile &&
                        (long)(p->N2 / p->tA->gAC) * nfc <= (long)c->sm_count * c->setup_done[p->N1 + 65536 * p->d.precision].a;
     {
         dim3 g(148 * 2, batch * nfc);
@@ -1164,89 +1257,23 @@ extern "C" int pmx_fiber_exec(pmx_plan* p, pmx_devfield* fld, pmx_fiber_result* 
     }
     int par = 0;          // fused control: the block the next pass A reads
     int fused_first = 1;
-    if (!fld->has_maps) return set_err(c, PMX_ERR_INVALID, "field has no tensor maps (unsupported nfft)");
-    const pmx_ctx::Occ oA = c->setup_done[p->N1 + 65536 * p->d.precision], oB = c->setup_done[p->N2 + 65536 * p->d.precision];
-    // Realization groups.  The batch is split into groups that run on their own streams with full-size persistent
-    // grids: while the last CTAs of one group's pass drain (tile-count quantisation, stragglers, the launch gap and
-    // the one-CTA-per-realization step control), the other group's pass already fills the freed SM slots.
-    static const int env_groups = getenv("PMX_GROUPS") ? atoi(getenv("PMX_GROUPS")) : 0;
-    // two groups pay once a pass has more than about two rounds of tiles; below that a single group with
-    // programmatic dependent launches (prologue of the next kernel under the tail of the current one) is faster
-    const long tiles_all = (long)(p->N2 / p->tA->gAC) * batch * nfc;
-    const int want_groups = env_groups ? env_groups : (tiles_all > 2L * c->sm_count * oA.a ? 2 : 1);
-    const int ngroups = c->profile ? 1 : std::max(1, std::min(std::min(want_groups, 4), batch));
-    static const double grid_mul = getenv("PMX_GRID_MUL") ? atof(getenv("PMX_GRID_MUL")) : 1.0;  // tuning knob
-    for (int g = 1; g < ngroups; ++g)
-        if (!c->gstream[g - 1]) {
-            CK(c, cudaStreamCreateWithFlags(&c->gstream[g - 1], cudaStreamNonBlocking));
-            CK(c, cudaEventCreateWithFlags(&c->ev_join[g - 1], cudaEventDisableTiming));
-            if (!c->ev_fork) CK(c, cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming));
-        }
-    static const int stagB = getenv("PMX_STAGGER_B") ? atoi(getenv("PMX_STAGGER_B")) : 0;
-    static const int stagAC = getenv("PMX_STAGGER_AC") ? atoi(getenv("PMX_STAGGER_AC")) : 0;
-    // programmatic dependent launch pays when nothing else fills the gap between two kernels of a stream, i.e. with a
-    // single realization group (a batch of one: the reference-style fiber() call); PMX_PDL=0/1 overrides
-    static const int pdl_env = getenv("PMX_PDL") ? atoi(getenv("PMX_PDL")) : -1;
-    const int use_pdl = (pdl_env >= 0) ? pdl_env : (ngroups == 1 && !c->profile && !p->fc.xpm ? 1 : 0);
-    struct Grp {
-        cudaStream_t st;
-        PassParams pA, pB, pc;
-        FiberConst fc;
-        int nb, gA, gB, gC;
-    } grp[4];
-    static const int grid_div = getenv("PMX_GRID_DIV") ? std::max(1, atoi(getenv("PMX_GRID_DIV"))) : 1;  // tuning knob
+    PassGroups gs;
+    rc = plan_groups(p, fld, pa, pA, pB, c->setup_done[p->N1 + 65536 * p->d.precision].c, !c->profile && !p->fc.xpm, gs);
+    if (rc) return rc;
     const size_t N = (size_t)p->d.nfft;
-    for (int g = 0; g < ngroups; ++g) {
-        Grp& G = grp[g];
-        const int b0 = (int)((long long)g * batch / ngroups);
-        G.nb = (int)((long long)(g + 1) * batch / ngroups) - b0;
-        G.st = g == 0 ? c->stream : c->gstream[g - 1];
-        G.fc = p->fc;
-        for (PassParams* q : {&G.pA, &G.pB, &G.pc}) {
-            *q = (q == &G.pA) ? pA : (q == &G.pB ? pB : pa);
-            q->field = (char*)pa.field + (size_t)b0 * nfc * N * 2 * fld->cbytes();
-            q->ctl = pa.ctl + b0;
-            q->pkg = pa.pkg + b0;
-            if (p->fc.plate_sets > 1) q->plates = pa.plates + (size_t)b0 * p->fc.nplates;
-            if (pa.trace_dz) {
-                q->trace_dz = pa.trace_dz + (size_t)b0 * p->trace_cap;
-                q->trace_ntrunk = pa.trace_ntrunk + (size_t)b0 * p->trace_cap;
-            }
-            q->batch = G.nb;
-            q->bc0 = b0 * nfc;
-            q->stagger = (q == &G.pB) ? stagB : stagAC;
-            q->pdl = use_pdl;
-        }
-        const int tilesAC = (p->N2 / p->tA->gAC) * G.nb * nfc, tilesB = (p->N1 / p->tB->gB) * G.nb * nfc;
-        // Persistent grids of one CTA per resident slot -- except when a pass has between one and two rounds of
-        // tiles (a batch of one at N = 2^20: 1024 tiles on 592 slots): then one CTA per tile, so that the hardware
-        // hands the tiles of the partial second round to whichever slot frees first (measured +8 % at batch 1, N = 2^20;
-        // with more rounds the persistent grid is the faster one, PMX_GRID_MUL sweeps in DESIGN.md)
-        auto grid_of = [&](int tiles, int ctas_per_sm) {
-            const int slots = (int)(std::max(1, ctas_per_sm / grid_div) * c->sm_count * grid_mul);
-            if (!getenv("PMX_GRID_MUL") && tiles > slots && tiles <= 2 * slots) return tiles;
-            return std::min(tiles, slots);
-        };
-        G.gA = grid_of(tilesAC, oA.a);
-        G.gB = grid_of(tilesB, oB.b);
-        G.gC = grid_of(tilesAC, oA.c);
-    }
-    static const bool serp = !getenv("PMX_NO_SERPENTINE");
     int chunk = p->single_step ? 1 : 8;
     int rev[4] = {1, 1, 1, 1};
     long total_steps = 0;
     for (;;) {
-        if (ngroups > 1) {  // the other streams start after everything queued on the first one so far
-            CK(c, cudaEventRecord(c->ev_fork, c->stream));
-            for (int g = 1; g < ngroups; ++g) CK(c, cudaStreamWaitEvent(c->gstream[g - 1], c->ev_fork, 0));
-        }
+        rc = fork_groups(c, gs.n);
+        if (rc) return rc;
         for (int s = 0; s < chunk; ++s) {
-            for (int gi = 0; gi < ngroups; ++gi) {
-                Grp& G = grp[gi];
+            for (int gi = 0; gi < gs.n; ++gi) {
+                PassGroup& G = gs.g[gi];
                 // serpentine tile order: consecutive passes walk the realizations in opposite directions
-                G.pA.reverse = serp ? (rev[gi] ^= 1) : 0;
-                if (G.fc.xpm) {  // row sums of |u|^2 over the columns, parked in the (empty) Y slots for pass A
-                    p->tA->xpm_sum(dim3((unsigned)std::min<size_t>((N + 255) / 256, 148 * 8), G.nb), G.st, G.pA, G.fc);
+                G.pA.reverse = (rev[gi] ^= 1);
+                if (p->fc.xpm) {  // row sums of |u|^2 over the columns, parked in the (empty) Y slots for pass A
+                    p->tA->xpm_sum(dim3((unsigned)std::min<size_t>((N + 255) / 256, 148 * 8), G.nb), G.st, G.pA, p->fc);
                     c->launches++;
                 }
                 if (fused) {   // pass A reads block `par`, writes block `par ^ 1`; pass C gathers the maxima in the new one
@@ -1254,22 +1281,22 @@ extern "C" int pmx_fiber_exec(pmx_plan* p, pmx_devfield* fld, pmx_fiber_result* 
                     G.pA.ctl_out = p->ctl + (par ^ 1);
                     G.pA.first = fused_first;
                 }
-                { ProfScope ps(c, 0); CK(c, p->tA->passA(G.gA, G.st, G.pA, G.fc, fld->map_rows)); }
-                G.pB.reverse = serp ? (rev[gi] ^= 1) : 0;
-                { ProfScope ps(c, 1); CK(c, p->tB->passB(G.gB, G.st, G.pB, G.fc, fld->map_cols)); }
-                G.pA.reverse = serp ? (rev[gi] ^= 1) : 0;
+                { ProfScope ps(c, 0); CK(c, p->tA->passA(G.gA, G.st, G.pA, p->fc, fld->map_rows)); }
+                G.pB.reverse = (rev[gi] ^= 1);
+                { ProfScope ps(c, 1); CK(c, p->tB->passB(G.gB, G.st, G.pB, p->fc, fld->map_cols)); }
+                G.pA.reverse = (rev[gi] ^= 1);
                 if (fused) {
                     PassParams pC = G.pA;
                     pC.ctl = p->ctl + (par ^ 1);
                     pC.ctl_out = nullptr;
-                    CK(c, p->tA->passC(G.gC, G.st, pC, G.fc, fld->map_rows));
+                    CK(c, p->tA->passC(G.gC, G.st, pC, p->fc, fld->map_rows));
                     par ^= 1;
                     fused_first = 0;
                     c->launches += 3;
                     continue;
                 }
-                { ProfScope ps(c, 2); CK(c, p->tA->passC(G.gC, G.st, G.pA, G.fc, fld->map_rows)); }
-                if (use_pdl) {
+                { ProfScope ps(c, 2); CK(c, p->tA->passC(G.gC, G.st, G.pA, p->fc, fld->map_rows)); }
+                if (gs.pdl) {
                     cudaLaunchConfig_t cfg = {};
                     cfg.gridDim = dim3(G.nb);
                     cfg.blockDim = dim3(128);
@@ -1279,9 +1306,9 @@ extern "C" int pmx_fiber_exec(pmx_plan* p, pmx_devfield* fld, pmx_fiber_result* 
                     at[0].val.programmaticStreamSerializationAllowed = 1;
                     cfg.attrs = at;
                     cfg.numAttrs = 1;
-                    CK(c, cudaLaunchKernelEx(&cfg, pmx_k_ctl, G.pc, G.fc, 0));
+                    CK(c, cudaLaunchKernelEx(&cfg, pmx_k_ctl, G.pc, p->fc, 0));
                 } else {
-                    pmx_k_ctl<<<G.nb, 128, 0, G.st>>>(G.pc, G.fc, 0);
+                    pmx_k_ctl<<<G.nb, 128, 0, G.st>>>(G.pc, p->fc, 0);
                 }
                 c->launches += 4;
             }
@@ -1289,10 +1316,8 @@ extern "C" int pmx_fiber_exec(pmx_plan* p, pmx_devfield* fld, pmx_fiber_result* 
         }
         total_steps += chunk;
         CK(c, cudaGetLastError());
-        for (int g = 1; g < ngroups; ++g) {
-            CK(c, cudaEventRecord(c->ev_join[g - 1], c->gstream[g - 1]));
-            CK(c, cudaStreamWaitEvent(c->stream, c->ev_join[g - 1], 0));
-        }
+        rc = join_groups(c, gs.n);
+        if (rc) return rc;
         CK(c, cudaMemcpyAsync(c->h_ctl, p->ctl + (fused ? par : 0), (size_t)batch * sizeof(StepCtl), cudaMemcpyDeviceToHost, c->stream));
         CK(c, cudaStreamSynchronize(c->stream));
         bool all_done = true;
@@ -3329,7 +3354,7 @@ extern "C" int pmx_scalar_adaptive_run(pmx_ctx* c, const pmx_fiber_desc* d, doub
 
 // ---------------------------------------------------------------------------
 // Digital backpropagation (polmux_ssfm.h, pmx_dbp_desc): a step of length h is the three passes of a forward step --
-// pass A without the nonlinear step, pass B with the dispersion negated, pass C' (pmx_k_passC_nl) with the scale
+// pass A without the nonlinear step, pass B with the dispersion negated, pass C' (pmx_k_passC<..., NL = true>) with the scale
 // exp(+alpha*h/2)/N and the nonlinear step with gam -> -xi*gam -- in the order N(-xi*gam) L(-h) A(-h), the inverse of the
 // forward A(h) L(h) N(h).  The schedule is known when the plan is made: every step's package is built here and the host
 // enqueues the whole link without reading anything back.
@@ -3579,16 +3604,6 @@ extern "C" int pmx_dbp_create(pmx_ctx* c, const pmx_fiber_desc* fd, const pmx_db
     p->fc_a.spm = 0;                            // pass A: the transform only
     p->fc_c = p->fc;
     for (int k = 0; k < p->fc.nfc; ++k) p->fc_c.gam[k] = -g->xi * p->fc.gam[k];   // (gam carries the Manakov 8/9)
-    const int key = p->tA->L + 65536 * p->tA->precision;
-    if (c->setup_done[key].cnl < 1) {
-        int n = 0;
-        cudaError_t err = p->tA->passC_nl_setup(&n);
-        if (err != cudaSuccess || n < 1) {
-            pmx_plan_destroy(p);
-            return set_err(c, PMX_ERR_CUDA, "kernel setup (pass C', L=%d) failed: %s", p->tA->L, cudaGetErrorString(err));
-        }
-        c->setup_done[key].cnl = n;
-    }
     if (pmd) {   // one package per step and realization, built by pmx_dbp_set_plates from the geometry table
         const size_t bytes = geo.size() * (size_t)p->d.batch * sizeof(StepPkg);
         cudaError_t err = cudaMallocAsync(&p->sched, bytes, c->stream);
@@ -3662,86 +3677,24 @@ extern "C" int pmx_dbp_exec(pmx_plan* p, pmx_devfield* fld) {
     if (!p->dbp) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_exec: the plan was not made by pmx_dbp_create");
     if (p->dbp_pmd && !p->dbp_plates_set)
         return set_err(c, PMX_ERR_INVALID, "pmx_dbp_exec: a PMD-aware plan needs its plates (pmx_dbp_set_plates) first");
-    if (fld->ctx != c && fld->ctx->device != c->device)
-        return set_err(c, PMX_ERR_INVALID, "field and plan belong to contexts on different devices");
-    if (fld->precision != p->d.precision)
-        return set_err(c, PMX_ERR_INVALID, "field precision %d does not match the plan's %d", fld->precision, p->d.precision);
-    if (fld->nfft != p->d.nfft || fld->nfc != p->d.nfc || fld->batch != p->d.batch)
-        return set_err(c, PMX_ERR_INVALID, "field shape (%lld,%d,%d) does not match the plan (%lld,%d,%d)",
-                       (long long)fld->nfft, fld->nfc, fld->batch, (long long)p->d.nfft, p->d.nfc, p->d.batch);
-    if (!fld->has_maps) return set_err(c, PMX_ERR_INVALID, "field has no tensor maps (unsupported nfft)");
-    CK(c, cudaSetDevice(c->device));
-    const int batch = p->d.batch, nfc = p->d.nfc;
-    const void *tw4A = nullptr, *tw4B = nullptr, *twA = nullptr, *twB = nullptr;
-    int rc = get_four_tw(c, p->d.nfft, p->tA, p->N2, &tw4A);
-    if (!rc) rc = get_four_tw(c, p->d.nfft, p->tB, p->N1, &tw4B);
-    if (!rc) rc = get_stage_tw(c, p->tA, &twA);
-    if (!rc) rc = get_stage_tw(c, p->tB, &twB);
+    int rc = check_field(p, fld);
     if (rc) return rc;
-    PassParams pa;
-    memset(&pa, 0, sizeof pa);
-    pa.field = fld->data;
-    pa.ctl = p->ctl;
-    pa.betat_p = p->betat_p;
-    pa.plates = p->plates;
-    pa.N1 = p->N1;
-    pa.N2 = p->N2;
-    pa.log2N1 = p->log2N1;
-    pa.log2N2 = p->log2N2;
-    pa.dbg = g_dbg;
-    PassParams pA = pa, pB = pa;
-    pA.tw_stage = twA;
-    pA.tw4 = tw4A;
-    pB.tw_stage = twB;
-    pB.tw4 = tw4B;
-    const pmx_ctx::Occ oA = c->setup_done[p->N1 + 65536 * p->d.precision], oB = c->setup_done[p->N2 + 65536 * p->d.precision];
-    // realization groups and dependent launches as in pmx_fiber_exec: two groups on two streams once a pass has more
-    // than about two rounds of tiles, else one group with programmatic dependent launch
-    const long tiles_all = (long)(p->N2 / p->tA->gAC) * batch * nfc;
-    const int ngroups = std::min(tiles_all > 2L * c->sm_count * oA.a ? 2 : 1, batch);
-    for (int gi = 1; gi < ngroups; ++gi)
-        if (!c->gstream[gi - 1]) {
-            CK(c, cudaStreamCreateWithFlags(&c->gstream[gi - 1], cudaStreamNonBlocking));
-            CK(c, cudaEventCreateWithFlags(&c->ev_join[gi - 1], cudaEventDisableTiming));
-            if (!c->ev_fork) CK(c, cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming));
-        }
-    struct Grp {
-        cudaStream_t st;
-        PassParams pA, pB;
-        int b0, gA, gB, gC;
-    } grp[2];
-    const size_t N = (size_t)p->d.nfft;
-    auto grid_of = [&](int tiles, int ctas_per_sm) {   // one CTA per tile between one and two rounds, else persistent
-        const int slots = ctas_per_sm * c->sm_count;
-        if (tiles > slots && tiles <= 2 * slots) return tiles;
-        return std::min(tiles, slots);
-    };
-    for (int gi = 0; gi < ngroups; ++gi) {
-        Grp& G = grp[gi];
-        G.b0 = (int)((long long)gi * batch / ngroups);
-        const int nb = (int)((long long)(gi + 1) * batch / ngroups) - G.b0;
-        G.st = gi == 0 ? c->stream : c->gstream[gi - 1];
-        for (PassParams* q : {&G.pA, &G.pB}) {
-            *q = (q == &G.pA) ? pA : pB;
-            q->field = (char*)pa.field + (size_t)G.b0 * nfc * N * 2 * fld->cbytes();
-            q->batch = nb;
-            q->bc0 = G.b0 * nfc;
-            q->pdl = ngroups == 1 ? 1 : 0;
-        }
-        const int tilesAC = (p->N2 / p->tA->gAC) * nb * nfc, tilesB = (p->N1 / p->tB->gB) * nb * nfc;
-        G.gA = grid_of(tilesAC, oA.a);
-        G.gB = grid_of(tilesB, oB.b);
-        G.gC = grid_of(tilesAC, c->setup_done[p->N1 + 65536 * p->d.precision].cnl);
-    }
-    if (ngroups > 1) {   // the other stream starts after everything queued on the first one so far
-        CK(c, cudaEventRecord(c->ev_fork, c->stream));
-        for (int gi = 1; gi < ngroups; ++gi) CK(c, cudaStreamWaitEvent(c->gstream[gi - 1], c->ev_fork, 0));
-    }
-    int rev[2] = {1, 1};
+    CK(c, cudaSetDevice(c->device));
+    const int batch = p->d.batch;
+    PassParams pa, pA, pB;
+    rc = pass_params(p, fld, pa, pA, pB);
+    if (rc) return rc;
+    // realization groups and dependent launches as in pmx_fiber_exec; pass C' has an occupancy of its own
+    PassGroups gs;
+    rc = plan_groups(p, fld, pa, pA, pB, c->setup_done[p->N1 + 65536 * p->d.precision].cnl, true, gs);
+    if (rc) return rc;
+    rc = fork_groups(c, gs.n);
+    if (rc) return rc;
+    int rev[4] = {1, 1, 1, 1};
     for (size_t s = 0; s < p->sched_idx.size(); ++s) {
         StepPkg* pk = p->sched + (size_t)p->sched_idx[s] * batch;
-        for (int gi = 0; gi < ngroups; ++gi) {
-            Grp& G = grp[gi];
+        for (int gi = 0; gi < gs.n; ++gi) {
+            PassGroup& G = gs.g[gi];
             G.pA.pkg = G.pB.pkg = pk + G.b0;
             if (p->dbp_pmd)   // the step's span: trunks beyond the package's PMX_PKG_PLATES are read from its table
                 G.pB.plates = p->plates + ((size_t)p->sched_span[s] * p->fc.plate_sets + (p->fc.plate_sets > 1 ? G.b0 : 0)) *
@@ -3756,10 +3709,8 @@ extern "C" int pmx_dbp_exec(pmx_plan* p, pmx_devfield* fld) {
         }
     }
     CK(c, cudaGetLastError());
-    for (int gi = 1; gi < ngroups; ++gi) {
-        CK(c, cudaEventRecord(c->ev_join[gi - 1], c->gstream[gi - 1]));
-        CK(c, cudaStreamWaitEvent(c->stream, c->ev_join[gi - 1], 0));
-    }
+    rc = join_groups(c, gs.n);
+    if (rc) return rc;
     CK(c, cudaStreamSynchronize(c->stream));
     return PMX_OK;
 }

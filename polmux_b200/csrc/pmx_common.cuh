@@ -157,7 +157,6 @@ struct PassParams {
     int bc0;                // first realization-column of this launch inside the field (tensor-map coordinate offset)
     int pdl;                // launched with programmatic stream serialization: the prologue overlaps the tail of the
                             // previous kernel of the stream, griddepcontrol.wait orders the dependent accesses
-    int stagger;            // cycles by which the CTAs sharing an SM start apart (de-phases their load / exchange / math phases)
     int reverse;            // walk the tile list backwards (alternates from pass to pass: the tiles the previous
                             // pass wrote last are still in L2 when this pass reads them first)
     long long* dbg;         // optional per-CTA phase cycle counters (PMX_TIMING builds only)

@@ -9,7 +9,7 @@
 //   pass C  rows    : W_N^(-n2*k1) -> IFFT over k1 -> 1/N * exp(-alpha/2 dz) (:531-532) ->
 //                     max |u|^2 (warp shuffle + one atomicMax per CTA and realization)
 //   ctl     one CTA per realization: nextstep + checkstep for the next step, step package for the passes
-//   pass C' rows    : (digital backpropagation, pmx_k_passC_nl) as pass C, scale exp(+alpha/2 h)/N, then the nonlinear
+//   pass C' rows    : (digital backpropagation, pmx_k_passC<..., NL = true>) as pass C, scale exp(+alpha/2 h)/N, then the nonlinear
 //                     step with -xi*gam; A without the NL step and B with the dispersion negated complete the step
 #pragma once
 #include "pmx_fft.cuh"
@@ -362,19 +362,6 @@ __device__ __forceinline__ bool pmx_is_done(const unsigned char* sdone, const Pa
     return (p.batch <= PMX_LIVE_CAP) ? (sdone[b] != 0) : (p.pkg[b].state >= PMX_ST_DONE);
 }
 
-// CTAs that share an SM would otherwise run their phases (tile load, shared-memory exchanges, FP64 math) in
-// lockstep and queue on one resource at a time while the others idle: start them apart.  Blocks are placed
-// round-robin over the SMs, so blockIdx.x / #SM is the slot of a CTA on its SM.
-__device__ __forceinline__ void pmx_stagger(const PassParams& p) {
-    if (p.stagger > 0) {
-        unsigned nsm;
-        asm("mov.u32 %0, %%nsmid;" : "=r"(nsm));
-        const long long d = (long long)(blockIdx.x / nsm) * p.stagger, t0 = clock64();
-        while (clock64() - t0 < d) {
-        }
-    }
-}
-
 // realization / column of a flat realization-column index
 __device__ __forceinline__ void pmx_split_bc(int bc, const FiberConst& f, int& b, int& col) {
     if (f.nfc == 1) {
@@ -536,13 +523,9 @@ __global__ void __launch_bounds__(G*(L / 8), PMX_MINB(G*(L / 8), PF))
     auto issue = [&](int tl, int buf) {  // one thread
         pmx_fence_proxy_async();
         const int tt = wk.phys(tl), bc = tt >> wk.ltpb, row0 = (tt & wk.tpb_mask) * G;
-#ifdef PMX_AC_LDG
-        pmx_mbar_expect_tx(mbar, S::AUX_BYTES);
-#else
         pmx_mbar_expect_tx(mbar, S::LOAD_BYTES);
         for (int l0 = 0; l0 < LINES; l0 += 256)
             pmx_tma_load_3d(in + l0 * 128, &tmap, 0, (tt & wk.tpb_mask) * LINES + l0, p.bc0 + bc, mbar);
-#endif
         int b_, col_;
         pmx_split_bc(bc, f, b_, col_);
         unsigned char* a = aux0 + buf * S::AUX_BYTES;
@@ -598,7 +581,6 @@ __global__ void __launch_bounds__(G*(L / 8), PMX_MINB(G*(L / 8), PF))
         }
         fpkg = sp;
     }
-    pmx_stagger(p);
     PMX_T_DECL
     while (tile < total) {
         const int tt = wk.phys(tile), bc = tt >> wk.ltpb, row0 = (tt & wk.tpb_mask) * G;
@@ -612,17 +594,6 @@ __global__ void __launch_bounds__(G*(L / 8), PMX_MINB(G*(L / 8), PF))
         const int next = live(tile + gridDim.x);
         cpx x[8], y[8];
         PMX_T_MARK(0)
-#ifdef PMX_AC_LDG
-        {   // the row is contiguous: 32 lanes x 32 B per load instruction, straight into registers
-            const cpx* src = reinterpret_cast<const cpx*>(p.field) + ((size_t)bc * N + (size_t)(row0 + rl) * L) * 2;
-#pragma unroll
-            for (int q = 0; q < 8; ++q) ld_sa(src + (size_t)(t + q * T) * 2, x[q], y[q]);
-        }
-        pmx_mbar_wait(mbar, phase);
-        phase ^= 1u;
-        __syncthreads();  // every thread has seen this phase complete before the barrier is armed again
-        if (threadIdx.x == 0 && next < total) issue(next, (it + 1) & 1);
-#else
         pmx_mbar_wait(mbar, phase);
         phase ^= 1u;
         PMX_T_MARK(1)
@@ -630,26 +601,17 @@ __global__ void __launch_bounds__(G*(L / 8), PMX_MINB(G*(L / 8), PF))
         for (int q = 0; q < 8; ++q) lds_sa(in, pmx_swz<7>((uint32_t)((rl * L + t + q * T) * PMX_SA_BYTES)), x[q], y[q]);
         __syncthreads();
         if (PF && threadIdx.x == 0 && next < total) issue(next, (it + 1) & 1);
-#endif
         PMX_T_MARK(2)
         pmx_nl_step(x, y, st, f, col);   // ---- nonlinear step, fiber.m:832-851
         cpx* sx = work + rl * PmxSmem<L, G>::STRIDE;
         cpx* sy = sx + L;
         PMX_T_MARK(3)
-#if defined(PMX_AC_LDG) || defined(PMX_AC_LATE_ISSUE)
-        CtaFFT<R, L>::run(x, y, sx, sy, t, stw);
-        PMX_T_MARK(4)
-#ifndef PMX_AC_LDG
-        if (!PF && threadIdx.x == 0 && next < total) issue(next, (it + 1) & 1);  // the exchange buffer is free again
-#endif
-#else
         // the next tile lands in the exchange buffer: its load goes out as soon as the last exchange is read, under the
         // last butterfly stage and the store
         CtaFFT<R, L>::run(x, y, sx, sy, t, stw, [&] {
             if (!PF && threadIdx.x == 0 && next < total) issue(next, (it + 1) & 1);
         });
         PMX_T_MARK(4)
-#endif
         // four-step twiddle W_N^(n2*k1), k1 = t + q*T, from the row's two-level table; straight to HBM (the row is
         // contiguous: 32 lanes x 32 B per store instruction)
         {
@@ -673,11 +635,6 @@ __global__ void __launch_bounds__(G*(L / 8), PMX_MINB(G*(L / 8), PF))
 
 // ---------------------------------------------------------------------------
 // pass B: G adjacent columns (k1) of the [n2][k1] matrix per tile, thread (cl fastest, t)
-#ifdef PMX_B_CTAS   // experiment knob: resident 128-thread-equivalent CTAs targeted for pass B
-#define PMX_MINB_B(threads, pf) (((PMX_B_CTAS * 128 * (32 / PMX_SA_BYTES)) / (threads)) > 0 ? ((PMX_B_CTAS * 128 * (32 / PMX_SA_BYTES)) / (threads)) : 1)
-#else
-#define PMX_MINB_B(threads, pf) PMX_MINB(threads, pf)
-#endif
 
 // u <- M*u for the eight bins of a thread, M row-major (re,im) in shared memory
 __device__ __forceinline__ void pmx_apply2x2(cpx (&x)[8], cpx (&y)[8], const double* M) {
@@ -963,44 +920,37 @@ __device__ __forceinline__ void pmx_linear_bins(cpx (&x)[8], cpx (&y)[8], const 
                              scr[2 * scr_stride], dmk(st->gd3_r, st->gd3_i));
             else if (f.pmd)
                 pmx_b_common(x, y, dmk(S4.x, -S4.y), dmk(Gacc.x, -Gacc.y), dmk(1.0, 0.0), dmk(1.0, 0.0));
-        } else
-#ifdef PMX_EXP_NO_COMMON
-        if (false) {
-#else
-        if (f.gvd_any) {  // common phase exp(-i*betat*sum(dzb))  (:924,927-928)
-#endif
-            {
-                double a[8];
-                if constexpr (SC) {  // betat regenerated per bin (:355-356)
-                    const double b1 = f.beta1[col], b2 = f.beta2[col];
-#pragma unroll
-                    for (int q = 0; q < 8; ++q) {
-                        const double fn = (q < 4) ? fn0 + (double)q * dfn : fn4 + (double)(q - 4) * dfn;  // exact
-                        const double w = __dmul_rn(f.w0, fn);
-                        const double w2 = __dmul_rn(w, w);
-                        double bt = __dadd_rn(__dmul_rn(w, b1), __dmul_rn(__dmul_rn(0.5, w2), b2));
-                        bt = __dadd_rn(bt, __dmul_rn(__dmul_rn(w2, w), f.b30_6));
-                        a[q] = -(bt * dz_cur);
-                    }
-                } else {
-                    const double* bt = p.betat_p + (size_t)col * N + (size_t)k1 * p.N2;
-#pragma unroll
-                    for (int q = 0; q < 8; ++q) a[q] = -(__ldg(&bt[t + q * T]) * dz_cur);
-                }
-                cpx e[8];
-#pragma unroll
-                for (int q = 0; q < 8; ++q) e[q] = pmx_cis(a[q]);
+        } else if (f.gvd_any) {  // common phase exp(-i*betat*sum(dzb))  (:924,927-928)
+            double a[8];
+            if constexpr (SC) {  // betat regenerated per bin (:355-356)
+                const double b1 = f.beta1[col], b2 = f.beta2[col];
 #pragma unroll
                 for (int q = 0; q < 8; ++q) {
-                    x[q] = cmul(x[q], e[q]);
-                    y[q] = cmul(y[q], e[q]);
+                    const double fn = (q < 4) ? fn0 + (double)q * dfn : fn4 + (double)(q - 4) * dfn;  // exact
+                    const double w = __dmul_rn(f.w0, fn);
+                    const double w2 = __dmul_rn(w, w);
+                    double bt = __dadd_rn(__dmul_rn(w, b1), __dmul_rn(__dmul_rn(0.5, w2), b2));
+                    bt = __dadd_rn(bt, __dmul_rn(__dmul_rn(w2, w), f.b30_6));
+                    a[q] = -(bt * dz_cur);
                 }
+            } else {
+                const double* bt = p.betat_p + (size_t)col * N + (size_t)k1 * p.N2;
+#pragma unroll
+                for (int q = 0; q < 8; ++q) a[q] = -(__ldg(&bt[t + q * T]) * dz_cur);
+            }
+            cpx e[8];
+#pragma unroll
+            for (int q = 0; q < 8; ++q) e[q] = pmx_cis(a[q]);
+#pragma unroll
+            for (int q = 0; q < 8; ++q) {
+                x[q] = cmul(x[q], e[q]);
+                y[q] = cmul(y[q], e[q]);
             }
         }
 }
 
 template <typename R, int L, int G, bool PF, bool SC>
-__global__ void __launch_bounds__(G*(L / 8), PMX_MINB_B(G*(L / 8), PF))
+__global__ void __launch_bounds__(G*(L / 8), PMX_MINB(G*(L / 8), PF))
     pmx_k_passB(PassParams p, FiberConst f, const __grid_constant__ CUtensorMap tmap) {
     using S = PassSmem<L, G, PF, 1>;
     constexpr int T = L / 8, SA = PMX_SA_BYTES, PITCH = G * SA, MASK = PITCH / 16 - 1;
@@ -1035,9 +985,6 @@ __global__ void __launch_bounds__(G*(L / 8), PMX_MINB_B(G*(L / 8), PF))
     };
     // The step package travels on its own mbarrier: it is a few KB out of the L2 and lands long before the tile, so
     // the threads can evaluate everything that does not depend on the field while the tile is still in flight.
-    // (PMX_B_EARLY_PKG: the next tile's package is fetched while the current tile is still being worked on -- its buffer and
-    // its barrier are free from the moment every thread has picked up the current one -- so that the data-independent
-    // phasors of the next tile start the moment the tile's store has been issued, under the tile load)
     auto issue_pkg = [&](int tl, int buf) {  // one thread
         pmx_fence_proxy_async();
         const int tt = wk.phys(tl), bc = tt >> wk.ltpb;
@@ -1053,11 +1000,7 @@ __global__ void __launch_bounds__(G*(L / 8), PMX_MINB_B(G*(L / 8), PF))
         for (int r0 = 0; r0 < L; r0 += 256) pmx_tma_load_3d(in + r0 * PITCH, &tmap, c0 * 4, r0, p.bc0 + bc, mbar);
     };
     auto issue = [&](int tl, int buf) {  // one thread
-#ifndef PMX_B_EARLY_PKG
         issue_pkg(tl, buf);
-#else
-        (void)buf;
-#endif
         issue_tile(tl);
     };
     if (threadIdx.x == 0) {
@@ -1073,11 +1016,7 @@ __global__ void __launch_bounds__(G*(L / 8), PMX_MINB_B(G*(L / 8), PF))
     pmx_cache_live(sdone, p);
     __syncthreads();
     int tile = live(blockIdx.x), it = 0;
-#ifdef PMX_B_EARLY_PKG
-    if (threadIdx.x == 0 && tile < total) issue_pkg(tile, 0);
-#endif
     if (threadIdx.x == 0 && tile < total) issue(tile, 0);
-    pmx_stagger(p);
     uint32_t phase = 0;
     PMX_T_DECL
     while (tile < total) {
@@ -1112,9 +1051,6 @@ __global__ void __launch_bounds__(G*(L / 8), PMX_MINB_B(G*(L / 8), PF))
         for (int q = 0; q < 8; ++q) lds_sa(in, pmx_swz<MASK>((uint32_t)((t + q * T) * PITCH + cl * SA)), x[q], y[q]);
         if (threadIdx.x == 0) pmx_tma_wait_read();  // previous tile's store has left the exchange buffer
         __syncthreads();
-#ifdef PMX_B_EARLY_PKG
-        if (threadIdx.x == 0 && next < total) issue_pkg(next, (it + 1) & 1);   // every thread is past this tile's package wait
-#endif
         if (PF && threadIdx.x == 0 && next < total) issue(next, (it + 1) & 1);
         cpx* sx = work + cl * PmxSmem<L, G>::STRIDE;
         cpx* sy = sx + L;
@@ -1123,18 +1059,12 @@ __global__ void __launch_bounds__(G*(L / 8), PMX_MINB_B(G*(L / 8), PF))
         // the transform code, run twice
 #pragma unroll 1
         for (int dir = 0; dir < 2; ++dir) {
-#ifndef PMX_EXP_NO_FFT
             CtaFFT<R, L>::run(x, y, sx, sy, t, stw);
-#endif
             if (dir == 1) break;
             PMX_T_MARK(3)
 
             // ---- linear step in the frequency domain, fiber.m:907-933
-#ifdef PMX_EXP_NO_PHYS
-            if (false) {
-#else
             if (ntrunk > 0) {
-#endif
                 pmx_linear_bins<SC, PRE>(x, y, st, f, p, scr, S::THREADS, schunk, b, col, k1, t, T, N, fn0, fn4, dfn, any_full);
             }
 #pragma unroll
@@ -1147,17 +1077,6 @@ __global__ void __launch_bounds__(G*(L / 8), PMX_MINB_B(G*(L / 8), PF))
         PMX_T_MARK(5)
         // the second transform was run on conj(spectrum): conj(result) is the inverse transform.  Its four-step
         // twiddle W_N^(-n2*k1) is applied by pass C when it loads the sample (pass C has FP64 slots to spare).
-#ifdef PMX_B_STG
-        // direct scattered stores (one 32-byte sector per lane): the exchange buffer is free for the next tile's load
-        // as soon as the last exchange is read out
-        if (!PF && threadIdx.x == 0 && next < total) issue(next, (it + 1) & 1);
-        {
-            cpx* base = reinterpret_cast<cpx*>(p.field) + ((size_t)bc * N + (size_t)k1) * 2;
-#pragma unroll
-            for (int q = 0; q < 8; ++q) st_sa(base + (size_t)(t + q * T) * p.N1 * 2, cconj(x[q]), cconj(y[q]));
-        }
-        __syncthreads();  // everyone is done with this tile's auxiliary buffer and plate chunk
-#else
         // The column tile is staged (same swizzled layout as it landed) in the exchange buffer and TMA-stored.
         unsigned char* outb = reinterpret_cast<unsigned char*>(work);
 #pragma unroll
@@ -1173,7 +1092,6 @@ __global__ void __launch_bounds__(G*(L / 8), PMX_MINB_B(G*(L / 8), PF))
                 issue(next, (it + 1) & 1);
             }
         }
-#endif
         tile = next;
         ++it;
         PMX_T_MARK(6)
@@ -1186,13 +1104,12 @@ __global__ void __launch_bounds__(G*(L / 8), PMX_MINB_B(G*(L / 8), PF))
 // pass C: rows like pass A: four-step twiddle, inverse transform over k1, attenuation, max reduction.  The
 // running maximum stays in registers across the tiles a CTA handles for one realization-column and is published
 // (one atomicMax per CTA) when the CTA moves on to another one.
-#ifdef PMX_C_CTAS
-#define PMX_MINB_C(threads, pf) (((PMX_C_CTAS * 128 * (32 / PMX_SA_BYTES)) / (threads)) > 0 ? ((PMX_C_CTAS * 128 * (32 / PMX_SA_BYTES)) / (threads)) : 1)
-#else
-#define PMX_MINB_C(threads, pf) PMX_MINB(threads, pf)
-#endif
-template <typename R, int L, int G, bool PF>
-__global__ void __launch_bounds__(G*(L / 8), PMX_MINB_C(G*(L / 8), PF))
+// NL (pass C' of a digital-backpropagation step, pmx_dbp_exec): after the scale exp(+alpha/2*h)/N of the step package
+// (times 1/sqrt(G) on the first step of a span), the nonlinear step N(-xi*gam) of pmx_nl_step on the rows the CTA holds,
+// in time, before the store.  The caller hands in a FiberConst whose gam is -xi*gam and a package whose bmode has no
+// PMX_BM_NL_SMALL.  The schedule is known before the first launch, so there is no max reduction and no step control.
+template <typename R, int L, int G, bool PF, bool NL>
+__global__ void __launch_bounds__(G*(L / 8), PMX_MINB(G*(L / 8), PF))
     pmx_k_passC(PassParams p, FiberConst f, const __grid_constant__ CUtensorMap tmap) {
     using S = PassSmem<L, G, PF, 2>;
     using W = PmxTw4<L>;
@@ -1229,13 +1146,9 @@ __global__ void __launch_bounds__(G*(L / 8), PMX_MINB_C(G*(L / 8), PF))
     auto issue = [&](int tl, int buf) {  // one thread
         pmx_fence_proxy_async();
         const int tt = wk.phys(tl), bc = tt >> wk.ltpb, row0 = (tt & wk.tpb_mask) * G;
-#ifdef PMX_AC_LDG
-        pmx_mbar_expect_tx(mbar, S::AUX_BYTES);
-#else
         pmx_mbar_expect_tx(mbar, S::LOAD_BYTES);
         for (int l0 = 0; l0 < LINES; l0 += 256)
             pmx_tma_load_3d(in + l0 * 128, &tmap, 0, (tt & wk.tpb_mask) * LINES + l0, p.bc0 + bc, mbar);
-#endif
         int b_, col_;
         pmx_split_bc(bc, f, b_, col_);
         unsigned char* a = aux0 + buf * S::AUX_BYTES;
@@ -1255,7 +1168,6 @@ __global__ void __launch_bounds__(G*(L / 8), PMX_MINB_C(G*(L / 8), PF))
     __syncthreads();
     int tile = live(blockIdx.x), it = 0;
     if (threadIdx.x == 0 && tile < total) issue(tile, 0);
-    pmx_stagger(p);
     uint32_t phase = 0;
     unsigned long long vmax = 0ull;  // running max of this thread for the current realization-column
     PMX_T_DECL
@@ -1271,20 +1183,11 @@ __global__ void __launch_bounds__(G*(L / 8), PMX_MINB_C(G*(L / 8), PF))
         const int next = live(tile + gridDim.x);
         cpx x[8], y[8];
         PMX_T_MARK(0)
-#ifdef PMX_AC_LDG
-        {
-            const cpx* src = reinterpret_cast<const cpx*>(p.field) + ((size_t)bc * N + (size_t)(row0 + rl) * L) * 2;
-#pragma unroll
-            for (int q = 0; q < 8; ++q) ld_sa(src + (size_t)(t + q * T) * 2, x[q], y[q]);
-        }
-#endif
         pmx_mbar_wait(mbar, phase);
         phase ^= 1u;
         PMX_T_MARK(1)
-#ifndef PMX_AC_LDG
 #pragma unroll
         for (int q = 0; q < 8; ++q) lds_sa(in, pmx_swz<7>((uint32_t)((rl * L + t + q * T) * PMX_SA_BYTES)), x[q], y[q]);
-#endif
         {   // Pass B left v = conj(z), z = its transform output before the four-step twiddle W_N^(-n2*k1), k1 = t + q*T.
             // The inverse transform over k1 = conj o forward o conj applied to conj(z)*conj(W): its input is z*W.
             const cpx* tb = gtab + rl * W::PER;
@@ -1298,199 +1201,48 @@ __global__ void __launch_bounds__(G*(L / 8), PMX_MINB_C(G*(L / 8), PF))
         }
         const real sc = (real)st->scale, nsc = -sc;
         __syncthreads();  // every thread has seen this phase complete before the barrier is armed again
-#ifdef PMX_AC_LDG
-        if (threadIdx.x == 0 && next < total) issue(next, (it + 1) & 1);
-#else
         if (PF && threadIdx.x == 0 && next < total) issue(next, (it + 1) & 1);
-#endif
         PMX_T_MARK(2)
         cpx* sx = work + rl * PmxSmem<L, G>::STRIDE;
         cpx* sy = sx + L;
         PMX_T_MARK(3)
-#if defined(PMX_AC_LDG) || defined(PMX_AC_LATE_ISSUE)
-        CtaFFT<R, L>::run(x, y, sx, sy, t, stw);
-        PMX_T_MARK(4)
-#ifndef PMX_AC_LDG
-        if (!PF && threadIdx.x == 0 && next < total) issue(next, (it + 1) & 1);
-#endif
-#else
         CtaFFT<R, L>::run(x, y, sx, sy, t, stw, [&] {
             if (!PF && threadIdx.x == 0 && next < total) issue(next, (it + 1) & 1);
         });
         PMX_T_MARK(4)
-#endif
         {
             cpx* base = reinterpret_cast<cpx*>(p.field) + ((size_t)bc * N + (size_t)(row0 + rl) * L) * 2;
+            if constexpr (NL) {
 #pragma unroll
-            for (int q = 0; q < 8; ++q) {
-                x[q] = mkc(x[q].x * sc, x[q].y * nsc);
-                y[q] = mkc(y[q].x * sc, y[q].y * nsc);
-                unsigned long long key = pmx_pow_key((double)power_ref(x[q], y[q]));
-                vmax = key > vmax ? key : vmax;
-                st_sa(base + (size_t)(t + q * T) * 2, x[q], y[q]);
+                for (int q = 0; q < 8; ++q) {
+                    x[q] = mkc(x[q].x * sc, x[q].y * nsc);
+                    y[q] = mkc(y[q].x * sc, y[q].y * nsc);
+                }
+                pmx_nl_step(x, y, st, f, col);   // ---- N(-xi*gam): the gam of f is the backpropagated one
+#pragma unroll
+                for (int q = 0; q < 8; ++q) st_sa(base + (size_t)(t + q * T) * 2, x[q], y[q]);
+            } else {
+#pragma unroll
+                for (int q = 0; q < 8; ++q) {
+                    x[q] = mkc(x[q].x * sc, x[q].y * nsc);
+                    y[q] = mkc(y[q].x * sc, y[q].y * nsc);
+                    unsigned long long key = pmx_pow_key((double)power_ref(x[q], y[q]));
+                    vmax = key > vmax ? key : vmax;
+                    st_sa(base + (size_t)(t + q * T) * 2, x[q], y[q]);
+                }
             }
         }
         PMX_T_MARK(5)
-        if (next >= total || (wk.phys(next) >> wk.ltpb) != bc) {  // moving on: publish the maximum (pmx_k_ctl consumes it)
-            pmx_block_max(vmax, sred, &p.ctl[b], col);
-            vmax = 0ull;
+        if constexpr (!NL) {
+            if (next >= total || (wk.phys(next) >> wk.ltpb) != bc) {  // moving on: publish the maximum (pmx_k_ctl consumes it)
+                pmx_block_max(vmax, sred, &p.ctl[b], col);
+                vmax = 0ull;
+            }
         }
         tile = next;
         ++it;
         __syncthreads();  // everyone is done with this tile's auxiliary buffer
         PMX_T_MARK(6)
     }
-    PMX_T_FLUSH(2)
-}
-
-// ---------------------------------------------------------------------------
-// pass C of a digital-backpropagation step (pmx_dbp_exec): the same tile walk, twiddle and inverse transform over k1 as
-// pmx_k_passC, then the scale exp(+alpha/2*h)/N of the step package (times 1/sqrt(G) on the first step of a span), then
-// the nonlinear step N(-xi*gam) of pmx_nl_step on the rows the CTA holds, in time, before the store.  The caller hands
-// in a FiberConst whose gam is -xi*gam and a package whose bmode has no PMX_BM_NL_SMALL.  The schedule is known before
-// the first launch, so there is no max reduction and no step control.  (A kernel of its own: pmx_k_passC stays as it is.)
-template <typename R, int L, int G, bool PF>
-__global__ void __launch_bounds__(G*(L / 8), PMX_MINB_C(G*(L / 8), PF))
-    pmx_k_passC_nl(PassParams p, FiberConst f, const __grid_constant__ CUtensorMap tmap) {
-    using S = PassSmem<L, G, PF, 2>;
-    using W = PmxTw4<L>;
-    constexpr int T = L / 8;
-    constexpr int LINES = G * L * PMX_SA_BYTES / 128;
-    extern __shared__ __align__(1024) unsigned char smraw[];
-    unsigned char* sm = pmx_checked1024(smraw);
-    unsigned char* in = sm;
-    cpx* work = reinterpret_cast<cpx*>(sm + S::WORK_OFF);
-    cpx* stw = reinterpret_cast<cpx*>(sm + S::TW_OFF);
-    unsigned char* aux0 = sm + S::AUX_OFF;
-    unsigned char* sdone = sm + S::LIVE_OFF;
-    uint64_t* mbar = reinterpret_cast<uint64_t*>(sm + S::MBAR_OFF);
-    const int rl = threadIdx.x / T, t = threadIdx.x % T;
-    const size_t N = (size_t)p.N1 * p.N2;
-    PmxWalk wk;
-    wk.ltpb = p.log2N2 - pmx_ilog2(G);
-    wk.tpb_mask = (1 << wk.ltpb) - 1;
-    wk.total = (p.batch * f.nfc) << wk.ltpb;
-    wk.reverse = p.reverse;
-    const int total = wk.total;
-
-    auto live = [&](int tl) {
-        while (tl < total) {
-            int b_, col_;
-            pmx_split_bc(wk.phys(tl) >> wk.ltpb, f, b_, col_);
-            if (!pmx_is_done(sdone, p, b_)) break;
-            tl += gridDim.x;
-        }
-        return tl;
-    };
-    // a tile = G adjacent rows of the [N2][N1] time-domain matrix = G*L contiguous Sa
-    auto issue = [&](int tl, int buf) {  // one thread
-        pmx_fence_proxy_async();
-        const int tt = wk.phys(tl), bc = tt >> wk.ltpb, row0 = (tt & wk.tpb_mask) * G;
-#ifdef PMX_AC_LDG
-        pmx_mbar_expect_tx(mbar, S::AUX_BYTES);
-#else
-        pmx_mbar_expect_tx(mbar, S::LOAD_BYTES);
-        for (int l0 = 0; l0 < LINES; l0 += 256)
-            pmx_tma_load_3d(in + l0 * 128, &tmap, 0, (tt & wk.tpb_mask) * LINES + l0, p.bc0 + bc, mbar);
-#endif
-        int b_, col_;
-        pmx_split_bc(bc, f, b_, col_);
-        unsigned char* a = aux0 + buf * S::AUX_BYTES;
-        pmx_bulk_load(a, &p.pkg[b_], S::PKG_BYTES, mbar);
-        pmx_bulk_load(a + S::PKG_BYTES, reinterpret_cast<const cpx*>(p.tw4) + (size_t)row0 * W::PER, S::TAB_BYTES, mbar);
-    };
-    if (threadIdx.x == 0) {
-        pmx_mbar_init(mbar, 1);
-        pmx_fence_mbar_init();
-    }
-    pmx_load_stage_tw<L>(stw, p.tw_stage);
-    if (p.pdl) {  // everything above is independent of the previous kernel of the stream
-        pmx_pdl_launch_dependents();
-        pmx_pdl_wait();
-    }
-    pmx_cache_live(sdone, p);
-    __syncthreads();
-    int tile = live(blockIdx.x), it = 0;
-    if (threadIdx.x == 0 && tile < total) issue(tile, 0);
-    pmx_stagger(p);
-    uint32_t phase = 0;
-    PMX_T_DECL
-    while (tile < total) {
-        const int tt = wk.phys(tile), bc = tt >> wk.ltpb, row0 = (tt & wk.tpb_mask) * G;
-        int b, col;
-        pmx_split_bc(bc, f, b, col);
-        PMX_ASSERT(tt >= 0 && tt < total && bc < p.batch * f.nfc && b < p.batch && col < f.nfc && b * f.nfc + col == bc);
-        PMX_ASSERT(row0 + G <= p.N2 && L == p.N1);
-        const unsigned char* aux = aux0 + (it & 1) * S::AUX_BYTES;
-        const StepPkg* st = reinterpret_cast<const StepPkg*>(aux);
-        const cpx* gtab = reinterpret_cast<const cpx*>(aux + S::PKG_BYTES);
-        const int next = live(tile + gridDim.x);
-        cpx x[8], y[8];
-        PMX_T_MARK(0)
-#ifdef PMX_AC_LDG
-        {
-            const cpx* src = reinterpret_cast<const cpx*>(p.field) + ((size_t)bc * N + (size_t)(row0 + rl) * L) * 2;
-#pragma unroll
-            for (int q = 0; q < 8; ++q) ld_sa(src + (size_t)(t + q * T) * 2, x[q], y[q]);
-        }
-#endif
-        pmx_mbar_wait(mbar, phase);
-        phase ^= 1u;
-        PMX_T_MARK(1)
-#ifndef PMX_AC_LDG
-#pragma unroll
-        for (int q = 0; q < 8; ++q) lds_sa(in, pmx_swz<7>((uint32_t)((rl * L + t + q * T) * PMX_SA_BYTES)), x[q], y[q]);
-#endif
-        {   // Pass B left v = conj(z), z = its transform output before the four-step twiddle W_N^(-n2*k1), k1 = t + q*T.
-            // The inverse transform over k1 = conj o forward o conj applied to conj(z)*conj(W): its input is z*W.
-            const cpx* tb = gtab + rl * W::PER;
-            const cpx wl = tb[t & (W::NLO - 1)];
-#pragma unroll
-            for (int q = 0; q < 8; ++q) {
-                const cpx w = cmul(wl, tb[W::NLO + ((t + q * T) >> W::LO)]);
-                x[q] = cmul(cconj(x[q]), w);
-                y[q] = cmul(cconj(y[q]), w);
-            }
-        }
-        const real sc = (real)st->scale, nsc = -sc;
-        __syncthreads();  // every thread has seen this phase complete before the barrier is armed again
-#ifdef PMX_AC_LDG
-        if (threadIdx.x == 0 && next < total) issue(next, (it + 1) & 1);
-#else
-        if (PF && threadIdx.x == 0 && next < total) issue(next, (it + 1) & 1);
-#endif
-        PMX_T_MARK(2)
-        cpx* sx = work + rl * PmxSmem<L, G>::STRIDE;
-        cpx* sy = sx + L;
-        PMX_T_MARK(3)
-#if defined(PMX_AC_LDG) || defined(PMX_AC_LATE_ISSUE)
-        CtaFFT<R, L>::run(x, y, sx, sy, t, stw);
-        PMX_T_MARK(4)
-#ifndef PMX_AC_LDG
-        if (!PF && threadIdx.x == 0 && next < total) issue(next, (it + 1) & 1);
-#endif
-#else
-        CtaFFT<R, L>::run(x, y, sx, sy, t, stw, [&] {
-            if (!PF && threadIdx.x == 0 && next < total) issue(next, (it + 1) & 1);
-        });
-        PMX_T_MARK(4)
-#endif
-        {
-            cpx* base = reinterpret_cast<cpx*>(p.field) + ((size_t)bc * N + (size_t)(row0 + rl) * L) * 2;
-#pragma unroll
-            for (int q = 0; q < 8; ++q) {
-                x[q] = mkc(x[q].x * sc, x[q].y * nsc);
-                y[q] = mkc(y[q].x * sc, y[q].y * nsc);
-            }
-            pmx_nl_step(x, y, st, f, col);   // ---- N(-xi*gam): the gam of f is the backpropagated one
-#pragma unroll
-            for (int q = 0; q < 8; ++q) st_sa(base + (size_t)(t + q * T) * 2, x[q], y[q]);
-        }
-        PMX_T_MARK(5)
-        tile = next;
-        ++it;
-        __syncthreads();  // everyone is done with this tile's auxiliary buffer
-        PMX_T_MARK(6)
-    }
-    PMX_T_FLUSH(3)
+    PMX_T_FLUSH(NL ? 3 : 2)
 }

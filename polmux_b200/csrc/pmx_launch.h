@@ -16,8 +16,8 @@ struct PmxLaunchTable {
     int tw4_lo_bits, tw4_per;  // four-step twiddle row layout (PmxTw4<L>)
     int precision;             // 0 = FP64, 1 = FP32 (pmx_precision)
     int cpx_bytes;             // sizeof one complex number of that precision
-    // opt in to the dynamic shared memory, report resident CTAs per SM of each kernel
-    cudaError_t (*setup)(int* ctasA, int* ctasB, int* ctasC);
+    // opt in to the dynamic shared memory, report resident CTAs per SM of each kernel (ctasCnl: passC_nl)
+    cudaError_t (*setup)(int* ctasA, int* ctasB, int* ctasC, int* ctasCnl);
     // grid_x persistent CTAs
     // (every launcher returns the launch status)
     cudaError_t (*passA)(int grid_x, cudaStream_t s, const PassParams& p, const FiberConst& f, const CUtensorMap& cols);
@@ -33,9 +33,7 @@ struct PmxLaunchTable {
     size_t smemOnchip;
     cudaError_t (*onchip_setup)();
     cudaError_t (*onchip)(int nfc, int batch, cudaStream_t s, const PassParams& p, const FiberConst& f);
-    // digital backpropagation: pass C with the nonlinear step after the scale and no max reduction (pmx_k_passC_nl);
-    // the setup opts in to the shared memory and reports its resident CTAs per SM
-    cudaError_t (*passC_nl_setup)(int* ctas);
+    // digital backpropagation: pass C with the nonlinear step after the scale and no max reduction (pmx_k_passC<..., true>)
     cudaError_t (*passC_nl)(int grid_x, cudaStream_t s, const PassParams& p, const FiberConst& f, const CUtensorMap& cols);
 };
 

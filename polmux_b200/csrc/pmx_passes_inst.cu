@@ -15,37 +15,21 @@ constexpr int L = PMX_L;
 // landing buffer + exchange buffer then fit three CTAs per SM with the next tile prefetched.  Longer
 // transforms land in the exchange buffer itself (no separate prefetch).
 constexpr int PSCALE = 32 / PMX_SA_BYTES;  // 1 (FP64) or 2 (FP32)
-#ifndef PMX_GAC
 constexpr int GAC = PSCALE * ((L >= 1024) ? 1 : (L == 512 ? 2 : 4));
-#else
-constexpr int GAC = PMX_GAC;
-#endif
-#ifdef PMX_GB
-constexpr int GB = PMX_GB;
-#else
 constexpr int GB = (PSCALE * ((L >= 1024) ? 1 : (L == 512 ? 2 : 4)) * (L / 8) > 1024) ? 1 : PSCALE * ((L >= 1024) ? 1 : (L == 512 ? 2 : 4));
-#endif
 constexpr int TILE_CAP = 32 * 1024;
-#ifndef PMX_PFAC
 // Since passes A and C read and write contiguous rows straight from / to registers they no longer stage a
 // tile for a TMA store, and a fourth resident CTA (the tile lands in the exchange buffer, 42 KB per CTA) beats a
 // separate prefetch buffer with three (measured 49.0 against 50.3 ps per Sa and step at N = 2^20).
 constexpr bool PFAC = false;
-#else
-constexpr bool PFAC = (PMX_PFAC != 0) && (GAC * L * PMX_SA_BYTES <= TILE_CAP);
-#endif
-#ifndef PMX_PFB
 // pass B is compute-bound: it prefers a fourth resident CTA to a separate prefetch buffer
 constexpr bool PFB = (GB * L * PMX_SA_BYTES <= TILE_CAP / 2);
-#else
-constexpr bool PFB = (PMX_PFB != 0) && (GB * L * PMX_SA_BYTES <= TILE_CAP);
-#endif
 static_assert(GAC * (L / 8) <= 1024 && GB * (L / 8) <= 1024, "CTA too large");
 using SA = PassSmem<L, GAC, PFAC, 0>;
 using SB = PassSmem<L, GB, PFB, 1>;
 using SC = PassSmem<L, GAC, PFAC, 2>;
 
-cudaError_t setup(int* ctasA, int* ctasB, int* ctasC) {
+cudaError_t setup(int* ctasA, int* ctasB, int* ctasC, int* ctasCnl) {
     cudaError_t e;
     auto prep = [](auto kern, int smem, int threads, int* ctas) -> cudaError_t {
         cudaError_t r = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
@@ -64,7 +48,9 @@ cudaError_t setup(int* ctasA, int* ctasB, int* ctasC) {
     if (e != cudaSuccess) return e;
     e = prep(pmx_k_passB<real, L, GB, PFB, true>, SB::TOTAL, SB::THREADS, ctasB);
     if (e != cudaSuccess) return e;
-    return prep(pmx_k_passC<real, L, GAC, PFAC>, SC::TOTAL, SC::THREADS, ctasC);
+    e = prep(pmx_k_passC<real, L, GAC, PFAC, false>, SC::TOTAL, SC::THREADS, ctasC);
+    if (e != cudaSuccess) return e;
+    return prep(pmx_k_passC<real, L, GAC, PFAC, true>, SC::TOTAL, SC::THREADS, ctasCnl);
 }
 // p.pdl: launch with programmatic stream serialization (the kernel's prologue then overlaps the previous kernel's tail)
 template <typename K>
@@ -92,16 +78,10 @@ cudaError_t passB(int gx, cudaStream_t s, const PassParams& p, const FiberConst&
     return launch(pmx_k_passB<real, L, GB, PFB, false>, gx, SB::THREADS, SB::TOTAL, s, p, f, m);
 }
 cudaError_t passC(int gx, cudaStream_t s, const PassParams& p, const FiberConst& f, const CUtensorMap& m) {
-    return launch(pmx_k_passC<real, L, GAC, PFAC>, gx, SC::THREADS, SC::TOTAL, s, p, f, m);
-}
-cudaError_t passC_nl_setup(int* ctas) {
-    cudaError_t e = cudaFuncSetAttribute(pmx_k_passC_nl<real, L, GAC, PFAC>, cudaFuncAttributeMaxDynamicSharedMemorySize, SC::TOTAL);
-    if (e != cudaSuccess) return e;
-    cudaFuncSetAttribute(pmx_k_passC_nl<real, L, GAC, PFAC>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas, pmx_k_passC_nl<real, L, GAC, PFAC>, SC::THREADS, SC::TOTAL);
+    return launch(pmx_k_passC<real, L, GAC, PFAC, false>, gx, SC::THREADS, SC::TOTAL, s, p, f, m);
 }
 cudaError_t passC_nl(int gx, cudaStream_t s, const PassParams& p, const FiberConst& f, const CUtensorMap& m) {
-    return launch(pmx_k_passC_nl<real, L, GAC, PFAC>, gx, SC::THREADS, SC::TOTAL, s, p, f, m);
+    return launch(pmx_k_passC<real, L, GAC, PFAC, true>, gx, SC::THREADS, SC::TOTAL, s, p, f, m);
 }
 // precision-dependent helpers that do not depend on L (every table carries them)
 void init_max(dim3 grid, cudaStream_t s, const PassParams& p, const FiberConst& f) {
@@ -150,5 +130,4 @@ cudaError_t onchip(int nfc, int batch, cudaStream_t s, const PassParams& p, cons
 extern const PmxLaunchTable PMX_TABLE_NAME = {
     L, GAC, GB, PFAC ? 1 : 0, PFB ? 1 : 0, SA::THREADS, SB::THREADS, (size_t)SA::TOTAL, (size_t)SB::TOTAL,
     pmx_tw_total(L), pmx_tw_layout(L), PmxTw4<L>::LO, PmxTw4<L>::PER, PMX_PRECISION, (int)sizeof(cpx),
-    setup, passA, passB, passC, init_max, fill_tw4, xpm_sum, (size_t)SO::TOTAL, onchip_setup, onchip, passC_nl_setup,
-    passC_nl};
+    setup, passA, passB, passC, init_max, fill_tw4, xpm_sum, (size_t)SO::TOTAL, onchip_setup, onchip, passC_nl};

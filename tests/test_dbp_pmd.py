@@ -276,6 +276,20 @@ def test_dbp_pmd_matches_the_oracle_fp32(ctx):
 
 
 @pytest.mark.gpu
+def test_dbp_pmd_vector_dispersion_mode_matches_the_oracle(ctx):
+    """betat and db1 uploaded per bin (disp_mode='vector'): pass B of every step reads the plan's negated db1 table"""
+    gs, s = _setup(256, 16, manakov=True)
+    brfs = _brfs(s, 2)
+    g = 10 ** (GAIN_DB / 10)
+    gx, gy = _run_device(ctx, s, _cols(gs.FIELDX), _cols(gs.FIELDY), _plates(brfs), nspan=2, gain_db=GAIN_DB,
+                         steps_per_span=5, disp_mode='vector')
+    wx, wy = _oracle(gs.FIELDX, gs.FIELDY, s, [r[0] for r in brfs], nspan=2, gain=g, steps_per_span=5)
+    err = rel_l2(gx[0].T, gy[0].T, wx, wy)
+    print('dbp pmd parity, vector dispersion mode: rel_l2 %.3e' % err)
+    assert err <= 1e-10
+
+
+@pytest.mark.gpu
 @pytest.mark.parametrize('case', ['c1', 'c2_span'])
 def test_dbp_pmd_inverts_fiber_on_the_device(case):
     """pmx.fiber(fib, 'gps-', trace=True) then pmx.dbp(fib, 'gps-', step_len=trace_dz, brf=brf): the Tx field back.
