@@ -250,9 +250,11 @@ int pmx_link_run(pmx_ctx* ctx, const pmx_fiber_desc* desc, const pmx_link_desc* 
  *     u <- ifft( fft(u) .* exp(+i*betat*h) )                     per column
  *     u <- N(-xi*gam, h) u                                       matrix_nl_step (fiber.m:827-851) with gam -> -xi*gam and
  *                                                                the forward leff(h) = (1 - exp(-alpha*h))/alpha
+ *     (scalar path, scalar_field = 1: nl_step (fiber.m:786-803) with gam -> -xi*gam; with the 'x' flag its power is
+ *      that of the cross-phase modulation over the sum of |u_j|^2 of all backpropagated columns j, taken after the scale)
  * With xi = 1 and the forward run's own steps (pmx_fiber_result.trace_dz), DBP inverts a noise-free fiber without PMD up
- * to rounding.  With pmd = 0, DBP ignores the 'p' flag, the plates and dgdrms; the 'x' flag fails with
- * PMX_ERR_XPM_VECTOR as in fiber.
+ * to rounding, on the scalar path with the 'x' flag as well.  With pmd = 0, DBP ignores the 'p' flag, the plates and
+ * dgdrms; the 'x' flag on a two-polarization field fails with PMX_ERR_XPM_VECTOR as in fiber.
  * PMD-aware DBP (pmd = 1, the fiber's 'p' flag, plates from pmx_dbp_set_plates): the linear operator of a step is the
  * inverse of the forward step's trunk product (matrix_step, fiber.m:904-935): the same trunk pieces in reverse order,
  * the plates last to first, db0, db1 (dgdrms) and betat negated, from and back to the laboratory basis.  The trunk
@@ -260,9 +262,13 @@ int pmx_link_run(pmx_ctx* ctx, const pmx_fiber_desc* desc, const pmx_link_desc* 
  * zprop accumulated step by step and the last step ending at the fiber length, so that trace_dz reproduces the forward
  * run's partition exactly.  Steps that would index past the last plate fail with PMX_ERR_PLATE_INDEX as fiber would.
  * With xi = 1 and trace_dz, PMD-aware DBP inverts a noise-free 'gps-' link up to rounding.
- * Two-polarization fields (scalar_field = 0), nfc <= 64, nfft from 2^12 to 2^24, FP64 or FP32; other fields fail with
- * PMX_ERR_UNSUPPORTED.  Every step is the three HBM passes of a forward step; the step packages of the whole schedule
- * are built when the plan is created, so pmx_dbp_exec enqueues every step without reading anything back. */
+ * Sizes, FP64 or FP32 (PMX_ERR_UNSUPPORTED otherwise, checked before a context is needed):
+ *   two-polarization fields, nfft from 2^12 to 2^24, nfc <= 64: every step is the three HBM passes of a forward step;
+ *   two-polarization fields, nfft from 2^6 to 2^11, and the scalar path, nfft from 2^6 to 2^12 (flags 's' and / or 'x'),
+ *   nfc <= 8: the whole link in one launch of the single-launch kernel of small fields, one CTA per column and the
+ *   columns of a realization in one thread-block cluster (PMX_NO_ONCHIP does not apply: these fields have no other route).
+ * The step packages of the whole schedule are built when the plan is created, so pmx_dbp_exec runs every step without
+ * reading anything back. */
 typedef struct pmx_dbp_desc {
     int32_t nspan;
     int32_t steps_per_span;    /* > 0: uniform steps of length/steps_per_span; 0: the explicit schedule below           */

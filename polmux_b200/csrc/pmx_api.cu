@@ -243,6 +243,9 @@ struct pmx_plan {
     int dbp_nspan = 0;
     DbpGeo* geo_d = nullptr;
     std::vector<int> sched_span;
+    // DBP of a small field (onchip): sched_idx and sched_span on the device, the on-chip kernel's step table
+    int* sched_idx_d = nullptr;
+    int* sched_span_d = nullptr;
 };
 
 static int set_err(pmx_ctx* ctx, int code, const char* fmt, ...) {
@@ -751,11 +754,16 @@ extern "C" void pmx_plan_destroy(pmx_plan* p) {
     if (p->trace_ntrunk) cudaFreeAsync(p->trace_ntrunk, st);
     if (p->sched) cudaFreeAsync(p->sched, st);
     if (p->geo_d) cudaFreeAsync(p->geo_d, st);
+    if (p->sched_idx_d) cudaFreeAsync(p->sched_idx_d, st);
+    if (p->sched_span_d) cudaFreeAsync(p->sched_span_d, st);
     delete p;
 }
 
-// passes_only: 2^12 fields run on the three passes instead of the single-launch kernel (digital backpropagation)
-static int plan_create(pmx_ctx* c, const pmx_fiber_desc* d, pmx_plan** out, bool passes_only) {
+// Which kernels a plan runs.  PLAN_AUTO: the single-launch kernel up to 2^12 samples and 8 columns (PMX_NO_ONCHIP=1 sends
+// 2^12 through the three passes), the passes above.  Digital backpropagation fixes the route itself: PLAN_PASSES for
+// two-polarization fields of 2^12 samples and more, PLAN_ONCHIP for everything smaller and for the scalar path.
+enum PlanRoute { PLAN_AUTO, PLAN_PASSES, PLAN_ONCHIP };
+static int plan_create(pmx_ctx* c, const pmx_fiber_desc* d, pmx_plan** out, PlanRoute route) {
     if (!c || !d || !out) return set_err(c, PMX_ERR_INVALID, "pmx_plan_create: null argument");
     *out = nullptr;
     if (d->precision != PMX_F64 && d->precision != PMX_F32)
@@ -767,7 +775,7 @@ static int plan_create(pmx_ctx* c, const pmx_fiber_desc* d, pmx_plan** out, bool
     // Fields of up to 4096 samples run in the single-launch on-chip kernel (one CTA per column, the columns of a
     // realization in one thread-block cluster): at most 8 columns.  PMX_NO_ONCHIP=1 sends 2^12 through the three passes.
     const bool no_onchip = getenv("PMX_NO_ONCHIP") && atoi(getenv("PMX_NO_ONCHIP"));
-    const bool onchip = lg <= 12 && d->nfc <= 8 && !(no_onchip && lg == 12) && !passes_only;
+    const bool onchip = lg <= 12 && d->nfc <= 8 && route != PLAN_PASSES && !(no_onchip && lg == 12 && route == PLAN_AUTO);
     if (lg < 12 && !onchip)
         return set_err(c, PMX_ERR_UNSUPPORTED, "nfft=%lld (< 2^12) with nfc=%d: small fields take at most 8 columns",
                        (long long)d->nfft, d->nfc);
@@ -948,7 +956,7 @@ static int plan_create(pmx_ctx* c, const pmx_fiber_desc* d, pmx_plan** out, bool
     return PMX_OK;
 }
 
-extern "C" int pmx_plan_create(pmx_ctx* c, const pmx_fiber_desc* d, pmx_plan** out) { return plan_create(c, d, out, false); }
+extern "C" int pmx_plan_create(pmx_ctx* c, const pmx_fiber_desc* d, pmx_plan** out) { return plan_create(c, d, out, PLAN_AUTO); }
 
 // ---------------------------------------------------------------------------
 // A linear filter as a plan: one step of a fiber without dispersion, birefringence, nonlinearity or loss whose per-bin
@@ -3502,17 +3510,46 @@ extern "C" int pmx_dbp_set_plates(pmx_plan* p, int32_t sets, const double* db0, 
     return PMX_OK;
 }
 
+// An on-chip DBP plan walks its step table on the device: the package index of every step and, PMD-aware, its span.
+static int dbp_upload_steps(pmx_plan* p) {
+    if (!p->onchip) return PMX_OK;
+    pmx_ctx* c = p->ctx;
+    const size_t n = p->sched_idx.size();
+    cudaError_t err = cudaMallocAsync(&p->sched_idx_d, n * sizeof(int), c->stream);
+    if (err == cudaSuccess)
+        err = cudaMemcpyAsync(p->sched_idx_d, p->sched_idx.data(), n * sizeof(int), cudaMemcpyHostToDevice, c->stream);
+    if (err == cudaSuccess && p->dbp_pmd) {
+        err = cudaMallocAsync(&p->sched_span_d, n * sizeof(int), c->stream);
+        if (err == cudaSuccess)
+            err = cudaMemcpyAsync(p->sched_span_d, p->sched_span.data(), n * sizeof(int), cudaMemcpyHostToDevice, c->stream);
+    }
+    if (err == cudaSuccess) err = cudaStreamSynchronize(c->stream);
+    if (err != cudaSuccess) return set_err(c, PMX_ERR_CUDA, "pmx_dbp_create: step index table: %s", cudaGetErrorString(err));
+    return PMX_OK;
+}
+
 extern "C" int pmx_dbp_create(pmx_ctx* c, const pmx_fiber_desc* fd, const pmx_dbp_desc* g, pmx_plan** out) {
     // (the descriptors are checked before the context, so that the checks run without a device)
     if (!fd || !g || !out) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: null argument");
     *out = nullptr;
-    if (fd->scalar_field)
-        return set_err(c, PMX_ERR_UNSUPPORTED, "digital backpropagation is built for two-polarization fields, not the scalar path");
-    if (fd->fls[3]) return set_err(c, PMX_ERR_XPM_VECTOR, "The CNLSE with separate fields is not yet implemented");
+    // The route follows from the field: the scalar path and fields below 2^12 samples run the whole link in one launch of
+    // the on-chip kernel (one CTA per column, the columns of a realization in one cluster: at most 8), two-polarization
+    // fields of 2^12 samples and more the three passes of every step.
+    const bool scalar = fd->scalar_field != 0;
+    if (fd->fls[3] && !scalar) return set_err(c, PMX_ERR_XPM_VECTOR, "The CNLSE with separate fields is not yet implemented");
     const int lg = ilog2_exact(fd->nfft);
-    if (lg < 12 || lg > 24)
-        return set_err(c, PMX_ERR_UNSUPPORTED, "digital backpropagation: nfft=%lld, built for powers of two from 2^12 to 2^24",
+    if (scalar && (lg < 6 || lg > 12))
+        return set_err(c, PMX_ERR_UNSUPPORTED,
+                       "digital backpropagation on the scalar path: nfft=%lld, built for powers of two from 2^6 to 2^12",
                        (long long)fd->nfft);
+    if (lg < 6 || lg > 24)
+        return set_err(c, PMX_ERR_UNSUPPORTED, "digital backpropagation: nfft=%lld, built for powers of two from 2^6 to 2^24",
+                       (long long)fd->nfft);
+    const bool onchip = scalar || lg < 12;
+    if (onchip && (fd->nfc < 1 || fd->nfc > 8))
+        return set_err(c, PMX_ERR_UNSUPPORTED,
+                       "digital backpropagation %s: nfc=%d, built for 1 to 8 columns (the columns of a realization form one "
+                       "thread-block cluster)", scalar ? "on the scalar path" : "below 2^12 samples", fd->nfc);
     if (g->nspan < 1) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: nspan must be >= 1");
     if (!std::isfinite(g->xi)) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: xi must be finite");
     if (!(g->gain >= 0) || !std::isfinite(g->gain)) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_create: gain must be >= 0 (0: none)");
@@ -3597,7 +3634,7 @@ extern "C" int pmx_dbp_create(pmx_ctx* c, const pmx_fiber_desc* fd, const pmx_db
         e.betat = nbt.data();
     }
     pmx_plan* p = nullptr;
-    int rc = plan_create(c, &e, &p, true);
+    int rc = plan_create(c, &e, &p, onchip ? PLAN_ONCHIP : PLAN_PASSES);
     if (rc) return rc;
     p->dbp = true;
     p->fc_a = p->fc;
@@ -3621,6 +3658,11 @@ extern "C" int pmx_dbp_create(pmx_ctx* c, const pmx_fiber_desc* fd, const pmx_db
         for (size_t s = 0; s < geo.size(); ++s) {
             p->sched_idx.push_back((int)s);
             p->sched_span.push_back(geo[s].span);
+        }
+        rc = dbp_upload_steps(p);
+        if (rc) {
+            pmx_plan_destroy(p);
+            return rc;
         }
         *out = p;
         return PMX_OK;
@@ -3667,6 +3709,11 @@ extern "C" int pmx_dbp_create(pmx_ctx* c, const pmx_fiber_desc* fd, const pmx_db
         pmx_plan_destroy(p);
         return set_err(c, PMX_ERR_CUDA, "pmx_dbp_create: step table: %s", cudaGetErrorString(err));
     }
+    rc = dbp_upload_steps(p);
+    if (rc) {
+        pmx_plan_destroy(p);
+        return rc;
+    }
     *out = p;
     return PMX_OK;
 }
@@ -3684,6 +3731,26 @@ extern "C" int pmx_dbp_exec(pmx_plan* p, pmx_devfield* fld) {
     PassParams pa, pA, pB;
     rc = pass_params(p, fld, pa, pA, pB);
     if (rc) return rc;
+    if (p->onchip) {   // small field or scalar path: the whole link of every realization in one launch
+        PassParams q = pa;
+        rc = get_stage_tw(c, p->tB, &q.tw_stage);
+        if (rc) return rc;
+        q.N1 = 1;
+        q.N2 = (int)p->d.nfft;
+        q.log2N1 = fld->log2N1;   // layout of the resident column (transposed for 2^12, natural below)
+        q.log2N2 = fld->log2N2;
+        DbpSteps ds;
+        ds.pkg = p->sched;
+        ds.idx = p->sched_idx_d;
+        ds.span = p->dbp_pmd ? p->sched_span_d : nullptr;
+        ds.nstep = (int)p->sched_idx.size();
+        ds.pkg_bytes = p->dbp_pmd ? (int)sizeof(StepPkg) : PMX_PKG_HEAD;   // without PMD no step reads past the header
+        ds.plate_stride = (long long)p->fc.plate_sets * p->fc.nplates;
+        CK(c, p->tB->onchip_dbp(p->d.nfc, batch, c->stream, q, p->fc_c, ds));
+        c->launches += 1;
+        CK(c, cudaStreamSynchronize(c->stream));
+        return PMX_OK;
+    }
     // realization groups and dependent launches as in pmx_fiber_exec; pass C' has an occupancy of its own
     PassGroups gs;
     rc = plan_groups(p, fld, pa, pA, pB, c->setup_done[p->N1 + 65536 * p->d.precision].cnl, true, gs);

@@ -162,6 +162,18 @@ struct PassParams {
     long long* dbg;         // optional per-CTA phase cycle counters (PMX_TIMING builds only)
 };
 
+// The fixed schedule of a digital-backpropagation plan for the single-launch kernel of small fields (pmx_k_onchip with
+// DBP = true, its third argument): step s runs package pkg[idx[s]][b]; a PMD-aware plan reads the plates of span span[s],
+// at plates + span[s] * plate_stride.
+struct DbpSteps {
+    const StepPkg* pkg;     // [npkg][batch]
+    const int* idx;         // [nstep]
+    const int* span;        // [nstep], or null without PMD
+    int nstep;
+    int pkg_bytes;          // bytes of a package the steps read: the header alone without PMD, all of it with
+    long long plate_stride; // PlateConst per span: plate_sets * nplates
+};
+
 __device__ __forceinline__ cpx cmul(cpx a, cpx b) { return mkc(a.x * b.x - a.y * b.y, a.x * b.y + a.y * b.x); }
 __device__ __forceinline__ cpx cmulc(cpx a, cpx b) {  // a * conj(b)
     return mkc(a.x * b.x + a.y * b.y, a.y * b.x - a.x * b.y);

@@ -35,6 +35,9 @@ struct PmxLaunchTable {
     cudaError_t (*onchip)(int nfc, int batch, cudaStream_t s, const PassParams& p, const FiberConst& f);
     // digital backpropagation: pass C with the nonlinear step after the scale and no max reduction (pmx_k_passC<..., true>)
     cudaError_t (*passC_nl)(int grid_x, cudaStream_t s, const PassParams& p, const FiberConst& f, const CUtensorMap& cols);
+    // digital backpropagation of a small field: the on-chip kernel walking the plan's step table (pmx_k_onchip<..., true>),
+    // launched like onchip (set up by onchip_setup)
+    cudaError_t (*onchip_dbp)(int nfc, int batch, cudaStream_t s, const PassParams& p, const FiberConst& f, const DbpSteps& ds);
 };
 
 const PmxLaunchTable* pmx_get_table(int L, int precision = 0);  // nullptr if L is not built

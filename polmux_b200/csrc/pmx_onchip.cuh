@@ -9,6 +9,13 @@
 // fiber.m:793-799): the nfc CTAs of a realization form a THREAD-BLOCK CLUSTER and read each other's maxima / powers
 // through distributed shared memory; every CTA runs the (deterministic) scalar step control redundantly, so no
 // broadcast is needed and all CTAs leave the loop in the same iteration.
+//
+// Digital backpropagation (DBP = true, pmx_dbp_exec on fields of up to 4096 samples): the same kernel walks the plan's
+// fixed step table (DbpSteps) instead of running the step control.  A step is the forward transform, the linear step of
+// the package (dispersion negated; for a PMD-aware plan the inverse trunk product), the inverse transform, the scale
+// exp(+alpha*h/2)/N (times 1/sqrt(G) on the first step of a span), on the scalar path with 'x' the cluster-wide
+// sum_j |u_j|^2, and the nonlinear step with gam -> -xi*gam: pass A, B and C' of a DBP step on the three-pass route.
+// No max reduction, no step control, no StepCtl write-back; the next step's package is fetched while this step runs.
 #pragma once
 #include <cooperative_groups.h>
 #include "pmx_kernels.cuh"
@@ -52,8 +59,10 @@ __device__ __forceinline__ unsigned long long pmx_block_max_t0(unsigned long lon
     return m;
 }
 
-template <typename R, int L, bool SC>
-__global__ void __launch_bounds__((L / 8) < 32 ? 32 : (L / 8), 1) pmx_k_onchip(PassParams p, FiberConst f) {
+// The DBP instances take the step table as a third argument (Steps = DbpSteps); the forward instances keep their two.
+template <typename R, int L, bool SC, bool DBP = false, typename... Steps>
+__global__ void __launch_bounds__((L / 8) < 32 ? 32 : (L / 8), 1) pmx_k_onchip(PassParams p, FiberConst f, Steps... steps) {
+    static_assert(sizeof...(Steps) == (DBP ? 1 : 0), "the DBP instances take one DbpSteps, the forward ones nothing");
     using S = OnchipSmem<L>;
     constexpr int T = L / 8;
     constexpr bool PRE = SC;
@@ -78,95 +87,158 @@ __global__ void __launch_bounds__((L / 8) < 32 ? 32 : (L / 8), 1) pmx_k_onchip(P
     PMX_ASSERT(col < f.nfc && b < p.batch && mem(L - 1) < N && (int)blockDim.x >= T && (int)gridDim.x == f.nfc);
 
     pmx_load_stage_tw<L>(stw, p.tw_stage);
-    for (int i = t; i < (int)(sizeof(StepCtl) / 4); i += blockDim.x) reinterpret_cast<int*>(c)[i] = 0;
     cpx x[8], y[8];
-    unsigned long long vmax = 0ull;
+    // ---- scalar path with the 'x' flag: sum over the columns of |u|^2 per sample, left to right (fiber.m:793-799), into y
+    auto xpm_sum = [&]() {
+        real* pw = reinterpret_cast<real*>(work);
+        if (live) {
 #pragma unroll
-    for (int q = 0; q < 8; ++q) {
-        ld_sa(fld + 2 * mem(tt + q * T), x[q], y[q]);
-        const unsigned long long key = pmx_pow_key((double)power_ref(x[q], y[q]));
-        if (live) vmax = key > vmax ? key : vmax;
-    }
-    __syncthreads();
-    int first = 1, parity = 0;
-    // a thread's bins after the full-length transform: k = t + q*T, q < 4 positive frequencies, q >= 4 negative
-    const double dfn = (double)T * f.inv_nsymb;
-    const double fn0 = (double)tt * f.inv_nsymb;
-    const double fn4 = (double)(tt + 4 * T - L) * f.inv_nsymb;
-    for (;;) {
-        // ---- max |u|^2 of every column of the realization (nextstep, fiber.m:693-698)
-        const unsigned long long m = pmx_block_max_t0(vmax, sred);
-        if (f.nfc > 1) {
-            if (t == 0) xch[parity] = m;
-            cluster.sync();
-            if (t < f.nfc) c->umax_bits[t] = *cluster.map_shared_rank(&xch[parity], t);
-            parity ^= 1;
-        } else if (t == 0) {
-            c->umax_bits[0] = m;
+            for (int q = 0; q < 8; ++q) pw[t + q * T] = R_ADD(R_MUL(x[q].x, x[q].x), R_MUL(x[q].y, x[q].y));
         }
-        __syncthreads();
-        // ---- nextstep + checkstep + step package (all CTAs of the cluster compute the same schedule)
-        const bool go = pmx_ctl_step(c, st, p, f, first, b, s_go);
-        __syncthreads();
-        if (!go) break;
-        first = 0;
-        const int ntrunk = st->ntrunk;
-        const bool any_full = (ntrunk > 2) || (st->dzb_first == f.lcorr) || (st->dzb_last == f.lcorr);
-        if constexpr (PRE) {
-            if (ntrunk > 0) pmx_b_pre(scr, T, st, f, col, fn4, fn0, any_full);
+        cluster.sync();
+        real sum[8];
+#pragma unroll
+        for (int q = 0; q < 8; ++q) sum[q] = (real)0;
+        for (int k = 0; k < f.nfc; ++k) {
+            const real* rp = cluster.map_shared_rank(pw, k);
+#pragma unroll
+            for (int q = 0; q < 8; ++q) sum[q] = R_ADD(sum[q], rp[tt + q * T]);
         }
-        // ---- scalar path with the 'x' flag: sum over the columns of |u|^2 per sample, left to right (fiber.m:793-799)
-        if (f.xpm) {
-            real* pw = reinterpret_cast<real*>(work);
-            if (live) {
 #pragma unroll
-                for (int q = 0; q < 8; ++q) pw[t + q * T] = R_ADD(R_MUL(x[q].x, x[q].x), R_MUL(x[q].y, x[q].y));
-            }
-            cluster.sync();
-            real sum[8];
-#pragma unroll
-            for (int q = 0; q < 8; ++q) sum[q] = (real)0;
-            for (int k = 0; k < f.nfc; ++k) {
-                const real* rp = cluster.map_shared_rank(pw, k);
-#pragma unroll
-                for (int q = 0; q < 8; ++q) sum[q] = R_ADD(sum[q], rp[tt + q * T]);
-            }
-#pragma unroll
-            for (int q = 0; q < 8; ++q) y[q] = mkc(sum[q], (real)0);
-            cluster.sync();   // everybody has read this CTA's powers: the buffer goes back to the transforms
-        }
-        pmx_nl_step(x, y, st, f, col);
-        // ---- linear step: full-length transform, the step's trunks, inverse transform (= conj o forward o conj)
+        for (int q = 0; q < 8; ++q) y[q] = mkc(sum[q], (real)0);
+        cluster.sync();   // everybody has read this CTA's powers: the buffer goes back to the transforms
+    };
+    // ---- linear step: full-length transform, the step's trunks, inverse transform (= conj o forward o conj)
+    auto linear_step = [&](const PassParams& pp, int ntrunk, bool any_full, double fn0, double fn4, double dfn) {
 #pragma unroll 1
         for (int dir = 0; dir < 2; ++dir) {
             CtaFFT<R, L>::run(x, y, work, work + L, tt, stw);
             if (dir == 1) break;
             if (ntrunk > 0)
-                pmx_linear_bins<SC, PRE>(x, y, st, f, p, scr, T, schunk, b, col, 0, tt, T, N, fn0, fn4, dfn, any_full);
+                pmx_linear_bins<SC, PRE>(x, y, st, f, pp, scr, T, schunk, b, col, 0, tt, T, N, fn0, fn4, dfn, any_full);
 #pragma unroll
             for (int q = 0; q < 8; ++q) {
                 x[q] = cconj(x[q]);
                 y[q] = cconj(y[q]);
             }
         }
-        // ---- 1/N and attenuation exp(-alpha/2*dz) (fiber.m:531-532), running max for the next step
-        const real sc = (real)st->scale, nsc = -sc;
-        vmax = 0ull;
+    };
+    if constexpr (DBP) {
+        const DbpSteps ds{steps...};
+        // a thread's bins after the full-length transform: k = t + q*T, q < 4 positive frequencies, q >= 4 negative
+        const double dfn = (double)T * f.inv_nsymb;
+        const double fn0 = (double)tt * f.inv_nsymb;
+        const double fn4 = (double)(tt + 4 * T - L) * f.inv_nsymb;
+        // the package of step s: every thread fetches its 16-byte words into registers (issued a step ahead, landed in
+        // shared memory between two steps)
+        constexpr int NTH = (L / 8) < 32 ? 32 : (L / 8);
+        constexpr int PW = ((int)(sizeof(StepPkg) / 16) + NTH - 1) / NTH;
+        const int nw = ds.pkg_bytes / 16;
+        uint4 nxt[PW];
+        const PlateConst* nxt_pl = p.plates;
+        auto fetch = [&](int s) {
+            const uint4* src = reinterpret_cast<const uint4*>(ds.pkg + (size_t)__ldg(&ds.idx[s]) * p.batch + b);
+#pragma unroll
+            for (int i = 0; i < PW; ++i)
+                if (t + i * NTH < nw) nxt[i] = __ldg(&src[t + i * NTH]);
+            if (ds.span) nxt_pl = p.plates + (size_t)__ldg(&ds.span[s]) * ds.plate_stride;
+        };
+        auto land = [&]() {
+#pragma unroll
+            for (int i = 0; i < PW; ++i)
+                if (t + i * NTH < nw) reinterpret_cast<uint4*>(st)[t + i * NTH] = nxt[i];
+        };
+        PMX_ASSERT(ds.nstep >= 1 && (ds.pkg_bytes == PMX_PKG_HEAD || ds.pkg_bytes == (int)sizeof(StepPkg)));
+#pragma unroll
+        for (int q = 0; q < 8; ++q) ld_sa(fld + 2 * mem(tt + q * T), x[q], y[q]);
+        fetch(0);
+        land();
+        __syncthreads();
+        PassParams ps = p;   // the step's plate table: its span's (PMD-aware plans)
+        for (int s = 0; s < ds.nstep; ++s) {
+            ps.plates = nxt_pl;
+            if (s + 1 < ds.nstep) fetch(s + 1);
+            const int ntrunk = st->ntrunk;
+            const bool any_full = (ntrunk > 2) || (st->dzb_first == f.lcorr) || (st->dzb_last == f.lcorr);
+            if constexpr (PRE) {
+                if (ntrunk > 0) pmx_b_pre(scr, T, st, f, col, fn4, fn0, any_full);
+            }
+            linear_step(ps, ntrunk, any_full, fn0, fn4, dfn);   // ---- L(-h): dispersion negated, the package's trunks
+            // ---- 1/N and the loss exp(+alpha/2*h), 1/sqrt(G) on the first step of a span
+            const real sc = (real)st->scale, nsc = -sc;
+#pragma unroll
+            for (int q = 0; q < 8; ++q) {
+                x[q] = mkc(x[q].x * sc, x[q].y * nsc);
+                y[q] = mkc(y[q].x * sc, y[q].y * nsc);
+            }
+            if (f.xpm) xpm_sum();   // over the backpropagated columns (the transform has released the exchange buffer)
+            pmx_nl_step(x, y, st, f, col);   // ---- N(-xi*gam): the gam of f is the backpropagated one
+            __syncthreads();   // the package is read: the next one lands
+            if (s + 1 < ds.nstep) {
+                land();
+                __syncthreads();
+            }
+        }
+    } else {
+        for (int i = t; i < (int)(sizeof(StepCtl) / 4); i += blockDim.x) reinterpret_cast<int*>(c)[i] = 0;
+        unsigned long long vmax = 0ull;
 #pragma unroll
         for (int q = 0; q < 8; ++q) {
-            x[q] = mkc(x[q].x * sc, x[q].y * nsc);
-            y[q] = mkc(y[q].x * sc, y[q].y * nsc);
+            ld_sa(fld + 2 * mem(tt + q * T), x[q], y[q]);
             const unsigned long long key = pmx_pow_key((double)power_ref(x[q], y[q]));
             if (live) vmax = key > vmax ? key : vmax;
         }
-        __syncthreads();   // the package and the exchange buffer are rewritten by the next step
+        __syncthreads();
+        int first = 1, parity = 0;
+        const double dfn = (double)T * f.inv_nsymb;   // (the thread's bins, as above)
+        const double fn0 = (double)tt * f.inv_nsymb;
+        const double fn4 = (double)(tt + 4 * T - L) * f.inv_nsymb;
+        for (;;) {
+            // ---- max |u|^2 of every column of the realization (nextstep, fiber.m:693-698)
+            const unsigned long long m = pmx_block_max_t0(vmax, sred);
+            if (f.nfc > 1) {
+                if (t == 0) xch[parity] = m;
+                cluster.sync();
+                if (t < f.nfc) c->umax_bits[t] = *cluster.map_shared_rank(&xch[parity], t);
+                parity ^= 1;
+            } else if (t == 0) {
+                c->umax_bits[0] = m;
+            }
+            __syncthreads();
+            // ---- nextstep + checkstep + step package (all CTAs of the cluster compute the same schedule)
+            const bool go = pmx_ctl_step(c, st, p, f, first, b, s_go);
+            __syncthreads();
+            if (!go) break;
+            first = 0;
+            const int ntrunk = st->ntrunk;
+            const bool any_full = (ntrunk > 2) || (st->dzb_first == f.lcorr) || (st->dzb_last == f.lcorr);
+            if constexpr (PRE) {
+                if (ntrunk > 0) pmx_b_pre(scr, T, st, f, col, fn4, fn0, any_full);
+            }
+            if (f.xpm) xpm_sum();
+            pmx_nl_step(x, y, st, f, col);
+            linear_step(p, ntrunk, any_full, fn0, fn4, dfn);
+            // ---- 1/N and attenuation exp(-alpha/2*dz) (fiber.m:531-532), running max for the next step
+            const real sc = (real)st->scale, nsc = -sc;
+            vmax = 0ull;
+#pragma unroll
+            for (int q = 0; q < 8; ++q) {
+                x[q] = mkc(x[q].x * sc, x[q].y * nsc);
+                y[q] = mkc(y[q].x * sc, y[q].y * nsc);
+                const unsigned long long key = pmx_pow_key((double)power_ref(x[q], y[q]));
+                if (live) vmax = key > vmax ? key : vmax;
+            }
+            __syncthreads();   // the package and the exchange buffer are rewritten by the next step
+        }
     }
     if (live) {
 #pragma unroll
         for (int q = 0; q < 8; ++q) st_sa(fld + 2 * mem(t + q * T), x[q], y[q]);
     }
-    if (col == 0)
-        for (int i = t; i < (int)(sizeof(StepCtl) / 4); i += blockDim.x)
-            reinterpret_cast<int*>(&p.ctl[b])[i] = reinterpret_cast<const int*>(c)[i];
+    if constexpr (!DBP) {
+        if (col == 0)
+            for (int i = t; i < (int)(sizeof(StepCtl) / 4); i += blockDim.x)
+                reinterpret_cast<int*>(&p.ctl[b])[i] = reinterpret_cast<const int*>(c)[i];
+    }
     if (f.nfc > 1) cluster.sync();   // no CTA of the cluster exits while another may still read its shared memory
 }

@@ -100,9 +100,15 @@ constexpr int ONCHIP_THREADS = (L / 8) < 32 ? 32 : (L / 8);
 cudaError_t onchip_setup() {
     cudaError_t e = cudaFuncSetAttribute(pmx_k_onchip<real, L, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SO::TOTAL);
     if (e != cudaSuccess) return e;
-    return cudaFuncSetAttribute(pmx_k_onchip<real, L, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SO::TOTAL);
+    e = cudaFuncSetAttribute(pmx_k_onchip<real, L, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SO::TOTAL);
+    if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(pmx_k_onchip<real, L, true, true, DbpSteps>, cudaFuncAttributeMaxDynamicSharedMemorySize, SO::TOTAL);
+    if (e != cudaSuccess) return e;
+    return cudaFuncSetAttribute(pmx_k_onchip<real, L, false, true, DbpSteps>, cudaFuncAttributeMaxDynamicSharedMemorySize, SO::TOTAL);
 }
-cudaError_t onchip(int nfc, int batch, cudaStream_t s, const PassParams& p, const FiberConst& f) {
+// the forward run (no step table) or digital backpropagation (one DbpSteps)
+template <bool DBP, typename... Steps>
+cudaError_t onchip_launch(int nfc, int batch, cudaStream_t s, const PassParams& p, const FiberConst& f, const Steps&... steps) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(nfc, batch);
     cfg.blockDim = dim3(ONCHIP_THREADS);
@@ -115,8 +121,14 @@ cudaError_t onchip(int nfc, int batch, cudaStream_t s, const PassParams& p, cons
     at[0].val.clusterDim.z = 1;
     cfg.attrs = at;
     cfg.numAttrs = nfc > 1 ? 1 : 0;
-    if (f.disp_scalar) return cudaLaunchKernelEx(&cfg, pmx_k_onchip<real, L, true>, p, f);
-    return cudaLaunchKernelEx(&cfg, pmx_k_onchip<real, L, false>, p, f);
+    if (f.disp_scalar) return cudaLaunchKernelEx(&cfg, pmx_k_onchip<real, L, true, DBP, Steps...>, p, f, steps...);
+    return cudaLaunchKernelEx(&cfg, pmx_k_onchip<real, L, false, DBP, Steps...>, p, f, steps...);
+}
+cudaError_t onchip(int nfc, int batch, cudaStream_t s, const PassParams& p, const FiberConst& f) {
+    return onchip_launch<false>(nfc, batch, s, p, f);
+}
+cudaError_t onchip_dbp(int nfc, int batch, cudaStream_t s, const PassParams& p, const FiberConst& f, const DbpSteps& ds) {
+    return onchip_launch<true>(nfc, batch, s, p, f, ds);
 }
 }  // namespace
 
@@ -130,4 +142,4 @@ cudaError_t onchip(int nfc, int batch, cudaStream_t s, const PassParams& p, cons
 extern const PmxLaunchTable PMX_TABLE_NAME = {
     L, GAC, GB, PFAC ? 1 : 0, PFB ? 1 : 0, SA::THREADS, SB::THREADS, (size_t)SA::TOTAL, (size_t)SB::TOTAL,
     pmx_tw_total(L), pmx_tw_layout(L), PmxTw4<L>::LO, PmxTw4<L>::PER, PMX_PRECISION, (int)sizeof(cpx),
-    setup, passA, passB, passC, init_max, fill_tw4, xpm_sum, (size_t)SO::TOTAL, onchip_setup, onchip, passC_nl};
+    setup, passA, passB, passC, init_max, fill_tw4, xpm_sum, (size_t)SO::TOTAL, onchip_setup, onchip, passC_nl, onchip_dbp};

@@ -1,13 +1,18 @@
 """dbp(x, flag, ...): digital backpropagation of a link on the received field.
 
 An extension: the reference has no DBP.  The field is run back through a virtual copy of the link -- dispersion,
-nonlinearity and loss negated, spans last first, the amplifier gain undone before each span -- on the same three-pass
-kernels as fiber() (pmx_dbp_create / pmx_dbp_exec, include/polmux_ssfm.h).  With xi = 1 and the forward run's own
-steps (fiber(..., trace=True) leaves them in FIBER_LAST['trace_dz']) it inverts a noise-free link without PMD up to
-rounding; with fewer steps or xi < 1 it is the receiver-side nonlinear compensation a Monte-Carlo run can count errors
-behind (McRunner(compensation='dbp')).  Given the link's waveplates (dbp_plan(plates=...), dbp(brf=...)) it is PMD-aware:
-every step undoes the forward step's own trunk product as well, so that it inverts a 'gps-' link too
-(McRunner(compensation='dbp_pmd')).  There is no CPU fallback.
+nonlinearity and loss negated, spans last first, the amplifier gain undone before each span -- on the kernels fiber()
+uses for the same field (pmx_dbp_create / pmx_dbp_exec, include/polmux_ssfm.h): the three passes per step for
+two-polarization fields of 2^12 to 2^24 samples, the single-launch on-chip kernel (the whole link in one launch) for
+smaller fields and for the scalar path (FIELDY empty, 2^6 to 2^12 samples, at most 8 columns).  On the scalar path
+with the 'x' flag every step's nonlinear phase includes the cross-phase modulation of all backpropagated columns
+(nl_step with gam -> -xi*gam), so a 'sepfields' multiplex is backpropagated as a whole; without 'x' each column is
+backpropagated on its own self-phase alone.  With xi = 1 and the forward run's own steps (fiber(..., trace=True) leaves
+them in FIBER_LAST['trace_dz']) it inverts a noise-free link without PMD up to rounding; with fewer steps or xi < 1 it is
+the receiver-side nonlinear compensation a Monte-Carlo run can count errors behind (McRunner(compensation='dbp')).
+Given the link's waveplates (dbp_plan(plates=...), dbp(brf=...)) it is PMD-aware: every step undoes the forward step's
+own trunk product as well, so that it inverts a 'gps-' link too (McRunner(compensation='dbp_pmd')).  There is no CPU
+fallback.
 """
 from __future__ import annotations
 
@@ -50,7 +55,8 @@ def dbp_plan(ctx: _lib.Context, setup: FiberSetup, nspan: int = 1, gain_db: Opti
 def dbp(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, steps_per_span: Optional[int] = None, step_len=None,
         span_steps=None, xi: float = 1.0, ctx: Optional[_lib.Context] = None, precision: Optional[str] = None, brf=None):
     """Backpropagates GSTATE.FIELDX / FIELDY in place through nspan spans of the fiber x, the amplifier of gain_db [dB]
-    after each (None: no amplifier).  x and flag are what fiber() takes.  Without brf the flag's 'p' is dropped (no plates
+    after each (None: no amplifier).  x and flag are what fiber() takes; a field without FIELDY runs the scalar path, the
+    'x' flag there backpropagating the cross-phase modulation of all columns.  Without brf the flag's 'p' is dropped (no plates
     are drawn, nothing is taken from the global random stream) but the fiber's nonlinear model stays the one fiber() used:
     Manakov when x.manakov is 'yes' and the flag has 'p', else the CNLSE.  brf: the struct fiber() returned (every span
     the same plates) or a list of nspan of them in forward span order, with 'p' in the flag: PMD-aware DBP through those
@@ -76,14 +82,30 @@ def dbp(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, steps_per
                 raise ValueError('dbp: brf has %d plates, the fiber %d' % (np.asarray(b['theta']).size, s.nplates))
         plates = tuple(np.stack([np.asarray(b[k], dtype=np.float64).reshape(1, -1) for b in brfs])
                        for k in ('db0', 'theta', 'epsilon'))
-    if not (s.isv and G.has_y()):
-        raise NotImplementedError('dbp: two-polarization fields only (the scalar path has no DBP)')
-    if s.fls[3]:
+    if s.fls[3] and s.isv:
         raise NotImplementedError('The CNLSE with separate fields is not yet implemented')    # fiber.m:854
+    if s.isv and not G.has_y():                                  # the 'p' flag on a single-polarization field (:285-289)
+        G.FIELDY = np.zeros_like(G.FIELDX)
     s.manakov = f[1] == 'p' and str(_get(x, 'manakov', 'no')) == 'yes'
     ctx = ctx or _lib.default_context()
     from .fiber import PRECISION                                 # (the module default, read at call time)
     prec = {'f64': _lib.PMX_F64, 'f32': _lib.PMX_F32}[precision or PRECISION]
+    if not s.isv:
+        # scalar path: host buffers like the scalar fiber() -- upload, plan, execute, download into FIELDX
+        fx = np.ascontiguousarray(np.asarray(G.FIELDX, dtype=np.complex128).T)[None]     # [1][nfc][nfft]
+        fld = _lib.DeviceField(ctx, s.nfft, s.nfc, 1, precision=prec)
+        try:
+            fld.upload(fx, np.zeros_like(fx))
+            plan = dbp_plan(ctx, s, nspan, gain_db, steps_per_span, step_len, span_steps, xi, precision=precision)
+            try:
+                plan.execute(fld)
+            finally:
+                plan.close()
+            ux, _ = fld.download()
+        finally:
+            fld.close()
+        G.FIELDX = np.ascontiguousarray(ux[0].T)
+        return
     fld, hx, hy = G.take_device(ctx, prec)
     try:
         plan = dbp_plan(ctx, s, nspan, gain_db, steps_per_span, step_len, span_steps, xi, precision=precision, plates=plates)
