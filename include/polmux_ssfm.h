@@ -79,7 +79,7 @@ void* pmx_ctx_stream(pmx_ctx* ctx);
 typedef struct pmx_fiber_desc {
     int64_t nfft;        /* rows of FIELDX = NSYMB*NT (fiber.m:133); power of two, 2^6..2^24 */
     int32_t nfc;         /* columns of FIELDX (fiber.m:132): <= 64; <= 8 for nfft < 2^12 (on-chip: one cluster) */
-    int32_t batch;       /* independent realizations propagated by one call (>=1)            */
+    int32_t batch;       /* independent realizations propagated by one call (>=1); batch*nfc <= 65535 */
     int32_t precision;   /* pmx_precision                                                     */
     int32_t manakov;     /* strcmp(manakov,'yes')   fiber.m:499                               */
     double length;       /* Lf        fiber.m:459 */
@@ -150,6 +150,8 @@ typedef struct pmx_fiber_result {
 int pmx_fiber_run(pmx_ctx* ctx, const pmx_fiber_desc* desc, pmx_field* io, pmx_fiber_result* out);
 
 /* ---- HBM-resident API (span loops, Monte-Carlo batches, benchmarks) --------- */
+/* batch*nfc <= 65535 (the kernels put a field's realization-columns in one grid dimension); larger fields return
+ * PMX_ERR_UNSUPPORTED, as does a plan (pmx_plan_create, pmx_filter_create, pmx_dbp_create) with batch*nfc above it. */
 int pmx_field_create(pmx_ctx* ctx, int64_t nfft, int32_t nfc, int32_t batch, int32_t precision,
                      pmx_devfield** f);
 void pmx_field_destroy(pmx_devfield* f);

@@ -437,12 +437,24 @@ static int get_four_tw(pmx_ctx* c, long long N, const PmxLaunchTable* t, int row
 
 // ---------------------------------------------------------------------------
 // fields
+
+// The pointwise kernels and the step kernels put a field's realization-columns (batch*nfc, or batch) in gridDim.y, which
+// CUDA caps at 65535.  Refused up front, so that no kernel on a field or plan fails to launch.
+#define PMX_MAX_BATCH_COLS 65535
+static int check_batch_cols(pmx_ctx* c, const char* who, int64_t batch, int64_t nfc) {
+    if (batch * nfc > PMX_MAX_BATCH_COLS)
+        return set_err(c, PMX_ERR_UNSUPPORTED, "%s: batch*nfc = %lld x %lld = %lld realization-columns, at most %d", who,
+                       (long long)batch, (long long)nfc, (long long)(batch * nfc), PMX_MAX_BATCH_COLS);
+    return PMX_OK;
+}
+
 extern "C" int pmx_field_create(pmx_ctx* c, int64_t nfft, int32_t nfc, int32_t batch, int32_t precision,
                                 pmx_devfield** out) {
     if (!c || !out) return set_err(c, PMX_ERR_INVALID, "pmx_field_create: null argument");
     *out = nullptr;
     if (precision != PMX_F64 && precision != PMX_F32) return set_err(c, PMX_ERR_INVALID, "unknown precision %d", precision);
     if (nfft <= 0 || nfc <= 0 || batch <= 0) return set_err(c, PMX_ERR_INVALID, "non-positive field size");
+    if (int rc = check_batch_cols(c, "pmx_field_create", batch, nfc)) return rc;
     CK(c, cudaSetDevice(c->device));
     pmx_devfield* f = new (std::nothrow) pmx_devfield();
     if (!f) return set_err(c, PMX_ERR_INVALID, "out of host memory");
@@ -782,6 +794,7 @@ static int plan_create(pmx_ctx* c, const pmx_fiber_desc* d, pmx_plan** out, Plan
     if (d->nfc < 1 || d->nfc > PMX_MAX_NFC)
         return set_err(c, PMX_ERR_UNSUPPORTED, "nfc=%d outside [1,%d]", d->nfc, PMX_MAX_NFC);
     if (d->batch < 1) return set_err(c, PMX_ERR_INVALID, "batch must be >= 1");
+    if (int rc = check_batch_cols(c, "pmx_plan_create", d->batch, d->nfc)) return rc;
     if (d->nplates < 1) return set_err(c, PMX_ERR_INVALID, "nplates must be >= 1");
     if (!(d->length > 0)) return set_err(c, PMX_ERR_INVALID, "length must be > 0");
     const bool scalar = d->disp_mode == PMX_DISP_SCALAR;
@@ -826,6 +839,7 @@ static int plan_create(pmx_ctx* c, const pmx_fiber_desc* d, pmx_plan** out, Plan
         if (!c->setup_done.count(key)) {
             cudaError_t e = p->tB->onchip_setup();
             if (e != cudaSuccess) {
+                cudaGetLastError();   // (the failed attribute call is not sticky: clear it, or the next check reports it)
                 delete p;
                 return set_err(c, PMX_ERR_CUDA, "on-chip kernel setup (L=%d) failed: %s", (int)d->nfft, cudaGetErrorString(e));
             }
@@ -838,6 +852,7 @@ static int plan_create(pmx_ctx* c, const pmx_fiber_desc* d, pmx_plan** out, Plan
             pmx_ctx::Occ o;
             cudaError_t e = t->setup(&o.a, &o.b, &o.c, &o.cnl);
             if (e != cudaSuccess || o.a < 1 || o.b < 1 || o.c < 1 || o.cnl < 1) {
+                cudaGetLastError();   // (as above)
                 delete p;
                 return set_err(c, PMX_ERR_CUDA, "kernel setup (L=%d) failed: %s (resident CTAs %d/%d/%d/%d)", t->L,
                                cudaGetErrorString(e), o.a, o.b, o.c, o.cnl);
@@ -1664,6 +1679,7 @@ extern "C" int pmx_count_errors(pmx_ctx* c, const uint8_t* hat, const uint8_t* p
                                 int64_t* counts_dev) {
     if (!c || !hat || !pat || !counts_dev || n <= 0 || batch <= 0)
         return set_err(c, PMX_ERR_INVALID, "pmx_count_errors: bad argument");
+    if (int rc = check_batch_cols(c, "pmx_count_errors", batch, 1)) return rc;
     CK(c, cudaSetDevice(c->device));
     CK(c, cudaMemsetAsync(counts_dev, 0, (size_t)batch * sizeof(int64_t), c->stream));
     dim3 g((unsigned)std::min<size_t>(((size_t)n + 255) / 256, 148 * 4), batch);

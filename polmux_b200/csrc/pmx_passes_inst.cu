@@ -16,8 +16,11 @@ constexpr int L = PMX_L;
 // transforms land in the exchange buffer itself (no separate prefetch).
 constexpr int PSCALE = 32 / PMX_SA_BYTES;  // 1 (FP64) or 2 (FP32)
 constexpr int GAC = PSCALE * ((L >= 1024) ? 1 : (L == 512 ? 2 : 4));
-constexpr int GB = (PSCALE * ((L >= 1024) ? 1 : (L == 512 ? 2 : 4)) * (L / 8) > 1024) ? 1 : PSCALE * ((L >= 1024) ? 1 : (L == 512 ? 2 : 4));
+constexpr int GB_ROWS = (PSCALE * ((L >= 1024) ? 1 : (L == 512 ? 2 : 4)) * (L / 8) > 1024) ? 1 : PSCALE * ((L >= 1024) ? 1 : (L == 512 ? 2 : 4));
 constexpr int TILE_CAP = 32 * 1024;
+// ... unless pass B would then need more shared memory than a CTA can have (227 KiB): FP32 at L = 4096 takes one column
+// per tile (as FP64 does), since two would need 251 KB and the kernel could not be launched at all.
+constexpr int GB = (PassSmem<L, GB_ROWS, (GB_ROWS * L * PMX_SA_BYTES <= TILE_CAP / 2), 1>::TOTAL > 227 * 1024) ? 1 : GB_ROWS;
 // Since passes A and C read and write contiguous rows straight from / to registers they no longer stage a
 // tile for a TMA store, and a fourth resident CTA (the tile lands in the exchange buffer, 42 KB per CTA) beats a
 // separate prefetch buffer with three (measured 49.0 against 50.3 ps per Sa and step at N = 2^20).

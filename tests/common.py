@@ -30,5 +30,20 @@ def make_tx(nsymb, nt, nch=1, rate=28.0, pavg_mw=2.0, ftype='unique', real=np.fl
     return gs
 
 
+def scalar_tx(nsymb, nt, nch, rate=10.0, pavg=4.0):
+    """-> oracle GState; the product's GSTATE holds the same single-polarization field (FIELDY empty), 'sepfields' for
+    nch > 1"""
+    ex, _, _, _ = synth.pdm_qpsk(nsymb, nt, nch)
+    lams = synth.wdm_lambdas(nch, 1550.0, 0.4)
+    gs = orc.reset_all(nsymb, nt, nch)
+    gs.SYMBOLRATE, gs.LAMBDA, gs.POWER = rate, lams.copy(), np.full(nch, pavg)
+    orc.create_field(gs, 'sepfields' if nch > 1 else 'unique', ex, None, power_average=True)
+    pmx.reset_all(nsymb, nt, nch)
+    G = pmx.GSTATE
+    G.SYMBOLRATE, G.LAMBDA, G.POWER = rate, lams.copy(), np.full(nch, pavg)
+    pmx.create_field('sepfields' if nch > 1 else 'unique', ex, None, {'power': 'average'})
+    return gs
+
+
 def rel_l2(ux, uy, rx, ry):
     return orc.rel_l2(ux, uy, rx, ry)

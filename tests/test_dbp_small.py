@@ -17,27 +17,13 @@ import dbp_oracle
 import dbp_pmd_oracle as dpo
 import dbp_scalar_oracle as dso
 import polmux_b200 as pmx
-from polmux_b200 import _lib, mc, synth
+from polmux_b200 import _lib, mc
 from polmux_b200.dbp import dbp_plan
 from polmux_b200.fiber import fiber_setup, setup_to_desc
-from common import base_fiber, make_tx, rel_l2
+from common import base_fiber, make_tx, rel_l2, scalar_tx as _scalar_tx
 
 GAIN_DB = 16.0
 G16 = 10 ** (GAIN_DB / 10)
-
-
-def _scalar_tx(nsymb, nt, nch, rate=10.0, pavg=4.0):
-    """-> oracle GState; the product's GSTATE holds the same single-polarization field (FIELDY empty)"""
-    ex, _, _, _ = synth.pdm_qpsk(nsymb, nt, nch)
-    lams = synth.wdm_lambdas(nch, 1550.0, 0.4)
-    gs = orc.reset_all(nsymb, nt, nch)
-    gs.SYMBOLRATE, gs.LAMBDA, gs.POWER = rate, lams.copy(), np.full(nch, pavg)
-    orc.create_field(gs, 'sepfields' if nch > 1 else 'unique', ex, None, power_average=True)
-    pmx.reset_all(nsymb, nt, nch)
-    G = pmx.GSTATE
-    G.SYMBOLRATE, G.LAMBDA, G.POWER = rate, lams.copy(), np.full(nch, pavg)
-    pmx.create_field('sepfields' if nch > 1 else 'unique', ex, None, {'power': 'average'})
-    return gs
 
 
 def _scalar_setup(nsymb, nt, nch, flag, pavg=4.0, length=1e5, dphimax=3e-3):

@@ -10,17 +10,17 @@ import pytest
 
 import oracle.fiber_oracle as orc
 import polmux_b200 as pmx
-from polmux_b200 import _lib, mc, synth
+from polmux_b200 import _lib, mc
 from polmux_b200.fiber import fiber_setup, setup_to_desc
-from common import base_fiber, make_tx, rel_l2
+from common import base_fiber, make_tx, rel_l2, scalar_tx as _scalar_tx
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-10
 
 
-def _check(gs, fib, flag, seed=7, two_pol=True):
+def _check(gs, fib, flag, seed=7, two_pol=True, disp_mode=None):
     orc.fiber(gs, fib, flag, rng=np.random.Generator(np.random.PCG64(seed)))
-    pmx.fiber(fib, flag, rng=np.random.Generator(np.random.PCG64(seed)), trace=two_pol)
+    pmx.fiber(fib, flag, rng=np.random.Generator(np.random.PCG64(seed)), trace=two_pol, disp_mode=disp_mode)
     G, L = pmx.GSTATE, pmx.FIBER_LAST
     assert L['ncycle'] == gs.log['ncycle']
     if two_pol:
@@ -39,6 +39,31 @@ def test_two_pol_pmd_every_small_size(lg, manakov):
     assert _check(gs, fib, 'gps-') < TOL
 
 
+@pytest.mark.parametrize('manakov', ['yes', 'no'])
+@pytest.mark.parametrize('lg', [6, 7, 8, 9, 10, 11])
+def test_two_pol_pmd_every_small_size_vector_dispersion(lg, manakov):
+    """the same in vector dispersion mode (betat / db1 uploaded, pmx_k_onchip<..., SC = false>)"""
+    nt = 8 if lg < 9 else 16
+    gs = make_tx((1 << lg) // nt, nt)
+    fib = base_fiber(length=5e4, dgd=0.4, nplates=12, manakov=manakov)
+    assert _check(gs, fib, 'gps-', disp_mode='vector') < TOL
+
+
+@pytest.mark.parametrize('nch,lg', [(3, 10), (8, 9)])
+def test_sepfields_in_one_cluster_vector_dispersion(nch, lg):
+    """per-column betat / db1 tables of a cluster in vector dispersion mode"""
+    gs = make_tx((1 << lg) // 16, 16, nch=nch, ftype='sepfields', pavg_mw=1.5)
+    fib = base_fiber(length=4e4, dgd=0.3, nplates=10, manakov='yes', slope=0.057)
+    assert _check(gs, fib, 'gps-', disp_mode='vector') < TOL
+
+
+@pytest.mark.parametrize('nsymb,nt,nch,flag', [(32, 32, 1, 'g-sx'), (64, 32, 5, 'g-sx')])
+def test_scalar_path_vector_dispersion(nsymb, nt, nch, flag):
+    gs = _scalar_tx(nsymb, nt, nch)
+    fib = base_fiber(length=1e5, dphimax=3e-3, slope=0.057)
+    assert _check(gs, fib, flag, two_pol=False, disp_mode='vector') < TOL
+
+
 @pytest.mark.parametrize('flag', ['g---', 'gp--', '--s-', 'g-s-', '-ps-'])
 def test_flags_small(flag):
     gs = make_tx(64, 16)
@@ -53,19 +78,6 @@ def test_sepfields_columns_in_one_cluster(nch, lg):
     gs = make_tx((1 << lg) // 16, 16, nch=nch, ftype='sepfields', pavg_mw=1.5)
     fib = base_fiber(length=4e4, dgd=0.3, nplates=10, manakov='yes', slope=0.057)
     assert _check(gs, fib, 'gps-') < TOL
-
-
-def _scalar_tx(nsymb, nt, nch, rate=10.0, pavg=4.0):
-    ex, _, _, _ = synth.pdm_qpsk(nsymb, nt, nch)
-    lams = synth.wdm_lambdas(nch, 1550.0, 0.4)
-    gs = orc.reset_all(nsymb, nt, nch)
-    gs.SYMBOLRATE, gs.LAMBDA, gs.POWER = rate, lams.copy(), np.full(nch, pavg)
-    orc.create_field(gs, 'sepfields' if nch > 1 else 'unique', ex, None, power_average=True)
-    pmx.reset_all(nsymb, nt, nch)
-    G = pmx.GSTATE
-    G.SYMBOLRATE, G.LAMBDA, G.POWER = rate, lams.copy(), np.full(nch, pavg)
-    pmx.create_field('sepfields' if nch > 1 else 'unique', ex, None, {'power': 'average'})
-    return gs
 
 
 @pytest.mark.parametrize('nsymb,nt,nch,flag', [(32, 32, 1, 'g-sx'), (64, 32, 5, 'g-sx'), (64, 32, 5, 'g--x'), (32, 16, 3, 'g-s-'),
