@@ -298,6 +298,31 @@ int pmx_dbp_set_plates(pmx_plan* plan, int32_t plate_sets, const double* db0, co
  * plan with pmx_plan_destroy. */
 int pmx_dbp_exec(pmx_plan* plan, pmx_devfield* f);
 
+/* ---- single-channel digital backpropagation: one channel of a 'unique' multiplex at a reduced sample rate ------------
+ * A coherent receiver sees its own channel only.  For a field of N = fiber->nfft samples in one column (nfc = 1, every
+ * channel in it) and band = {m, r}, M = N/r, the plan runs per realization, in place:
+ *   down : u <- ifft(fft(u) .* H), H = 1 on the M bins (k - m) mod N of the signed k in [-M/2, M/2), 0 elsewhere (a filter
+ *          plan, pmx_filter_create); v[n] = u[n*r] * exp(+2*pi*i*m*n*r/N), n < M: the channel at baseband, decimated
+ *   DBP  : pmx_dbp_exec on v, a plan of pmx_dbp_create at M samples (same schedule, xi, gain, model, precision and
+ *          PMD-aware variant) whose dispersion is the channel's own: betat_M[k] = betat_N[(k - m) mod N], db1 likewise
+ *   up   : u[n] = r * v[n/r] * exp(-2*pi*i*m*n/N) where r divides n, 0 elsewhere; u <- ifft(fft(u) .* H)
+ * Afterwards the field holds the backpropagated channel on its own bins and zeros elsewhere, so a receiver downstream
+ * (pmx_field_modulate by m, its filters) is unchanged.  The phase indices are reduced modulo N in integers, as in
+ * pmx_field_modulate.  With PMX_DISP_VECTOR the channel's betat / db1 are cropped from fiber's tables; with PMX_DISP_SCALAR
+ * the host evaluates them at the channel's signed bins k - m (betat = omega*beta1 + 0.5*omega^2*beta2 + omega^3*b30/6,
+ * db1 = dgdrms*omega, omega = 2*pi*symbolrate*FN).  The M-sample plan takes the route pmx_dbp_create gives M samples. */
+typedef struct pmx_dbp_band {
+    int64_t shift;    /* bins that bring the channel to baseband (as pmx_field_modulate's m; the receiver's ndfn) */
+    int32_t decim;    /* r: power of two >= 2; the channel is backpropagated on nfft/r samples                    */
+    int32_t reserved;
+} pmx_dbp_band;
+/* fiber describes the link at N samples.  Checked before a context is needed: PMX_ERR_INVALID for decim not a power of
+ * two >= 2 or nfft/decim < 2^6; PMX_ERR_UNSUPPORTED for nfc != 1 and for the scalar path with nfft/decim > 2^12; and
+ * everything pmx_dbp_create rejects.  pmx_dbp_set_plates, pmx_dbp_exec (fields of nfft samples, one column) and
+ * pmx_plan_destroy take the returned plan; it owns the M-sample DBP plan, the band filter and an M x batch work field. */
+int pmx_dbp_channel_create(pmx_ctx* ctx, const pmx_fiber_desc* fiber, const pmx_dbp_desc* dbp, const pmx_dbp_band* band,
+                           pmx_plan** plan);
+
 /* ---- create_field('unique'): the WDM multiplex on the device (create_field.m:113-149,180-199) ----------------
  * The reference builds the single field as
  *   FIELDX = ifft( sum_ch fastshift( fft(sigx(:,ch)), -ndfn(ch) ) ),   ndfn = round(deltafn/SYMBOLRATE/minfreq)

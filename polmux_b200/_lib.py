@@ -34,7 +34,7 @@ EXPORTS = [
     'pmx_host_is_pinned', 'pmx_scalar_adaptive_run', 'pmx_mc_run', 'pmx_mc_nccl_available',
     'pmx_ampliflat_exec_at', 'pmx_dsp_count', 'pmx_field_mean_power', 'pmx_pmd_matrix', 'pmx_field_jones', 'pmx_filter_create', 'pmx_field_copy_cols', 'pmx_field_modulate',
     'pmx_cohmix_exec', 'pmx_field_mean_power_xy', 'pmx_cohmix_run', 'pmx_dsp_phases', 'pmx_field_quantize', 'pmx_inverse_pmd_run',
-    'pmx_dbp_create', 'pmx_dbp_exec', 'pmx_dbp_set_plates',
+    'pmx_dbp_create', 'pmx_dbp_exec', 'pmx_dbp_set_plates', 'pmx_dbp_channel_create',
 ]
 
 
@@ -82,6 +82,10 @@ class DspDesc(C.Structure):
 class DbpDesc(C.Structure):
     _fields_ = [('nspan', C.c_int32), ('steps_per_span', C.c_int32), ('span_steps', _ip), ('step_len', _dp),
                 ('xi', C.c_double), ('gain', C.c_double), ('pmd', C.c_int32), ('reserved', C.c_int32)]
+
+
+class DbpBand(C.Structure):
+    _fields_ = [('shift', C.c_int64), ('decim', C.c_int32), ('reserved', C.c_int32)]
 
 
 class McReceiver(C.Structure):
@@ -181,6 +185,7 @@ def load():
     lib.pmx_dbp_create.argtypes = [vp, C.POINTER(FiberDesc), C.POINTER(DbpDesc), C.POINTER(vp)]
     lib.pmx_dbp_exec.argtypes = [vp, vp]
     lib.pmx_dbp_set_plates.argtypes = [vp, C.c_int32, _dp, _dp, _dp]
+    lib.pmx_dbp_channel_create.argtypes = [vp, C.POINTER(FiberDesc), C.POINTER(DbpDesc), C.POINTER(DbpBand), C.POINTER(vp)]
     _lib = lib
     return lib
 
@@ -521,12 +526,17 @@ class Plan:
 
 
 class DbpPlan(Plan):
-    """Digital backpropagation of a link (pmx_dbp_create): execute(field) runs it in place on a resident field."""
+    """Digital backpropagation of a link (pmx_dbp_create): execute(field) runs it in place on a resident field.  With a
+    band (DbpBand: shift, decim) it is the DBP of one channel of a one-column field at nfft/decim samples
+    (pmx_dbp_channel_create)."""
 
-    def __init__(self, ctx: Context, desc: FiberDesc, keep, dbp: DbpDesc, dbp_keep):
-        self.ctx, self.desc, self.keep, self.dbp, self.dbp_keep = ctx, desc, keep, dbp, dbp_keep
+    def __init__(self, ctx: Context, desc: FiberDesc, keep, dbp: DbpDesc, dbp_keep, band: 'DbpBand' = None):
+        self.ctx, self.desc, self.keep, self.dbp, self.dbp_keep, self.band = ctx, desc, keep, dbp, dbp_keep, band
         h = C.c_void_p()
-        ctx.check(ctx.lib.pmx_dbp_create(ctx.h, C.byref(desc), C.byref(dbp), C.byref(h)))
+        if band is None:
+            ctx.check(ctx.lib.pmx_dbp_create(ctx.h, C.byref(desc), C.byref(dbp), C.byref(h)))
+        else:
+            ctx.check(ctx.lib.pmx_dbp_channel_create(ctx.h, C.byref(desc), C.byref(dbp), C.byref(band), C.byref(h)))
         self.h = h
 
     def execute(self, field: DeviceField, trace_cap=0):
@@ -540,6 +550,14 @@ class DbpPlan(Plan):
         if not (a.size == b.size == c.size == n):
             raise ValueError('plates must be [nspan][plate_sets][nplates] = %d values each' % n)
         self.ctx.check(self.ctx.lib.pmx_dbp_set_plates(self.h, int(plate_sets), _ptr(a), _ptr(b), _ptr(c)))
+
+
+def make_band(shift, decim):
+    """-> DbpBand: the channel brought to baseband by `shift` bins (pmx_field_modulate's m), backpropagated on nfft/decim
+    samples"""
+    b = DbpBand()
+    b.shift, b.decim = int(shift), int(decim)
+    return b
 
 
 def make_dbp(nspan, gain=0.0, steps_per_span=None, step_len=None, span_steps=None, xi=1.0, pmd=False):

@@ -246,6 +246,13 @@ struct pmx_plan {
     // DBP of a small field (onchip): sched_idx and sched_span on the device, the on-chip kernel's step table
     int* sched_idx_d = nullptr;
     int* sched_span_d = nullptr;
+    // single-channel DBP (pmx_dbp_channel_create): the DBP plan at nfft/decim samples, the band filter at nfft, the
+    // work field of the decimated channel, and the channel's shift (mod nfft) and log2(decim)
+    pmx_plan* ch_dbp = nullptr;
+    pmx_plan* ch_band = nullptr;
+    pmx_devfield* ch_work = nullptr;
+    long long ch_shift = 0;
+    int ch_log2r = 0;
 };
 
 static int set_err(pmx_ctx* ctx, int code, const char* fmt, ...) {
@@ -768,6 +775,9 @@ extern "C" void pmx_plan_destroy(pmx_plan* p) {
     if (p->geo_d) cudaFreeAsync(p->geo_d, st);
     if (p->sched_idx_d) cudaFreeAsync(p->sched_idx_d, st);
     if (p->sched_span_d) cudaFreeAsync(p->sched_span_d, st);
+    pmx_plan_destroy(p->ch_dbp);
+    pmx_plan_destroy(p->ch_band);
+    pmx_field_destroy(p->ch_work);
     delete p;
 }
 
@@ -2999,6 +3009,63 @@ extern "C" int pmx_field_modulate(pmx_ctx* c, pmx_devfield* f, int64_t m) {
     return PMX_OK;
 }
 
+// Resampling of single-channel DBP (pmx_dbp_channel_create) between a one-column field of N samples (layout l1/l2) and
+// the M = N/r = N >> lr samples of the channel (layout m1/m2); one realization per blockIdx.y.  The phase index is
+// reduced modulo N in integers and the argument of sincospi is exact, as in pmx_k_modulate.
+// Gather: v[n] = u[n*r] * exp(+i*2*pi*m*n*r/N) -- the band-passed channel at baseband, decimated.
+template <typename E>
+__global__ void __launch_bounds__(256) pmx_k_band_gather(const E* __restrict__ field, int l1, int l2, E* __restrict__ chan,
+                                                         int m1, int m2, size_t N, int lr, long long m) {
+    const size_t M = N >> lr;
+    const E* src = field + (size_t)blockIdx.y * N * 2;
+    E* dst = chan + (size_t)blockIdx.y * M * 2;
+    for (size_t pos = (size_t)blockIdx.x * blockDim.x + threadIdx.x; pos < M; pos += (size_t)gridDim.x * blockDim.x) {
+        const size_t t = pmx_time_index(pos, m1, m2) << lr;
+        const size_t sp = pmx_mem_index(t, l1, l2);
+        PMX_ASSERT(t < N && sp < N && m >= 0 && (unsigned long long)m < N);
+        const unsigned long long r = ((unsigned long long)m * (unsigned long long)t) & (N - 1);   // m*n*r mod N
+        double sn, cs;
+        sincospi(2.0 * (double)r / (double)N, &sn, &cs);
+        const E x = src[2 * sp], y = src[2 * sp + 1];
+        E ox, oy;
+        ox.x = (double)x.x * cs - (double)x.y * sn;
+        ox.y = (double)x.x * sn + (double)x.y * cs;
+        oy.x = (double)y.x * cs - (double)y.y * sn;
+        oy.y = (double)y.x * sn + (double)y.y * cs;
+        dst[2 * pos] = ox;
+        dst[2 * pos + 1] = oy;
+    }
+}
+
+// Stuff: u[n] = r * v[n/r] * exp(-i*2*pi*m*n/N) where r divides n, 0 elsewhere; the band filter that follows interpolates.
+template <typename E>
+__global__ void __launch_bounds__(256) pmx_k_band_stuff(const E* __restrict__ chan, int m1, int m2, E* __restrict__ field,
+                                                        int l1, int l2, size_t N, int lr, long long m) {
+    const size_t M = N >> lr;
+    const E* src = chan + (size_t)blockIdx.y * M * 2;
+    E* dst = field + (size_t)blockIdx.y * N * 2;
+    const double rr = (double)(1 << lr);
+    for (size_t pos = (size_t)blockIdx.x * blockDim.x + threadIdx.x; pos < N; pos += (size_t)gridDim.x * blockDim.x) {
+        const size_t n = pmx_time_index(pos, l1, l2);
+        E ox, oy;
+        ox.x = ox.y = oy.x = oy.y = 0;
+        if ((n & (((size_t)1 << lr) - 1)) == 0) {
+            const size_t sp = pmx_mem_index(n >> lr, m1, m2);
+            PMX_ASSERT(n < N && sp < M && m >= 0 && (unsigned long long)m < N);
+            const unsigned long long r = ((unsigned long long)m * (unsigned long long)n) & (N - 1);   // m*n mod N
+            double sn, cs;
+            sincospi(2.0 * (double)r / (double)N, &sn, &cs);
+            const E x = src[2 * sp], y = src[2 * sp + 1];
+            ox.x = rr * ((double)x.x * cs + (double)x.y * sn);
+            ox.y = rr * ((double)x.y * cs - (double)x.x * sn);
+            oy.x = rr * ((double)y.x * cs + (double)y.y * sn);
+            oy.y = rr * ((double)y.y * cs - (double)y.x * sn);
+        }
+        dst[2 * pos] = ox;
+        dst[2 * pos + 1] = oy;
+    }
+}
+
 // The four mixer outputs and the photocurrents of one polarization (receiver_cohmix.m:253-277), as the interpreter forms
 // them: E1 = j*s + j*lo, E2 = s - lo, E3 = j*s - lo, E4 = -s + j*lo, I_k = real(E_k .* conj(E_k)); balanced detection
 // returns (I1 - I2, I3 - I4), single photodiodes (I1, I3).  The pair is stored as one complex sample.
@@ -3486,8 +3553,11 @@ __global__ void __launch_bounds__(128) pmx_k_dbp_pkg(const DbpGeo* __restrict__ 
     pmx_pkg_fill(&c, g, f, plates + ((size_t)G.span * f.plate_sets + (f.plate_sets > 1 ? b : 0)) * f.nplates);
 }
 
+static int dbp_channel_exec(pmx_plan* p, pmx_devfield* fld);
+
 extern "C" int pmx_dbp_set_plates(pmx_plan* p, int32_t sets, const double* db0, const double* theta, const double* epsilon) {
     if (!p) return set_err(nullptr, PMX_ERR_INVALID, "pmx_dbp_set_plates: null plan");
+    if (p->ch_dbp) return pmx_dbp_set_plates(p->ch_dbp, sets, db0, theta, epsilon);   // single-channel DBP: its M-sample plan
     pmx_ctx* c = p->ctx;
     if (!p->dbp_pmd) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_set_plates: not a PMD-aware DBP plan (pmx_dbp_create with pmd = 1)");
     if (sets != 1 && sets != p->d.batch)
@@ -3738,6 +3808,7 @@ extern "C" int pmx_dbp_exec(pmx_plan* p, pmx_devfield* fld) {
     if (!p || !fld) return set_err(nullptr, PMX_ERR_INVALID, "pmx_dbp_exec: null argument");
     pmx_ctx* c = p->ctx;
     if (!p->dbp) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_exec: the plan was not made by pmx_dbp_create");
+    if (p->ch_dbp) return dbp_channel_exec(p, fld);
     if (p->dbp_pmd && !p->dbp_plates_set)
         return set_err(c, PMX_ERR_INVALID, "pmx_dbp_exec: a PMD-aware plan needs its plates (pmx_dbp_set_plates) first");
     int rc = check_field(p, fld);
@@ -3796,4 +3867,122 @@ extern "C" int pmx_dbp_exec(pmx_plan* p, pmx_devfield* fld) {
     if (rc) return rc;
     CK(c, cudaStreamSynchronize(c->stream));
     return PMX_OK;
+}
+
+// ---------------------------------------------------------------------------
+// Single-channel DBP (polmux_ssfm.h, pmx_dbp_band): band filter at N, gather to M = N/r, the DBP plan of M samples, stuff
+// back to N, band filter.  The M-sample plan is an ordinary pmx_dbp_create plan on vector tables: the channel's own
+// dispersion, so that nothing in the step kernels knows about the channel's offset.
+extern "C" int pmx_dbp_channel_create(pmx_ctx* c, const pmx_fiber_desc* fd, const pmx_dbp_desc* g, const pmx_dbp_band* band,
+                                      pmx_plan** out) {
+    // (checked before the context, like pmx_dbp_create)
+    if (!fd || !g || !band || !out) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_channel_create: null argument");
+    *out = nullptr;
+    const int lg = ilog2_exact(fd->nfft), lr = ilog2_exact(band->decim);
+    if (band->decim < 2 || lr < 1)
+        return set_err(c, PMX_ERR_INVALID, "pmx_dbp_channel_create: decim=%d, must be a power of two >= 2", band->decim);
+    if (lg < 6 || lg > 24)
+        return set_err(c, PMX_ERR_UNSUPPORTED, "single-channel digital backpropagation: nfft=%lld, built for powers of two from "
+                       "2^6 to 2^24", (long long)fd->nfft);
+    if (lg - lr < 6)
+        return set_err(c, PMX_ERR_INVALID, "pmx_dbp_channel_create: nfft/decim = %lld/%d samples, at least 2^6 are needed",
+                       (long long)fd->nfft, band->decim);
+    if (fd->nfc != 1)
+        return set_err(c, PMX_ERR_UNSUPPORTED, "single-channel digital backpropagation: nfc=%d, built for one column holding "
+                       "every channel (a 'unique' multiplex)", fd->nfc);
+    const int64_t N = fd->nfft, M = N >> lr;
+    if (fd->scalar_field && lg - lr > 12)
+        return set_err(c, PMX_ERR_UNSUPPORTED, "single-channel digital backpropagation on the scalar path: nfft/decim=%lld, "
+                       "built for at most 2^12 samples", (long long)M);
+    const long long m = ((band->shift % N) + N) % N;
+    auto bin = [&](int64_t j) { return (size_t)((((j < M / 2 ? j : j - M) - m) % N + N) % N); };   // N-grid bin of M-grid bin j
+    const bool pmd = g->pmd == 1 && fd->fls[1];
+    std::vector<double> bt((size_t)M), d1;
+    if (fd->disp_mode == PMX_DISP_SCALAR) {
+        if (!fd->beta1 || !fd->beta2) return set_err(c, PMX_ERR_INVALID, "scalar dispersion mode needs beta1 and beta2");
+        if (fd->nsymb <= 0 || fd->nt <= 0 || (int64_t)fd->nsymb * fd->nt != N)
+            return set_err(c, PMX_ERR_INVALID, "scalar dispersion mode: nsymb*nt must equal nfft");
+        // fiber.m:350-358 at the channel's bins, in the host's operation order: FN = fftshift(-NT/2 + (0:N-1)/NSYMB)
+        // (reset_all.m:153), omega = 2*pi*symbolrate*FN
+        if (pmd) d1.resize((size_t)M);
+        for (int64_t j = 0; j < M; ++j) {
+            const int64_t i = (int64_t)((bin(j) + (size_t)(N / 2)) & (size_t)(N - 1));   // index before the fftshift
+            const double fn = -fd->nt / 2.0 + (double)i * (1.0 / fd->nsymb);
+            const double om = 2 * M_PI * fd->symbolrate * fn;
+            bt[j] = om * fd->beta1[0] + 0.5 * (om * om) * fd->beta2[0] + std::pow(om, 3) * fd->b30 / 6;
+            if (pmd) d1[j] = fd->dgdrms * om;
+        }
+    } else {
+        if (!fd->betat) return set_err(c, PMX_ERR_INVALID, "betat is required in vector dispersion mode");
+        for (int64_t j = 0; j < M; ++j) bt[j] = fd->betat[bin(j)];
+        if (pmd && fd->db1) {
+            d1.resize((size_t)M);
+            for (int64_t j = 0; j < M; ++j) d1[j] = fd->db1[bin(j)];
+        }
+    }
+    pmx_fiber_desc e = *fd;
+    e.nfft = M;
+    e.disp_mode = PMX_DISP_VECTOR;
+    e.betat = bt.data();
+    e.db1 = d1.empty() ? nullptr : d1.data();
+    pmx_plan* inner = nullptr;
+    int rc = pmx_dbp_create(c, &e, g, &inner);   // validates the rest before it needs the context
+    if (rc) return rc;
+    std::vector<double> H(2 * (size_t)N, 0.0);   // 1 on the channel's M bins
+    for (int64_t j = 0; j < M; ++j) H[2 * bin(j)] = 1.0;
+    pmx_plan* p = new (std::nothrow) pmx_plan();
+    if (!p) {
+        pmx_plan_destroy(inner);
+        return set_err(c, PMX_ERR_INVALID, "out of host memory");
+    }
+    p->ctx = c;
+    p->d = *fd;
+    p->d.gam = p->d.db0 = p->d.theta = p->d.epsilon = p->d.betat = p->d.db1 = p->d.beta1 = p->d.beta2 = nullptr;
+    p->dbp = true;
+    p->ch_dbp = inner;
+    p->ch_shift = m;
+    p->ch_log2r = lr;
+    rc = pmx_filter_create(c, N, 1, fd->batch, fd->precision, H.data(), 1, &p->ch_band);
+    if (!rc) rc = pmx_field_create(c, M, 1, fd->batch, fd->precision, &p->ch_work);
+    if (rc) {
+        pmx_plan_destroy(p);
+        return rc;
+    }
+    *out = p;
+    return PMX_OK;
+}
+
+static int dbp_channel_exec(pmx_plan* p, pmx_devfield* fld) {
+    pmx_ctx* c = p->ctx;
+    int rc = check_field(p->ch_band, fld);   // device, precision, nfft, one column, batch
+    if (!rc) rc = pmx_fiber_exec(p->ch_band, fld, nullptr);
+    if (rc) return rc;
+    CK(c, cudaSetDevice(c->device));
+    pmx_devfield* w = p->ch_work;
+    const size_t N = (size_t)fld->nfft, M = (size_t)w->nfft;
+    const dim3 gm((unsigned)std::min<size_t>((M + 255) / 256, 148 * 8), fld->batch);
+    if (fld->precision == PMX_F32)
+        pmx_k_band_gather<float2><<<gm, 256, 0, c->stream>>>(reinterpret_cast<const float2*>(fld->data), fld->log2N1, fld->log2N2,
+                                                              reinterpret_cast<float2*>(w->data), w->log2N1, w->log2N2, N,
+                                                              p->ch_log2r, p->ch_shift);
+    else
+        pmx_k_band_gather<double2><<<gm, 256, 0, c->stream>>>(reinterpret_cast<const double2*>(fld->data), fld->log2N1,
+                                                               fld->log2N2, reinterpret_cast<double2*>(w->data), w->log2N1,
+                                                               w->log2N2, N, p->ch_log2r, p->ch_shift);
+    c->launches++;
+    CK(c, cudaGetLastError());
+    rc = pmx_dbp_exec(p->ch_dbp, w);
+    if (rc) return rc;
+    const dim3 gn((unsigned)std::min<size_t>((N + 255) / 256, 148 * 8), fld->batch);
+    if (fld->precision == PMX_F32)
+        pmx_k_band_stuff<float2><<<gn, 256, 0, c->stream>>>(reinterpret_cast<const float2*>(w->data), w->log2N1, w->log2N2,
+                                                             reinterpret_cast<float2*>(fld->data), fld->log2N1, fld->log2N2, N,
+                                                             p->ch_log2r, p->ch_shift);
+    else
+        pmx_k_band_stuff<double2><<<gn, 256, 0, c->stream>>>(reinterpret_cast<const double2*>(w->data), w->log2N1, w->log2N2,
+                                                              reinterpret_cast<double2*>(fld->data), fld->log2N1, fld->log2N2, N,
+                                                              p->ch_log2r, p->ch_shift);
+    c->launches++;
+    CK(c, cudaGetLastError());
+    return pmx_fiber_exec(p->ch_band, fld, nullptr);
 }

@@ -13,6 +13,12 @@ the receiver-side nonlinear compensation a Monte-Carlo run can count errors behi
 Given the link's waveplates (dbp_plan(plates=...), dbp(brf=...)) it is PMD-aware: every step undoes the forward step's
 own trunk product as well, so that it inverts a 'gps-' link too (McRunner(compensation='dbp_pmd')).  There is no CPU
 fallback.
+
+Single-channel DBP (dbp(..., ich=, decim=), dbp_plan(..., shift=, decim=); pmx_dbp_channel_create): a coherent receiver sees
+its own channel only.  Channel ich of a 'unique' multiplex (one column holding every channel) is cut out by an ideal
+band-pass, brought to baseband and decimated to nfft/decim samples, backpropagated there on the channel's own dispersion
+-- on the route DBP takes for that size -- then interpolated back and returned to its own bins; the other channels are
+dropped.  A receiver downstream is unchanged: receiver_cohmix still shifts the channel by its ndfn and filters it.
 """
 from __future__ import annotations
 
@@ -27,21 +33,27 @@ from .gstate import GSTATE
 
 def dbp_plan(ctx: _lib.Context, setup: FiberSetup, nspan: int = 1, gain_db: Optional[float] = None,
              steps_per_span: Optional[int] = None, step_len=None, span_steps=None, xi: float = 1.0, batch: int = 1,
-             precision: Optional[str] = None, disp_mode: Optional[str] = None, plates=None) -> _lib.DbpPlan:
+             precision: Optional[str] = None, disp_mode: Optional[str] = None, plates=None, shift: Optional[int] = None,
+             decim: Optional[int] = None) -> _lib.DbpPlan:
     """The DBP of nspan spans of the fiber `setup` describes, for resident fields of `batch` realizations.  Schedule:
     steps_per_span uniform steps per span (default 1), or step_len -- one span's steps in forward order for every span,
     or with span_steps [nspan] all spans' steps concatenated.  plates: None -- the 'p' flag, plates and dgdrms are
     ignored; (db0, theta, epsilon), each [nspan][plate_sets][nplates] in forward order (plate_sets 1 or batch) -- PMD-aware
-    DBP through those waveplates (setup must carry the 'p' flag; DbpPlan.set_plates swaps in another draw)."""
+    DBP through those waveplates (setup must carry the 'p' flag; DbpPlan.set_plates swaps in another draw).
+    decim: single-channel DBP of a one-column field -- the channel that `shift` bins bring to baseband (the receiver's
+    ndfn; default 0), backpropagated on nfft/decim samples (pmx_dbp_channel_create)."""
     if plates is not None and not setup.fls[1]:
         raise ValueError("PMD-aware DBP (plates given) needs a fiber with the 'p' flag")
+    if decim is None and shift is not None:
+        raise ValueError('dbp_plan: shift selects a channel for single-channel DBP and needs decim')
     desc, keep = setup_to_desc(setup, batch=batch, disp_mode=disp_mode, precision=precision)
     gain = 0.0 if gain_db is None else 10 ** (gain_db * 0.1)
     if step_len is None and steps_per_span is None:
         steps_per_span = 1
     d, dkeep = _lib.make_dbp(nspan, gain, steps_per_span=steps_per_span, step_len=step_len, span_steps=span_steps, xi=xi,
                              pmd=plates is not None)
-    plan = _lib.DbpPlan(ctx, desc, keep, d, dkeep)
+    band = None if decim is None else _lib.make_band(shift or 0, decim)
+    plan = _lib.DbpPlan(ctx, desc, keep, d, dkeep, band)
     if plates is not None:
         try:
             arrs = [np.asarray(a, dtype=np.float64).reshape(int(nspan), -1, setup.nplates) for a in plates]
@@ -53,19 +65,33 @@ def dbp_plan(ctx: _lib.Context, setup: FiberSetup, nspan: int = 1, gain_db: Opti
 
 
 def dbp(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, steps_per_span: Optional[int] = None, step_len=None,
-        span_steps=None, xi: float = 1.0, ctx: Optional[_lib.Context] = None, precision: Optional[str] = None, brf=None):
+        span_steps=None, xi: float = 1.0, ctx: Optional[_lib.Context] = None, precision: Optional[str] = None, brf=None,
+        ich: Optional[int] = None, decim: Optional[int] = None):
     """Backpropagates GSTATE.FIELDX / FIELDY in place through nspan spans of the fiber x, the amplifier of gain_db [dB]
     after each (None: no amplifier).  x and flag are what fiber() takes; a field without FIELDY runs the scalar path, the
     'x' flag there backpropagating the cross-phase modulation of all columns.  Without brf the flag's 'p' is dropped (no plates
     are drawn, nothing is taken from the global random stream) but the fiber's nonlinear model stays the one fiber() used:
     Manakov when x.manakov is 'yes' and the flag has 'p', else the CNLSE.  brf: the struct fiber() returned (every span
     the same plates) or a list of nspan of them in forward span order, with 'p' in the flag: PMD-aware DBP through those
-    plates.  xi: fraction of gamma backpropagated.  The field stays resident on the device like fiber() and ampliflat()
-    leave it."""
+    plates.  xi: fraction of gamma backpropagated.  ich, decim: single-channel DBP of channel ich (1-based) of a 'unique'
+    multiplex on nfft/decim samples; afterwards the field holds that channel alone, on its own bins.  The field stays
+    resident on the device like fiber() and ampliflat() leave it."""
     G = GSTATE
     f = str(flag).lower()
     if len(f) != 4:
         raise ValueError("wrong flag. E.g. flag can be 'g---','gp--','-s--', etc")
+    shift = None
+    if decim is not None:
+        if ich is None:
+            raise ValueError('dbp: single-channel DBP (decim) needs the channel ich')
+        if ich < 1 or ich > G.NCH:
+            raise ValueError('The channel does not exist')
+        if G.field_shape()[1] != 1:
+            raise ValueError("dbp: single-channel DBP takes a field holding every channel in one column ('unique')")
+        from .receiver import channel_ndfn
+        shift = int(channel_ndfn(ich, G)) if G.NCH > 1 else 0
+    elif ich is not None:
+        raise ValueError('dbp: ich selects a channel for single-channel DBP and needs decim')
     plates = None
     if brf is None:
         s = fiber_setup(x, f[0] + '-' + f[2:])
@@ -96,7 +122,8 @@ def dbp(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, steps_per
         fld = _lib.DeviceField(ctx, s.nfft, s.nfc, 1, precision=prec)
         try:
             fld.upload(fx, np.zeros_like(fx))
-            plan = dbp_plan(ctx, s, nspan, gain_db, steps_per_span, step_len, span_steps, xi, precision=precision)
+            plan = dbp_plan(ctx, s, nspan, gain_db, steps_per_span, step_len, span_steps, xi, precision=precision,
+                            shift=shift, decim=decim)
             try:
                 plan.execute(fld)
             finally:
@@ -108,7 +135,8 @@ def dbp(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, steps_per
         return
     fld, hx, hy = G.take_device(ctx, prec)
     try:
-        plan = dbp_plan(ctx, s, nspan, gain_db, steps_per_span, step_len, span_steps, xi, precision=precision, plates=plates)
+        plan = dbp_plan(ctx, s, nspan, gain_db, steps_per_span, step_len, span_steps, xi, precision=precision, plates=plates,
+                        shift=shift, decim=decim)
     except Exception:
         G.restore_host(fld, hx, hy)     # nothing ran: the caller's field is as it was
         raise

@@ -219,7 +219,9 @@ class McRunner:
         compensation ('blind' and 'cohmix'): 'cd' -- the all-pass step that undoes the link's dispersion; 'dbp' -- digital
         backpropagation of the link (polmux_b200/dbp.py) with dbp_params (steps_per_span, step_len, span_steps, xi; default
         one step per span, xi = 1), the amplifier gain undone before each span.  'dbp_pmd' (every receiver) -- PMD-aware
-        DBP through each group's own plate draws (Link.plates); with 'genie' it replaces the linear equaliser"""
+        DBP through each group's own plate draws (Link.plates); with 'genie' it replaces the linear equaliser.
+        dbp_params with 'decim' (a power of two >= 2; 'blind' and 'cohmix', a one-column 'unique' field): single-channel DBP
+        on nfft/decim samples -- of channel `ich` for 'cohmix', of the channel at the centre of the grid for 'blind'"""
         import torch
         from . import dsp as _dsp
         self.receiver, self.dsp_params = receiver, dict(dsp_params or {})
@@ -229,6 +231,8 @@ class McRunner:
             raise ValueError("compensation must be 'cd', 'dbp' or 'dbp_pmd'")
         if compensation == 'dbp' and receiver == 'genie':
             raise ValueError("the genie receiver undoes the link with the known plates: compensation='dbp' needs 'blind' or 'cohmix'")
+        if receiver == 'genie' and dict(dbp_params or {}).get('decim') is not None:
+            raise ValueError("single-channel DBP (dbp_params 'decim') needs the 'blind' or 'cohmix' receiver")
         self.ref_patmat = _dsp.reference_pattern(np.asarray(sym)[0], np.asarray(sym)[1]) if receiver != 'genie' else None
         self.passes = []
         self.ctx, self.setup, self.sym, self.nsymb, self.nt = ctx, setup, sym, nsymb, nt
@@ -255,18 +259,23 @@ class McRunner:
                                       **dict(dbp_params or {}))
         if receiver != 'genie':
             self.rxctx = _lib.Context(ctx.device) if self.pipelined else ctx
-            if compensation in ('dbp', 'dbp_pmd'):
-                from .dbp import dbp_plan
-                comp = dbp_plan(self.rxctx, setup, nspan, gain_db, batch=batch, precision='f64',
-                                plates=self._link_plates() if compensation == 'dbp_pmd' else None, **dict(dbp_params or {}))
-            else:
-                comp = self.link.cd_plan(self.rxctx)
-            self.rx = dict(cd=comp, S=None)
+            S = None
             if receiver == 'cohmix':
                 from . import receiver as _rx
                 from .gstate import GSTATE
                 x = dict(rx_params or {'oftype': 'gauss', 'obw': 1.9, 'eftype': 'bessel5', 'ebw': 0.65})   # ex20_coherent_polmux.m:47-50
                 S = _rx.CohmixSetup(ich, x, GSTATE, nfc=setup.nfc)
+            if compensation in ('dbp', 'dbp_pmd'):
+                from .dbp import dbp_plan
+                dp = dict(dbp_params or {})
+                if dp.get('decim') is not None:      # single-channel DBP of the receiver's channel
+                    dp['shift'] = S.ndfn if S is not None else 0
+                comp = dbp_plan(self.rxctx, setup, nspan, gain_db, batch=batch, precision='f64',
+                                plates=self._link_plates() if compensation == 'dbp_pmd' else None, **dp)
+            else:
+                comp = self.link.cd_plan(self.rxctx)
+            self.rx = dict(cd=comp, S=None)
+            if receiver == 'cohmix':
                 delay = _rx.evaldelay(x['oftype'], x['obw'] * 0.5) + _rx.evaldelay(x['eftype'], x['ebw']) + S.x['post_delay']
                 self.rx.update(S=S, ich=ich, shift=int(round(delay * nt)),
                                peak=4.0 * math.sqrt(float(np.asarray(GSTATE.POWER).ravel()[ich - 1])),

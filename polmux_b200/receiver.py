@@ -94,6 +94,18 @@ def hermitian_part(h):
     return 0.5 * (h + mirror)
 
 
+def channel_ndfn(ich, G=None):
+    """The offset of channel ich in a field holding every channel (receiver_cohmix.m:85-105), in FFT bins: the shift
+    pmx_field_modulate takes to bring the channel to baseband (its spectrum sits on the bins k - ndfn)."""
+    G = G or GSTATE
+    fn = np.asarray(G.FN, dtype=np.float64).ravel()
+    lam = np.asarray(G.LAMBDA, dtype=np.float64).ravel()
+    maxl, minl = lam.max(), lam.min()
+    lamc = 2 * maxl * minl / (maxl + minl)
+    minfreq = fn[1] - fn[0]
+    return round(CONSTANTS.CLIGHT * (1 / lamc - 1 / lam[ich - 1]) / G.SYMBOLRATE / minfreq)
+
+
 class CohmixSetup:
     """What receiver_cohmix.m:78-169,178-219 derives from (ich, x) and GSTATE before it touches the samples."""
 
@@ -112,12 +124,10 @@ class CohmixSetup:
         if ich > G.NCH or ich < 1:
             raise ValueError('The channel does not exist')
         if nfc != G.NCH:                                                      # one field for all the channels (:85-105)
-            minfreq = fn[1] - fn[0]
-            dfn = lambda l: clight * (1 / lamc - 1 / l)
-            self.ndfn = int(round(dfn(lam[ich - 1]) / G.SYMBOLRATE / minfreq))
+            self.ndfn = int(channel_ndfn(ich, G))
             self.nch = 1
-            self.ndfnl = nfft // 2 if ich == 1 else int(round((self.ndfn - round(dfn(lam[ich - 2]) / G.SYMBOLRATE / minfreq)) * 0.5))
-            self.ndfnr = nfft // 2 if ich == G.NCH else int(round((round(dfn(lam[ich]) / G.SYMBOLRATE / minfreq) - self.ndfn) * 0.5))
+            self.ndfnl = nfft // 2 if ich == 1 else int(round((self.ndfn - channel_ndfn(ich - 1, G)) * 0.5))
+            self.ndfnr = nfft // 2 if ich == G.NCH else int(round((channel_ndfn(ich + 1, G) - self.ndfn) * 0.5))
         else:
             self.ndfn, self.nch, self.ndfnl, self.ndfnr = 0, ich, nfft // 2, nfft // 2
         self.b2b = False
