@@ -7,7 +7,8 @@ function zbrf = fiber(x, flag)
 %   GSTATE.DELAY and GSTATE.DISP, and the same birefringence struct ZBRF when an output is asked for.
 %
 %   Put this directory BEFORE the toolbox on the path.  Everything up to the SSFM dispatch is plain
-%   interpreter arithmetic in the toolbox's operation order; the propagation loop itself -- the
+%   interpreter arithmetic in the toolbox's operation order (the part before the plate draw lives in
+%   FIBER_SETUP, which DBP shares); the propagation loop itself -- the
 %   toolbox's matrix_ssfm, scalar_ssfm and scalar_a_ssfm sub-functions -- runs inside the MEX gateway
 %   ssfm_mex (mex/ssfm_mex.c -> libpolmux_ssfm.so).  There is no CPU fallback: without the gateway
 %   the call fails.
@@ -25,158 +26,52 @@ if nargin < 2
 end
 c0 = CONSTANTS.CLIGHT;
 ncol = size(GSTATE.FIELDX, 2);
-nfft = GSTATE.NSYMB * GSTATE.NT;
 
-% ---- step-size policy
-if ~isfield(x, 'dzmax') || x.dzmax > x.length
-    x.dzmax = x.length;
-end
-tolflag = 0;
-ltol = 0;
-if isfield(x, 'ltol')
-    if ~isfield(x, 'dphimax')
-        x.dphimax = Inf;
-    end
-    ltol = x.ltol;
-    tolflag = 2;
-    if isfield(x, 'dphiadapt') && x.dphiadapt
-        tolflag = 1;
-    end
-end
+% ---- everything up to the plate draw: step-size policy, flag, birefringence parameters, unit conversions,
+%      front-end options, dispersion vectors (fiber_setup.m, shared with dbp.m)
+[s, x] = fiber_setup(x, flag, nargout > 0);
+fls = s.fls;
+tolflag = s.tolflag;
+ltol = s.ltol;
+dphimaxt = s.dphimaxt;
+dzmaxt = s.dzmaxt;
+isy = s.isy;
+vector = s.vector;
+manakov = s.manakov;
+ispmf = s.ispmf;
+nplates = s.nplates;
+alphalin = s.alphalin;
+b30 = s.b30;
+b1 = s.b1;
+gam = s.gam;
+dch = s.dch;
+prec = s.prec;
+resident = s.resident;
+betat = s.betat;
+db1 = s.db1;
+scal = s.scal;
 
-% ---- flag -> [g p s x]
-f = lower(flag);
-if ~ischar(f) || length(f) ~= 4
-    error('wrong flag. E.g. flag can be ''g---'',''gp--'',''-s--'', etc');
-end
-letters = 'gpsx';
-fls = [0 0 0 0];
-for k = 1:4
-    if f(k) == letters(k)
-        fls(k) = 1;
-    elseif f(k) ~= '-'
-        error('wrong flag. E.g. flag can be ''g---'',''gp--'',''-s--'', etc');
-    end
-end
-if fls(4) && ncol == 1
-    if ~fls(3)
-        error(['flag ''', f, ''' available only for channels separated']);
-    end
-    fls(4) = 0;                                  % a single field has no cross-phase partner
-end
-onestep = ~fls(3) && ~fls(4);                    % linear flags: one step over the whole fiber
-if ncol == 1 && fls(3) && ~fls(1) && ~fls(2)
-    onestep = true;                              % pure SPM of one field has an exact solution
-end
-if onestep
-    dphimaxt = Inf;
-    dzmaxt = x.length;
-else
-    dphimaxt = x.dphimax;
-    dzmaxt = x.dzmax;
-end
-
-% ---- birefringence
-isy = ~isempty(GSTATE.FIELDY);
-vector = fls(2) || isy;
+% ---- birefringence: the waveplates
 if fls(2)
-    manakov = isfield(x, 'manakov') && strcmp(x.manakov, 'yes');
-    if ~isfield(x, 'dgd')
-        error('Missing DGD in fiber');
-    end
-    given = isfield(x, 'db0') + isfield(x, 'theta') + isfield(x, 'epsilon');
-    ispmf = (given == 3);
-    if given == 3                                % user-defined plates (e.g. a PMF)
-        nplates = length(x.theta);
-        x.nplates = nplates;
+    if ispmf                                     % user-defined plates (e.g. a PMF)
         brf.db0 = x.db0;
         brf.theta = x.theta;
         brf.epsilon = x.epsilon;
-        dgdrms = x.dgd / nplates;
-    elseif given == 0                            % random plates, three uniform draws in this order
-        if ~isfield(x, 'nplates')
-            x.nplates = 100;
-        end
-        nplates = x.nplates;
+    else                                         % random plates, three uniform draws in this order
         brf.db0 = rand(nplates, 1) * 2 * pi - pi;
         brf.theta = rand(nplates, 1) * pi - 0.5 * pi;
         brf.epsilon = 0.5 * asin(rand(nplates, 1) * 2 - 1);
-        dgdrms = sqrt((3 * pi) / 8) * x.dgd / sqrt(nplates);
-    else
-        error('Missing one of db0, theta or epsilon in fiber');
     end
     brf.dgd = x.dgd;
-    dgdrms = dgdrms / GSTATE.SYMBOLRATE;
     if ~isy                                      % (isy keeps its value: the DELAY / DISP rows below follow it)
         GSTATE.FIELDY = zeros(size(GSTATE.FIELDX));
         warning('optilux:fiber', ['You are working with two polarizations ', ...
             'but in create_field you initialized just one polarization']);
     end
 else
-    manakov = false;
-    nplates = 1;
-    dgdrms = 0;
     brf.db0 = 0;
     brf.theta = 0;
     brf.epsilon = 0;
-end
-
-% ---- unit conversions
-alphalin = (log(10) * 1e-4) * x.alphadB;
-b20 = -x.lambda^2 / 2 / pi / c0 * x.disp * 1e-6;
-b30 = (x.lambda / 2 / pi / c0)^2 * (2 * x.lambda * x.disp + x.lambda^2 * x.slope) * 1e-6;
-b30 = b30 * fls(1);
-maxl = max(GSTATE.LAMBDA);
-minl = min(GSTATE.LAMBDA);
-lamc = 2 * maxl * minl / (maxl + minl);
-w_i0 = 2 * pi * c0 * (1 ./ GSTATE.LAMBDA - 1 / x.lambda);
-w_ic = 2 * pi * c0 * (1 ./ GSTATE.LAMBDA - 1 / lamc);
-w_c0 = 2 * pi * c0 * (1 ./ lamc - 1 / x.lambda);
-b1 = b20 * w_ic + 0.5 * b30 * (w_i0.^2 - w_c0^2);
-if ncol == 1
-    beta1 = 0;
-    w_i0 = 2 * pi * c0 * (1 / lamc - 1 / x.lambda);
-    gam = 2 * pi * x.n2 / (lamc * x.aeff) * 1e18;
-else
-    beta1 = b1;
-    gam = 2 * pi * x.n2 ./ (GSTATE.LAMBDA * x.aeff) * 1e18;
-end
-beta2 = (b20 + b30 * w_i0) * fls(1);
-dch = x.disp + x.slope * (GSTATE.LAMBDA - x.lambda);
-
-% ---- front-end options
-prec = 0;
-resident = 1;
-scalmode = 1;
-if isstruct(PMXOPT)
-    if isfield(PMXOPT, 'precision') && strcmp(PMXOPT.precision, 'f32')
-        prec = 1;
-    end
-    if isfield(PMXOPT, 'resident')
-        resident = double(PMXOPT.resident ~= 0);
-    end
-    if isfield(PMXOPT, 'scalar')
-        scalmode = double(PMXOPT.scalar ~= 0);
-    end
-end
-
-% ---- dispersion vectors (only built when they are returned or uploaded)
-betat = [];
-db1 = [];
-if nargout || ~scalmode
-    omega = 2 * pi * GSTATE.SYMBOLRATE * GSTATE.FN';
-    betat = zeros(nfft, ncol);
-    db1 = zeros(nfft, ncol);
-    for k = 1:ncol
-        betat(:, k) = omega * beta1(k) + 0.5 * omega.^2 * beta2(k) + omega.^3 * b30 / 6;
-        if fls(2)
-            db1(:, k) = dgdrms * omega;
-        end
-    end
-end
-scal = [];
-if scalmode
-    scal = [GSTATE.SYMBOLRATE, GSTATE.NSYMB, GSTATE.NT, b30, dgdrms, beta1(:)', beta2(:)'];
 end
 
 % ---- side effects on the global state

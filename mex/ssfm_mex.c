@@ -47,6 +47,16 @@
  *   [ux,uy] = ssfm_mex('ampliflat', ux, uy, gain, sigma, noise, asepol, opt)
  *       gain   linear power gain; sigma 1 x nfc; noise = Nfft x 2*nfc complex (options.noise, ampliflat.m:123-129) or a
  *              scalar seed of the device generator; asepol 1 = X, 2 = Y, 3 = both (options.onepol); opt as above
+ *   [ux,uy] = ssfm_mex('dbp', ux, uy, betat, db1, P, gam, fls, plates, scal, D, steplen, spansteps, band, opt)
+ *       digital backpropagation of a link (matlab/dbp.m; pmx_dbp_create / pmx_dbp_channel_create, pmx_dbp_exec)
+ *       ux ... scal, opt   as for 'fiber' (opt = [scalar_field precision resident]); the resident field is used the same way
+ *       D      [nspan gain steps_per_span xi pmd]: linear amplifier gain after every span (0: none), uniform steps per span
+ *              (0: the explicit schedule), fraction of gamma backpropagated, 1 = PMD-aware DBP
+ *       steplen   [] or the steps in forward order: one span's steps for every span, or with spansteps (1 x nspan step
+ *              counts) all spans' steps concatenated
+ *       plates [] or (nplates*nspan) x 3 [db0 theta epsilon], span k in rows (k-1)*nplates+1 .. k*nplates, forward order
+ *              (needs pmd = 1 and the 'p' flag)
+ *       band   [] or [shift decim]: single-channel DBP of the channel shift bins bring to baseband, on Nfft/decim samples
  *   ssfm_mex('reset')                    drops the resident field
  *   c = ssfm_mex('stats')                [uploads downloads resident_hits] since the MEX file was loaded
  *
@@ -587,6 +597,175 @@ static void cmd_ampliflat(int nlhs, mxArray *plhs[], int nrhs, const mxArray *pr
     release(f, nfft, nfc, precision, 1, resident, nlhs, plhs);
 }
 
+static void cmd_dbp(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[])
+{
+    /* prhs: 'dbp', ux, uy, betat, db1, P, gam, fls, plates, scal, D, steplen, spansteps, band, opt */
+    pmx_fiber_desc d;
+    pmx_dbp_desc g;
+    pmx_dbp_band b;
+    pmx_plan *plan = NULL;
+    pmx_devfield *f;
+    double gam_buf[PMX_MEX_MAX_NFC], beta_buf[2 * PMX_MEX_MAX_NFC];
+    const double *P, *D, *pl = NULL;
+    size_t nfft, nfc, n, k, j, np, nspan, nsteps = 0;
+    int scalar_field, precision, resident, rc, has_y, channel;
+    mxArray *work = NULL;
+    const mxArray *opt = prhs[14];
+
+    if (nrhs != 15 || nlhs > 2)
+        mexErrMsgTxt("[ux,uy] = ssfm_mex('dbp',ux,uy,betat,db1,P,gam,fls,plates,scal,D,steplen,spansteps,band,opt): "
+                     "wrong number of arguments.");
+    nfft = mxGetM(prhs[1]);
+    nfc = mxGetN(prhs[1]);
+    n = nfft * nfc;
+    if (n == 0)
+        mexErrMsgTxt("ssfm_mex: empty x field.");
+    if (nfc > PMX_MEX_MAX_NFC)
+        mexErrMsgTxt("ssfm_mex: at most 64 field columns.");
+    has_y = mxGetNumberOfElements(prhs[2]) != 0;
+    if (has_y && (mxGetM(prhs[2]) != nfft || mxGetN(prhs[2]) != nfc))
+        mexErrMsgTxt("ssfm_mex: ux and uy must have the same size.");
+    if (mxGetNumberOfElements(prhs[5]) != 6)
+        mexErrMsgTxt("ssfm_mex: P must be [dzmaxt dphimaxt alphalin Lf nplates manakov].");
+    if (mxGetNumberOfElements(prhs[7]) != 4)
+        mexErrMsgTxt("ssfm_mex: fls must have 4 elements.");
+    if (mxGetNumberOfElements(prhs[10]) != 5)
+        mexErrMsgTxt("ssfm_mex: D must be [nspan gain steps_per_span xi pmd].");
+    scalar_field = opt_at(opt, 0, 0.0) != 0.0;
+    precision = opt_at(opt, 1, 0.0) != 0.0 ? PMX_F32 : PMX_F64;
+    resident = opt_at(opt, 2, 0.0) != 0.0;
+    if (scalar_field && has_y)
+        mexErrMsgTxt("ssfm_mex: the scalar path takes no y field (fiber.m:253).");
+
+    /* the fiber: the same parsing as 'fiber' */
+    P = mxGetPr(prhs[5]);
+    memset(&d, 0, sizeof d);
+    d.nfft = (int64_t)nfft;
+    d.nfc = (int32_t)nfc;
+    d.batch = 1;
+    d.precision = precision;
+    d.dzmaxt = P[0];
+    d.dphimaxt = P[1];
+    d.alphalin = P[2];
+    d.length = P[3];
+    d.nplates = (int32_t)P[4];
+    d.manakov = P[5] != 0.0;
+    d.scalar_field = scalar_field;
+    for (k = 0; k < 4; k++)
+        d.fls[k] = mxGetPr(prhs[7])[k] != 0.0;
+    for (k = 0; k < nfc; k++)
+        gam_buf[k] = mxGetPr(prhs[6])[mxGetNumberOfElements(prhs[6]) == 1 ? 0 : k];
+    d.gam = gam_buf;
+    d.plate_sets = 1;
+    if (mxGetNumberOfElements(prhs[9]) != 0) {
+        const double *s = mxGetPr(prhs[9]);
+        if (mxGetNumberOfElements(prhs[9]) != 5 + 2 * nfc)
+            mexErrMsgTxt("ssfm_mex: scal must be [symbolrate nsymb nt b30 dgdrms beta1(1:nfc) beta2(1:nfc)].");
+        d.disp_mode = PMX_DISP_SCALAR;
+        d.symbolrate = s[0];
+        d.nsymb = (int32_t)s[1];
+        d.nt = (int32_t)s[2];
+        d.b30 = s[3];
+        d.dgdrms = s[4];
+        for (k = 0; k < 2 * nfc; k++)
+            beta_buf[k] = s[5 + k];
+        d.beta1 = beta_buf;
+        d.beta2 = beta_buf + nfc;
+    } else {
+        if (mxGetM(prhs[3]) != nfft || mxGetN(prhs[3]) != nfc)
+            mexErrMsgTxt("ssfm_mex: betat must be Nfft x nfc.");
+        d.disp_mode = PMX_DISP_VECTOR;
+        d.betat = mxGetPr(prhs[3]);
+        d.db1 = (mxGetNumberOfElements(prhs[4]) == n) ? mxGetPr(prhs[4]) : NULL;
+    }
+
+    /* the link: D, the step schedule, the waveplates of every span */
+    D = mxGetPr(prhs[10]);
+    memset(&g, 0, sizeof g);
+    g.nspan = (int32_t)D[0];
+    g.gain = D[1];
+    g.steps_per_span = (int32_t)D[2];
+    g.xi = D[3];
+    g.pmd = D[4] != 0.0;
+    if (g.nspan < 1)
+        mexErrMsgTxt("ssfm_mex: D(1), the number of spans, must be at least 1.");
+    nspan = (size_t)g.nspan;
+    np = (size_t)(d.nplates > 0 ? d.nplates : 0);
+    if (g.pmd) {
+        if (mxGetM(prhs[8]) != np * nspan || mxGetN(prhs[8]) != 3 || np == 0)
+            mexErrMsgTxt("ssfm_mex: PMD-aware DBP: plates must be (nplates*nspan) x 3 [db0 theta epsilon].");
+        pl = mxGetPr(prhs[8]);
+    } else if (mxGetNumberOfElements(prhs[8]) != 0) {
+        mexErrMsgTxt("ssfm_mex: plates are given only for PMD-aware DBP (D(5) = 1).");
+    }
+    if (mxGetNumberOfElements(prhs[11]) != 0) { /* explicit schedule: steplen in forward order, spansteps per span */
+        const double *sl = mxGetPr(prhs[11]), *ss = mxGetPr(prhs[12]);
+        const size_t nl = mxGetNumberOfElements(prhs[11]), nss = mxGetNumberOfElements(prhs[12]);
+        double *buf;
+        int32_t *cnt;
+        if (g.steps_per_span != 0)
+            mexErrMsgTxt("ssfm_mex: give steps_per_span (D(3)) or steplen, not both.");
+        if (nss != 0 && nss != nspan)
+            mexErrMsgTxt("ssfm_mex: spansteps must give the steps of every span.");
+        nsteps = nss ? nl : nl * nspan; /* without spansteps, steplen is one span's steps, repeated for every span */
+        work = mxCreateDoubleMatrix(nsteps + nspan, 1, mxREAL);
+        buf = mxGetPr(work);
+        cnt = (int32_t *)(buf + nsteps);
+        if (nss) {
+            size_t tot = 0;
+            for (k = 0; k < nspan; k++) {
+                if (!(ss[k] >= 1.0) || ss[k] != floor(ss[k]))
+                    mexErrMsgTxt("ssfm_mex: spansteps must hold positive integers.");
+                cnt[k] = (int32_t)ss[k];
+                tot += (size_t)cnt[k];
+            }
+            if (tot != nl)
+                mexErrMsgTxt("ssfm_mex: steplen must hold sum(spansteps) steps.");
+            memcpy(buf, sl, nl * sizeof(double));
+        } else {
+            for (k = 0; k < nspan; k++) {
+                cnt[k] = (int32_t)nl;
+                for (j = 0; j < nl; j++)
+                    buf[k * nl + j] = sl[j];
+            }
+        }
+        g.step_len = buf;
+        g.span_steps = cnt;
+    } else if (mxGetNumberOfElements(prhs[12]) != 0) {
+        mexErrMsgTxt("ssfm_mex: spansteps needs steplen.");
+    }
+    channel = mxGetNumberOfElements(prhs[13]) != 0;
+    if (channel) {
+        if (mxGetNumberOfElements(prhs[13]) != 2)
+            mexErrMsgTxt("ssfm_mex: band must be [shift decim].");
+        memset(&b, 0, sizeof b);
+        b.shift = (int64_t)mxGetPr(prhs[13])[0];
+        b.decim = (int32_t)mxGetPr(prhs[13])[1];
+    }
+
+    ensure_ctx();
+    rc = channel ? pmx_dbp_channel_create(g_ctx, &d, &g, &b, &plan) : pmx_dbp_create(g_ctx, &d, &g, &plan);
+    if (work)
+        mxDestroyArray(work); /* the plan has taken the schedule */
+    if (rc != PMX_OK) {
+        if (d.fls[3] && !scalar_field)
+            mexErrMsgTxt("The CNLSE with separate fields is not yet implemented"); /* fiber.m:854 */
+        fail("ssfm_mex: DBP plan creation failed");
+    }
+    if (g.pmd && pmx_dbp_set_plates(plan, 1, pl, pl + np * nspan, pl + 2 * np * nspan) != PMX_OK) {
+        pmx_plan_destroy(plan);
+        fail("ssfm_mex: DBP waveplates rejected");
+    }
+    f = acquire(prhs[1], prhs[2], precision);
+    rc = pmx_dbp_exec(plan, f);
+    pmx_plan_destroy(plan);
+    if (rc != PMX_OK) {
+        pmx_field_destroy(f); /* part-way through the link: not usable */
+        fail("ssfm_mex: backpropagation failed");
+    }
+    release(f, nfft, nfc, precision, !scalar_field, resident, nlhs, plhs);
+}
+
 /* complex mxArray (split storage) -> interleaved re,im in a fresh mxArray-owned buffer of 2*n doubles */
 static double *interleave(const mxArray *a, size_t n, mxArray **owner)
 {
@@ -771,12 +950,14 @@ static void command(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[])
         cmd_cohmix(nlhs, plhs, nrhs, prhs);
     } else if (!strcmp(cmd, "invpmd")) {
         cmd_invpmd(nlhs, plhs, nrhs, prhs);
+    } else if (!strcmp(cmd, "dbp")) {
+        cmd_dbp(nlhs, plhs, nrhs, prhs);
     } else if (!strcmp(cmd, "reset")) {
         drop_resident();
     } else if (!strcmp(cmd, "stats")) {
         plhs[0] = mxCreateDoubleMatrix(1, 3, mxREAL);
         memcpy(mxGetPr(plhs[0]), g_stats, sizeof g_stats);
     } else {
-        mexErrMsgTxt("ssfm_mex: unknown command (fiber, ampliflat, cohmix, invpmd, reset, stats).");
+        mexErrMsgTxt("ssfm_mex: unknown command (fiber, ampliflat, cohmix, invpmd, dbp, reset, stats).");
     }
 }
