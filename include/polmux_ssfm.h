@@ -293,6 +293,19 @@ int pmx_dbp_create(pmx_ctx* ctx, const pmx_fiber_desc* fiber, const pmx_dbp_desc
  * and sign, as pmx_link_desc takes them; plate_sets is 1 (shared by the batch) or batch.  The library reverses and
  * negates them and rebuilds the step packages on the device; calling it again swaps in a new draw. */
 int pmx_dbp_set_plates(pmx_plan* plan, int32_t plate_sets, const double* db0, const double* theta, const double* epsilon);
+/* Filtered DBP (Du & Lowery 2010): a Gaussian low-pass with a one-sided -3 dB bandwidth bw, in DFT bins of the plan's grid,
+ *   H[k] = exp(-(ln 2 / 2) * (k_s / bw)^2),  k_s the signed bin in [-N/2, N/2)
+ * (H(0) = 1, |H(bw)|^2 = 1/2, real, even, a real and positive impulse response), on the intensity of every backward
+ * nonlinear step N(-xi*gam, h): each quantity the step computes from |u|^2 is replaced by ifft(fft(q) .* H), the rest of
+ * the step is unchanged.  Two polarizations: the phase uses the filtered |ux|^2+|uy|^2 and, CNLSE, the s3 rotation the
+ * filtered s3 (P + i*s3 is filtered as one complex signal).  Scalar path: every |u_j|^2 of nl_step is the filtered one;
+ * with the 'x' flag the sum over the columns is taken over the filtered powers.  bw = 0: no filter (the plan runs as it
+ * did before any call).  Calling it again swaps the bandwidth.  On a single-channel plan (pmx_dbp_channel_create) it applies
+ * to the M-sample plan: the bins are equally spaced on both grids, so the same bw is the same frequency.
+ * On the three passes a filtered step adds pass C' without its nonlinear epilogue, two pointwise kernels and a filter
+ * plan (pmx_filter_create) on a work field of ceil(batch*nfc/2) columns.  PMX_ERR_INVALID for a negative or non-finite
+ * bw and for a plan that is not a DBP plan. */
+int pmx_dbp_set_filter(pmx_plan* plan, double bw);
 /* In place on a resident field; returns when the field is backpropagated.  The field may belong to another context of
  * the same device (as for pmx_fiber_exec).  A PMD-aware plan needs its plates first (PMX_ERR_INVALID).  Destroy the
  * plan with pmx_plan_destroy. */

@@ -19,6 +19,8 @@ function dbp(x, flag, options)
 %                span order; needs the 'p' flag: PMD-aware DBP through those waveplates
 %     ich, decim single-channel DBP of channel ICH of a one-column ('unique') field, on Nfft/DECIM samples;
 %                afterwards the field holds that channel alone, on its own bins
+%     filter_bw  filtered DBP: one-sided -3 dB bandwidth [GHz] of a Gaussian low-pass on the intensity of every
+%                nonlinear step (absent: none)
 %
 %   Without brf the 'p' flag is dropped: no plates are drawn and nothing is taken from the RAND stream.  The
 %   nonlinear model stays the one FIBER used: Manakov when x.manakov is 'yes' and the flag has 'p', else the
@@ -136,6 +138,9 @@ manakov = pflag && isfield(x, 'manakov') && strcmp(x.manakov, 'yes');
 % ---- the backpropagation: one gateway call for the whole link
 P = [s.dzmaxt, s.dphimaxt, s.alphalin, x.length, s.nplates, double(manakov)];
 D = [nspan, gain, steps, xi, double(pmd)];
+if isfield(options, 'filter_bw')                 % in bins of GSTATE.FN
+    D = [D, options.filter_bw * GSTATE.NSYMB / GSTATE.SYMBOLRATE];
+end
 if s.vector
     [GSTATE.FIELDX, GSTATE.FIELDY] = ssfm_mex('dbp', GSTATE.FIELDX, GSTATE.FIELDY, s.betat, s.db1, P, s.gam, fls, ...
         plates, s.scal, D, steplen, spansteps, band, [0, s.prec, s.resident]);

@@ -50,8 +50,9 @@
  *   [ux,uy] = ssfm_mex('dbp', ux, uy, betat, db1, P, gam, fls, plates, scal, D, steplen, spansteps, band, opt)
  *       digital backpropagation of a link (matlab/dbp.m; pmx_dbp_create / pmx_dbp_channel_create, pmx_dbp_exec)
  *       ux ... scal, opt   as for 'fiber' (opt = [scalar_field precision resident]); the resident field is used the same way
- *       D      [nspan gain steps_per_span xi pmd]: linear amplifier gain after every span (0: none), uniform steps per span
- *              (0: the explicit schedule), fraction of gamma backpropagated, 1 = PMD-aware DBP
+ *       D      [nspan gain steps_per_span xi pmd] or [nspan gain steps_per_span xi pmd bw]: linear amplifier gain after
+ *              every span (0: none), uniform steps per span (0: the explicit schedule), fraction of gamma backpropagated,
+ *              1 = PMD-aware DBP, and for filtered DBP the Gaussian's one-sided -3 dB bandwidth in bins (pmx_dbp_set_filter)
  *       steplen   [] or the steps in forward order: one span's steps for every span, or with spansteps (1 x nspan step
  *              counts) all spans' steps concatenated
  *       plates [] or (nplates*nspan) x 3 [db0 theta epsilon], span k in rows (k-1)*nplates+1 .. k*nplates, forward order
@@ -629,8 +630,8 @@ static void cmd_dbp(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[])
         mexErrMsgTxt("ssfm_mex: P must be [dzmaxt dphimaxt alphalin Lf nplates manakov].");
     if (mxGetNumberOfElements(prhs[7]) != 4)
         mexErrMsgTxt("ssfm_mex: fls must have 4 elements.");
-    if (mxGetNumberOfElements(prhs[10]) != 5)
-        mexErrMsgTxt("ssfm_mex: D must be [nspan gain steps_per_span xi pmd].");
+    if (mxGetNumberOfElements(prhs[10]) != 5 && mxGetNumberOfElements(prhs[10]) != 6)
+        mexErrMsgTxt("ssfm_mex: D must be [nspan gain steps_per_span xi pmd] or [nspan gain steps_per_span xi pmd bw].");
     scalar_field = opt_at(opt, 0, 0.0) != 0.0;
     precision = opt_at(opt, 1, 0.0) != 0.0 ? PMX_F32 : PMX_F64;
     resident = opt_at(opt, 2, 0.0) != 0.0;
@@ -755,6 +756,10 @@ static void cmd_dbp(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[])
     if (g.pmd && pmx_dbp_set_plates(plan, 1, pl, pl + np * nspan, pl + 2 * np * nspan) != PMX_OK) {
         pmx_plan_destroy(plan);
         fail("ssfm_mex: DBP waveplates rejected");
+    }
+    if (mxGetNumberOfElements(prhs[10]) == 6 && pmx_dbp_set_filter(plan, D[5]) != PMX_OK) {
+        pmx_plan_destroy(plan);
+        fail("ssfm_mex: DBP filter bandwidth rejected");
     }
     f = acquire(prhs[1], prhs[2], precision);
     rc = pmx_dbp_exec(plan, f);

@@ -34,7 +34,7 @@ EXPORTS = [
     'pmx_host_is_pinned', 'pmx_scalar_adaptive_run', 'pmx_mc_run', 'pmx_mc_nccl_available',
     'pmx_ampliflat_exec_at', 'pmx_dsp_count', 'pmx_field_mean_power', 'pmx_pmd_matrix', 'pmx_field_jones', 'pmx_filter_create', 'pmx_field_copy_cols', 'pmx_field_modulate',
     'pmx_cohmix_exec', 'pmx_field_mean_power_xy', 'pmx_cohmix_run', 'pmx_dsp_phases', 'pmx_field_quantize', 'pmx_inverse_pmd_run',
-    'pmx_dbp_create', 'pmx_dbp_exec', 'pmx_dbp_set_plates', 'pmx_dbp_channel_create',
+    'pmx_dbp_create', 'pmx_dbp_exec', 'pmx_dbp_set_plates', 'pmx_dbp_channel_create', 'pmx_dbp_set_filter',
 ]
 
 
@@ -185,6 +185,7 @@ def load():
     lib.pmx_dbp_create.argtypes = [vp, C.POINTER(FiberDesc), C.POINTER(DbpDesc), C.POINTER(vp)]
     lib.pmx_dbp_exec.argtypes = [vp, vp]
     lib.pmx_dbp_set_plates.argtypes = [vp, C.c_int32, _dp, _dp, _dp]
+    lib.pmx_dbp_set_filter.argtypes = [vp, C.c_double]
     lib.pmx_dbp_channel_create.argtypes = [vp, C.POINTER(FiberDesc), C.POINTER(DbpDesc), C.POINTER(DbpBand), C.POINTER(vp)]
     _lib = lib
     return lib
@@ -550,6 +551,11 @@ class DbpPlan(Plan):
         if not (a.size == b.size == c.size == n):
             raise ValueError('plates must be [nspan][plate_sets][nplates] = %d values each' % n)
         self.ctx.check(self.ctx.lib.pmx_dbp_set_plates(self.h, int(plate_sets), _ptr(a), _ptr(b), _ptr(c)))
+
+    def set_filter(self, bw_bins):
+        """filtered DBP (pmx_dbp_set_filter): a Gaussian low-pass of one-sided -3 dB bandwidth bw_bins, in DFT bins of the
+        plan's grid, on the intensity of every nonlinear step; 0 switches it off"""
+        self.ctx.check(self.ctx.lib.pmx_dbp_set_filter(self.h, float(bw_bins)))
 
 
 def make_band(shift, decim):

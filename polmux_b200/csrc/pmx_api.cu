@@ -253,6 +253,12 @@ struct pmx_plan {
     pmx_devfield* ch_work = nullptr;
     long long ch_shift = 0;
     int ch_log2r = 0;
+    // filtered DBP (pmx_dbp_set_filter, bw > 0): on-chip, H/N over the transform length; on the three passes, the filter plan
+    // of the Gaussian response and its work field (the intensity of two realization-columns per Sa)
+    double filt_bw = 0.0;
+    double* filt_hn_d = nullptr;
+    pmx_plan* filt = nullptr;
+    pmx_devfield* filt_work = nullptr;
 };
 
 static int set_err(pmx_ctx* ctx, int code, const char* fmt, ...) {
@@ -778,6 +784,9 @@ extern "C" void pmx_plan_destroy(pmx_plan* p) {
     pmx_plan_destroy(p->ch_dbp);
     pmx_plan_destroy(p->ch_band);
     pmx_field_destroy(p->ch_work);
+    if (p->filt_hn_d) cudaFreeAsync(p->filt_hn_d, st);
+    pmx_plan_destroy(p->filt);
+    pmx_field_destroy(p->filt_work);
     delete p;
 }
 
@@ -3555,6 +3564,53 @@ __global__ void __launch_bounds__(128) pmx_k_dbp_pkg(const DbpGeo* __restrict__ 
 
 static int dbp_channel_exec(pmx_plan* p, pmx_devfield* fld);
 
+// Filtered DBP (polmux_ssfm.h): the Gaussian H[k] = exp(-(ln 2/2) (k_s/bw)^2) at the signed bin k_s of the plan's grid.
+extern "C" int pmx_dbp_set_filter(pmx_plan* p, double bw) {
+    if (!(bw >= 0) || !std::isfinite(bw))
+        return set_err(p ? p->ctx : nullptr, PMX_ERR_INVALID, "pmx_dbp_set_filter: bw must be finite and >= 0 (0: no filter), got %g", bw);
+    if (!p) return set_err(nullptr, PMX_ERR_INVALID, "pmx_dbp_set_filter: null plan");
+    pmx_ctx* c = p->ctx;
+    if (!p->dbp) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_set_filter: not a digital-backpropagation plan");
+    if (p->ch_dbp) return pmx_dbp_set_filter(p->ch_dbp, bw);   // single-channel DBP: the same bins on the M-sample grid
+    CK(c, cudaSetDevice(c->device));
+    CK(c, cudaStreamSynchronize(c->stream));   // no queued work still reads the old response
+    if (p->filt_hn_d) CK(c, cudaFreeAsync(p->filt_hn_d, c->stream));
+    p->filt_hn_d = nullptr;
+    pmx_plan_destroy(p->filt);
+    p->filt = nullptr;
+    pmx_field_destroy(p->filt_work);
+    p->filt_work = nullptr;
+    p->filt_bw = 0.0;
+    if (bw == 0.0) return PMX_OK;
+    const int64_t N = p->d.nfft;
+    const double a = 0.5 * std::log(2.0);
+    std::vector<double> H((size_t)N);
+    for (int64_t k = 0; k < N; ++k) {
+        const double ks = (double)(k < N / 2 ? k : k - N) / bw;
+        H[k] = std::exp(-a * (ks * ks));
+    }
+    int rc = PMX_OK;
+    if (p->onchip) {   // H/N: the kernel's inverse transform is unscaled
+        for (auto& v : H) v *= p->fc.invN;
+        CK(c, cudaMallocAsync(&p->filt_hn_d, H.size() * sizeof(double), c->stream));
+        CK(c, cudaMemcpyAsync(p->filt_hn_d, H.data(), H.size() * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+        CK(c, cudaStreamSynchronize(c->stream));
+    } else {
+        std::vector<double> Hc(2 * (size_t)N, 0.0);
+        for (int64_t k = 0; k < N; ++k) Hc[2 * k] = H[k];
+        const int nw = (p->d.batch * p->d.nfc + 1) / 2;   // two realization-columns per Sa
+        rc = pmx_filter_create(c, N, 1, nw, p->d.precision, Hc.data(), 1, &p->filt);
+        if (!rc) rc = pmx_field_create(c, N, 1, nw, p->d.precision, &p->filt_work);
+        if (rc) {
+            pmx_plan_destroy(p->filt);
+            p->filt = nullptr;
+            return rc;
+        }
+    }
+    p->filt_bw = bw;
+    return PMX_OK;
+}
+
 extern "C" int pmx_dbp_set_plates(pmx_plan* p, int32_t sets, const double* db0, const double* theta, const double* epsilon) {
     if (!p) return set_err(nullptr, PMX_ERR_INVALID, "pmx_dbp_set_plates: null plan");
     if (p->ch_dbp) return pmx_dbp_set_plates(p->ch_dbp, sets, db0, theta, epsilon);   // single-channel DBP: its M-sample plan
@@ -3804,6 +3860,50 @@ extern "C" int pmx_dbp_create(pmx_ctx* c, const pmx_fiber_desc* fd, const pmx_db
     return PMX_OK;
 }
 
+// Filtered DBP on the three passes, per step: passes A and B, pass C' without its nonlinear epilogue (spm = 0 makes
+// pmx_nl_step a no-op), the intensity into the work field, the filter plan on it, and the nonlinear step from the filtered
+// intensity.  The filter plan runs on the context's stream, so the realization groups join before it.
+static int dbp_filtered_passes(pmx_plan* p, pmx_devfield* fld, const PassParams& pa, PassGroups& gs) {
+    pmx_ctx* c = p->ctx;
+    const int batch = p->d.batch;
+    FiberConst fc_lin = p->fc_c;
+    fc_lin.spm = 0;
+    const dim3 grid((unsigned)std::min<int64_t>((p->d.nfft + 255) / 256, 148 * 4), (unsigned)(batch * p->d.nfc));
+    int rev[4] = {1, 1, 1, 1};
+    for (size_t s = 0; s < p->sched_idx.size(); ++s) {
+        StepPkg* pk = p->sched + (size_t)p->sched_idx[s] * batch;
+        int rc = fork_groups(c, gs.n);
+        if (rc) return rc;
+        for (int gi = 0; gi < gs.n; ++gi) {
+            PassGroup& G = gs.g[gi];
+            G.pA.pkg = G.pB.pkg = pk + G.b0;
+            if (p->dbp_pmd)
+                G.pB.plates = p->plates + ((size_t)p->sched_span[s] * p->fc.plate_sets + (p->fc.plate_sets > 1 ? G.b0 : 0)) *
+                                              p->fc.nplates;
+            G.pA.reverse = (rev[gi] ^= 1);
+            CK(c, p->tA->passA(G.gA, G.st, G.pA, p->fc_a, fld->map_rows));
+            G.pB.reverse = (rev[gi] ^= 1);
+            CK(c, p->tB->passB(G.gB, G.st, G.pB, p->fc_c, fld->map_cols));
+            G.pA.reverse = (rev[gi] ^= 1);
+            CK(c, p->tA->passC_nl(G.gC, G.st, G.pA, fc_lin, fld->map_rows));
+            c->launches += 3;
+        }
+        CK(c, cudaGetLastError());
+        rc = join_groups(c, gs.n);
+        if (rc) return rc;
+        p->tA->dbp_intensity(grid, c->stream, pa, p->fc_c, p->filt_work->data);
+        c->launches++;
+        CK(c, cudaGetLastError());
+        rc = pmx_fiber_exec(p->filt, p->filt_work, nullptr);
+        if (rc) return rc;
+        p->tA->dbp_nl_filt(grid, c->stream, pa, p->fc_c, p->filt_work->data, pk);
+        c->launches++;
+        CK(c, cudaGetLastError());
+    }
+    CK(c, cudaStreamSynchronize(c->stream));
+    return PMX_OK;
+}
+
 extern "C" int pmx_dbp_exec(pmx_plan* p, pmx_devfield* fld) {
     if (!p || !fld) return set_err(nullptr, PMX_ERR_INVALID, "pmx_dbp_exec: null argument");
     pmx_ctx* c = p->ctx;
@@ -3833,7 +3933,10 @@ extern "C" int pmx_dbp_exec(pmx_plan* p, pmx_devfield* fld) {
         ds.nstep = (int)p->sched_idx.size();
         ds.pkg_bytes = p->dbp_pmd ? (int)sizeof(StepPkg) : PMX_PKG_HEAD;   // without PMD no step reads past the header
         ds.plate_stride = (long long)p->fc.plate_sets * p->fc.nplates;
-        CK(c, p->tB->onchip_dbp(p->d.nfc, batch, c->stream, q, p->fc_c, ds));
+        if (p->filt_bw > 0)
+            CK(c, p->tB->onchip_dbp_filt(p->d.nfc, batch, c->stream, q, p->fc_c, DbpFiltSteps{ds, p->filt_hn_d}));
+        else
+            CK(c, p->tB->onchip_dbp(p->d.nfc, batch, c->stream, q, p->fc_c, ds));
         c->launches += 1;
         CK(c, cudaStreamSynchronize(c->stream));
         return PMX_OK;
@@ -3842,6 +3945,7 @@ extern "C" int pmx_dbp_exec(pmx_plan* p, pmx_devfield* fld) {
     PassGroups gs;
     rc = plan_groups(p, fld, pa, pA, pB, c->setup_done[p->N1 + 65536 * p->d.precision].cnl, true, gs);
     if (rc) return rc;
+    if (p->filt_bw > 0) return dbp_filtered_passes(p, fld, pa, gs);
     rc = fork_groups(c, gs.n);
     if (rc) return rc;
     int rev[4] = {1, 1, 1, 1};

@@ -173,6 +173,14 @@ struct DbpSteps {
     int pkg_bytes;          // bytes of a package the steps read: the header alone without PMD, all of it with
     long long plate_stride; // PlateConst per span: plate_sets * nplates
 };
+// Filtered DBP on the single-launch kernel (pmx_dbp_set_filter): the step table and the Gaussian response over the
+// transform length, hn[k] = H(k)/N at the unsigned bin k.  Its own type, so that its instances are new ones.
+struct DbpFiltSteps {
+    DbpSteps s;
+    const double* hn;       // [L]
+};
+__host__ __device__ __forceinline__ DbpSteps pmx_dbp_steps(const DbpSteps& s) { return s; }
+__host__ __device__ __forceinline__ DbpSteps pmx_dbp_steps(const DbpFiltSteps& s) { return s.s; }
 
 __device__ __forceinline__ cpx cmul(cpx a, cpx b) { return mkc(a.x * b.x - a.y * b.y, a.x * b.y + a.y * b.x); }
 __device__ __forceinline__ cpx cmulc(cpx a, cpx b) {  // a * conj(b)

@@ -461,6 +461,83 @@ __device__ __forceinline__ void pmx_nl_step(cpx (&x)[8], cpx (&y)[8], const Step
     }
 }
 
+// pmx_nl_step of filtered DBP (pmx_dbp_set_filter): every quantity the step computes from |u|^2 comes filtered, the rest
+// is unchanged.  pw: the filtered power (|ux|^2+|uy|^2, on the scalar path |u|^2 of the column); aux: the filtered s3
+// (CNLSE) or, on the scalar path with the 'x' flag, the sum over the columns of the filtered powers.
+template <int NQ>
+__device__ __forceinline__ void pmx_nl_step_filt(cpx (&x)[NQ], cpx (&y)[NQ], const real (&pw)[NQ], const real (&aux)[NQ],
+                                                 double leff, const FiberConst& f, int col) {
+    if (f.scalar_field) {
+        if (f.spm || f.xpm) {
+            const real ngam = (real)(-f.gam[col]), rl = (real)leff;
+#pragma unroll
+            for (int q = 0; q < NQ; ++q) {
+                real p = pw[q];
+                if (f.xpm) p = f.spm ? R_ADD(R_MUL((real)2, aux[q]), -p) : R_MUL((real)2, R_ADD(aux[q], -p));
+                x[q] = cmul(x[q], pmx_cis_r(R_MUL(R_MUL(ngam, p), rl)));
+            }
+        }
+#pragma unroll
+        for (int q = 0; q < NQ; ++q) y[q] = mkc((real)0, (real)0);
+    } else if (f.spm) {
+        const real gamleff = (real)__dmul_rn(f.gam[col], leff);
+#pragma unroll
+        for (int q = 0; q < NQ; ++q) {
+            const cpx e = pmx_cis_r(R_MUL(-gamleff, pw[q]));
+            x[q] = cmul(x[q], e);
+            y[q] = cmul(y[q], e);
+        }
+        if (!f.manakov) {   // the s3 rotation with the filtered s3
+#pragma unroll
+            for (int q = 0; q < NQ; ++q) {
+                const cpx e = pmx_cis_r(R_MUL(gamleff, aux[q]) / (real)3.0);
+                const cpx ux = x[q], uy = y[q];
+                x[q] = mkc(e.x * ux.x + e.y * uy.x, e.x * ux.y + e.y * uy.y);
+                y[q] = mkc(e.x * uy.x - e.y * ux.x, e.x * uy.y - e.y * ux.y);
+            }
+        }
+    }
+}
+
+// The intensity filtered DBP low-passes, P + i*s3 (s3 = 0 for Manakov) of the two-polarization sample (x, y).
+__device__ __forceinline__ cpx pmx_dbp_intensity(cpx x, cpx y, const FiberConst& f) {
+    return mkc(power_ref(x, y), f.manakov ? (real)0 : (real)2.0 * (x.x * y.y - x.y * y.x));
+}
+
+// Filtered DBP on the three passes, two pointwise kernels around the filter plan (grid.y: realization-columns bc).
+// pmx_k_dbp_intensity writes P + i*s3 of column bc into the work field, two columns per Sa: column bc/2, slot bc&1 (X, Y);
+// an odd last column leaves its Y slot zero.  Both fields have N samples per column in the same layout.
+static __global__ void __launch_bounds__(256) pmx_k_dbp_intensity(PassParams p, FiberConst f, cpx* __restrict__ work) {
+    const int bc = blockIdx.y, nbc = p.batch * f.nfc;
+    const size_t N = (size_t)p.N1 * p.N2;
+    const cpx* fld = reinterpret_cast<const cpx*>(p.field) + (size_t)bc * N * 2;
+    cpx* w = work + (size_t)(bc >> 1) * N * 2 + (bc & 1);
+    const bool pad = (bc & 1) == 0 && bc + 1 == nbc;
+    for (size_t n = (size_t)blockIdx.x * blockDim.x + threadIdx.x; n < N; n += (size_t)gridDim.x * blockDim.x) {
+        cpx x, y;
+        ld_sa(fld + 2 * n, x, y);
+        w[2 * n] = pmx_dbp_intensity(x, y, f);
+        if (pad) w[2 * n + 1] = mkc((real)0, (real)0);
+    }
+}
+// pmx_k_dbp_nl_filt: N(-xi*gam, h) of the step package pkg[b] from the filtered intensity in the work field
+static __global__ void __launch_bounds__(256) pmx_k_dbp_nl_filt(PassParams p, FiberConst f, const cpx* __restrict__ work,
+                                                                const StepPkg* __restrict__ pkg) {
+    const int bc = blockIdx.y, b = bc / f.nfc, col = bc - b * f.nfc;
+    const size_t N = (size_t)p.N1 * p.N2;
+    cpx* fld = reinterpret_cast<cpx*>(p.field) + (size_t)bc * N * 2;
+    const cpx* w = work + (size_t)(bc >> 1) * N * 2 + (bc & 1);
+    const double leff = pkg[b].leff;
+    for (size_t n = (size_t)blockIdx.x * blockDim.x + threadIdx.x; n < N; n += (size_t)gridDim.x * blockDim.x) {
+        cpx x[1], y[1];
+        ld_sa(fld + 2 * n, x[0], y[0]);
+        const cpx q = w[2 * n];
+        const real pw[1] = {q.x}, s3[1] = {q.y};
+        pmx_nl_step_filt(x, y, pw, s3, leff, f, col);
+        st_sa(fld + 2 * n, x[0], y[0]);
+    }
+}
+
 // ---------------------------------------------------------------------------
 // Tile walk shared by the three passes (persistent CTAs): tile -> (realization-column bc, group inside it),
 // serpentine direction, skipping finished realizations.

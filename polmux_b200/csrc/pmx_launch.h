@@ -38,6 +38,12 @@ struct PmxLaunchTable {
     // digital backpropagation of a small field: the on-chip kernel walking the plan's step table (pmx_k_onchip<..., true>),
     // launched like onchip (set up by onchip_setup)
     cudaError_t (*onchip_dbp)(int nfc, int batch, cudaStream_t s, const PassParams& p, const FiberConst& f, const DbpSteps& ds);
+    // filtered DBP (pmx_dbp_set_filter): the on-chip kernel with the Gaussian response (pmx_k_onchip<..., DbpFiltSteps>), and
+    // on the three passes the intensity into the work field and the nonlinear step from the filtered one (grid.y = batch*nfc)
+    cudaError_t (*onchip_dbp_filt)(int nfc, int batch, cudaStream_t s, const PassParams& p, const FiberConst& f,
+                                   const DbpFiltSteps& ds);
+    void (*dbp_intensity)(dim3 grid, cudaStream_t s, const PassParams& p, const FiberConst& f, void* work);
+    void (*dbp_nl_filt)(dim3 grid, cudaStream_t s, const PassParams& p, const FiberConst& f, const void* work, const StepPkg* pkg);
 };
 
 const PmxLaunchTable* pmx_get_table(int L, int precision = 0);  // nullptr if L is not built

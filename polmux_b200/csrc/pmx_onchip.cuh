@@ -16,7 +16,11 @@
 // exp(+alpha*h/2)/N (times 1/sqrt(G) on the first step of a span), on the scalar path with 'x' the cluster-wide
 // sum_j |u_j|^2, and the nonlinear step with gam -> -xi*gam: pass A, B and C' of a DBP step on the three-pass route.
 // No max reduction, no step control, no StepCtl write-back; the next step's package is fetched while this step runs.
+// Filtered DBP (the step table is a DbpFiltSteps: pmx_dbp_set_filter): after the scale the field is parked in registers,
+// the intensity it drives the nonlinear step with (P + i*s3, on the scalar path |u|^2) is transformed in the CTA,
+// multiplied by H/N at the thread's bins and transformed back, and the nonlinear step runs from the filtered quantities.
 #pragma once
+#include <type_traits>
 #include <cooperative_groups.h>
 #include "pmx_kernels.cuh"
 
@@ -63,6 +67,7 @@ __device__ __forceinline__ unsigned long long pmx_block_max_t0(unsigned long lon
 template <typename R, int L, bool SC, bool DBP = false, typename... Steps>
 __global__ void __launch_bounds__((L / 8) < 32 ? 32 : (L / 8), 1) pmx_k_onchip(PassParams p, FiberConst f, Steps... steps) {
     static_assert(sizeof...(Steps) == (DBP ? 1 : 0), "the DBP instances take one DbpSteps, the forward ones nothing");
+    constexpr bool FILT = (std::is_same<Steps, DbpFiltSteps>::value || ... || false);
     using S = OnchipSmem<L>;
     constexpr int T = L / 8;
     constexpr bool PRE = SC;
@@ -124,7 +129,7 @@ __global__ void __launch_bounds__((L / 8) < 32 ? 32 : (L / 8), 1) pmx_k_onchip(P
         }
     };
     if constexpr (DBP) {
-        const DbpSteps ds{steps...};
+        const DbpSteps ds = pmx_dbp_steps(steps...);
         // a thread's bins after the full-length transform: k = t + q*T, q < 4 positive frequencies, q >= 4 negative
         const double dfn = (double)T * f.inv_nsymb;
         const double fn0 = (double)tt * f.inv_nsymb;
@@ -171,8 +176,58 @@ __global__ void __launch_bounds__((L / 8) < 32 ? 32 : (L / 8), 1) pmx_k_onchip(P
                 x[q] = mkc(x[q].x * sc, x[q].y * nsc);
                 y[q] = mkc(y[q].x * sc, y[q].y * nsc);
             }
-            if (f.xpm) xpm_sum();   // over the backpropagated columns (the transform has released the exchange buffer)
-            pmx_nl_step(x, y, st, f, col);   // ---- N(-xi*gam): the gam of f is the backpropagated one
+            if constexpr (FILT) {
+                const double* hn = (steps.hn, ...);
+                cpx u[8], v[8];   // the field, parked while its intensity is filtered
+                real pw[8], aux[8];
+#pragma unroll
+                for (int q = 0; q < 8; ++q) {
+                    u[q] = x[q];
+                    v[q] = y[q];
+                    x[q] = f.scalar_field ? mkc(R_ADD(R_MUL(u[q].x, u[q].x), R_MUL(u[q].y, u[q].y)), (real)0)
+                                          : pmx_dbp_intensity(u[q], v[q], f);
+                    y[q] = mkc((real)0, (real)0);
+                }
+                // ifft(fft(q) .* H): forward transform, H/N at the thread's bins (conjugated), forward transform = conj(result)
+                CtaFFT<R, L>::run(x, y, work, work + L, tt, stw);
+#pragma unroll
+                for (int q = 0; q < 8; ++q) {
+                    const real h = (real)__ldg(&hn[tt + q * T]);
+                    x[q] = mkc(x[q].x * h, -(x[q].y * h));
+                    y[q] = mkc((real)0, (real)0);
+                }
+                CtaFFT<R, L>::run(x, y, work, work + L, tt, stw);
+#pragma unroll
+                for (int q = 0; q < 8; ++q) {
+                    pw[q] = x[q].x;
+                    aux[q] = -x[q].y;
+                }
+                if (f.scalar_field && f.xpm) {   // sum over the columns of the filtered powers, left to right
+                    real* sp = reinterpret_cast<real*>(work);
+                    if (live) {
+#pragma unroll
+                        for (int q = 0; q < 8; ++q) sp[t + q * T] = pw[q];
+                    }
+                    cluster.sync();
+#pragma unroll
+                    for (int q = 0; q < 8; ++q) aux[q] = (real)0;
+                    for (int k = 0; k < f.nfc; ++k) {
+                        const real* rp = cluster.map_shared_rank(sp, k);
+#pragma unroll
+                        for (int q = 0; q < 8; ++q) aux[q] = R_ADD(aux[q], rp[tt + q * T]);
+                    }
+                    cluster.sync();
+                }
+#pragma unroll
+                for (int q = 0; q < 8; ++q) {
+                    x[q] = u[q];
+                    y[q] = v[q];
+                }
+                pmx_nl_step_filt(x, y, pw, aux, st->leff, f, col);   // ---- N(-xi*gam) from the filtered intensity
+            } else {
+                if (f.xpm) xpm_sum();   // over the backpropagated columns (the transform has released the exchange buffer)
+                pmx_nl_step(x, y, st, f, col);   // ---- N(-xi*gam): the gam of f is the backpropagated one
+            }
             __syncthreads();   // the package is read: the next one lands
             if (s + 1 < ds.nstep) {
                 land();

@@ -107,7 +107,13 @@ cudaError_t onchip_setup() {
     if (e != cudaSuccess) return e;
     e = cudaFuncSetAttribute(pmx_k_onchip<real, L, true, true, DbpSteps>, cudaFuncAttributeMaxDynamicSharedMemorySize, SO::TOTAL);
     if (e != cudaSuccess) return e;
-    return cudaFuncSetAttribute(pmx_k_onchip<real, L, false, true, DbpSteps>, cudaFuncAttributeMaxDynamicSharedMemorySize, SO::TOTAL);
+    e = cudaFuncSetAttribute(pmx_k_onchip<real, L, false, true, DbpSteps>, cudaFuncAttributeMaxDynamicSharedMemorySize, SO::TOTAL);
+    if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(pmx_k_onchip<real, L, true, true, DbpFiltSteps>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             SO::TOTAL);
+    if (e != cudaSuccess) return e;
+    return cudaFuncSetAttribute(pmx_k_onchip<real, L, false, true, DbpFiltSteps>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                SO::TOTAL);
 }
 // the forward run (no step table) or digital backpropagation (one DbpSteps)
 template <bool DBP, typename... Steps>
@@ -133,6 +139,16 @@ cudaError_t onchip(int nfc, int batch, cudaStream_t s, const PassParams& p, cons
 cudaError_t onchip_dbp(int nfc, int batch, cudaStream_t s, const PassParams& p, const FiberConst& f, const DbpSteps& ds) {
     return onchip_launch<true>(nfc, batch, s, p, f, ds);
 }
+cudaError_t onchip_dbp_filt(int nfc, int batch, cudaStream_t s, const PassParams& p, const FiberConst& f, const DbpFiltSteps& ds) {
+    return onchip_launch<true>(nfc, batch, s, p, f, ds);
+}
+// filtered DBP on the three passes: the pointwise kernels around the filter plan (grid.y = batch * nfc)
+void dbp_intensity(dim3 grid, cudaStream_t s, const PassParams& p, const FiberConst& f, void* work) {
+    pmx_k_dbp_intensity<<<grid, 256, 0, s>>>(p, f, reinterpret_cast<cpx*>(work));
+}
+void dbp_nl_filt(dim3 grid, cudaStream_t s, const PassParams& p, const FiberConst& f, const void* work, const StepPkg* pkg) {
+    pmx_k_dbp_nl_filt<<<grid, 256, 0, s>>>(p, f, reinterpret_cast<const cpx*>(work), pkg);
+}
 }  // namespace
 
 #define PMX_CAT2(a, b) a##b
@@ -145,4 +161,5 @@ cudaError_t onchip_dbp(int nfc, int batch, cudaStream_t s, const PassParams& p, 
 extern const PmxLaunchTable PMX_TABLE_NAME = {
     L, GAC, GB, PFAC ? 1 : 0, PFB ? 1 : 0, SA::THREADS, SB::THREADS, (size_t)SA::TOTAL, (size_t)SB::TOTAL,
     pmx_tw_total(L), pmx_tw_layout(L), PmxTw4<L>::LO, PmxTw4<L>::PER, PMX_PRECISION, (int)sizeof(cpx),
-    setup, passA, passB, passC, init_max, fill_tw4, xpm_sum, (size_t)SO::TOTAL, onchip_setup, onchip, passC_nl, onchip_dbp};
+    setup, passA, passB, passC, init_max, fill_tw4, xpm_sum, (size_t)SO::TOTAL, onchip_setup, onchip, passC_nl, onchip_dbp,
+    onchip_dbp_filt, dbp_intensity, dbp_nl_filt};

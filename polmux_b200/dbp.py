@@ -34,14 +34,16 @@ from .gstate import GSTATE
 def dbp_plan(ctx: _lib.Context, setup: FiberSetup, nspan: int = 1, gain_db: Optional[float] = None,
              steps_per_span: Optional[int] = None, step_len=None, span_steps=None, xi: float = 1.0, batch: int = 1,
              precision: Optional[str] = None, disp_mode: Optional[str] = None, plates=None, shift: Optional[int] = None,
-             decim: Optional[int] = None) -> _lib.DbpPlan:
+             decim: Optional[int] = None, filter_bw: Optional[float] = None) -> _lib.DbpPlan:
     """The DBP of nspan spans of the fiber `setup` describes, for resident fields of `batch` realizations.  Schedule:
     steps_per_span uniform steps per span (default 1), or step_len -- one span's steps in forward order for every span,
     or with span_steps [nspan] all spans' steps concatenated.  plates: None -- the 'p' flag, plates and dgdrms are
     ignored; (db0, theta, epsilon), each [nspan][plate_sets][nplates] in forward order (plate_sets 1 or batch) -- PMD-aware
     DBP through those waveplates (setup must carry the 'p' flag; DbpPlan.set_plates swaps in another draw).
     decim: single-channel DBP of a one-column field -- the channel that `shift` bins bring to baseband (the receiver's
-    ndfn; default 0), backpropagated on nfft/decim samples (pmx_dbp_channel_create)."""
+    ndfn; default 0), backpropagated on nfft/decim samples (pmx_dbp_channel_create).
+    filter_bw [GHz]: filtered DBP -- a Gaussian low-pass of that one-sided -3 dB bandwidth on the intensity of every
+    nonlinear step (DbpPlan.set_filter, in bins of GSTATE.FN: filter_bw * NSYMB / SYMBOLRATE); None or 0: none."""
     if plates is not None and not setup.fls[1]:
         raise ValueError("PMD-aware DBP (plates given) needs a fiber with the 'p' flag")
     if decim is None and shift is not None:
@@ -54,19 +56,21 @@ def dbp_plan(ctx: _lib.Context, setup: FiberSetup, nspan: int = 1, gain_db: Opti
                              pmd=plates is not None)
     band = None if decim is None else _lib.make_band(shift or 0, decim)
     plan = _lib.DbpPlan(ctx, desc, keep, d, dkeep, band)
-    if plates is not None:
-        try:
+    try:
+        if plates is not None:
             arrs = [np.asarray(a, dtype=np.float64).reshape(int(nspan), -1, setup.nplates) for a in plates]
             plan.set_plates(*arrs, plate_sets=arrs[0].shape[1])
-        except Exception:
-            plan.close()
-            raise
+        if filter_bw is not None:
+            plan.set_filter(float(filter_bw) * GSTATE.NSYMB / GSTATE.SYMBOLRATE)
+    except Exception:
+        plan.close()
+        raise
     return plan
 
 
 def dbp(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, steps_per_span: Optional[int] = None, step_len=None,
         span_steps=None, xi: float = 1.0, ctx: Optional[_lib.Context] = None, precision: Optional[str] = None, brf=None,
-        ich: Optional[int] = None, decim: Optional[int] = None):
+        ich: Optional[int] = None, decim: Optional[int] = None, filter_bw: Optional[float] = None):
     """Backpropagates GSTATE.FIELDX / FIELDY in place through nspan spans of the fiber x, the amplifier of gain_db [dB]
     after each (None: no amplifier).  x and flag are what fiber() takes; a field without FIELDY runs the scalar path, the
     'x' flag there backpropagating the cross-phase modulation of all columns.  Without brf the flag's 'p' is dropped (no plates
@@ -74,7 +78,8 @@ def dbp(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, steps_per
     Manakov when x.manakov is 'yes' and the flag has 'p', else the CNLSE.  brf: the struct fiber() returned (every span
     the same plates) or a list of nspan of them in forward span order, with 'p' in the flag: PMD-aware DBP through those
     plates.  xi: fraction of gamma backpropagated.  ich, decim: single-channel DBP of channel ich (1-based) of a 'unique'
-    multiplex on nfft/decim samples; afterwards the field holds that channel alone, on its own bins.  The field stays
+    multiplex on nfft/decim samples; afterwards the field holds that channel alone, on its own bins.  filter_bw [GHz]:
+    filtered DBP, a Gaussian low-pass of that one-sided -3 dB bandwidth on the intensity of every nonlinear step.  The field stays
     resident on the device like fiber() and ampliflat() leave it."""
     G = GSTATE
     f = str(flag).lower()
@@ -123,7 +128,7 @@ def dbp(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, steps_per
         try:
             fld.upload(fx, np.zeros_like(fx))
             plan = dbp_plan(ctx, s, nspan, gain_db, steps_per_span, step_len, span_steps, xi, precision=precision,
-                            shift=shift, decim=decim)
+                            shift=shift, decim=decim, filter_bw=filter_bw)
             try:
                 plan.execute(fld)
             finally:
@@ -136,7 +141,7 @@ def dbp(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, steps_per
     fld, hx, hy = G.take_device(ctx, prec)
     try:
         plan = dbp_plan(ctx, s, nspan, gain_db, steps_per_span, step_len, span_steps, xi, precision=precision, plates=plates,
-                        shift=shift, decim=decim)
+                        shift=shift, decim=decim, filter_bw=filter_bw)
     except Exception:
         G.restore_host(fld, hx, hy)     # nothing ran: the caller's field is as it was
         raise

@@ -64,6 +64,8 @@ def scalar_case(nsymb, nt, nch, flag):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--reps', type=int, default=20)
+    ap.add_argument('--filter-bw', type=float, default=None,
+                    help='also filtered DBP [GHz] with the same steps, alternated with the forward run and plain DBP')
     ap.add_argument('--out', default=None, help='directory for dbp_small_time.json')
     a = ap.parse_args()
     ctx = _lib.default_context(0)
@@ -86,9 +88,16 @@ def main():
         dbp = dbp_plan(ctx, s, 1, None, step_len=dz, batch=B)
         fld.broadcast_from(tx)
         dbp.execute(fld)                                           # warm-up
-        t = {'forward': [], 'dbp': []}
-        for _ in range(a.reps):                                    # the two alternate
-            for what, run in (('forward', lambda: fwd.execute(fld)), ('dbp', lambda: dbp.execute(fld))):
+        runs = [('forward', lambda: fwd.execute(fld)), ('dbp', lambda: dbp.execute(fld))]
+        filt = None
+        if a.filter_bw is not None:
+            filt = dbp_plan(ctx, s, 1, None, step_len=dz, batch=B, filter_bw=a.filter_bw)
+            fld.broadcast_from(tx)
+            filt.execute(fld)                                      # warm-up
+            runs.append(('filtered', lambda: filt.execute(fld)))
+        t = {what: [] for what, _ in runs}
+        for _ in range(a.reps):                                    # they alternate
+            for what, run in runs:
                 fld.broadcast_from(tx)
                 ctx.sync()
                 t0 = time.perf_counter()
@@ -96,6 +105,8 @@ def main():
                 t[what].append(time.perf_counter() - t0)
         fwd.close()
         dbp.close()
+        if filt is not None:
+            filt.close()
         fld.close()
         tx.close()
         row = dict(case=name, batch=B, nfft=n, nfc=nfc, steps=steps)
@@ -105,6 +116,10 @@ def main():
                              gsa_steps_per_s=B * nfc * n * steps / med / 1e9)
         row['dbp_vs_forward'] = row['dbp']['gsa_steps_per_s'] / row['forward']['gsa_steps_per_s']
         rows.append(row)
+        if filt is not None:
+            print('%-26s batch %5d  filtered dbp %8.2f us/step %7.2f GSa*steps/s | filtered/dbp %.3f'
+                  % (name, B, row['filtered']['us_per_step'], row['filtered']['gsa_steps_per_s'],
+                     row['filtered']['gsa_steps_per_s'] / row['dbp']['gsa_steps_per_s']))
         print('%-26s batch %5d  %3d steps | forward %8.2f us/step %7.2f GSa*steps/s | dbp %8.2f us/step %7.2f GSa*steps/s'
               ' | dbp/forward %.3f' % (name, B, steps, row['forward']['us_per_step'], row['forward']['gsa_steps_per_s'],
                                        row['dbp']['us_per_step'], row['dbp']['gsa_steps_per_s'], row['dbp_vs_forward']))

@@ -48,6 +48,8 @@ def main():
     ap.add_argument('--nspan', type=int, default=10)
     ap.add_argument('--reps', type=int, default=3)
     ap.add_argument('--pmd', action='store_true', help="the 'gps-' link with 100 plates; PMD-aware DBP and the equaliser too")
+    ap.add_argument('--filter-bw', type=float, default=None,
+                    help='filtered DBP [GHz] at 1, 2 and 4 steps per span, alternated with the plain plan in this process')
     ap.add_argument('--out', default=None, help='directory for dbp_time.json')
     a = ap.parse_args()
     try:
@@ -78,8 +80,8 @@ def main():
     link, lkeep = _lib.make_link(a.nspan, gain)
     rows = []
 
-    def timed(name, run, steps_of):
-        for rep in range(a.reps + 1):              # the first call warms up (module load, tables)
+    def timed(name, run, steps_of, reps=None):
+        for rep in range((a.reps if reps is None else reps) + 1):   # the first call warms up (module load, tables)
             fld.broadcast_from(tx)
             ctx.sync()
             t0 = time.perf_counter()
@@ -106,6 +108,15 @@ def main():
         plan = dbp_plan(ctx, s, a.nspan, 16.0, steps_per_span=m, batch=B)
         timed('dbp M=%d' % m, lambda: plan.execute(fld), lambda _r, m=m: m * a.nspan * B)
         plan.close()
+    if a.filter_bw is not None:
+        for m in (1, 2, 4):
+            plans = [('dbp M=%d' % m, dbp_plan(ctx, s, a.nspan, 16.0, steps_per_span=m, batch=B)),
+                     ('filtered M=%d' % m, dbp_plan(ctx, s, a.nspan, 16.0, steps_per_span=m, batch=B, filter_bw=a.filter_bw))]
+            for _ in range(a.reps):
+                for name, pl in plans:
+                    timed(name, lambda pl=pl: pl.execute(fld), lambda _r, m=m: m * a.nspan * B, reps=1)
+            for _, pl in plans:
+                pl.close()
     if a.pmd:
         for m in (1, 4, 16):
             plan = dbp_plan(ctx, s, a.nspan, 16.0, steps_per_span=m, batch=B, plates=plates)
