@@ -304,8 +304,24 @@ int pmx_dbp_set_plates(pmx_plan* plan, int32_t plate_sets, const double* db0, co
  * to the M-sample plan: the bins are equally spaced on both grids, so the same bw is the same frequency.
  * On the three passes a filtered step adds pass C' without its nonlinear epilogue, two pointwise kernels and a filter
  * plan (pmx_filter_create) on a work field of ceil(batch*nfc/2) columns.  PMX_ERR_INVALID for a negative or non-finite
- * bw and for a plan that is not a DBP plan. */
+ * bw, for a plan that is not a DBP plan, and for bw > 0 on a plan that has taps (pmx_dbp_set_taps). */
 int pmx_dbp_set_filter(pmx_plan* plan, double bw);
+/* Enhanced split-step DBP (ESSFM; Secondini, Marsella, Forestieri, ECOC 2014): a real circular FIR on the intensity of
+ * every backward nonlinear step N(-xi*gam, h).  taps c[0..2K], ntaps = 2K+1 odd, 1 <= ntaps <= 65 (K <= 32) and at most
+ * the number of samples of the plan's grid; c[K] is lag 0.  At time index n of the grid (indices mod N, the sum taken
+ * left to right in m)
+ *   q~[n] = sum_{m=-K..K} c[m+K] * q[(n - m) mod N],
+ * and every quantity the step computes from |u|^2 is replaced by its q~; the rest of the step is unchanged.  Two
+ * polarizations: q = P + i*s3 (s3 = 0 for Manakov), as filtered DBP filters it; scalar path: every |u_j|^2, with the
+ * 'x' flag the column sum taken over the filtered powers.  This is filtered DBP with H = fft(c placed circularly), but
+ * it costs a time-domain FIR, not a transform: on the three passes a step adds pass C' without its nonlinear epilogue,
+ * the intensity into a work field of ceil(batch*nfc/2) columns and one kernel that applies the FIR and the nonlinear
+ * step.  The same taps serve every step.  ntaps = 0 (taps may then be NULL): no taps, the plan runs as it did before any
+ * call.  Calling it again swaps the taps.  On a single-channel plan (pmx_dbp_channel_create) the taps act on the
+ * M-sample grid: one tap there spans r = N/M samples of the full field.  PMX_ERR_INVALID for an even ntaps or more than
+ * 65, a non-finite tap, more taps than samples, a plan that is not a DBP plan, and taps on a plan that has a filter
+ * bandwidth (pmx_dbp_set_filter). */
+int pmx_dbp_set_taps(pmx_plan* plan, int32_t ntaps, const double* taps);
 /* In place on a resident field; returns when the field is backpropagated.  The field may belong to another context of
  * the same device (as for pmx_fiber_exec).  A PMD-aware plan needs its plates first (PMX_ERR_INVALID).  Destroy the
  * plan with pmx_plan_destroy. */

@@ -21,6 +21,9 @@ function dbp(x, flag, options)
 %                afterwards the field holds that channel alone, on its own bins
 %     filter_bw  filtered DBP: one-sided -3 dB bandwidth [GHz] of a Gaussian low-pass on the intensity of every
 %                nonlinear step (absent: none)
+%     taps       enhanced split-step DBP: a row or column of 2K+1 <= 65 real FIR taps, taps(K+1) at lag 0, applied
+%                circularly on the time grid to the intensity of every nonlinear step (absent or []: none; not with
+%                filter_bw).  With decim the grid is the channel's Nfft/DECIM samples: one tap spans DECIM samples
 %
 %   Without brf the 'p' flag is dropped: no plates are drawn and nothing is taken from the RAND stream.  The
 %   nonlinear model stays the one FIBER used: Manakov when x.manakov is 'yes' and the flag has 'p', else the
@@ -141,10 +144,30 @@ D = [nspan, gain, steps, xi, double(pmd)];
 if isfield(options, 'filter_bw')                 % in bins of GSTATE.FN
     D = [D, options.filter_bw * GSTATE.NSYMB / GSTATE.SYMBOLRATE];
 end
-if s.vector
+taps = [];                                       % the gateway's optional last argument
+if isfield(options, 'taps') && ~isempty(options.taps)
+    taps = double(options.taps(:)');
+    if mod(numel(taps), 2) ~= 1 || numel(taps) > 65
+        error('pmx_dbp_set_taps: ntaps must be odd and at most 65 (0: no taps), got %d', numel(taps));
+    end
+    bad = find(isnan(taps) | isinf(taps));
+    if ~isempty(bad)
+        error('pmx_dbp_set_taps: tap %d is not finite', bad(1) - 1);
+    end
+    if isfield(options, 'filter_bw') && options.filter_bw ~= 0
+        error('pmx_dbp_set_taps: the plan has a filter bandwidth (pmx_dbp_set_filter); a plan takes one or the other');
+    end
+end
+if s.vector && isempty(taps)
     [GSTATE.FIELDX, GSTATE.FIELDY] = ssfm_mex('dbp', GSTATE.FIELDX, GSTATE.FIELDY, s.betat, s.db1, P, s.gam, fls, ...
         plates, s.scal, D, steplen, spansteps, band, [0, s.prec, s.resident]);
-else
+elseif s.vector
+    [GSTATE.FIELDX, GSTATE.FIELDY] = ssfm_mex('dbp', GSTATE.FIELDX, GSTATE.FIELDY, s.betat, s.db1, P, s.gam, fls, ...
+        plates, s.scal, D, steplen, spansteps, band, [0, s.prec, s.resident], taps);
+elseif isempty(taps)
     GSTATE.FIELDX = ssfm_mex('dbp', GSTATE.FIELDX, [], s.betat, s.db1, P, s.gam, fls, [], s.scal, D, steplen, ...
         spansteps, band, [1, s.prec, s.resident]);
+else
+    GSTATE.FIELDX = ssfm_mex('dbp', GSTATE.FIELDX, [], s.betat, s.db1, P, s.gam, fls, [], s.scal, D, steplen, ...
+        spansteps, band, [1, s.prec, s.resident], taps);
 end

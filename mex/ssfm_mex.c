@@ -47,7 +47,7 @@
  *   [ux,uy] = ssfm_mex('ampliflat', ux, uy, gain, sigma, noise, asepol, opt)
  *       gain   linear power gain; sigma 1 x nfc; noise = Nfft x 2*nfc complex (options.noise, ampliflat.m:123-129) or a
  *              scalar seed of the device generator; asepol 1 = X, 2 = Y, 3 = both (options.onepol); opt as above
- *   [ux,uy] = ssfm_mex('dbp', ux, uy, betat, db1, P, gam, fls, plates, scal, D, steplen, spansteps, band, opt)
+ *   [ux,uy] = ssfm_mex('dbp', ux, uy, betat, db1, P, gam, fls, plates, scal, D, steplen, spansteps, band, opt[, taps])
  *       digital backpropagation of a link (matlab/dbp.m; pmx_dbp_create / pmx_dbp_channel_create, pmx_dbp_exec)
  *       ux ... scal, opt   as for 'fiber' (opt = [scalar_field precision resident]); the resident field is used the same way
  *       D      [nspan gain steps_per_span xi pmd] or [nspan gain steps_per_span xi pmd bw]: linear amplifier gain after
@@ -58,6 +58,8 @@
  *       plates [] or (nplates*nspan) x 3 [db0 theta epsilon], span k in rows (k-1)*nplates+1 .. k*nplates, forward order
  *              (needs pmd = 1 and the 'p' flag)
  *       band   [] or [shift decim]: single-channel DBP of the channel shift bins bring to baseband, on Nfft/decim samples
+ *       taps   absent or [], or enhanced split-step DBP: the real FIR c(1..2K+1) on the intensity of every nonlinear step,
+ *              c(K+1) at lag 0 (pmx_dbp_set_taps)
  *   ssfm_mex('reset')                    drops the resident field
  *   c = ssfm_mex('stats')                [uploads downloads resident_hits] since the MEX file was loaded
  *
@@ -600,7 +602,7 @@ static void cmd_ampliflat(int nlhs, mxArray *plhs[], int nrhs, const mxArray *pr
 
 static void cmd_dbp(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[])
 {
-    /* prhs: 'dbp', ux, uy, betat, db1, P, gam, fls, plates, scal, D, steplen, spansteps, band, opt */
+    /* prhs: 'dbp', ux, uy, betat, db1, P, gam, fls, plates, scal, D, steplen, spansteps, band, opt[, taps] */
     pmx_fiber_desc d;
     pmx_dbp_desc g;
     pmx_dbp_band b;
@@ -613,8 +615,8 @@ static void cmd_dbp(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[])
     mxArray *work = NULL;
     const mxArray *opt = prhs[14];
 
-    if (nrhs != 15 || nlhs > 2)
-        mexErrMsgTxt("[ux,uy] = ssfm_mex('dbp',ux,uy,betat,db1,P,gam,fls,plates,scal,D,steplen,spansteps,band,opt): "
+    if ((nrhs != 15 && nrhs != 16) || nlhs > 2)
+        mexErrMsgTxt("[ux,uy] = ssfm_mex('dbp',ux,uy,betat,db1,P,gam,fls,plates,scal,D,steplen,spansteps,band,opt[,taps]): "
                      "wrong number of arguments.");
     nfft = mxGetM(prhs[1]);
     nfc = mxGetN(prhs[1]);
@@ -760,6 +762,11 @@ static void cmd_dbp(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[])
     if (mxGetNumberOfElements(prhs[10]) == 6 && pmx_dbp_set_filter(plan, D[5]) != PMX_OK) {
         pmx_plan_destroy(plan);
         fail("ssfm_mex: DBP filter bandwidth rejected");
+    }
+    if (nrhs == 16 && mxGetNumberOfElements(prhs[15]) != 0 &&
+        pmx_dbp_set_taps(plan, (int32_t)mxGetNumberOfElements(prhs[15]), mxGetPr(prhs[15])) != PMX_OK) {
+        pmx_plan_destroy(plan);
+        fail("ssfm_mex: DBP taps rejected");
     }
     f = acquire(prhs[1], prhs[2], precision);
     rc = pmx_dbp_exec(plan, f);

@@ -35,6 +35,7 @@ EXPORTS = [
     'pmx_ampliflat_exec_at', 'pmx_dsp_count', 'pmx_field_mean_power', 'pmx_pmd_matrix', 'pmx_field_jones', 'pmx_filter_create', 'pmx_field_copy_cols', 'pmx_field_modulate',
     'pmx_cohmix_exec', 'pmx_field_mean_power_xy', 'pmx_cohmix_run', 'pmx_dsp_phases', 'pmx_field_quantize', 'pmx_inverse_pmd_run',
     'pmx_dbp_create', 'pmx_dbp_exec', 'pmx_dbp_set_plates', 'pmx_dbp_channel_create', 'pmx_dbp_set_filter',
+    'pmx_dbp_set_taps',
 ]
 
 
@@ -186,6 +187,7 @@ def load():
     lib.pmx_dbp_exec.argtypes = [vp, vp]
     lib.pmx_dbp_set_plates.argtypes = [vp, C.c_int32, _dp, _dp, _dp]
     lib.pmx_dbp_set_filter.argtypes = [vp, C.c_double]
+    lib.pmx_dbp_set_taps.argtypes = [vp, C.c_int32, _dp]
     lib.pmx_dbp_channel_create.argtypes = [vp, C.POINTER(FiberDesc), C.POINTER(DbpDesc), C.POINTER(DbpBand), C.POINTER(vp)]
     _lib = lib
     return lib
@@ -556,6 +558,27 @@ class DbpPlan(Plan):
         """filtered DBP (pmx_dbp_set_filter): a Gaussian low-pass of one-sided -3 dB bandwidth bw_bins, in DFT bins of the
         plan's grid, on the intensity of every nonlinear step; 0 switches it off"""
         self.ctx.check(self.ctx.lib.pmx_dbp_set_filter(self.h, float(bw_bins)))
+
+    def set_taps(self, taps):
+        """enhanced split-step DBP (pmx_dbp_set_taps): the real circular FIR taps c[0..2K] (c[K] at lag 0) on the intensity
+        of every nonlinear step, on the plan's grid; None or [] switches them off"""
+        a = check_taps(taps)
+        self.ctx.check(self.ctx.lib.pmx_dbp_set_taps(self.h, int(a.size), _ptr(a) if a.size else None))
+
+
+MAX_TAPS = 65
+
+
+def check_taps(taps) -> np.ndarray:
+    """-> the taps as a contiguous float64 vector (empty: no taps); ValueError with pmx_dbp_set_taps's message for what
+    it refuses without a plan: an even count, more than MAX_TAPS, a non-finite tap"""
+    a = np.ascontiguousarray(np.asarray([] if taps is None else taps, dtype=np.float64).ravel())
+    if a.size > MAX_TAPS or (a.size and a.size % 2 == 0):
+        raise ValueError('pmx_dbp_set_taps: ntaps must be odd and at most %d (0: no taps), got %d' % (MAX_TAPS, a.size))
+    bad = np.flatnonzero(~np.isfinite(a))
+    if bad.size:
+        raise ValueError('pmx_dbp_set_taps: tap %d is not finite' % bad[0])
+    return a
 
 
 def make_band(shift, decim):

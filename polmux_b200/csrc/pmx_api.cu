@@ -259,6 +259,11 @@ struct pmx_plan {
     double* filt_hn_d = nullptr;
     pmx_plan* filt = nullptr;
     pmx_devfield* filt_work = nullptr;
+    // enhanced split-step DBP (pmx_dbp_set_taps, ntaps > 0): the taps, and on the three passes the work field the intensity
+    // goes to before its FIR (two realization-columns per Sa)
+    int ntaps = 0;
+    DbpTaps taps{};
+    pmx_devfield* tap_work = nullptr;
 };
 
 static int set_err(pmx_ctx* ctx, int code, const char* fmt, ...) {
@@ -787,6 +792,7 @@ extern "C" void pmx_plan_destroy(pmx_plan* p) {
     if (p->filt_hn_d) cudaFreeAsync(p->filt_hn_d, st);
     pmx_plan_destroy(p->filt);
     pmx_field_destroy(p->filt_work);
+    pmx_field_destroy(p->tap_work);
     delete p;
 }
 
@@ -3572,6 +3578,8 @@ extern "C" int pmx_dbp_set_filter(pmx_plan* p, double bw) {
     pmx_ctx* c = p->ctx;
     if (!p->dbp) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_set_filter: not a digital-backpropagation plan");
     if (p->ch_dbp) return pmx_dbp_set_filter(p->ch_dbp, bw);   // single-channel DBP: the same bins on the M-sample grid
+    if (bw > 0 && p->ntaps > 0)
+        return set_err(c, PMX_ERR_INVALID, "pmx_dbp_set_filter: the plan has FIR taps (pmx_dbp_set_taps); a plan takes one or the other");
     CK(c, cudaSetDevice(c->device));
     CK(c, cudaStreamSynchronize(c->stream));   // no queued work still reads the old response
     if (p->filt_hn_d) CK(c, cudaFreeAsync(p->filt_hn_d, c->stream));
@@ -3608,6 +3616,39 @@ extern "C" int pmx_dbp_set_filter(pmx_plan* p, double bw) {
         }
     }
     p->filt_bw = bw;
+    return PMX_OK;
+}
+
+// Enhanced split-step DBP (polmux_ssfm.h): the taps c[0..2k] of the FIR on the intensity of every nonlinear step.
+extern "C" int pmx_dbp_set_taps(pmx_plan* p, int32_t ntaps, const double* taps) {
+    pmx_ctx* c = p ? p->ctx : nullptr;
+    if (ntaps < 0 || ntaps > PMX_MAX_TAPS || (ntaps > 0 && ntaps % 2 == 0))
+        return set_err(c, PMX_ERR_INVALID, "pmx_dbp_set_taps: ntaps must be odd and at most %d (0: no taps), got %d", PMX_MAX_TAPS, ntaps);
+    if (ntaps > 0 && !taps) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_set_taps: null taps");
+    for (int j = 0; j < ntaps; ++j)
+        if (!std::isfinite(taps[j])) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_set_taps: tap %d is not finite", j);
+    if (!p) return set_err(nullptr, PMX_ERR_INVALID, "pmx_dbp_set_taps: null plan");
+    if (!p->dbp) return set_err(c, PMX_ERR_INVALID, "pmx_dbp_set_taps: not a digital-backpropagation plan");
+    if (p->ch_dbp) return pmx_dbp_set_taps(p->ch_dbp, ntaps, taps);   // single-channel DBP: the taps act on the M-sample grid
+    if (ntaps > 0 && p->filt_bw > 0)
+        return set_err(c, PMX_ERR_INVALID, "pmx_dbp_set_taps: the plan has a filter bandwidth (pmx_dbp_set_filter); a plan takes one or the other");
+    if (ntaps > p->d.nfft)
+        return set_err(c, PMX_ERR_INVALID, "pmx_dbp_set_taps: %d taps on a grid of %lld samples", ntaps, (long long)p->d.nfft);
+    CK(c, cudaSetDevice(c->device));
+    CK(c, cudaStreamSynchronize(c->stream));   // no queued work still reads the old work field
+    pmx_field_destroy(p->tap_work);
+    p->tap_work = nullptr;
+    p->ntaps = 0;
+    p->taps = DbpTaps{};
+    if (ntaps == 0) return PMX_OK;
+    if (!p->onchip) {
+        const int nw = (p->d.batch * p->d.nfc + 1) / 2;   // two realization-columns per Sa
+        const int rc = pmx_field_create(c, p->d.nfft, 1, nw, p->d.precision, &p->tap_work);
+        if (rc) return rc;
+    }
+    p->taps.k = ntaps / 2;
+    for (int j = 0; j < ntaps; ++j) p->taps.c[j] = taps[j];
+    p->ntaps = ntaps;
     return PMX_OK;
 }
 
@@ -3860,9 +3901,10 @@ extern "C" int pmx_dbp_create(pmx_ctx* c, const pmx_fiber_desc* fd, const pmx_db
     return PMX_OK;
 }
 
-// Filtered DBP on the three passes, per step: passes A and B, pass C' without its nonlinear epilogue (spm = 0 makes
-// pmx_nl_step a no-op), the intensity into the work field, the filter plan on it, and the nonlinear step from the filtered
-// intensity.  The filter plan runs on the context's stream, so the realization groups join before it.
+// Filtered and enhanced split-step DBP on the three passes, per step: passes A and B, pass C' without its nonlinear
+// epilogue (spm = 0 makes pmx_nl_step a no-op), the intensity into the work field, then either the filter plan on it and
+// the nonlinear step from the filtered intensity, or the nonlinear step from the FIR of the taps (pmx_k_dbp_nl_fir).  The
+// filter plan runs on the context's stream, so the realization groups join before it.
 static int dbp_filtered_passes(pmx_plan* p, pmx_devfield* fld, const PassParams& pa, PassGroups& gs) {
     pmx_ctx* c = p->ctx;
     const int batch = p->d.batch;
@@ -3891,6 +3933,12 @@ static int dbp_filtered_passes(pmx_plan* p, pmx_devfield* fld, const PassParams&
         CK(c, cudaGetLastError());
         rc = join_groups(c, gs.n);
         if (rc) return rc;
+        if (p->ntaps > 0) {
+            p->tA->dbp_intensity(grid, c->stream, pa, p->fc_c, p->tap_work->data);
+            CK(c, p->tA->dbp_nl_fir(c->stream, pa, p->fc_c, p->tap_work->data, pk, p->taps));
+            c->launches += 2;
+            continue;
+        }
         p->tA->dbp_intensity(grid, c->stream, pa, p->fc_c, p->filt_work->data);
         c->launches++;
         CK(c, cudaGetLastError());
@@ -3933,7 +3981,9 @@ extern "C" int pmx_dbp_exec(pmx_plan* p, pmx_devfield* fld) {
         ds.nstep = (int)p->sched_idx.size();
         ds.pkg_bytes = p->dbp_pmd ? (int)sizeof(StepPkg) : PMX_PKG_HEAD;   // without PMD no step reads past the header
         ds.plate_stride = (long long)p->fc.plate_sets * p->fc.nplates;
-        if (p->filt_bw > 0)
+        if (p->ntaps > 0)
+            CK(c, p->tB->onchip_dbp_taps(p->d.nfc, batch, c->stream, q, p->fc_c, DbpTapSteps{ds, p->taps}));
+        else if (p->filt_bw > 0)
             CK(c, p->tB->onchip_dbp_filt(p->d.nfc, batch, c->stream, q, p->fc_c, DbpFiltSteps{ds, p->filt_hn_d}));
         else
             CK(c, p->tB->onchip_dbp(p->d.nfc, batch, c->stream, q, p->fc_c, ds));
@@ -3945,7 +3995,7 @@ extern "C" int pmx_dbp_exec(pmx_plan* p, pmx_devfield* fld) {
     PassGroups gs;
     rc = plan_groups(p, fld, pa, pA, pB, c->setup_done[p->N1 + 65536 * p->d.precision].cnl, true, gs);
     if (rc) return rc;
-    if (p->filt_bw > 0) return dbp_filtered_passes(p, fld, pa, gs);
+    if (p->filt_bw > 0 || p->ntaps > 0) return dbp_filtered_passes(p, fld, pa, gs);
     rc = fork_groups(c, gs.n);
     if (rc) return rc;
     int rev[4] = {1, 1, 1, 1};

@@ -179,8 +179,20 @@ struct DbpFiltSteps {
     DbpSteps s;
     const double* hn;       // [L]
 };
+// Enhanced split-step DBP (pmx_dbp_set_taps): the real FIR c[0..2k] on the intensity of every nonlinear step, c[k] at
+// lag 0.  A kernel parameter, by value: every thread reads the same tap at the same time.
+#define PMX_MAX_TAPS 65
+struct DbpTaps {
+    int k;                  // half-length: 2k+1 taps, 0 <= k <= 32
+    double c[PMX_MAX_TAPS];
+};
+struct DbpTapSteps {
+    DbpSteps s;
+    DbpTaps taps;
+};
 __host__ __device__ __forceinline__ DbpSteps pmx_dbp_steps(const DbpSteps& s) { return s; }
 __host__ __device__ __forceinline__ DbpSteps pmx_dbp_steps(const DbpFiltSteps& s) { return s.s; }
+__host__ __device__ __forceinline__ DbpSteps pmx_dbp_steps(const DbpTapSteps& s) { return s.s; }
 
 __device__ __forceinline__ cpx cmul(cpx a, cpx b) { return mkc(a.x * b.x - a.y * b.y, a.x * b.y + a.y * b.x); }
 __device__ __forceinline__ cpx cmulc(cpx a, cpx b) {  // a * conj(b)

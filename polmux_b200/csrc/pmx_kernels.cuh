@@ -538,6 +538,94 @@ static __global__ void __launch_bounds__(256) pmx_k_dbp_nl_filt(PassParams p, Fi
     }
 }
 
+// Enhanced split-step DBP on the three passes (pmx_dbp_set_taps): N(-xi*gam, h) of the step package pkg[b] from the FIR
+//   q~[n] = sum_{m=-k..k} c[m+k] * q[(n - m) mod N]   (left to right in m)
+// of the intensity pmx_k_dbp_intensity left in the work field (grid.y: the work column, realization-columns 2y and 2y+1).
+// The resident column is time-transposed: sample n1*N2 + n2 sits at n2*N1 + n1, so the time neighbour n - m is row n2 - m
+// at the same n1, or across the row wrap row n2 - m +- N2 at n1 -+ 1 (mod N1: circular at n = 0 and n = N - 1; k <= 32
+// < N2 wraps once at most).  A CTA takes PMX_FIR_ROWS rows of PMX_FIR_COLS positions along n1 and lands them with a k-row
+// halo on either side in shared memory.  It reads the intensity only from the work field, never a sample another CTA
+// has already rotated, so the result does not depend on the order the CTAs run in.
+#define PMX_FIR_ROWS 64
+#define PMX_FIR_COLS 16
+#define PMX_FIR_RB 4
+static __global__ void __launch_bounds__(256) pmx_k_dbp_nl_fir(PassParams p, FiberConst f, const cpx* __restrict__ work,
+                                                               const StepPkg* __restrict__ pkg, DbpTaps tp) {
+    constexpr int TY = 256 / PMX_FIR_COLS;
+    static_assert(TY * PMX_FIR_RB == PMX_FIR_ROWS, "a thread row per PMX_FIR_RB rows of the tile");
+    extern __shared__ __align__(16) unsigned char smf[];
+    cpx* sq = reinterpret_cast<cpx*>(smf);   // [PMX_FIR_ROWS + 2k][PMX_FIR_COLS][2]: time row r0 - k + r at row r
+    const int K = tp.k, N1 = p.N1, N2 = p.N2;
+    const int tiles1 = N1 / PMX_FIR_COLS;
+    const int c0 = (int)(blockIdx.x % tiles1) * PMX_FIR_COLS, r0 = (int)(blockIdx.x / tiles1) * PMX_FIR_ROWS;
+    const int tx = threadIdx.x % PMX_FIR_COLS, ty = threadIdx.x / PMX_FIR_COLS;
+    const size_t N = (size_t)N1 * N2;
+    PMX_ASSERT(K >= 0 && K <= 32 && K < N2 && r0 + PMX_FIR_ROWS <= N2 && blockDim.x == 256);
+    const cpx* w = work + (size_t)blockIdx.y * N * 2;
+    for (int r = ty; r < PMX_FIR_ROWS + 2 * K; r += TY) {
+        int rr = r0 - K + r, n1 = c0 + tx;
+        if (rr < 0) {
+            rr += N2;
+            n1 = (n1 - 1) & (N1 - 1);
+        } else if (rr >= N2) {
+            rr -= N2;
+            n1 = (n1 + 1) & (N1 - 1);
+        }
+        cpx a, b;
+        ld_sa(w + 2 * ((size_t)rr * N1 + n1), a, b);
+        sq[2 * (r * PMX_FIR_COLS + tx)] = a;
+        sq[2 * (r * PMX_FIR_COLS + tx) + 1] = b;
+    }
+    __syncthreads();
+    // a thread takes PMX_FIR_RB consecutive rows: the rows the taps read slide by one from tap to tap, so every tap lands
+    // one new row per thread and feeds PMX_FIR_RB independent sums
+    const int i0 = ty * PMX_FIR_RB;
+    cpx qa[PMX_FIR_RB], qb[PMX_FIR_RB], wa[PMX_FIR_RB], wb[PMX_FIR_RB];
+    const cpx* s = sq + 2 * ((i0 + 2 * K) * PMX_FIR_COLS + tx);   // tap 0 (lag m = -k) of row i0 + r: row i0 + r + 2k
+#pragma unroll
+    for (int r = 0; r < PMX_FIR_RB; ++r) {
+        qa[r] = qb[r] = mkc((real)0, (real)0);
+        wa[r] = s[2 * r * PMX_FIR_COLS];
+        wb[r] = s[2 * r * PMX_FIR_COLS + 1];
+    }
+    for (int j = 0;;) {
+        const real c = (real)tp.c[j];
+#pragma unroll
+        for (int r = 0; r < PMX_FIR_RB; ++r) {
+            qa[r] = mkc(fma(c, wa[r].x, qa[r].x), fma(c, wa[r].y, qa[r].y));
+            qb[r] = mkc(fma(c, wb[r].x, qb[r].x), fma(c, wb[r].y, qb[r].y));
+        }
+        if (++j > 2 * K) break;
+#pragma unroll
+        for (int r = PMX_FIR_RB - 1; r > 0; --r) {
+            wa[r] = wa[r - 1];
+            wb[r] = wb[r - 1];
+        }
+        s -= 2 * PMX_FIR_COLS;
+        wa[0] = s[0];
+        wb[0] = s[1];
+    }
+    const int nbc = p.batch * f.nfc;
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+        const int bc = 2 * (int)blockIdx.y + h;
+        if (bc >= nbc) break;   // an odd last work column: its Y slot is padding
+        const int b = bc / f.nfc, col = bc - b * f.nfc;
+        cpx* fld = reinterpret_cast<cpx*>(p.field) + (size_t)bc * N * 2;
+        const double leff = pkg[b].leff;
+#pragma unroll
+        for (int r = 0; r < PMX_FIR_RB; ++r) {
+            const size_t pos = (size_t)(r0 + i0 + r) * N1 + c0 + tx;
+            cpx x[1], y[1];
+            ld_sa(fld + 2 * pos, x[0], y[0]);
+            const cpx q = h ? qb[r] : qa[r];
+            const real pw[1] = {q.x}, s3[1] = {q.y};
+            pmx_nl_step_filt(x, y, pw, s3, leff, f, col);
+            st_sa(fld + 2 * pos, x[0], y[0]);
+        }
+    }
+}
+
 // ---------------------------------------------------------------------------
 // Tile walk shared by the three passes (persistent CTAs): tile -> (realization-column bc, group inside it),
 // serpentine direction, skipping finished realizations.

@@ -44,6 +44,12 @@ struct PmxLaunchTable {
                                    const DbpFiltSteps& ds);
     void (*dbp_intensity)(dim3 grid, cudaStream_t s, const PassParams& p, const FiberConst& f, void* work);
     void (*dbp_nl_filt)(dim3 grid, cudaStream_t s, const PassParams& p, const FiberConst& f, const void* work, const StepPkg* pkg);
+    // enhanced split-step DBP (pmx_dbp_set_taps): the on-chip kernel with the taps (pmx_k_onchip<..., DbpTapSteps>), and on
+    // the three passes the nonlinear step from the FIR of dbp_intensity's work field (pmx_k_dbp_nl_fir, its own grid)
+    cudaError_t (*onchip_dbp_taps)(int nfc, int batch, cudaStream_t s, const PassParams& p, const FiberConst& f,
+                                   const DbpTapSteps& ds);
+    cudaError_t (*dbp_nl_fir)(cudaStream_t s, const PassParams& p, const FiberConst& f, const void* work, const StepPkg* pkg,
+                              const DbpTaps& taps);
 };
 
 const PmxLaunchTable* pmx_get_table(int L, int precision = 0);  // nullptr if L is not built

@@ -19,6 +19,8 @@
 // Filtered DBP (the step table is a DbpFiltSteps: pmx_dbp_set_filter): after the scale the field is parked in registers,
 // the intensity it drives the nonlinear step with (P + i*s3, on the scalar path |u|^2) is transformed in the CTA,
 // multiplied by H/N at the thread's bins and transformed back, and the nonlinear step runs from the filtered quantities.
+// Enhanced split-step DBP (a DbpTapSteps: pmx_dbp_set_taps): after the scale the intensity goes to shared memory in time
+// order and every thread takes the circular FIR of the taps at its own samples; the nonlinear step runs from that.
 #pragma once
 #include <type_traits>
 #include <cooperative_groups.h>
@@ -68,6 +70,7 @@ template <typename R, int L, bool SC, bool DBP = false, typename... Steps>
 __global__ void __launch_bounds__((L / 8) < 32 ? 32 : (L / 8), 1) pmx_k_onchip(PassParams p, FiberConst f, Steps... steps) {
     static_assert(sizeof...(Steps) == (DBP ? 1 : 0), "the DBP instances take one DbpSteps, the forward ones nothing");
     constexpr bool FILT = (std::is_same<Steps, DbpFiltSteps>::value || ... || false);
+    constexpr bool TAPS = (std::is_same<Steps, DbpTapSteps>::value || ... || false);
     using S = OnchipSmem<L>;
     constexpr int T = L / 8;
     constexpr bool PRE = SC;
@@ -224,6 +227,47 @@ __global__ void __launch_bounds__((L / 8) < 32 ? 32 : (L / 8), 1) pmx_k_onchip(P
                     y[q] = v[q];
                 }
                 pmx_nl_step_filt(x, y, pw, aux, st->leff, f, col);   // ---- N(-xi*gam) from the filtered intensity
+            } else if constexpr (TAPS) {
+                const DbpTaps& tp = (steps.taps, ...);
+                // the intensity in time order (q at n = t + q*T), then its circular FIR, left to right in the lag
+                cpx* sq = work;
+                if (live) {
+#pragma unroll
+                    for (int q = 0; q < 8; ++q)
+                        sq[t + q * T] = f.scalar_field ? mkc(R_ADD(R_MUL(x[q].x, x[q].x), R_MUL(x[q].y, x[q].y)), (real)0)
+                                                       : pmx_dbp_intensity(x[q], y[q], f);
+                }
+                __syncthreads();
+                real pw[8], aux[8];
+#pragma unroll
+                for (int q = 0; q < 8; ++q) {
+                    const int n = tt + q * T;
+                    cpx a = mkc((real)0, (real)0);
+                    for (int j = 0; j <= 2 * tp.k; ++j) {
+                        const real c = (real)tp.c[j];
+                        const cpx v = sq[(n + tp.k - j) & (L - 1)];
+                        a = mkc(fma(c, v.x, a.x), fma(c, v.y, a.y));
+                    }
+                    pw[q] = a.x;
+                    aux[q] = a.y;
+                }
+                if (f.scalar_field && f.xpm) {   // sum over the columns of the filtered powers, left to right
+                    real* sp = reinterpret_cast<real*>(work + L);   // (the intensity may still be read)
+                    if (live) {
+#pragma unroll
+                        for (int q = 0; q < 8; ++q) sp[t + q * T] = pw[q];
+                    }
+                    cluster.sync();
+#pragma unroll
+                    for (int q = 0; q < 8; ++q) aux[q] = (real)0;
+                    for (int k = 0; k < f.nfc; ++k) {
+                        const real* rp = cluster.map_shared_rank(sp, k);
+#pragma unroll
+                        for (int q = 0; q < 8; ++q) aux[q] = R_ADD(aux[q], rp[tt + q * T]);
+                    }
+                    cluster.sync();
+                }
+                pmx_nl_step_filt(x, y, pw, aux, st->leff, f, col);   // ---- N(-xi*gam) from the FIR of the intensity
             } else {
                 if (f.xpm) xpm_sum();   // over the backpropagated columns (the transform has released the exchange buffer)
                 pmx_nl_step(x, y, st, f, col);   // ---- N(-xi*gam): the gam of f is the backpropagated one

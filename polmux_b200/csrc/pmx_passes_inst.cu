@@ -112,7 +112,13 @@ cudaError_t onchip_setup() {
     e = cudaFuncSetAttribute(pmx_k_onchip<real, L, true, true, DbpFiltSteps>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              SO::TOTAL);
     if (e != cudaSuccess) return e;
-    return cudaFuncSetAttribute(pmx_k_onchip<real, L, false, true, DbpFiltSteps>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    e = cudaFuncSetAttribute(pmx_k_onchip<real, L, false, true, DbpFiltSteps>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             SO::TOTAL);
+    if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(pmx_k_onchip<real, L, true, true, DbpTapSteps>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             SO::TOTAL);
+    if (e != cudaSuccess) return e;
+    return cudaFuncSetAttribute(pmx_k_onchip<real, L, false, true, DbpTapSteps>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 SO::TOTAL);
 }
 // the forward run (no step table) or digital backpropagation (one DbpSteps)
@@ -149,6 +155,20 @@ void dbp_intensity(dim3 grid, cudaStream_t s, const PassParams& p, const FiberCo
 void dbp_nl_filt(dim3 grid, cudaStream_t s, const PassParams& p, const FiberConst& f, const void* work, const StepPkg* pkg) {
     pmx_k_dbp_nl_filt<<<grid, 256, 0, s>>>(p, f, reinterpret_cast<const cpx*>(work), pkg);
 }
+// enhanced split-step DBP: the taps on the M-sample grid of a single-launch plan, and on the three passes the nonlinear
+// step from the FIR of the intensity in the work field (one CTA per tile of rows and work column)
+cudaError_t onchip_dbp_taps(int nfc, int batch, cudaStream_t s, const PassParams& p, const FiberConst& f, const DbpTapSteps& ds) {
+    return onchip_launch<true>(nfc, batch, s, p, f, ds);
+}
+cudaError_t dbp_nl_fir(cudaStream_t s, const PassParams& p, const FiberConst& f, const void* work, const StepPkg* pkg,
+                       const DbpTaps& taps) {
+    const int smem = (PMX_FIR_ROWS + 2 * taps.k) * PMX_FIR_COLS * 2 * (int)sizeof(cpx);
+    cudaError_t e = cudaFuncSetAttribute(pmx_k_dbp_nl_fir, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (e != cudaSuccess) return e;
+    const dim3 grid((unsigned)((p.N1 / PMX_FIR_COLS) * (p.N2 / PMX_FIR_ROWS)), (unsigned)((p.batch * f.nfc + 1) / 2));
+    pmx_k_dbp_nl_fir<<<grid, 256, smem, s>>>(p, f, reinterpret_cast<const cpx*>(work), pkg, taps);
+    return cudaGetLastError();
+}
 }  // namespace
 
 #define PMX_CAT2(a, b) a##b
@@ -162,4 +182,4 @@ extern const PmxLaunchTable PMX_TABLE_NAME = {
     L, GAC, GB, PFAC ? 1 : 0, PFB ? 1 : 0, SA::THREADS, SB::THREADS, (size_t)SA::TOTAL, (size_t)SB::TOTAL,
     pmx_tw_total(L), pmx_tw_layout(L), PmxTw4<L>::LO, PmxTw4<L>::PER, PMX_PRECISION, (int)sizeof(cpx),
     setup, passA, passB, passC, init_max, fill_tw4, xpm_sum, (size_t)SO::TOTAL, onchip_setup, onchip, passC_nl, onchip_dbp,
-    onchip_dbp_filt, dbp_intensity, dbp_nl_filt};
+    onchip_dbp_filt, dbp_intensity, dbp_nl_filt, onchip_dbp_taps, dbp_nl_fir};

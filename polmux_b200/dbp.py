@@ -34,7 +34,7 @@ from .gstate import GSTATE
 def dbp_plan(ctx: _lib.Context, setup: FiberSetup, nspan: int = 1, gain_db: Optional[float] = None,
              steps_per_span: Optional[int] = None, step_len=None, span_steps=None, xi: float = 1.0, batch: int = 1,
              precision: Optional[str] = None, disp_mode: Optional[str] = None, plates=None, shift: Optional[int] = None,
-             decim: Optional[int] = None, filter_bw: Optional[float] = None) -> _lib.DbpPlan:
+             decim: Optional[int] = None, filter_bw: Optional[float] = None, nl_taps=None) -> _lib.DbpPlan:
     """The DBP of nspan spans of the fiber `setup` describes, for resident fields of `batch` realizations.  Schedule:
     steps_per_span uniform steps per span (default 1), or step_len -- one span's steps in forward order for every span,
     or with span_steps [nspan] all spans' steps concatenated.  plates: None -- the 'p' flag, plates and dgdrms are
@@ -43,7 +43,11 @@ def dbp_plan(ctx: _lib.Context, setup: FiberSetup, nspan: int = 1, gain_db: Opti
     decim: single-channel DBP of a one-column field -- the channel that `shift` bins bring to baseband (the receiver's
     ndfn; default 0), backpropagated on nfft/decim samples (pmx_dbp_channel_create).
     filter_bw [GHz]: filtered DBP -- a Gaussian low-pass of that one-sided -3 dB bandwidth on the intensity of every
-    nonlinear step (DbpPlan.set_filter, in bins of GSTATE.FN: filter_bw * NSYMB / SYMBOLRATE); None or 0: none."""
+    nonlinear step (DbpPlan.set_filter, in bins of GSTATE.FN: filter_bw * NSYMB / SYMBOLRATE); None or 0: none.
+    nl_taps: enhanced split-step DBP -- the real circular FIR c[0..2K] (c[K] at lag 0, 2K+1 <= 65 taps) on the intensity of
+    every nonlinear step, on the plan's grid (DbpPlan.set_taps; with decim the channel's nfft/decim samples); None or []:
+    none.  Not together with filter_bw."""
+    taps = _check_taps(nl_taps, filter_bw)
     if plates is not None and not setup.fls[1]:
         raise ValueError("PMD-aware DBP (plates given) needs a fiber with the 'p' flag")
     if decim is None and shift is not None:
@@ -62,15 +66,25 @@ def dbp_plan(ctx: _lib.Context, setup: FiberSetup, nspan: int = 1, gain_db: Opti
             plan.set_plates(*arrs, plate_sets=arrs[0].shape[1])
         if filter_bw is not None:
             plan.set_filter(float(filter_bw) * GSTATE.NSYMB / GSTATE.SYMBOLRATE)
+        if taps.size:
+            plan.set_taps(taps)
     except Exception:
         plan.close()
         raise
     return plan
 
 
+def _check_taps(nl_taps, filter_bw) -> np.ndarray:
+    """the taps as float64 (empty: none), refused with pmx_dbp_set_taps's messages before any plan is made"""
+    taps = _lib.check_taps(nl_taps)
+    if taps.size and filter_bw:
+        raise ValueError('pmx_dbp_set_taps: the plan has a filter bandwidth (pmx_dbp_set_filter); a plan takes one or the other')
+    return taps
+
+
 def dbp(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, steps_per_span: Optional[int] = None, step_len=None,
         span_steps=None, xi: float = 1.0, ctx: Optional[_lib.Context] = None, precision: Optional[str] = None, brf=None,
-        ich: Optional[int] = None, decim: Optional[int] = None, filter_bw: Optional[float] = None):
+        ich: Optional[int] = None, decim: Optional[int] = None, filter_bw: Optional[float] = None, nl_taps=None):
     """Backpropagates GSTATE.FIELDX / FIELDY in place through nspan spans of the fiber x, the amplifier of gain_db [dB]
     after each (None: no amplifier).  x and flag are what fiber() takes; a field without FIELDY runs the scalar path, the
     'x' flag there backpropagating the cross-phase modulation of all columns.  Without brf the flag's 'p' is dropped (no plates
@@ -79,12 +93,14 @@ def dbp(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, steps_per
     the same plates) or a list of nspan of them in forward span order, with 'p' in the flag: PMD-aware DBP through those
     plates.  xi: fraction of gamma backpropagated.  ich, decim: single-channel DBP of channel ich (1-based) of a 'unique'
     multiplex on nfft/decim samples; afterwards the field holds that channel alone, on its own bins.  filter_bw [GHz]:
-    filtered DBP, a Gaussian low-pass of that one-sided -3 dB bandwidth on the intensity of every nonlinear step.  The field stays
-    resident on the device like fiber() and ampliflat() leave it."""
+    filtered DBP, a Gaussian low-pass of that one-sided -3 dB bandwidth on the intensity of every nonlinear step.  nl_taps:
+    enhanced split-step DBP, the real circular FIR c[0..2K] (c[K] at lag 0) on the intensity of every nonlinear step
+    (dbp_plan).  The field stays resident on the device like fiber() and ampliflat() leave it."""
     G = GSTATE
     f = str(flag).lower()
     if len(f) != 4:
         raise ValueError("wrong flag. E.g. flag can be 'g---','gp--','-s--', etc")
+    _check_taps(nl_taps, filter_bw)
     shift = None
     if decim is not None:
         if ich is None:
@@ -128,7 +144,7 @@ def dbp(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, steps_per
         try:
             fld.upload(fx, np.zeros_like(fx))
             plan = dbp_plan(ctx, s, nspan, gain_db, steps_per_span, step_len, span_steps, xi, precision=precision,
-                            shift=shift, decim=decim, filter_bw=filter_bw)
+                            shift=shift, decim=decim, filter_bw=filter_bw, nl_taps=nl_taps)
             try:
                 plan.execute(fld)
             finally:
@@ -141,7 +157,7 @@ def dbp(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, steps_per
     fld, hx, hy = G.take_device(ctx, prec)
     try:
         plan = dbp_plan(ctx, s, nspan, gain_db, steps_per_span, step_len, span_steps, xi, precision=precision, plates=plates,
-                        shift=shift, decim=decim, filter_bw=filter_bw)
+                        shift=shift, decim=decim, filter_bw=filter_bw, nl_taps=nl_taps)
     except Exception:
         G.restore_host(fld, hx, hy)     # nothing ran: the caller's field is as it was
         raise

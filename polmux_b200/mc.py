@@ -222,7 +222,7 @@ class McRunner:
         DBP through each group's own plate draws (Link.plates); with 'genie' it replaces the linear equaliser.
         dbp_params with 'decim' (a power of two >= 2; 'blind' and 'cohmix', a one-column 'unique' field): single-channel DBP
         on nfft/decim samples -- of channel `ich` for 'cohmix', of the channel at the centre of the grid for 'blind'.
-        dbp_params with 'filter_bw' [GHz]: filtered DBP (dbp_plan)"""
+        dbp_params with 'filter_bw' [GHz]: filtered DBP (dbp_plan); with 'nl_taps': enhanced split-step DBP (dbp_plan)"""
         import torch
         from . import dsp as _dsp
         self.receiver, self.dsp_params = receiver, dict(dsp_params or {})
@@ -402,6 +402,9 @@ def run_mc_native(setup: FiberSetup, tx_x, tx_y, sym, nsymb: int, nt: int, nspan
     import ctypes as C
     if dict(dbp_params or {}).get('filter_bw') is not None:
         raise ValueError("run_mc_native: filtered DBP (dbp_params 'filter_bw') is not available in pmx_mc_run; use McRunner")
+    if _lib.check_taps(dict(dbp_params or {}).get('nl_taps')).size:
+        raise ValueError("run_mc_native: enhanced split-step DBP (dbp_params 'nl_taps') is not available in pmx_mc_run; "
+                         "use McRunner")
     lib = _lib.load()
     np_ = setup.nplates
     pl = np.empty((3, nspan, nreal, np_))

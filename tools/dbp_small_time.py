@@ -7,7 +7,9 @@ resident batch, then DBP (pmx_dbp_exec) of the same batch with the forward run's
 Cases: 2^10 two-polarization Manakov 'g-s-' at batch 1, 148 and 1184; the ex10_wdm.m shape (64 x 32 samples x 5
 'sepfields' columns, scalar path 'g-sx') at batch 148; 2^12 scalar 'g-s-' at batch 148.  Reported: the median wall time
 of a call (it returns synchronised), us per step and GSa*steps/s = batch*nfc*nfft*steps/time.  The card's name and power
-limit are printed with the numbers."""
+limit are printed with the numbers.
+--filter-bw BW / --taps K: also filtered DBP (BW GHz; with --taps alone 4 GHz) and, with --taps, enhanced split-step DBP
+with the 2K+1 taps of dbp_time.essfm_taps, with the same steps, alternated with the forward run and plain DBP."""
 import argparse
 import json
 import os
@@ -24,6 +26,7 @@ import polmux_b200 as pmx  # noqa: E402
 from polmux_b200 import _lib, synth  # noqa: E402
 from polmux_b200.dbp import dbp_plan  # noqa: E402
 from polmux_b200.fiber import fiber_setup, setup_to_desc  # noqa: E402
+from dbp_time import essfm_taps  # noqa: E402
 
 
 def card():
@@ -66,6 +69,8 @@ def main():
     ap.add_argument('--reps', type=int, default=20)
     ap.add_argument('--filter-bw', type=float, default=None,
                     help='also filtered DBP [GHz] with the same steps, alternated with the forward run and plain DBP')
+    ap.add_argument('--taps', type=int, default=None,
+                    help='also enhanced split-step DBP with 2K+1 taps, alternated with the others')
     ap.add_argument('--out', default=None, help='directory for dbp_small_time.json')
     a = ap.parse_args()
     ctx = _lib.default_context(0)
@@ -89,12 +94,17 @@ def main():
         fld.broadcast_from(tx)
         dbp.execute(fld)                                           # warm-up
         runs = [('forward', lambda: fwd.execute(fld)), ('dbp', lambda: dbp.execute(fld))]
-        filt = None
-        if a.filter_bw is not None:
-            filt = dbp_plan(ctx, s, 1, None, step_len=dz, batch=B, filter_bw=a.filter_bw)
+        filt = ess = None
+        if a.filter_bw is not None or a.taps is not None:
+            filt = dbp_plan(ctx, s, 1, None, step_len=dz, batch=B, filter_bw=4.0 if a.filter_bw is None else a.filter_bw)
             fld.broadcast_from(tx)
             filt.execute(fld)                                      # warm-up
             runs.append(('filtered', lambda: filt.execute(fld)))
+        if a.taps is not None:
+            ess = dbp_plan(ctx, s, 1, None, step_len=dz, batch=B, nl_taps=essfm_taps(a.taps))
+            fld.broadcast_from(tx)
+            ess.execute(fld)                                       # warm-up
+            runs.append(('essfm', lambda: ess.execute(fld)))
         t = {what: [] for what, _ in runs}
         for _ in range(a.reps):                                    # they alternate
             for what, run in runs:
@@ -107,6 +117,8 @@ def main():
         dbp.close()
         if filt is not None:
             filt.close()
+        if ess is not None:
+            ess.close()
         fld.close()
         tx.close()
         row = dict(case=name, batch=B, nfft=n, nfc=nfc, steps=steps)
@@ -120,6 +132,11 @@ def main():
             print('%-26s batch %5d  filtered dbp %8.2f us/step %7.2f GSa*steps/s | filtered/dbp %.3f'
                   % (name, B, row['filtered']['us_per_step'], row['filtered']['gsa_steps_per_s'],
                      row['filtered']['gsa_steps_per_s'] / row['dbp']['gsa_steps_per_s']))
+        if ess is not None:
+            print('%-26s batch %5d  essfm dbp %8.2f us/step %7.2f GSa*steps/s | essfm/dbp %.3f | essfm/filtered %.3f'
+                  % (name, B, row['essfm']['us_per_step'], row['essfm']['gsa_steps_per_s'],
+                     row['essfm']['gsa_steps_per_s'] / row['dbp']['gsa_steps_per_s'],
+                     row['essfm']['gsa_steps_per_s'] / row['filtered']['gsa_steps_per_s']))
         print('%-26s batch %5d  %3d steps | forward %8.2f us/step %7.2f GSa*steps/s | dbp %8.2f us/step %7.2f GSa*steps/s'
               ' | dbp/forward %.3f' % (name, B, steps, row['forward']['us_per_step'], row['forward']['gsa_steps_per_s'],
                                        row['dbp']['us_per_step'], row['dbp']['gsa_steps_per_s'], row['dbp_vs_forward']))

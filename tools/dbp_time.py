@@ -10,7 +10,9 @@ step moves per Sa in FP64 (3 passes x read + write x 32 B), against the same pea
 hbm_gbs, else 6650 GB/s).  The card's name and power limit are printed with the numbers.
 --pmd: the 'gps-' C2 link with 100 plates per span and a plate draw per span and realization; timed are the forward link,
 PMD-blind DBP and PMD-aware DBP (each at M = 1, 4, 16) and the genie equaliser (Link.equalize, one 100-trunk step per
-span)."""
+span).
+--taps K: enhanced split-step DBP with the 2K+1 taps of essfm_taps (symmetric, sum 1) at 1, 2 and 4 steps per span,
+alternated in this process with the plain plan and the filtered plan (--filter-bw, default 4 GHz)."""
 import argparse
 import json
 import os
@@ -29,6 +31,13 @@ from polmux_b200.dbp import dbp_plan  # noqa: E402
 from polmux_b200.fiber import fiber_setup, setup_to_desc  # noqa: E402
 
 BYTES_PER_SA_STEP = 192.0
+
+
+def essfm_taps(k):
+    """the fixed symmetric test tap set of --taps K: 2K+1 samples of a Gaussian, normalised to sum 1"""
+    m = np.arange(-k, k + 1, dtype=np.float64)
+    c = np.exp(-(m / (0.5 * k + 1)) ** 2)
+    return c / c.sum()
 
 
 def card():
@@ -50,6 +59,8 @@ def main():
     ap.add_argument('--pmd', action='store_true', help="the 'gps-' link with 100 plates; PMD-aware DBP and the equaliser too")
     ap.add_argument('--filter-bw', type=float, default=None,
                     help='filtered DBP [GHz] at 1, 2 and 4 steps per span, alternated with the plain plan in this process')
+    ap.add_argument('--taps', type=int, default=None,
+                    help='enhanced split-step DBP with 2K+1 taps, alternated with plain and filtered DBP in this process')
     ap.add_argument('--out', default=None, help='directory for dbp_time.json')
     a = ap.parse_args()
     try:
@@ -108,10 +119,14 @@ def main():
         plan = dbp_plan(ctx, s, a.nspan, 16.0, steps_per_span=m, batch=B)
         timed('dbp M=%d' % m, lambda: plan.execute(fld), lambda _r, m=m: m * a.nspan * B)
         plan.close()
-    if a.filter_bw is not None:
+    if a.filter_bw is not None or a.taps is not None:
+        bw = 4.0 if a.filter_bw is None else a.filter_bw
         for m in (1, 2, 4):
             plans = [('dbp M=%d' % m, dbp_plan(ctx, s, a.nspan, 16.0, steps_per_span=m, batch=B)),
-                     ('filtered M=%d' % m, dbp_plan(ctx, s, a.nspan, 16.0, steps_per_span=m, batch=B, filter_bw=a.filter_bw))]
+                     ('filtered M=%d' % m, dbp_plan(ctx, s, a.nspan, 16.0, steps_per_span=m, batch=B, filter_bw=bw))]
+            if a.taps is not None:
+                plans.append(('essfm M=%d' % m, dbp_plan(ctx, s, a.nspan, 16.0, steps_per_span=m, batch=B,
+                                                          nl_taps=essfm_taps(a.taps))))
             for _ in range(a.reps):
                 for name, pl in plans:
                     timed(name, lambda pl=pl: pl.execute(fld), lambda _r, m=m: m * a.nspan * B, reps=1)
