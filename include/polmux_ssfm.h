@@ -327,6 +327,8 @@ int pmx_dbp_set_taps(pmx_plan* plan, int32_t ntaps, const double* taps);
  * plan with pmx_plan_destroy. */
 int pmx_dbp_exec(pmx_plan* plan, pmx_devfield* f);
 
+/* (Perturbation-based nonlinearity compensation, a symbol-rate alternative to DBP: pmx_pb_create below.) */
+
 /* ---- single-channel digital backpropagation: one channel of a 'unique' multiplex at a reduced sample rate ------------
  * A coherent receiver sees its own channel only.  For a field of N = fiber->nfft samples in one column (nfc = 1, every
  * channel in it) and band = {m, r}, M = N/r, the plan runs per realization, in place:
@@ -351,6 +353,54 @@ typedef struct pmx_dbp_band {
  * pmx_plan_destroy take the returned plan; it owns the M-sample DBP plan, the band filter and an M x batch work field. */
 int pmx_dbp_channel_create(pmx_ctx* ctx, const pmx_fiber_desc* fiber, const pmx_dbp_desc* dbp, const pmx_dbp_band* band,
                            pmx_plan** plan);
+
+/* ---- perturbation-based nonlinearity compensation (PB-NLC): a first-order triplet correction at the symbol rate -----
+ * An extension (the reference has none; Mecozzi, Clausen & Shtaif, IEEE PTL 12(4), 2000; Tao et al., JLT 29(17), 2011).
+ * For a resident one-column two-polarization FP64 field of nfft = nsymb*nt samples holding one channel whose dispersion
+ * is already compensated (the all-pass step of the link), per realization, in place, with p the pulse table:
+ *   project : A^x_k = sum_j p[j] * ux[(k*nt - npulse/2 + j) mod nfft] / sum_j p[j]^2  (A^y likewise), k < nsymb: the
+ *             matched filter of the pulse of symbol k, centred at time index k*nt
+ *   triplets: Delta^x_k = sum_i C'_i * ( a*A^x_{k+m} A^x_{k+n} conj(A^x_{k+m+n}) + b*A^x_{k+m} A^y_{k+n} conj(A^y_{k+m+n})
+ *                                      + c*A^y_{k+m} A^y_{k+n} conj(A^x_{k+m+n}) ),     (x <-> y for Delta^y)
+ *             symbol indices mod nsymb, the sum over the list i = (m_i, n_i, C_i) in list order, C'_i = -j*gamma*s^2*C_i
+ *   apply   : u[t] -= xi * sum_k Delta_k * p[t - k*nt + npulse/2] over the k whose pulse covers t (k descending)
+ * The triplets are formed on s*A and subtracted in the field's units, which is gamma -> gamma*s^2: s brings the received
+ * field to launch scale, the field keeps its own.  (a, b, c) = (1, 1, 0) is Manakov (gamma then carries the 8/9), (1, 2/3,
+ * 1/3) the CNLSE.  xi = 0 runs no kernel and leaves the field bit for bit as it was.  The sum has a fixed order and no
+ * atomics: two executions give the same bits. */
+#define PMX_PB_MAX_K 128           /* |m|, |n| <= PMX_PB_MAX_K                                                           */
+#define PMX_PB_MAX_COEF 1000000    /* at most this many (m, n, C) entries                                                */
+typedef struct pmx_pb_desc {
+    int64_t nfft;           /* samples per column: nsymb*nt, a power of two from 2^6 to 2^24                          */
+    int32_t nsymb, nt;      /* symbols per block and samples per symbol                                                */
+    int32_t batch;          /* realizations of the fields the plan runs on                                             */
+    int32_t nfc;            /* columns of those fields: 1 (one channel)                                               */
+    int32_t precision;      /* PMX_F64                                                                                 */
+    int32_t npulse;         /* pulse samples: even, 2 .. min(16*nt, nfft)                                             */
+    const double* pulse;    /* [npulse] real pulse table (electricsource's 2*nt samples: symbol k from (k-1)*nt)        */
+    double weights[3];      /* (a, b, c)                                                                                */
+    double gamma;           /* [1/W/m] of the triplet sum (Manakov: with the 8/9)                                       */
+    double xi;              /* fraction of the perturbation subtracted                                                  */
+    double scale;           /* s: received field -> launch scale                                                        */
+    int32_t ncoef;          /* entries of the coefficient list, 1 .. PMX_PB_MAX_COEF                                    */
+    int32_t reserved;
+    const int32_t* m;       /* [ncoef] */
+    const int32_t* n;       /* [ncoef] */
+    const double* coef;     /* [ncoef][2] C = (re, im), finite                                                         */
+} pmx_pb_desc;
+typedef struct pmx_pb_plan pmx_pb_plan;
+/* Checked before a context is needed: PMX_ERR_UNSUPPORTED for nfc != 1 and for FP32; PMX_ERR_INVALID for nsymb*nt !=
+ * nfft, nfft not a power of two from 2^6 to 2^24, batch < 1, a bad pulse (odd or out-of-range npulse, NULL, non-finite,
+ * zero energy), non-finite weights, gamma, xi or scale, ncoef out of range, |m| or |n| > PMX_PB_MAX_K, and a non-finite
+ * coefficient.  The plan copies the pulse and the list to the device; it holds two [batch][2][nsymb] complex buffers. */
+int pmx_pb_create(pmx_ctx* ctx, const pmx_pb_desc* desc, pmx_pb_plan** plan);
+/* In place on a resident field of the same device: PMX_ERR_UNSUPPORTED for nfc != 1 or FP32, PMX_ERR_INVALID for a field
+ * whose nfft or batch differs from the plan's. */
+int pmx_pb_exec(pmx_pb_plan* plan, pmx_devfield* f);
+/* The projected symbols A and the perturbation Delta of the last pmx_pb_exec (with xi != 0), each [batch][2][nsymb] complex
+ * (re, im interleaved) into host buffers; either may be NULL.  Returns when the copies are done. */
+int pmx_pb_symbols(pmx_pb_plan* plan, double* A, double* delta);
+void pmx_pb_destroy(pmx_pb_plan* plan);
 
 /* ---- create_field('unique'): the WDM multiplex on the device (create_field.m:113-149,180-199) ----------------
  * The reference builds the single field as

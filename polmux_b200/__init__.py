@@ -10,6 +10,7 @@ from .ampliflat import ampliflat  # noqa: F401
 from .inverse_pmd import inverse_pmd  # noqa: F401
 from .link import link  # noqa: F401
 from .dbp import dbp  # noqa: F401
+from .pbnlc import pbnlc, pb_plan  # noqa: F401
 from .receiver import receiver_cohmix, myfilter, evaldelay  # noqa: F401
 from .dsp import dsp4cohdec  # noqa: F401
 from ._lib import PolmuxError, Context, DeviceField, Plan  # noqa: F401

@@ -35,7 +35,7 @@ EXPORTS = [
     'pmx_ampliflat_exec_at', 'pmx_dsp_count', 'pmx_field_mean_power', 'pmx_pmd_matrix', 'pmx_field_jones', 'pmx_filter_create', 'pmx_field_copy_cols', 'pmx_field_modulate',
     'pmx_cohmix_exec', 'pmx_field_mean_power_xy', 'pmx_cohmix_run', 'pmx_dsp_phases', 'pmx_field_quantize', 'pmx_inverse_pmd_run',
     'pmx_dbp_create', 'pmx_dbp_exec', 'pmx_dbp_set_plates', 'pmx_dbp_channel_create', 'pmx_dbp_set_filter',
-    'pmx_dbp_set_taps',
+    'pmx_dbp_set_taps', 'pmx_pb_create', 'pmx_pb_exec', 'pmx_pb_symbols', 'pmx_pb_destroy',
 ]
 
 
@@ -87,6 +87,13 @@ class DbpDesc(C.Structure):
 
 class DbpBand(C.Structure):
     _fields_ = [('shift', C.c_int64), ('decim', C.c_int32), ('reserved', C.c_int32)]
+
+
+class PbDesc(C.Structure):
+    _fields_ = [('nfft', C.c_int64), ('nsymb', C.c_int32), ('nt', C.c_int32), ('batch', C.c_int32), ('nfc', C.c_int32),
+                ('precision', C.c_int32), ('npulse', C.c_int32), ('pulse', _dp), ('weights', C.c_double * 3),
+                ('gamma', C.c_double), ('xi', C.c_double), ('scale', C.c_double), ('ncoef', C.c_int32),
+                ('reserved', C.c_int32), ('m', _ip), ('n', _ip), ('coef', _dp)]
 
 
 class McReceiver(C.Structure):
@@ -188,6 +195,11 @@ def load():
     lib.pmx_dbp_set_plates.argtypes = [vp, C.c_int32, _dp, _dp, _dp]
     lib.pmx_dbp_set_filter.argtypes = [vp, C.c_double]
     lib.pmx_dbp_set_taps.argtypes = [vp, C.c_int32, _dp]
+    lib.pmx_pb_create.argtypes = [vp, C.POINTER(PbDesc), C.POINTER(vp)]
+    lib.pmx_pb_exec.argtypes = [vp, vp]
+    lib.pmx_pb_symbols.argtypes = [vp, _dp, _dp]
+    lib.pmx_pb_destroy.argtypes = [vp]
+    lib.pmx_pb_destroy.restype = None
     lib.pmx_dbp_channel_create.argtypes = [vp, C.POINTER(FiberDesc), C.POINTER(DbpDesc), C.POINTER(DbpBand), C.POINTER(vp)]
     _lib = lib
     return lib
@@ -614,6 +626,67 @@ def make_dbp(nspan, gain=0.0, steps_per_span=None, step_len=None, span_steps=Non
     d.step_len = _ptr(keep['step_len'])
     d.span_steps = keep['span_steps'].ctypes.data_as(_ip)
     return d, keep
+
+
+PB_MAX_K = 128             # PMX_PB_MAX_K
+
+
+def check_pb_k(K):
+    """ValueError with pmx_pb_create's limit for a triplet table half-width K out of range, before any table is computed"""
+    if int(K) < 0 or int(K) > PB_MAX_K:
+        raise ValueError('pmx_pb_create: K=%d, |m| and |n| at most %d' % (int(K), PB_MAX_K))
+
+
+def make_pb(nsymb, nt, batch, pulse, weights, gamma, xi, scale, m, n, coef):
+    """-> (PbDesc, keep-alive dict) for one-column FP64 fields of nsymb*nt samples; (m, n, coef) the triplet table"""
+    keep = {'pulse': _f64(np.asarray(pulse, dtype=np.float64).ravel()),
+            'm': np.ascontiguousarray(np.asarray(m).ravel(), dtype=np.int32),
+            'n': np.ascontiguousarray(np.asarray(n).ravel(), dtype=np.int32),
+            'coef': np.ascontiguousarray(np.asarray(coef, dtype=np.complex128).ravel()).view(np.float64)}
+    if not (keep['m'].size == keep['n'].size == keep['coef'].size // 2):
+        raise ValueError('make_pb: m, n and coef must have one value per entry')
+    d = PbDesc()
+    d.nfft, d.nsymb, d.nt, d.batch, d.nfc, d.precision = int(nsymb) * int(nt), int(nsymb), int(nt), int(batch), 1, PMX_F64
+    d.npulse, d.pulse = keep['pulse'].size, _ptr(keep['pulse'])
+    d.weights = (C.c_double * 3)(*[float(w) for w in weights])
+    d.gamma, d.xi, d.scale = float(gamma), float(xi), float(scale)
+    d.ncoef = keep['m'].size
+    d.m, d.n, d.coef = keep['m'].ctypes.data_as(_ip), keep['n'].ctypes.data_as(_ip), _ptr(keep['coef'])
+    return d, keep
+
+
+class PbPlan:
+    """Perturbation-based nonlinearity compensation (pmx_pb_create): execute(field) runs it in place on a resident field."""
+
+    def __init__(self, ctx: Context, desc_keep):
+        self.ctx, (self.desc, self.keep) = ctx, desc_keep
+        h = C.c_void_p()
+        ctx.check(ctx.lib.pmx_pb_create(ctx.h, C.byref(self.desc), C.byref(h)))
+        self.h = h
+
+    def execute(self, field: DeviceField):
+        self.ctx.check(self.ctx.lib.pmx_pb_exec(self.h, field.h))
+
+    def symbols(self):
+        """-> (A, Delta) of the last execute, each [batch][2][nsymb] complex128 (pmx_pb_symbols)"""
+        a = np.zeros((self.desc.batch, 2, self.desc.nsymb), dtype=np.complex128)
+        d = np.zeros_like(a)
+        self.ctx.check(self.ctx.lib.pmx_pb_symbols(self.h, a.ctypes.data_as(_dp), d.ctypes.data_as(_dp)))
+        return a, d
+
+    def close(self):
+        if getattr(self, 'h', None):
+            self.ctx.lib.pmx_pb_destroy(self.h)
+            self.h = None
+
+    def __del__(self):
+        # at interpreter shutdown objects die in no particular order (a context before its plans): leave them to the process exit
+        if sys.is_finalizing():
+            return
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 class Filter(Plan):

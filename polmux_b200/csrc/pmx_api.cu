@@ -4140,3 +4140,279 @@ static int dbp_channel_exec(pmx_plan* p, pmx_devfield* fld) {
     CK(c, cudaGetLastError());
     return pmx_fiber_exec(p->ch_band, fld, nullptr);
 }
+
+// ---------------------------------------------------------------------------
+// Perturbation-based nonlinearity compensation (pmx_pb_create / pmx_pb_exec, see the header): projection onto the pulses,
+// the first-order triplet sum at the symbol rate, reconstruction.  FP64, one-column fields, either resident layout.
+struct PbCoef {   // one entry of the list, C' = -j*gamma*s^2*C folded on the host
+    double cr, ci;
+    int m, n;
+};
+struct pmx_pb_plan {
+    pmx_ctx* ctx;
+    int64_t nfft;
+    int nsymb, nt, batch, npulse, ncoef, K;
+    double wa, wb, wc, xi, inorm;
+    double* pulse = nullptr;  // [npulse]
+    PbCoef* coef = nullptr;   // [ncoef]
+    cpx* A = nullptr;         // [batch][2][nsymb] projected symbols
+    cpx* D = nullptr;         // [batch][2][nsymb] perturbation
+};
+
+// A^{x,y}_k = sum_j p[j] u[(k*nt - np/2 + j) mod N] * inorm (j ascending); thread per symbol, grid.y the realization
+__global__ void __launch_bounds__(256) pmx_k_pb_project(const cpx* __restrict__ field, size_t N, int l1, int l2, int nsymb,
+                                                        int nt, const double* __restrict__ pulse, int np, double inorm,
+                                                        cpx* __restrict__ A) {
+    const int b = blockIdx.y;
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= nsymb) return;
+    const cpx* fld = field + (size_t)b * N * 2;
+    const size_t t0 = ((size_t)k * nt + N - (size_t)(np / 2)) & (N - 1);
+    double axr = 0, axi = 0, ayr = 0, ayi = 0;
+    for (int j = 0; j < np; ++j) {
+        cpx x, y;
+        ld_sa(fld + 2 * pmx_mem_index((t0 + j) & (N - 1), l1, l2), x, y);
+        const double p = pulse[j];
+        axr = fma(p, x.x, axr);
+        axi = fma(p, x.y, axi);
+        ayr = fma(p, y.x, ayr);
+        ayi = fma(p, y.y, ayi);
+    }
+    A[(size_t)(2 * b) * nsymb + k] = make_double2(axr * inorm, axi * inorm);
+    A[(size_t)(2 * b + 1) * nsymb + k] = make_double2(ayr * inorm, ayi * inorm);
+}
+
+// The triplet sum.  A CTA takes PMX_PB_TILE symbols of one realization and lands them with a 2K-symbol halo on either side
+// (indices k+m, k+n, k+m+n with |m|, |n| <= K), both polarizations, in shared memory.  A thread owns PMX_PB_RB symbols, so
+// every coefficient it reads (the same entry for all threads: a broadcast) feeds PMX_PB_RB independent sums.  Its symbols are
+// PMX_PB_THREADS apart rather than adjacent: the loads of one coefficient share nothing between neighbouring symbols, and
+// a warp then reads 32 consecutive 16-byte samples per load, without bank conflicts.  Per entry and symbol the loop runs
+// 4 complex products xx, yy, xy, yx (8 FMA + 8 MUL), the weighted sums a*xx + c*yy, a*yy + c*xx (4 FMA + 4 MUL), b*xy,
+// b*yx (4 MUL), T^x = q^x conj(A^x_{k+m+n}) + b*xy conj(A^y_{k+m+n}) and T^y likewise (12 FMA + 4 MUL) and the two
+// accumulations C'*T (8 FMA): 52 FP64 instructions, 32 FMA and 20 MUL, 84 flops per entry and symbol (an FMA counted as
+// two), from 6 shared-memory loads of 16 bytes.  Fixed order, no atomics.
+#define PMX_PB_THREADS 128
+#define PMX_PB_RB 4
+#define PMX_PB_TILE (PMX_PB_THREADS * PMX_PB_RB)
+__device__ __forceinline__ double2 pb_mul(double2 a, double2 b) {
+    return make_double2(fma(a.x, b.x, -a.y * b.y), fma(a.x, b.y, a.y * b.x));
+}
+// a*conj(b), and acc + a*conj(b)
+__device__ __forceinline__ double2 pb_mul_conj(double2 a, double2 b) {
+    return make_double2(fma(a.x, b.x, a.y * b.y), fma(a.y, b.x, -a.x * b.y));
+}
+__device__ __forceinline__ double2 pb_mac_conj(double2 acc, double2 a, double2 b) {
+    return make_double2(fma(a.y, b.y, fma(a.x, b.x, acc.x)), fma(-a.x, b.y, fma(a.y, b.x, acc.y)));
+}
+__global__ void __launch_bounds__(PMX_PB_THREADS) pmx_k_pb_triplet(const cpx* __restrict__ A, int nsymb,
+                                                                   const PbCoef* __restrict__ coef, int ncoef, int K,
+                                                                   double wa, double wb, double wc, cpx* __restrict__ D) {
+    extern __shared__ __align__(16) unsigned char smp[];
+    const int H = 2 * K, span = PMX_PB_TILE + 2 * H;
+    cpx* sx = reinterpret_cast<cpx*>(smp);   // [span]: symbol k0 - H + i at i
+    cpx* sy = sx + span;
+    const int b = blockIdx.y, k0 = blockIdx.x * PMX_PB_TILE;
+    const cpx* ax = A + (size_t)(2 * b) * nsymb;
+    const cpx* ay = ax + nsymb;
+    for (int i = threadIdx.x; i < span; i += PMX_PB_THREADS) {
+        int k = (k0 - H + i) % nsymb;
+        if (k < 0) k += nsymb;
+        sx[i] = ax[k];
+        sy[i] = ay[k];
+    }
+    __syncthreads();
+    double2 dx[PMX_PB_RB], dy[PMX_PB_RB];
+#pragma unroll
+    for (int r = 0; r < PMX_PB_RB; ++r) dx[r] = dy[r] = make_double2(0.0, 0.0);
+    const int base = H + threadIdx.x;
+    for (int i = 0; i < ncoef; ++i) {
+        const double cr = __ldg(&coef[i].cr), ci = __ldg(&coef[i].ci);
+        const int m = __ldg(&coef[i].m), n = __ldg(&coef[i].n);
+#pragma unroll
+        for (int r = 0; r < PMX_PB_RB; ++r) {
+            const int o = base + r * PMX_PB_THREADS;
+            const double2 xm = sx[o + m], ym = sy[o + m], xn = sx[o + n], yn = sy[o + n];
+            const double2 xs = sx[o + m + n], ys = sy[o + m + n];
+            const double2 xx = pb_mul(xm, xn), yy = pb_mul(ym, yn), xy = pb_mul(xm, yn), yx = pb_mul(ym, xn);
+            const double2 qx = make_double2(fma(wa, xx.x, wc * yy.x), fma(wa, xx.y, wc * yy.y));
+            const double2 qy = make_double2(fma(wa, yy.x, wc * xx.x), fma(wa, yy.y, wc * xx.y));
+            const double2 bxy = make_double2(wb * xy.x, wb * xy.y), byx = make_double2(wb * yx.x, wb * yx.y);
+            const double2 tx = pb_mac_conj(pb_mul_conj(qx, xs), bxy, ys);
+            const double2 ty = pb_mac_conj(pb_mul_conj(qy, ys), byx, xs);
+            dx[r] = make_double2(fma(cr, tx.x, fma(-ci, tx.y, dx[r].x)), fma(cr, tx.y, fma(ci, tx.x, dx[r].y)));
+            dy[r] = make_double2(fma(cr, ty.x, fma(-ci, ty.y, dy[r].x)), fma(cr, ty.y, fma(ci, ty.x, dy[r].y)));
+        }
+    }
+#pragma unroll
+    for (int r = 0; r < PMX_PB_RB; ++r) {
+        const int k = k0 + threadIdx.x + r * PMX_PB_THREADS;
+        if (k < nsymb) {
+            D[(size_t)(2 * b) * nsymb + k] = dx[r];
+            D[(size_t)(2 * b + 1) * nsymb + k] = dy[r];
+        }
+    }
+}
+
+// u[t] -= xi * sum_k p[t - k*nt + np/2] * Delta_k, k descending from the last symbol whose pulse covers t
+__global__ void __launch_bounds__(256) pmx_k_pb_apply(cpx* __restrict__ field, size_t N, int l1, int l2, int nsymb, int nt,
+                                                      const double* __restrict__ pulse, int np, const cpx* __restrict__ D,
+                                                      double xi) {
+    const int b = blockIdx.y;
+    cpx* fld = field + (size_t)b * N * 2;
+    const cpx* dx = D + (size_t)(2 * b) * nsymb;
+    const cpx* dy = dx + nsymb;
+    for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < N; t += (size_t)gridDim.x * blockDim.x) {
+        const long long h = (long long)t + np / 2;
+        long long k = h / nt;
+        int j = (int)(h - k * nt);
+        double axr = 0, axi = 0, ayr = 0, ayi = 0;
+        for (; j < np; j += nt, --k) {
+            int kk = (int)(k % nsymb);
+            if (kk < 0) kk += nsymb;
+            const double p = pulse[j];
+            const cpx ex = dx[kk], ey = dy[kk];
+            axr = fma(p, ex.x, axr);
+            axi = fma(p, ex.y, axi);
+            ayr = fma(p, ey.x, ayr);
+            ayi = fma(p, ey.y, ayi);
+        }
+        const size_t pos = 2 * pmx_mem_index(t, l1, l2);
+        cpx x, y;
+        ld_sa(fld + pos, x, y);
+        x = make_double2(fma(-xi, axr, x.x), fma(-xi, axi, x.y));
+        y = make_double2(fma(-xi, ayr, y.x), fma(-xi, ayi, y.y));
+        st_sa(fld + pos, x, y);
+    }
+}
+
+extern "C" int pmx_pb_create(pmx_ctx* c, const pmx_pb_desc* d, pmx_pb_plan** out) {
+    // (the descriptor is checked before the context, so that the checks run without a device)
+    if (!d || !out) return set_err(c, PMX_ERR_INVALID, "pmx_pb_create: null argument");
+    *out = nullptr;
+    if (d->nfc != 1)
+        return set_err(c, PMX_ERR_UNSUPPORTED, "pmx_pb_create: nfc=%d, PB-NLC takes one-column fields holding one channel",
+                       d->nfc);
+    if (d->precision != PMX_F64) return set_err(c, PMX_ERR_UNSUPPORTED, "pmx_pb_create: FP64 fields only");
+    const int lg = ilog2_exact(d->nfft);
+    if (lg < 6 || lg > 24)
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_create: nfft=%lld, built for powers of two from 2^6 to 2^24",
+                       (long long)d->nfft);
+    if (d->nsymb < 1 || d->nt < 1 || (int64_t)d->nsymb * d->nt != d->nfft)
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_create: nsymb*nt = %d x %d must equal nfft = %lld", d->nsymb, d->nt,
+                       (long long)d->nfft);
+    if (d->batch < 1) return set_err(c, PMX_ERR_INVALID, "pmx_pb_create: batch must be >= 1");
+    if (int rc = check_batch_cols(c, "pmx_pb_create", d->batch, 1)) return rc;
+    if (!d->pulse || d->npulse < 2 || d->npulse % 2 || d->npulse > 16 * d->nt || d->npulse > d->nfft)
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_create: npulse=%d, the pulse must have an even count of 2 to min(16*nt, "
+                       "nfft) = %lld samples", d->npulse, (long long)std::min<int64_t>(16 * (int64_t)d->nt, d->nfft));
+    double e = 0;
+    for (int j = 0; j < d->npulse; ++j) {
+        if (!std::isfinite(d->pulse[j])) return set_err(c, PMX_ERR_INVALID, "pmx_pb_create: pulse sample %d is not finite", j);
+        e += d->pulse[j] * d->pulse[j];
+    }
+    if (!(e > 0) || !std::isfinite(e)) return set_err(c, PMX_ERR_INVALID, "pmx_pb_create: the pulse has no energy");
+    for (int i = 0; i < 3; ++i)
+        if (!std::isfinite(d->weights[i])) return set_err(c, PMX_ERR_INVALID, "pmx_pb_create: weight %d is not finite", i);
+    if (!std::isfinite(d->gamma) || !std::isfinite(d->xi) || !std::isfinite(d->scale))
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_create: gamma, xi and scale must be finite");
+    if (d->ncoef < 1 || d->ncoef > PMX_PB_MAX_COEF)
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_create: ncoef=%d, 1 to %d entries", d->ncoef, PMX_PB_MAX_COEF);
+    if (!d->m || !d->n || !d->coef) return set_err(c, PMX_ERR_INVALID, "pmx_pb_create: null coefficient list");
+    std::vector<PbCoef> list(d->ncoef);
+    const double g = d->gamma * d->scale * d->scale;
+    int K = 0;
+    for (int i = 0; i < d->ncoef; ++i) {
+        const int m = d->m[i], n = d->n[i];
+        if (std::abs(m) > PMX_PB_MAX_K || std::abs(n) > PMX_PB_MAX_K)
+            return set_err(c, PMX_ERR_INVALID, "pmx_pb_create: entry %d has (m, n) = (%d, %d), |m| and |n| at most %d", i, m,
+                           n, PMX_PB_MAX_K);
+        const double cr = d->coef[2 * i], ci = d->coef[2 * i + 1];
+        if (!std::isfinite(cr) || !std::isfinite(ci))
+            return set_err(c, PMX_ERR_INVALID, "pmx_pb_create: coefficient %d is not finite", i);
+        list[i] = PbCoef{g * ci, -(g * cr), m, n};   // -j*gamma*s^2*C
+        K = std::max(K, std::max(std::abs(m), std::abs(n)));
+    }
+    if (!c) return set_err(c, PMX_ERR_INVALID, "pmx_pb_create: null ctx");
+    CK(c, cudaSetDevice(c->device));
+    pmx_pb_plan* p = new (std::nothrow) pmx_pb_plan();
+    if (!p) return set_err(c, PMX_ERR_INVALID, "pmx_pb_create: out of host memory");
+    p->ctx = c;
+    p->nfft = d->nfft;
+    p->nsymb = d->nsymb;
+    p->nt = d->nt;
+    p->batch = d->batch;
+    p->npulse = d->npulse;
+    p->ncoef = d->ncoef;
+    p->K = K;
+    p->wa = d->weights[0];
+    p->wb = d->weights[1];
+    p->wc = d->weights[2];
+    p->xi = d->xi;
+    p->inorm = 1.0 / e;
+    const size_t sym_bytes = (size_t)d->batch * 2 * d->nsymb * sizeof(cpx);
+    cudaError_t err = cudaMallocAsync(&p->pulse, sizeof(double) * d->npulse, c->stream);
+    if (err == cudaSuccess) err = cudaMallocAsync(&p->coef, sizeof(PbCoef) * d->ncoef, c->stream);
+    if (err == cudaSuccess) err = cudaMallocAsync(&p->A, sym_bytes, c->stream);
+    if (err == cudaSuccess) err = cudaMallocAsync(&p->D, sym_bytes, c->stream);
+    if (err == cudaSuccess)
+        err = cudaMemcpyAsync(p->pulse, d->pulse, sizeof(double) * d->npulse, cudaMemcpyHostToDevice, c->stream);
+    if (err == cudaSuccess)
+        err = cudaMemcpyAsync(p->coef, list.data(), sizeof(PbCoef) * d->ncoef, cudaMemcpyHostToDevice, c->stream);
+    if (err == cudaSuccess) err = cudaMemsetAsync(p->A, 0, sym_bytes, c->stream);
+    if (err == cudaSuccess) err = cudaMemsetAsync(p->D, 0, sym_bytes, c->stream);
+    if (err == cudaSuccess) err = cudaStreamSynchronize(c->stream);   // the host tables are the caller's and this frame's
+    if (err != cudaSuccess) {
+        pmx_pb_destroy(p);
+        return set_err(c, PMX_ERR_CUDA, "pmx_pb_create: %s", cudaGetErrorString(err));
+    }
+    *out = p;
+    return PMX_OK;
+}
+
+extern "C" int pmx_pb_exec(pmx_pb_plan* p, pmx_devfield* f) {
+    if (!p || !f) return set_err(p ? p->ctx : nullptr, PMX_ERR_INVALID, "pmx_pb_exec: null argument");
+    pmx_ctx* c = p->ctx;
+    if (f->nfc != 1)
+        return set_err(c, PMX_ERR_UNSUPPORTED, "pmx_pb_exec: nfc=%d, PB-NLC takes one-column fields holding one channel",
+                       f->nfc);
+    if (f->precision != PMX_F64) return set_err(c, PMX_ERR_UNSUPPORTED, "pmx_pb_exec: FP64 fields only");
+    if (f->nfft != p->nfft)
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_exec: the field has nfft=%lld, the plan %lld", (long long)f->nfft,
+                       (long long)p->nfft);
+    if (f->batch != p->batch)
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_exec: the field has batch %d, the plan %d", f->batch, p->batch);
+    if (p->xi == 0) return PMX_OK;   // nothing to subtract: the field is left as it is
+    CK(c, cudaSetDevice(c->device));
+    const size_t N = (size_t)p->nfft;
+    const int l1 = f->log2N1, l2 = f->log2N2;
+    pmx_k_pb_project<<<dim3((unsigned)((p->nsymb + 255) / 256), p->batch), 256, 0, c->stream>>>(
+        f->data, N, l1, l2, p->nsymb, p->nt, p->pulse, p->npulse, p->inorm, p->A);
+    const int smem = (PMX_PB_TILE + 4 * p->K) * 2 * (int)sizeof(cpx);
+    if (smem > 48 * 1024) CK(c, cudaFuncSetAttribute(pmx_k_pb_triplet, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    pmx_k_pb_triplet<<<dim3((unsigned)((p->nsymb + PMX_PB_TILE - 1) / PMX_PB_TILE), p->batch), PMX_PB_THREADS, smem,
+                       c->stream>>>(p->A, p->nsymb, p->coef, p->ncoef, p->K, p->wa, p->wb, p->wc, p->D);
+    pmx_k_pb_apply<<<dim3((unsigned)std::min<size_t>((N + 255) / 256, 148 * 8), p->batch), 256, 0, c->stream>>>(
+        f->data, N, l1, l2, p->nsymb, p->nt, p->pulse, p->npulse, p->D, p->xi);
+    c->launches += 3;
+    CK(c, cudaGetLastError());
+    return PMX_OK;
+}
+
+extern "C" int pmx_pb_symbols(pmx_pb_plan* p, double* A, double* delta) {
+    if (!p) return set_err(nullptr, PMX_ERR_INVALID, "pmx_pb_symbols: null plan");
+    pmx_ctx* c = p->ctx;
+    const size_t bytes = (size_t)p->batch * 2 * p->nsymb * sizeof(cpx);
+    CK(c, cudaSetDevice(c->device));
+    if (A) CK(c, cudaMemcpyAsync(A, p->A, bytes, cudaMemcpyDeviceToHost, c->stream));
+    if (delta) CK(c, cudaMemcpyAsync(delta, p->D, bytes, cudaMemcpyDeviceToHost, c->stream));
+    CK(c, cudaStreamSynchronize(c->stream));
+    return PMX_OK;
+}
+
+extern "C" void pmx_pb_destroy(pmx_pb_plan* p) {
+    if (!p) return;
+    cudaSetDevice(p->ctx->device);
+    for (void* q : {(void*)p->pulse, (void*)p->coef, (void*)p->A, (void*)p->D})
+        if (q) cudaFreeAsync(q, p->ctx->stream);
+    delete p;
+}

@@ -119,22 +119,27 @@ class Link:
         return self._make_cd_plan(ctx)
 
     def _make_cd_plan(self, ctx):
-        s = self.setup
-        sc = dict(s.scalars)
-        sc.update(b30=-sc['b30'], dgdrms=0.0, beta1=-np.asarray(sc['beta1']), beta2=-np.asarray(sc['beta2']))
-        total = s.length * self.nspan
-        inv = FiberSetup(nfft=s.nfft, nfc=s.nfc, fls=(s.fls[0], 0, 0, 0), dphimaxt=math.inf, dzmaxt=total, length=total,
-                         alphalin=0.0, gam=s.gam, betat=-s.betat, db1=np.zeros_like(s.db1), manakov=False, nplates=1,
-                         brf={'db0': np.zeros(1), 'theta': np.zeros(1), 'epsilon': np.zeros(1)}, isv=True, isy=True,
-                         b1=s.b1, dch=s.dch, scalars=sc)
-        desc, keep = setup_to_desc(inv, batch=self.batch, plate_sets=1)
-        return _lib.Plan(ctx, desc, keep)
+        return cd_plan_of(ctx, self.setup, self.nspan, self.batch)
 
     def cd_compensate(self, field: _lib.DeviceField):
         """What a blind receiver knows: the accumulated chromatic dispersion of the link (dsp4cohdec's p.applydcf,
         dsp4cohdec.m:200-210, as an all-pass filter): one linear step with the dispersion of all spans negated.  The PMD
         stays in the field for the polarization demultiplexer."""
         self.cd_plan().execute(field)
+
+
+def cd_plan_of(ctx: _lib.Context, s: FiberSetup, nspan: int, batch: int, precision: Optional[str] = None) -> _lib.Plan:
+    """The all-pass step that undoes the chromatic dispersion of nspan spans of the fiber s: one linear step with the
+    dispersion of all spans negated (Link.cd_plan; pbnlc runs it ahead of the PB-NLC stage)"""
+    sc = dict(s.scalars)
+    sc.update(b30=-sc['b30'], dgdrms=0.0, beta1=-np.asarray(sc['beta1']), beta2=-np.asarray(sc['beta2']))
+    total = s.length * nspan
+    inv = FiberSetup(nfft=s.nfft, nfc=s.nfc, fls=(s.fls[0], 0, 0, 0), dphimaxt=math.inf, dzmaxt=total, length=total,
+                     alphalin=0.0, gam=s.gam, betat=-s.betat, db1=np.zeros_like(s.db1), manakov=False, nplates=1,
+                     brf={'db0': np.zeros(1), 'theta': np.zeros(1), 'epsilon': np.zeros(1)}, isv=True, isy=True,
+                     b1=s.b1, dch=s.dch, scalars=sc)
+    desc, keep = setup_to_desc(inv, batch=batch, plate_sets=1, precision=precision)
+    return _lib.Plan(ctx, desc, keep)
 
 
 # ------------------------------------------------------------------------------------------
@@ -207,7 +212,7 @@ class McRunner:
     def __init__(self, ctx: _lib.Context, setup: FiberSetup, tx_x, tx_y, sym, nsymb: int, nt: int, nspan: int,
                  gain_db: float, nf_db: float, nreal: int, batch: int, rank: int = 0, world: int = 1,
                  receiver: str = 'genie', dsp_params=None, rx_params=None, ich: int = 1, pipeline: bool = True,
-                 compensation: str = 'cd', dbp_params=None):
+                 compensation: str = 'cd', dbp_params=None, pb_params=None):
         """receiver: 'genie' -- ideal linear equaliser from the known plates + data-aided decision (pmx_qpsk_count);
         'blind' -- chromatic dispersion compensated, then the DSP core of dsp4cohdec (CMA polarization demultiplexer,
         Viterbi & Viterbi carrier recovery, differential decision: pmx_dsp_count, polmux_b200/dsp.py);
@@ -222,16 +227,24 @@ class McRunner:
         DBP through each group's own plate draws (Link.plates); with 'genie' it replaces the linear equaliser.
         dbp_params with 'decim' (a power of two >= 2; 'blind' and 'cohmix', a one-column 'unique' field): single-channel DBP
         on nfft/decim samples -- of channel `ich` for 'cohmix', of the channel at the centre of the grid for 'blind'.
-        dbp_params with 'filter_bw' [GHz]: filtered DBP (dbp_plan); with 'nl_taps': enhanced split-step DBP (dbp_plan)"""
+        dbp_params with 'filter_bw' [GHz]: filtered DBP (dbp_plan); with 'nl_taps': enhanced split-step DBP (dbp_plan).
+        'pbnlc' ('blind' and 'cohmix', one channel in a one-column field): the all-pass step, then perturbation-based
+        nonlinearity compensation (polmux_b200/pbnlc.py, pb_plan) with pb_params (xi, K, prune, pulse, nquad, window;
+        default xi = 1, K = 16) at the launch scale s of the link's loss and gain."""
         import torch
         from . import dsp as _dsp
         self.receiver, self.dsp_params = receiver, dict(dsp_params or {})
         if receiver not in ('genie', 'blind', 'cohmix'):
             raise ValueError("receiver must be 'genie', 'blind' or 'cohmix'")
-        if compensation not in ('cd', 'dbp', 'dbp_pmd'):
-            raise ValueError("compensation must be 'cd', 'dbp' or 'dbp_pmd'")
-        if compensation == 'dbp' and receiver == 'genie':
-            raise ValueError("the genie receiver undoes the link with the known plates: compensation='dbp' needs 'blind' or 'cohmix'")
+        if compensation not in ('cd', 'dbp', 'dbp_pmd', 'pbnlc'):
+            raise ValueError("compensation must be 'cd', 'dbp', 'dbp_pmd' or 'pbnlc'")
+        if compensation in ('dbp', 'pbnlc') and receiver == 'genie':
+            raise ValueError("the genie receiver undoes the link with the known plates: compensation='%s' needs 'blind' or "
+                             "'cohmix'" % compensation)
+        if compensation == 'pbnlc' and setup.nfc != 1:
+            raise ValueError("compensation='pbnlc' takes one-column fields holding one channel, got nfc=%d" % setup.nfc)
+        if pb_params is not None and compensation != 'pbnlc':
+            raise ValueError("pb_params needs compensation='pbnlc'")
         if receiver == 'genie' and dict(dbp_params or {}).get('decim') is not None:
             raise ValueError("single-channel DBP (dbp_params 'decim') needs the 'blind' or 'cohmix' receiver")
         self.ref_patmat = _dsp.reference_pattern(np.asarray(sym)[0], np.asarray(sym)[1]) if receiver != 'genie' else None
@@ -275,7 +288,10 @@ class McRunner:
                                 plates=self._link_plates() if compensation == 'dbp_pmd' else None, **dp)
             else:
                 comp = self.link.cd_plan(self.rxctx)
-            self.rx = dict(cd=comp, S=None)
+            self.rx = dict(cd=comp, S=None, pb=None)
+            if compensation == 'pbnlc':
+                from .pbnlc import pb_plan
+                self.rx['pb'] = pb_plan(self.rxctx, setup, nspan, gain_db, batch=batch, nt=nt, **dict(pb_params or {}))
             if receiver == 'cohmix':
                 delay = _rx.evaldelay(x['oftype'], x['obw'] * 0.5) + _rx.evaldelay(x['eftype'], x['ebw']) + S.x['post_delay']
                 self.rx.update(S=S, ich=ich, shift=int(round(delay * nt)),
@@ -293,6 +309,8 @@ class McRunner:
         from . import dsp as _dsp
         R, c = self.rx, self.rxctx
         R['cd'].execute(work)
+        if R['pb'] is not None:
+            R['pb'].execute(work)
         cur, extra = work, {}
         if self.receiver == 'cohmix':
             S = R['S']
@@ -374,6 +392,8 @@ class McRunner:
                     self.rx[k].close()
             if self.pipelined or isinstance(self.rx['cd'], _lib.DbpPlan):
                 self.rx['cd'].close()
+            if self.rx.get('pb') is not None:
+                self.rx['pb'].close()
 
 
 def run_mc(ctx: _lib.Context, setup: FiberSetup, tx_x, tx_y, sym, nsymb: int, nt: int, nspan: int, gain_db: float,

@@ -1,0 +1,184 @@
+"""pbnlc(x, flag, ...): perturbation-based nonlinearity compensation (PB-NLC) of a single-channel received field.
+
+An extension: the reference has none.  The first-order regular-perturbation term of the link is written as a sum of
+symbol triplets (Mecozzi, Clausen & Shtaif, IEEE PTL 12(4), 2000),
+
+    Delta^x_k = -j*gamma * sum_{m,n} C[m,n] * ( a*A^x_{k+m} A^x_{k+n} conj(A^x_{k+m+n})
+                                              + b*A^x_{k+m} A^y_{k+n} conj(A^y_{k+m+n})
+                                              + c*A^y_{k+m} A^y_{k+n} conj(A^x_{k+m+n}) )      (x <-> y for Y)
+
+and subtracted at the receiver from the received samples, scaled by xi (Tao et al., JLT 29(17), 2011).  A_k = <p_k, u> is
+the field projected onto the pulse of symbol k (centred at time index k*nt, circular over the block).  The weights are
+those of the library's nonlinear step: Manakov (1, 1, 0) with gam carrying the 8/9, the CNLSE (1, 2/3, 1/3) -- the
+first-order expansion of -j*gam*[P*u + (s3/3)*J*u] (fiber.m:827-851).
+
+The coefficient table C[m,n] of the whole link (pb_coefficients) is computed once on the host; the stage itself runs on the
+device in one pass at the symbol rate (pmx_pb_create / pmx_pb_exec, include/polmux_ssfm.h).  There is no CPU fallback.
+"""
+from __future__ import annotations
+
+import math
+from typing import Optional
+
+import numpy as np
+import scipy.fft as _sfft
+
+from . import _lib
+from . import synth
+from .fiber import FiberSetup, _get, fiber_setup
+from .gstate import GSTATE
+
+# model weights (a, b, c) of the triplet sum
+MANAKOV = (1.0, 1.0, 0.0)
+CNLSE = (1.0, 2.0 / 3.0, 1.0 / 3.0)
+
+
+def model_weights(setup: FiberSetup):
+    """(a, b, c) and the gamma of the triplet sum for the nonlinear model the fiber's nonlinear step uses"""
+    gam = float(np.asarray(setup.gam, dtype=np.float64).ravel()[0])
+    return (MANAKOV, gam * 8 / 9) if setup.manakov else (CNLSE, gam)
+
+
+def pb_nodes(length: float, nspan: int, alphalin: float, nquad: int):
+    """Gauss-Legendre nodes of every span -> (accumulated distance zeta [nspan*nquad], weight * exp(-alpha*z))"""
+    x, w = np.polynomial.legendre.leggauss(int(nquad))
+    z = 0.5 * length * (x + 1.0)
+    wz = 0.5 * length * w * np.exp(-alphalin * z)
+    zeta = np.concatenate([s * length + z for s in range(int(nspan))])
+    return zeta, np.tile(wz, int(nspan))
+
+
+def _lin_step(betaxdz, u):
+    """fiber.m:771-773: ifft(fft(u) .* exp(-i*betaxdz))"""
+    return _sfft.ifft(_sfft.fft(u) * (np.cos(betaxdz) - 1j * np.sin(betaxdz)))
+
+
+def default_window(setup: FiberSetup, nspan: int, pulse, nt: int, K: int, tol: float = 1e-9) -> int:
+    """The symbols of the circular window the table is computed on: the smallest power of two that holds the pulse
+    dispersed over the whole link (all but `tol` of its energy) plus the 2K symbols of the shifts, at most the block."""
+    N = setup.nfft
+    nsymb = N // nt
+    p0 = np.zeros(N, dtype=np.complex128)
+    p0[(np.arange(len(pulse)) - len(pulse) // 2) % N] = pulse
+    g = _lin_step(np.asarray(setup.betat, dtype=np.float64)[:, 0] * (setup.length * nspan), p0)
+    e = np.abs(np.fft.fftshift(g)) ** 2
+    c = np.cumsum(e) / e.sum()
+    lo, hi = np.searchsorted(c, 0.5 * tol), np.searchsorted(c, 1 - 0.5 * tol)
+    need = (hi - lo + 1) / nt + 2 * K + 8
+    w = 1
+    while w < need:
+        w *= 2
+    return int(min(w, nsymb))
+
+
+def pb_coefficients(setup: FiberSetup, nspan: int, pulse=None, K: int = 16, prune: float = 0.0, nt: Optional[int] = None,
+                    nquad: int = 32, window: Optional[int] = None):
+    """The triplet coefficients of nspan spans of the fiber `setup` describes:
+        C[m,n] = sum_s int_0^Ls exp(-alpha*z) <g_0, g_m g_n conj(g_{m+n})>(s*Ls + z) dz,   |m|, |n| <= K,
+    g_m(zeta) the pulse of symbol m (centred at m*nt) after lin_step(betat*zeta) (no loss), <u, v> = sum conj(u) v / sum p^2.
+    pulse: default synth.cosroll_pulse(nt, 0.2); nt: default GSTATE.NT.  nquad Gauss-Legendre nodes per span; the table is
+    computed on a circular window of `window` symbols (default_window; the link's frequency grid subsampled, so betat is
+    the link's own).  prune drops entries with |C| < prune*|C[0,0]|.
+    By translation invariance the row m is the autocorrelation of a_m = conj(g_0) g_m at symbol-spaced lags,
+    C[m,n] = sum_t a_m(t) conj(a_m(t - n*nt)): one FFT per row and node.  Only the rows m >= 0 are transformed: the
+    autocorrelation gives C[m,-n] = conj(C[m,n]), and with C[m,n] = C[n,m], C[-m,n] = conj(C[m,n]).
+    -> (m, n, C): int32 [ncoef], int32 [ncoef], complex128 [ncoef], m-major with n ascending."""
+    nt = int(nt or GSTATE.NT)
+    K = int(K)
+    if K < 0:
+        raise ValueError('pb_coefficients: K must be >= 0')
+    p = np.asarray(synth.cosroll_pulse(nt, 0.2) if pulse is None else pulse, dtype=np.float64).ravel()
+    N = int(setup.nfft)
+    nsymb = N // nt
+    W = int(window or default_window(setup, nspan, p, nt, K))
+    if nsymb % W or W < 1:
+        raise ValueError('pb_coefficients: the window (%d symbols) must divide the block (%d symbols)' % (W, nsymb))
+    Ws = W * nt
+    bt = np.asarray(setup.betat, dtype=np.float64)[:, 0][::N // Ws]      # the link's bins that fall on the window's grid
+    p0 = np.zeros(Ws, dtype=np.complex128)
+    p0[(np.arange(p.size) - p.size // 2) % Ws] = p
+    norm = float(np.sum(p * p))
+    zeta, wq = pb_nodes(setup.length, nspan, setup.alphalin, nquad)
+    spec = np.zeros((K + 1, W))                                            # sum_nodes w * (|fft a_m|^2 folded to W bins)
+    for z, w in zip(zeta, wq):
+        g0 = _lin_step(bt * z, p0)
+        a = np.conj(g0)[None, :] * np.stack([np.roll(g0, m * nt) for m in range(K + 1)])
+        s = np.abs(_sfft.fft(a, axis=1)) ** 2
+        spec += w * s.reshape(K + 1, nt, W).sum(axis=1)
+    row = _sfft.ifft(spec / nt, axis=1) / norm                            # [m >= 0][lag n mod W]
+    lags = np.arange(-K, K + 1)
+    C = np.empty((2 * K + 1, 2 * K + 1), dtype=np.complex128)
+    C[K:, :] = row[:, lags % W]
+    C[:K, :] = np.conj(row[1:, lags % W][::-1])
+    C = 0.5 * (C + C.T)                                                    # exactly symmetric
+    mm, nn = np.meshgrid(lags, lags, indexing='ij')
+    keep = np.abs(C) >= float(prune) * abs(C[K, K]) if prune else np.ones(C.shape, dtype=bool)
+    return mm[keep].astype(np.int32), nn[keep].astype(np.int32), C[keep]
+
+
+def scale_factor(setup: FiberSetup, nspan: int, gain_db: Optional[float] = None) -> float:
+    """s = (exp(alpha*Ls/2)/sqrt(G))^nspan (G = 1 without an amplifier): the factor that brings the received field to
+    launch scale, the net of DBP's per-step and per-span factors"""
+    g = 1.0 if gain_db is None else 10 ** (gain_db * 0.1)
+    return (math.exp(0.5 * setup.alphalin * setup.length) / math.sqrt(g)) ** int(nspan)
+
+
+def pb_plan(ctx: _lib.Context, setup: FiberSetup, nspan: int, gain_db: Optional[float] = None, xi: float = 1.0,
+            K: int = 16, prune: float = 0.0, pulse=None, batch: int = 1, nt: Optional[int] = None, nquad: int = 32,
+            window: Optional[int] = None, coefs=None) -> _lib.PbPlan:
+    """The PB-NLC stage of nspan spans of the fiber `setup` describes (amplifier of gain_db [dB] after each; None: none), for
+    resident one-column FP64 fields of `batch` realizations: pmx_pb_create with the table of pb_coefficients (or `coefs`,
+    a (m, n, C) table), the model and gamma of the fiber, and s = scale_factor(setup, nspan, gain_db)."""
+    nt = int(nt or GSTATE.NT)
+    p = np.asarray(synth.cosroll_pulse(nt, 0.2) if pulse is None else pulse, dtype=np.float64).ravel()
+    if setup.nfc != 1:
+        raise ValueError('pmx_pb_create: nfc=%d, PB-NLC takes one-column fields holding one channel' % setup.nfc)
+    _lib.check_pb_k(K)
+    m, n, C = pb_coefficients(setup, nspan, p, K, prune, nt, nquad, window) if coefs is None else coefs
+    w, gam = model_weights(setup)
+    return _lib.PbPlan(ctx, _lib.make_pb(setup.nfft // nt, nt, batch, p, w, gam, xi, scale_factor(setup, nspan, gain_db),
+                                         m, n, C))
+
+
+def pbnlc(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, xi: float = 1.0, K: int = 16, prune: float = 0.0,
+          pulse=None, ctx: Optional[_lib.Context] = None, nquad: int = 32, window: Optional[int] = None):
+    """Compensates GSTATE.FIELDX / FIELDY in place for nspan spans of the fiber x, the amplifier of gain_db [dB] after each
+    (None: no amplifier): the all-pass step that undoes the link's chromatic dispersion (as Link.cd_plan), then the PB-NLC
+    stage with the triplet table of K (pb_coefficients) at s = scale_factor(...), the fraction xi of the perturbation
+    subtracted.  The nonlinear model is the one fiber() used: Manakov when x.manakov is 'yes' and the flag has 'p', else the
+    CNLSE.  One channel (GSTATE.NCH == 1), two polarizations, FP64.  The field stays resident on the device like dbp()
+    leaves it."""
+    from .mc import cd_plan_of
+    G = GSTATE
+    f = str(flag).lower()
+    if len(f) != 4:
+        raise ValueError("wrong flag. E.g. flag can be 'g---','gp--','-s--', etc")
+    if G.NCH != 1:
+        raise ValueError('pbnlc: PB-NLC takes a field holding one channel (GSTATE.NCH == 1), got %d' % G.NCH)
+    if not G.has_y():
+        raise ValueError('pbnlc: PB-NLC takes two-polarization fields (FIELDY is empty)')
+    if G.field_shape()[1] != 1:
+        raise ValueError('pbnlc: PB-NLC takes one-column fields')
+    if int(nspan) < 1:
+        raise ValueError('pbnlc: nspan must be >= 1')
+    _lib.check_pb_k(K)
+    s = fiber_setup(x, f[0] + '-' + f[2:])
+    s.manakov = f[1] == 'p' and str(_get(x, 'manakov', 'no')) == 'yes'
+    ctx = ctx or _lib.default_context()
+    cd = cd_plan_of(ctx, s, int(nspan), 1, precision='f64')
+    try:
+        plan = pb_plan(ctx, s, nspan, gain_db, xi, K, prune, pulse, nquad=nquad, window=window)
+    except Exception:
+        cd.close()
+        raise
+    fld, hx, hy = G.take_device(ctx, _lib.PMX_F64)
+    try:
+        cd.execute(fld)
+        plan.execute(fld)
+    except Exception:
+        fld.close()
+        raise
+    finally:
+        plan.close()
+        cd.close()
+    G.put_device(fld, hx, hy)

@@ -1,0 +1,157 @@
+"""Times perturbation-based nonlinearity compensation (pmx_pb_create / pmx_pb_exec) on the C2 shape.
+
+    python tools/pbnlc_time.py [--nspan 10] [--reps 20] [--ks 4,8,16,32,64] [--out DIR]
+
+C2 (BASELINE.md): one 28-GBaud PDM-QPSK channel, 2^16 symbols x 16 samples = 2^20 samples, 80 km spans with 16 dB
+amplifiers, Manakov.  In one process:
+  1. the triplet kernel (pmx_k_pb_triplet) alone against the coefficient count (full tables of K in --ks, (2K+1)^2 entries)
+     at batch 1 and 16: its device time from torch.profiler over --reps executions, and its FP64 rate -- 52 FP64
+     instructions (32 DFMA, 20 DMUL) per entry and symbol, counted from the code -- as a share of the FP64 pipe rate
+     tools/ubench/fp64_rate.cu measures in the same call (its best DFMA/clk/SM x 148 SMs x the card's maximum SM clock);
+  2. per group of 16 realizations: the CD all-pass step + PB-NLC (K = 32, the table of the link) against DBP at one step per
+     span on the whole field (single-channel DBP of the one channel, decim 2) and full DBP, each the median wall time of
+     a call that ends synchronised (the PB-NLC plan with xi = 1e-9, so that the repeated runs on one field stay bounded).
+The card's name, power limit and maximum SM clock are read in the same run and printed with the numbers."""
+import argparse
+import json
+import os
+import re
+import subprocess
+import sys
+import tempfile
+import time
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+import polmux_b200 as pmx  # noqa: E402
+from polmux_b200 import _lib, mc, synth  # noqa: E402
+from polmux_b200.dbp import dbp_plan  # noqa: E402
+from polmux_b200.fiber import fiber_setup  # noqa: E402
+from polmux_b200.pbnlc import pb_coefficients, pb_plan, model_weights  # noqa: E402
+
+FP64_INSTR = 52
+
+
+def card():
+    try:
+        return subprocess.run(['nvidia-smi', '-i', '0', '--query-gpu=name,power.limit,clocks.max.sm',
+                               '--format=csv,noheader'], capture_output=True, text=True, timeout=30).stdout.strip()
+    except Exception as e:  # noqa: BLE001
+        return 'nvidia-smi unavailable (%s)' % e
+
+
+def fp64_pipe():
+    """best DFMA/clk/SM of tools/ubench/fp64_rate.cu, built into a temporary directory"""
+    with tempfile.TemporaryDirectory() as d:
+        exe = os.path.join(d, 'fp64_rate')
+        subprocess.run(['nvcc', '-arch=sm_100a', '-O3', os.path.join(ROOT, 'tools', 'ubench', 'fp64_rate.cu'), '-o', exe],
+                       check=True)
+        out = subprocess.run([exe], capture_output=True, text=True, check=True).stdout
+    return max(float(v) for v in re.findall(r'-> ([0-9.]+) DFMA/clk/SM', out))
+
+
+def kernel_ms(fn, reps, name):
+    """device time of kernel `name` per call of fn, from torch.profiler"""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    fn()
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(reps):
+            fn()
+        torch.cuda.synchronize()
+    tot = sum(e.device_time_total for e in prof.key_averages() if name in e.key)
+    return tot / reps / 1000.0
+
+
+def wall_ms(fn, reps):
+    fn()
+    ts = []
+    for _ in range(reps):
+        t = time.perf_counter()
+        fn()
+        ts.append(time.perf_counter() - t)
+    return 1000.0 * float(np.median(ts))
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument('--nsymb', type=int, default=1 << 16)
+    ap.add_argument('--nt', type=int, default=16)
+    ap.add_argument('--nspan', type=int, default=10)
+    ap.add_argument('--reps', type=int, default=20)
+    ap.add_argument('--ks', default='4,8,16,32,64')
+    ap.add_argument('--out', default=None, help='directory for pbnlc_time.json')
+    a = ap.parse_args()
+    import torch
+    torch.cuda.init()
+    info = card()
+    print('card:', info)
+    dfma = fp64_pipe()
+    mhz = float(re.findall(r'([0-9.]+) MHz', info)[-1]) if 'MHz' in info else float('nan')
+    pipe = dfma * 148 * mhz * 1e6                                   # DFMA instructions per second
+    print('FP64 pipe: %.1f DFMA/clk/SM (fp64_rate.cu) x 148 SMs x %.0f MHz = %.3g FP64 instr/s' % (dfma, mhz, pipe))
+    ex, ey, _, _ = synth.pdm_qpsk(a.nsymb, a.nt, 1)
+    pmx.reset_all(a.nsymb, a.nt, 1)
+    G = pmx.GSTATE
+    G.SYMBOLRATE, G.LAMBDA, G.POWER = 28.0, np.array([1550.0]), np.array([1.0])
+    pmx.create_field('unique', ex, ey, {'power': 'average'})
+    fib = dict(synth.SMF)
+    fib.update(length=8e4, manakov='yes')
+    s = fiber_setup(fib, 'g-s-')
+    s.manakov = True
+    ctx = _lib.Context(0)
+    N = a.nsymb * a.nt
+    res = {'card': info, 'dfma_per_clk_sm': dfma, 'triplet': [], 'chain': {}}
+    t0 = time.perf_counter()
+    m, n, C = pb_coefficients(s, a.nspan, None, 64, nt=a.nt)
+    res['table_s_K64'] = time.perf_counter() - t0
+    print('table of %d x 80 km, K = 64: %.1f s on one host thread' % (a.nspan, res['table_s_K64']))
+    w, gam = model_weights(s)
+    p = synth.cosroll_pulse(a.nt, 0.2)
+    for batch in (1, 16):
+        fld = _lib.DeviceField(ctx, N, 1, batch)
+        x = np.broadcast_to(np.asarray(G.FIELDX).T[None], (batch, 1, N))
+        y = np.broadcast_to(np.asarray(G.FIELDY).T[None], (batch, 1, N))
+        fld.upload(x, y)
+        for K in [int(k) for k in a.ks.split(',')]:
+            sel = (np.abs(m) <= K) & (np.abs(n) <= K)
+            plan = _lib.PbPlan(ctx, _lib.make_pb(a.nsymb, a.nt, batch, p, w, gam, 1e-9, 1.0, m[sel], n[sel], C[sel]))
+            ms = kernel_ms(lambda: (plan.execute(fld), ctx.sync()), a.reps, 'pmx_k_pb_triplet')
+            plan.close()
+            ncoef = int(sel.sum())
+            rate = FP64_INSTR * ncoef * a.nsymb * batch / (ms * 1e-3)
+            row = dict(batch=batch, K=K, ncoef=ncoef, triplet_ms=ms, fp64_instr_per_s=rate, pipe_share=rate / pipe)
+            res['triplet'].append(row)
+            print('triplet batch %2d K %2d ncoef %5d: %8.3f ms  %.3g FP64 instr/s  %.1f %% of the pipe'
+                  % (batch, K, ncoef, ms, rate, 100 * rate / pipe))
+        fld.close()
+    # per group of 16: CD + PB-NLC against DBP at one step per span
+    batch = 16
+    fld = _lib.DeviceField(ctx, N, 1, batch)
+    x = np.broadcast_to(np.asarray(G.FIELDX).T[None], (batch, 1, N))
+    y = np.broadcast_to(np.asarray(G.FIELDY).T[None], (batch, 1, N))
+    fld.upload(x, y)
+    cd = mc.cd_plan_of(ctx, s, a.nspan, batch, precision='f64')
+    sel = (np.abs(m) <= 32) & (np.abs(n) <= 32)
+    # (xi = 1e-9: the chain runs over and over on one field, which a full correction each time would drive to overflow;
+    # every xi != 0 costs the same launches and work)
+    pb = pb_plan(ctx, s, a.nspan, 16.0, xi=1e-9, batch=batch, nt=a.nt, coefs=(m[sel], n[sel], C[sel]))
+    res['chain']['cd_pbnlc_K32_ms'] = wall_ms(lambda: (cd.execute(fld), pb.execute(fld), ctx.sync()), a.reps)
+    res['chain']['cd_ms'] = wall_ms(lambda: (cd.execute(fld), ctx.sync()), a.reps)
+    for name, kw in (('dbp_channel_1step_ms', dict(decim=2, shift=0)), ('dbp_full_1step_ms', {})):
+        plan = dbp_plan(ctx, s, a.nspan, 16.0, steps_per_span=1, batch=batch, precision='f64', **kw)
+        res['chain'][name] = wall_ms(lambda: (plan.execute(fld), ctx.sync()), a.reps)
+        plan.close()
+    print('per group of 16 at 2^20, %d spans: %s' % (a.nspan, json.dumps({k: round(v, 3) for k, v in res['chain'].items()})))
+    if a.out:
+        os.makedirs(a.out, exist_ok=True)
+        with open(os.path.join(a.out, 'pbnlc_time.json'), 'w') as f:
+            json.dump(res, f, indent=1)
+
+
+if __name__ == '__main__':
+    main()
