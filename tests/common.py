@@ -4,6 +4,7 @@ import numpy as np
 import oracle.fiber_oracle as orc
 import polmux_b200 as pmx
 from polmux_b200 import synth
+from polmux_b200.fiber import fiber_setup
 
 
 def base_fiber(**kw):
@@ -47,3 +48,23 @@ def scalar_tx(nsymb, nt, nch, rate=10.0, pavg=4.0):
 
 def rel_l2(ux, uy, rx, ry):
     return orc.rel_l2(ux, uy, rx, ry)
+
+
+def _rel(a, b):
+    return float(np.linalg.norm(np.asarray(a) - np.asarray(b)) / np.linalg.norm(np.asarray(b)))
+
+
+def _cols(a):
+    return np.ascontiguousarray(np.asarray(a).T)[None]          # GSTATE [nfft, nfc] -> [1][nfc][nfft]
+
+
+def _mc_scenario(nsymb, nt, pavg_mw):
+    ex, ey, sx, sy = synth.pdm_qpsk(nsymb, nt, 1)
+    pmx.reset_all(nsymb, nt, 1)
+    G = pmx.GSTATE
+    G.SYMBOLRATE, G.LAMBDA, G.POWER = 28.0, np.array([1550.0]), np.array([float(pavg_mw)])
+    pmx.create_field('unique', ex, ey, {'power': 'average'})
+    fib = dict(synth.SMF)
+    fib.update(length=8e4, dgd=0.3, nplates=20, manakov='yes')
+    setup = fiber_setup(fib, 'gps-', rng=np.random.Generator(np.random.PCG64(0)))
+    return G, setup, np.stack([sx[:, 0], sy[:, 0]]).astype(np.uint8)

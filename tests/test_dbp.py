@@ -14,10 +14,10 @@ import pytest
 import oracle.fiber_oracle as orc
 import dbp_oracle
 import polmux_b200 as pmx
-from polmux_b200 import _lib, mc, synth
+from polmux_b200 import _lib, mc
 from polmux_b200.dbp import dbp_plan
 from polmux_b200.fiber import fiber_setup, setup_to_desc
-from common import base_fiber, make_tx, rel_l2
+from common import _cols, _mc_scenario, base_fiber, make_tx, rel_l2
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GAIN_DB = 16.0
@@ -151,10 +151,6 @@ def _run_device(ctx, s, xs, ys, precision='f64', **kw):
     return out
 
 
-def _cols(a):
-    return np.ascontiguousarray(np.asarray(a).T)[None]          # GSTATE [nfft, nfc] -> [1][nfc][nfft]
-
-
 PARITY = [  # nsymb, nt, nch, manakov, schedule, nspan, batch
     (256, 16, 1, False, 'uniform', 3, 1),
     (256, 16, 3, True, 'explicit', 1, 1),
@@ -251,18 +247,6 @@ def test_dbp_realizations_are_independent(ctx):
     for b in range(3):
         ox, oy = _run_device(ctx, s, xs[b:b + 1], ys[b:b + 1], **kw)
         assert np.array_equal(ox[0], bx[b]) and np.array_equal(oy[0], by[b]), b
-
-
-def _mc_scenario(nsymb, nt, pavg_mw):
-    ex, ey, sx, sy = synth.pdm_qpsk(nsymb, nt, 1)
-    pmx.reset_all(nsymb, nt, 1)
-    G = pmx.GSTATE
-    G.SYMBOLRATE, G.LAMBDA, G.POWER = 28.0, np.array([1550.0]), np.array([float(pavg_mw)])
-    pmx.create_field('unique', ex, ey, {'power': 'average'})
-    fib = dict(synth.SMF)
-    fib.update(length=8e4, dgd=0.3, nplates=20, manakov='yes')
-    setup = fiber_setup(fib, 'gps-', rng=np.random.Generator(np.random.PCG64(0)))
-    return G, setup, np.stack([sx[:, 0], sy[:, 0]]).astype(np.uint8)
 
 
 @pytest.mark.gpu

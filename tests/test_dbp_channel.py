@@ -2,7 +2,7 @@
 dbp_params 'decim'): one channel of a 'unique' multiplex cut out, backpropagated at nfft/decim samples on its own
 dispersion, and returned to its own bins.
 
-Oracle: tests/dbp_channel_oracle.py -- the full-field oracles on the cropped spectrum -- tied here to the full-field
+Oracle: tests/dbp_oracle.dbp_channel -- the full-field oracles on the cropped spectrum -- tied here to the full-field
 oracle (xi = 0: the full DBP followed by the ideal band-pass) and to the forward oracle (the exact inverse of a link run
 on the channel alone)."""
 import ctypes
@@ -14,14 +14,13 @@ import numpy as np
 import pytest
 
 import oracle.fiber_oracle as orc
-import dbp_channel_oracle as dco
 import dbp_oracle
 import polmux_b200 as pmx
 from polmux_b200 import _lib, mc, synth
 from polmux_b200.dbp import dbp_plan
 from polmux_b200.fiber import fiber_setup, setup_to_desc
 from polmux_b200.receiver import CohmixSetup, channel_ndfn
-from common import base_fiber, make_tx, rel_l2
+from common import _cols, _rel, base_fiber, make_tx, rel_l2
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GAIN_DB = 16.0
@@ -38,11 +37,8 @@ def _setup(nsymb, nt, nch=3, flag='g-s-', manakov=False, pavg_mw=4.0, length=8e4
 
 
 def _oracle(ux, uy, s, shift, decim, **kw):
-    return dco.dbp_channel(ux, uy, s.betat, s.gam, s.alphalin, s.length, 'yes' if s.manakov else 'no', shift, decim, **kw)
-
-
-def _rel(a, b):
-    return float(np.linalg.norm(np.asarray(a) - np.asarray(b)) / np.linalg.norm(np.asarray(b)))
+    return dbp_oracle.dbp_channel(ux, uy, s.betat, s.gam, s.alphalin, s.length, 'yes' if s.manakov else 'no', shift, decim,
+                                  **kw)
 
 
 def _scalar_unique(nsymb, nt, nch, pavg=4.0):
@@ -73,8 +69,8 @@ def test_oracle_linear_is_the_band_passed_full_field_dbp(manakov):
     kw = dict(nspan=2, gain=G16, steps_per_span=3, xi=0.0)
     cx, cy = _oracle(gs.FIELDX, gs.FIELDY, s, m, 8, **kw)
     fx, fy = dbp_oracle.dbp(gs.FIELDX, gs.FIELDY, s.betat, s.gam, s.alphalin, 1, s.length, 'yes' if manakov else 'no', **kw)
-    b = dco.channel_bins(s.nfft, m, 8)
-    err = rel_l2(cx, cy, dco.band_pass(fx, b), dco.band_pass(fy, b))
+    b = dbp_oracle.channel_bins(s.nfft, m, 8)
+    err = rel_l2(cx, cy, dbp_oracle.band_pass(fx, b), dbp_oracle.band_pass(fy, b))
     assert err <= 1e-13, err
 
 
@@ -84,8 +80,8 @@ def test_oracle_inverts_a_link_run_on_the_channel_alone(flag):
     embedded at shift 0 in N; single-channel DBP with the forward steps and xi = 1 returns the embedded Tx"""
     gs, s = _setup(256, 16, nch=1, flag=flag, dgd=0.5, nplates=20) if flag == 'gps-' else _setup(256, 16, nch=1)
     r, N = 4, s.nfft
-    b = dco.channel_bins(N, 0, r)
-    tx, ty = dco.crop(gs.FIELDX, b, r), dco.crop(gs.FIELDY, b, r)
+    b = dbp_oracle.channel_bins(N, 0, r)
+    tx, ty = dbp_oracle.crop(gs.FIELDX, b, r), dbp_oracle.crop(gs.FIELDY, b, r)
     bt, d1 = s.betat[b], s.db1[b]
     brfs = [dict(s.brf)] * 2                     # (without 'p' the forward oracle still reads the identity plates)
     if flag == 'gps-':
@@ -97,12 +93,12 @@ def test_oracle_inverts_a_link_run_on_the_channel_alone(flag):
         steps.append([st['dz'] for st in sched])
         ux, uy = ux * math.sqrt(G16), uy * math.sqrt(G16)
     assert sum(len(x) for x in steps) > 4
-    ex, ey = dco.embed(ux, b, N, r), dco.embed(uy, b, N, r)
+    ex, ey = dbp_oracle.embed(ux, b, N, r), dbp_oracle.embed(uy, b, N, r)
     kw = dict(nspan=2, gain=G16, step_len=np.concatenate(steps), span_steps=[len(x) for x in steps])
     if flag == 'gps-':
         kw.update(db1=s.db1, brfs=brfs)
     gx, gy = _oracle(ex, ey, s, 0, r, **kw)
-    err = rel_l2(gx, gy, dco.embed(tx, b, N, r), dco.embed(ty, b, N, r))
+    err = rel_l2(gx, gy, dbp_oracle.embed(tx, b, N, r), dbp_oracle.embed(ty, b, N, r))
     assert err <= 1e-12, err
 
 
@@ -185,10 +181,6 @@ def test_channel_dbp_has_no_cpu_fallback():
 
 
 # ---------------------------------------------------------------------------------------------------------------- GPU
-def _cols(a):
-    return np.ascontiguousarray(np.asarray(a).T)[None]          # GSTATE [nfft, nfc] -> [1][nfc][nfft]
-
-
 def _run_device(ctx, s, xs, ys, precision='f64', plates=None, **kw):
     """DBP of the fields xs, ys ([batch][1][nfft]) on the device -> (x, y) of the same shape"""
     b = xs.shape[0]
@@ -272,10 +264,10 @@ def test_channel_dbp_inverts_fiber_on_the_device(flag):
     rx, ry = G.FIELDX.copy(), G.FIELDY.copy()
     pmx.reset_all(nsymb, nt * r, 1)
     G.SYMBOLRATE, G.LAMBDA, G.POWER = rate, lam, power
-    b = dco.channel_bins(nsymb * nt * r, 0, r)
-    G.FIELDX, G.FIELDY = dco.embed(rx, b, nsymb * nt * r, r), dco.embed(ry, b, nsymb * nt * r, r)
+    b = dbp_oracle.channel_bins(nsymb * nt * r, 0, r)
+    G.FIELDX, G.FIELDY = dbp_oracle.embed(rx, b, nsymb * nt * r, r), dbp_oracle.embed(ry, b, nsymb * nt * r, r)
     pmx.dbp(fib, flag, step_len=steps, ich=1, decim=r, brf=brf if flag == 'gps-' else None)
-    err = rel_l2(G.FIELDX, G.FIELDY, dco.embed(tx, b, nsymb * nt * r, r), dco.embed(ty, b, nsymb * nt * r, r))
+    err = rel_l2(G.FIELDX, G.FIELDY, dbp_oracle.embed(tx, b, nsymb * nt * r, r), dbp_oracle.embed(ty, b, nsymb * nt * r, r))
     print('channel dbp exact inverse %s: %d steps, rel_l2 %.3e' % (flag, len(steps), err))
     assert err <= 1e-11
 
@@ -290,7 +282,7 @@ def test_channel_dbp_scalar_path_matches_the_oracle():
     u = G.FIELDX.copy()
     kw = dict(nspan=2, steps_per_span=3)
     pmx.dbp(fib, 'g-s-', gain_db=GAIN_DB, ich=3, decim=16, **kw)
-    want = dco.dbp_channel_scalar(u, s.betat, s.gam, s.alphalin, s.length, channel_ndfn(3), 16, gain=G16, **kw)
+    want = dbp_oracle.dbp_channel_scalar(u, s.betat, s.gam, s.alphalin, s.length, channel_ndfn(3), 16, gain=G16, **kw)
     err = _rel(G.FIELDX, want)
     print('channel dbp scalar parity: rel_l2 %.3e' % err)
     assert G.FIELDY is None or not np.size(G.FIELDY)
@@ -311,7 +303,7 @@ def test_linear_channel_dbp_is_full_field_dbp_then_the_band_filter(ctx):
     plan.execute(fld)
     plan.close()
     H = np.zeros(s.nfft)
-    H[dco.channel_bins(s.nfft, m, r)] = 1
+    H[dbp_oracle.channel_bins(s.nfft, m, r)] = 1
     band = _lib.Filter(ctx, s.nfft, 1, H, batch=2)
     band.execute(fld)
     band.close()
@@ -329,11 +321,11 @@ def test_without_dispersion_loss_or_nonlinearity_it_is_the_band_pass(ctx):
     m, r = channel_ndfn(3), 16
     xs, ys = _batch2(gs)
     gx, gy = _run_device(ctx, s, xs, ys, shift=m, decim=r, nspan=2, steps_per_span=2)
-    b = dco.channel_bins(s.nfft, m, r)
+    b = dbp_oracle.channel_bins(s.nfft, m, r)
     out = np.ones(s.nfft, bool)
     out[b] = False
     for k in range(2):
-        err = rel_l2(gx[k, 0], gy[k, 0], dco.band_pass(xs[k, 0], b), dco.band_pass(ys[k, 0], b))
+        err = rel_l2(gx[k, 0], gy[k, 0], dbp_oracle.band_pass(xs[k, 0], b), dbp_oracle.band_pass(ys[k, 0], b))
         spec = np.abs(np.fft.fft(gx[k, 0])) ** 2 + np.abs(np.fft.fft(gy[k, 0])) ** 2
         leak = spec[out].sum() / spec.sum()
         print('band only, realization %d: rel_l2 %.3e, energy outside the band %.3e' % (k, err, leak))

@@ -1,17 +1,15 @@
 """Enhanced split-step digital backpropagation (pmx_dbp_set_taps, DbpPlan.set_taps, dbp_plan / pmx.dbp nl_taps, dbp.m
-options.taps, tests/dbp_essfm_oracle.py): a circular FIR of real taps on the intensity of every backward nonlinear step."""
+options.taps, tests/dbp_oracle.py with taps=): a circular FIR of real taps on the intensity of every backward nonlinear
+step."""
 import numpy as np
 import pytest
 
-import dbp_essfm_oracle as deo
-import dbp_filtered_oracle as dfo
 import dbp_oracle
-import dbp_scalar_oracle
 import polmux_b200 as pmx
 from polmux_b200 import _lib, mc
 from polmux_b200.dbp import dbp_plan
 from polmux_b200.fiber import fiber_setup
-from common import base_fiber, make_tx, rel_l2, scalar_tx
+from common import _cols, _mc_scenario, base_fiber, make_tx, rel_l2, scalar_tx
 
 GAIN_DB = 16.0
 G16 = 10 ** (GAIN_DB / 10)
@@ -36,27 +34,20 @@ def _man(s):
 
 
 # ---------------------------------------------------------------------------------------------------------------- CPU
-def _as_filtered(monkeypatch, nfft, c):
-    """dbp_filtered_oracle with H = fft(c placed circularly) in place of its Gaussian (any bw selects it)"""
-    monkeypatch.setattr(dfo, 'gauss_response', lambda n, bw: deo.circular_response(n, c))
-
-
 @pytest.mark.parametrize('manakov', [False, True])
-def test_oracle_is_filtered_dbp_with_the_circular_response_two_pol(monkeypatch, manakov):
+def test_oracle_is_filtered_dbp_with_the_circular_response_two_pol(manakov):
     gs, s = _setup(64, 16, nch=3, pavg_mw=10.0, manakov=manakov)
     args = (gs.FIELDX, gs.FIELDY, s.betat, s.gam, s.alphalin, s.nfc, s.length, _man(s))
     kw = dict(nspan=2, gain=G16, steps_per_span=2)
     for k in (1, 16, 32):
         c = taps(k)
-        a = deo.dbp(*args, taps=c, **kw)
-        _as_filtered(monkeypatch, s.nfft, c)
-        b = dfo.dbp(*args, bw=1.0, **kw)
-        monkeypatch.undo()
+        a = dbp_oracle.dbp(*args, taps=c, **kw)
+        b = dbp_oracle.dbp(*args, response=dbp_oracle.circular_response(s.nfft, c), **kw)
         assert rel_l2(*a, *b) <= 1e-13, k
-        assert rel_l2(*a, *deo.dbp(*args, **kw)) > 1e-6
+        assert rel_l2(*a, *dbp_oracle.dbp(*args, **kw)) > 1e-6
 
 
-def test_oracle_is_filtered_dbp_with_the_circular_response_pmd_and_channel(monkeypatch):
+def test_oracle_is_filtered_dbp_with_the_circular_response_pmd_and_channel():
     gs = make_tx(64, 16, pavg_mw=10.0)
     s = fiber_setup(base_fiber(length=8e4, slope=0.057, dphimax=0.02, dgd=0.5, nplates=12, manakov='no'), 'gps-',
                     rng=np.random.Generator(np.random.PCG64(7)))
@@ -64,25 +55,23 @@ def test_oracle_is_filtered_dbp_with_the_circular_response_pmd_and_channel(monke
     c = taps(7)
     kw = dict(nspan=2, gain=G16, steps_per_span=2)
     pargs = (gs.FIELDX, gs.FIELDY, s.betat, np.asarray(s.db1), s.gam, s.alphalin, 1, s.length, 'no', brfs)
-    a = deo.dbp_pmd(*pargs, taps=c, **kw)
+    a = dbp_oracle.dbp_pmd(*pargs, taps=c, **kw)
     cargs = (gs.FIELDX, gs.FIELDY, s.betat, s.gam, s.alphalin, s.length, 'no', 0, 4)
-    ca = deo.dbp_channel(*cargs, taps=c, **kw)
-    _as_filtered(monkeypatch, s.nfft, c)
-    assert rel_l2(*a, *dfo.dbp_pmd(*pargs, bw=1.0, **kw)) <= 1e-13
-    monkeypatch.setattr(dfo, 'gauss_response', lambda n, bw: deo.circular_response(n, c))   # (on the channel's grid)
-    assert rel_l2(*ca, *dfo.dbp_channel(*cargs, bw=1.0, **kw)) <= 1e-13
+    ca = dbp_oracle.dbp_channel(*cargs, taps=c, **kw)
+    assert rel_l2(*a, *dbp_oracle.dbp_pmd(*pargs, response=dbp_oracle.circular_response(s.nfft, c), **kw)) <= 1e-13
+    H = dbp_oracle.circular_response(s.nfft // 4, c)                                 # on the channel's grid
+    assert rel_l2(*ca, *dbp_oracle.dbp_channel(*cargs, response=H, **kw)) <= 1e-13
 
 
 @pytest.mark.parametrize('flag', ['g-s-', 'g--x', 'g-sx'])
-def test_oracle_is_filtered_dbp_with_the_circular_response_scalar(monkeypatch, flag):
+def test_oracle_is_filtered_dbp_with_the_circular_response_scalar(flag):
     u = scalar_tx(32, 32, 3, pavg=8.0).FIELDX
     ss = fiber_setup(base_fiber(length=1e5, slope=0.057), flag)
     sa = (u, ss.betat, ss.gam, ss.alphalin, ss.nfc, ss.length, ss.fls[2], ss.fls[3])
     kw = dict(nspan=2, gain=G16, steps_per_span=3)
     c = taps(5)
-    a = deo.dbp_scalar(*sa, taps=c, **kw)
-    _as_filtered(monkeypatch, u.shape[0], c)
-    b = dfo.dbp_scalar(*sa, bw=1.0, **kw)
+    a = dbp_oracle.dbp_scalar(*sa, taps=c, **kw)
+    b = dbp_oracle.dbp_scalar(*sa, response=dbp_oracle.circular_response(u.shape[0], c), **kw)
     assert np.linalg.norm(a - b) <= 1e-13 * np.linalg.norm(b)
 
 
@@ -90,12 +79,12 @@ def test_oracle_single_unit_tap_is_plain_dbp():
     gs, s = _setup(64, 16, nch=2, pavg_mw=10.0)
     args = (gs.FIELDX, gs.FIELDY, s.betat, s.gam, s.alphalin, s.nfc, s.length, 'no')
     kw = dict(nspan=2, gain=G16, steps_per_span=3)
-    assert rel_l2(*deo.dbp(*args, taps=[1.0], **kw), *dbp_oracle.dbp(*args, **kw)) <= 1e-14
+    assert rel_l2(*dbp_oracle.dbp(*args, taps=[1.0], **kw), *dbp_oracle.dbp(*args, **kw)) <= 1e-14
     u = scalar_tx(32, 32, 3, pavg=8.0).FIELDX
     ss = fiber_setup(base_fiber(length=1e5, slope=0.057), 'g-sx')
     sa = (u, ss.betat, ss.gam, ss.alphalin, ss.nfc, ss.length, 1, 1)
-    a = deo.dbp_scalar(*sa, taps=[1.0], **kw)
-    b = dbp_scalar_oracle.dbp_scalar(*sa, **kw)
+    a = dbp_oracle.dbp_scalar(*sa, taps=[1.0], **kw)
+    b = dbp_oracle.dbp_scalar(*sa, **kw)
     assert np.linalg.norm(a - b) <= 1e-14 * np.linalg.norm(b)
 
 
@@ -125,32 +114,6 @@ def test_native_mc_rejects_nl_taps():
 
 
 # -------------------------------------------------------------------------------------------------- M front-end (dbp.m)
-def _taps_gateway(log):
-    """test_matlab_dbp's oracle-backed gateway; a 'dbp' call with the trailing taps (two polarizations, full field, no PMD)
-    is answered by the ESSFM oracle.  Every 'dbp' call logs its taps (None: the 15-argument call)."""
-    import test_matlab_dbp as tmd
-    base = tmd.oracle_gateway()
-
-    def call(it, a, nargout):
-        if a[0] != 'dbp':
-            return base(it, a, nargout)
-        log.append(np.asarray(a[15], dtype=np.float64) if len(a) > 15 else None)
-        if len(a) == 15:
-            return base(it, a, nargout)
-        assert len(a) == 16 and np.size(a[15]) > 0
-        ux, uy, betat, db1, P, gam = a[1:7]
-        scal, D, fls = a[9], np.asarray(a[10], dtype=np.float64).ravel(), [int(v) for v in np.asarray(a[7]).ravel()]
-        _, _, alphalin, lf, _, manakov = [float(v) for v in np.asarray(P).ravel()]
-        nfft, nfc = np.shape(ux)
-        if np.size(betat) == 0:
-            betat, db1 = tmd._vectors(scal, nfft, nfc, fls[1])
-        out = deo.dbp(ux, uy, betat, np.asarray(gam, dtype=np.float64).ravel(), alphalin, nfc, lf,
-                      'yes' if manakov else 'no', spm=fls[2], nspan=int(D[0]), gain=D[1] or None,
-                      steps_per_span=int(D[2]), xi=D[3], taps=np.asarray(a[15], dtype=np.float64).ravel())
-        return list(out)[:max(nargout, 1)]
-    return call
-
-
 @pytest.mark.parametrize('shape', ['row', 'column'])
 def test_m_front_end_sends_the_taps(shape):
     """dbp.m with options.taps (a row or a column): the gateway's trailing argument, and the field of the ESSFM oracle on
@@ -162,14 +125,17 @@ def test_m_front_end_sends_the_taps(shape):
     tx, ty = np.array(G.FIELDX), np.array(G.FIELDY)
     s = fiber_setup(fib, 'g-s-')
     c = taps(3)
-    want = deo.dbp(tx, ty, s.betat, s.gam, s.alphalin, 1, s.length, 'no', nspan=2, gain=G16, steps_per_span=2, taps=c)
-    log = []
-    it = tmd._interp(_taps_gateway(log))
+    want = dbp_oracle.dbp(tx, ty, s.betat, s.gam, s.alphalin, 1, s.length, 'no', nspan=2, gain=G16, steps_per_span=2,
+                          taps=c)
+    gw = tmd.oracle_gateway()
+    it = tmd._interp(gw)
     m = c.reshape(1, -1) if shape == 'row' else c.reshape(-1, 1)
     it.call('dbp', [tmd.to_m(fib), 'g-s-', tmd._opts(nspan=2, gain=GAIN_DB, steps=2, taps=m)], 0)
+    log = [e['taps'] for e in gw.log if e['cmd'] == 'dbp']
     assert len(log) == 1 and np.array_equal(log[0].ravel(), c)
     assert rel_l2(*tmd._m_field(it), *want) <= 1e-13
     it.call('dbp', [tmd.to_m(fib), 'g-s-', tmd._opts(nspan=2, gain=GAIN_DB, steps=2, taps=np.zeros((0, 0)))], 0)
+    log = [e['taps'] for e in gw.log if e['cmd'] == 'dbp']
     assert len(log) == 2 and log[1] is None
 
 
@@ -188,10 +154,6 @@ def test_m_front_end_refusals_are_pmx_dbp_s(case):
 
 
 # ---------------------------------------------------------------------------------------------------------------- GPU
-def _cols(a):
-    return np.ascontiguousarray(np.asarray(a).T)[None]
-
-
 def _run(ctx, s, xs, ys, c, precision='f64', plates=None, **kw):
     b = xs.shape[0]
     fld = _lib.DeviceField(ctx, s.nfft, s.nfc, b, precision={'f64': _lib.PMX_F64, 'f32': _lib.PMX_F32}[precision])
@@ -213,7 +175,8 @@ def _two_pol(ctx, nsymb, nt, nch, manakov, batch, k, steps=2, nspan=2, precision
     gx, gy = _run(ctx, s, xs, ys, c, precision=precision, gain_db=GAIN_DB, **kw)
     errs = []
     for b in range(batch):
-        wx, wy = deo.dbp(xs[b].T, ys[b].T, s.betat, s.gam, s.alphalin, s.nfc, s.length, _man(s), gain=G16, taps=c, **kw)
+        wx, wy = dbp_oracle.dbp(xs[b].T, ys[b].T, s.betat, s.gam, s.alphalin, s.nfc, s.length, _man(s), gain=G16, taps=c,
+                                **kw)
         errs.append(rel_l2(gx[b].T, gy[b].T, wx, wy))
     return errs
 
@@ -257,7 +220,7 @@ def test_scalar_essfm_matches_the_oracle(ctx, case):
     kw = dict(nspan=2, steps_per_span=3)
     c = taps(k, seed=2)
     gx, _ = _run(ctx, s, _cols(u), np.zeros_like(_cols(u)), c, gain_db=GAIN_DB, **kw)
-    w = deo.dbp_scalar(u, s.betat, s.gam, s.alphalin, s.nfc, s.length, s.fls[2], s.fls[3], gain=G16, taps=c, **kw)
+    w = dbp_oracle.dbp_scalar(u, s.betat, s.gam, s.alphalin, s.nfc, s.length, s.fls[2], s.fls[3], gain=G16, taps=c, **kw)
     err = np.linalg.norm(gx[0].T - w) / np.linalg.norm(w)
     print('essfm scalar %s: %.3e' % (case, err))
     assert err <= 1e-10
@@ -280,8 +243,8 @@ def test_pmd_essfm_matches_the_oracle(ctx, nsymb):
     kw = dict(nspan=nspan, steps_per_span=2)
     gx, gy = _run(ctx, s, xs, ys, c, plates=plates, gain_db=GAIN_DB, **kw)
     for b in range(batch):
-        wx, wy = deo.dbp_pmd(xs[b].T, ys[b].T, s.betat, np.asarray(s.db1), s.gam, s.alphalin, 1, s.length, 'no', brfs[b],
-                             gain=G16, taps=c, **kw)
+        wx, wy = dbp_oracle.dbp_pmd(xs[b].T, ys[b].T, s.betat, np.asarray(s.db1), s.gam, s.alphalin, 1, s.length, 'no',
+                                    brfs[b], gain=G16, taps=c, **kw)
         err = rel_l2(gx[b].T, gy[b].T, wx, wy)
         print('essfm pmd 2^%d b%d: %.3e' % (int(np.log2(s.nfft)), b, err))
         assert err <= 1e-10
@@ -293,8 +256,8 @@ def test_single_channel_essfm_matches_the_oracle(ctx):
     gs, s = _setup(4096, 16, pavg_mw=10.0)
     c, kw = taps(16), dict(nspan=2, steps_per_span=2)
     gx, gy = _run(ctx, s, _cols(gs.FIELDX), _cols(gs.FIELDY), c, gain_db=GAIN_DB, decim=16, shift=0, **kw)
-    wx, wy = deo.dbp_channel(gs.FIELDX, gs.FIELDY, s.betat, s.gam, s.alphalin, s.length, 'no', 0, 16, gain=G16, taps=c,
-                             **kw)
+    wx, wy = dbp_oracle.dbp_channel(gs.FIELDX, gs.FIELDY, s.betat, s.gam, s.alphalin, s.length, 'no', 0, 16, gain=G16,
+                                    taps=c, **kw)
     err = rel_l2(gx[0].T, gy[0].T, wx, wy)
     print('essfm single-channel 2^16 / 16: %.3e' % err)
     assert err <= 1e-10
@@ -381,9 +344,8 @@ def test_m_front_end_essfm_on_the_device():
 def test_mc_runner_with_essfm(ctx):
     """McRunner(compensation='dbp', dbp_params=dict(nl_taps=[1.0])) counts what plain DBP counts, behind the 'cohmix' and
     the 'blind' receiver"""
-    import test_dbp as td
     nsymb, nt, nspan, nreal, batch = 1 << 12, 16, 2, 8, 4
-    G, setup, sym = td._mc_scenario(nsymb, nt, 8.0)
+    G, setup, sym = _mc_scenario(nsymb, nt, 8.0)
     x = {'oftype': 'gauss', 'obw': 1.9, 'eftype': 'bessel5', 'ebw': 0.65, 'lopower': 0.0}
     for receiver in ('cohmix', 'blind'):
         counts = []

@@ -1,5 +1,5 @@
 """Filtered digital backpropagation (pmx_dbp_set_filter, DbpPlan.set_filter, dbp_plan / pmx.dbp filter_bw,
-tests/dbp_filtered_oracle.py): a Gaussian low-pass on the intensity of every backward nonlinear step."""
+tests/dbp_oracle.py with bw=): a Gaussian low-pass on the intensity of every backward nonlinear step."""
 import ctypes
 import math
 
@@ -7,15 +7,12 @@ import numpy as np
 import pytest
 
 import oracle.fiber_oracle as orc
-import dbp_filtered_oracle as dfo
 import dbp_oracle
-import dbp_pmd_oracle
-import dbp_scalar_oracle
 import polmux_b200 as pmx
 from polmux_b200 import _lib, mc
 from polmux_b200.dbp import dbp_plan
 from polmux_b200.fiber import fiber_setup
-from common import base_fiber, make_tx, rel_l2, scalar_tx
+from common import _cols, _mc_scenario, base_fiber, make_tx, rel_l2, scalar_tx
 
 GAIN_DB = 16.0
 G16 = 10 ** (GAIN_DB / 10)
@@ -45,13 +42,13 @@ def _forward(ux, uy, s, nspan, gain):
 def test_oracle_without_filter_is_the_existing_oracles():
     gs, s = _setup(64, 16, nch=3, manakov=False)
     kw = dict(nspan=2, gain=G16, steps_per_span=3)
-    a = dfo.dbp(gs.FIELDX, gs.FIELDY, s.betat, s.gam, s.alphalin, s.nfc, s.length, 'no', **kw)
+    a = dbp_oracle.dbp(gs.FIELDX, gs.FIELDY, s.betat, s.gam, s.alphalin, s.nfc, s.length, 'no', bw=None, **kw)
     b = dbp_oracle.dbp(gs.FIELDX, gs.FIELDY, s.betat, s.gam, s.alphalin, s.nfc, s.length, 'no', **kw)
     assert all(np.array_equal(x, y) for x, y in zip(a, b))
     u = scalar_tx(32, 32, 3, pavg=8.0).FIELDX
     ss = fiber_setup(base_fiber(length=1e5, slope=0.057), 'g-sx')
-    a = dfo.dbp_scalar(u, ss.betat, ss.gam, ss.alphalin, ss.nfc, ss.length, 1, 1, **kw)
-    b = dbp_scalar_oracle.dbp_scalar(u, ss.betat, ss.gam, ss.alphalin, ss.nfc, ss.length, 1, 1, **kw)
+    a = dbp_oracle.dbp_scalar(u, ss.betat, ss.gam, ss.alphalin, ss.nfc, ss.length, 1, 1, bw=None, **kw)
+    b = dbp_oracle.dbp_scalar(u, ss.betat, ss.gam, ss.alphalin, ss.nfc, ss.length, 1, 1, **kw)
     assert np.array_equal(a, b)
 
 
@@ -60,16 +57,16 @@ def test_oracle_wide_filter_is_unfiltered_and_xi0_ignores_the_filter(manakov):
     gs, s = _setup(16, 16, nch=2, pavg_mw=10.0, manakov=manakov)   # 2^8: 1 - H(N/2) = 5.7e-13 at bw = 1e8 bins
     args = (gs.FIELDX, gs.FIELDY, s.betat, s.gam, s.alphalin, s.nfc, s.length, _man(s))
     kw = dict(nspan=2, gain=G16, steps_per_span=2)
-    ref = dfo.dbp(*args, **kw)
-    wide = dfo.dbp(*args, bw=1e8, **kw)
+    ref = dbp_oracle.dbp(*args, **kw)
+    wide = dbp_oracle.dbp(*args, bw=1e8, **kw)
     assert rel_l2(*wide, *ref) <= 1e-12
-    lin = [dfo.dbp(*args, xi=0.0, bw=bw, **kw) for bw in (None, 3.0, 40.0)]
+    lin = [dbp_oracle.dbp(*args, xi=0.0, bw=bw, **kw) for bw in (None, 3.0, 40.0)]
     assert rel_l2(*lin[1], *lin[0]) <= 1e-15 and rel_l2(*lin[2], *lin[0]) <= 1e-15
     u = scalar_tx(32, 32, 3, pavg=8.0).FIELDX
     ss = fiber_setup(base_fiber(length=1e5, slope=0.057), 'g-sx')
     sa = (u, ss.betat, ss.gam, ss.alphalin, ss.nfc, ss.length, 1, 1)
-    r = dbp_scalar_oracle.dbp_scalar(*sa, **kw)
-    w = dfo.dbp_scalar(*sa, bw=1e9, **kw)   # 2^10: 1 - H(N/2) = 9e-14
+    r = dbp_oracle.dbp_scalar(*sa, **kw)
+    w = dbp_oracle.dbp_scalar(*sa, bw=1e9, **kw)   # 2^10: 1 - H(N/2) = 9e-14
     assert np.linalg.norm(w - r) <= 1e-12 * np.linalg.norm(r)
 
 
@@ -77,15 +74,15 @@ def test_oracle_wide_filter_is_unfiltered_and_xi0_ignores_the_filter(manakov):
 def test_filtered_nonlinear_step_keeps_every_modulus(manakov):
     gs, s = _setup(64, 16, pavg_mw=30.0, manakov=manakov)
     ux, uy = gs.FIELDX.copy(), gs.FIELDY.copy()
-    H = dfo.gauss_response(ux.shape[0], 5.0)
-    vx, vy = dfo.matrix_nl_step_filt(manakov, s.alphalin, -np.asarray(s.gam), s.length, ux.copy(), uy.copy(), 1, H)
+    op = dbp_oracle.intensity(ux.shape[0], bw=5.0)
+    vx, vy = dbp_oracle.matrix_nl_step(manakov, s.alphalin, -np.asarray(s.gam), s.length, ux.copy(), uy.copy(), 1, 1, op)
     p0 = np.abs(ux) ** 2 + np.abs(uy) ** 2
     p1 = np.abs(vx) ** 2 + np.abs(vy) ** 2
     assert np.max(np.abs(p1 - p0) / np.maximum(p0, 1e-300)) <= 1e-13
     if manakov:   # a common phase: each polarization keeps its own modulus
         assert np.max(np.abs(np.abs(vx) - np.abs(ux))) <= 1e-13 * np.max(np.abs(ux))
     u = scalar_tx(32, 32, 3, pavg=8.0).FIELDX
-    w = dfo.nl_step_filt(0.0, -1.3 * np.ones((1, 3)), 1e5, u, 3, 1, 1, dfo.gauss_response(u.shape[0], 4.0))
+    w = dbp_oracle.nl_step(0.0, -1.3 * np.ones((1, 3)), 1e5, u, 3, 1, 1, dbp_oracle.intensity(u.shape[0], bw=4.0))
     assert np.max(np.abs(np.abs(w) - np.abs(u))) <= 1e-13 * np.max(np.abs(u))
 
 
@@ -101,7 +98,7 @@ def test_filtered_dbp_beats_plain_dbp_at_one_step_per_span():
     bws_ghz = (2.0, 4.0, 8.0, 16.0)
 
     def res(**kw):
-        return rel_l2(*dfo.dbp(*args, nspan=3, gain=G16, **kw), gs.FIELDX, gs.FIELDY)
+        return rel_l2(*dbp_oracle.dbp(*args, nspan=3, gain=G16, **kw), gs.FIELDX, gs.FIELDY)
     plain = min(res(steps_per_span=1, xi=xi) for xi in xis)
     filt = min((res(steps_per_span=1, xi=xi, bw=b * nsymb / 28.0), b, xi) for b in bws_ghz for xi in xis)
     four = min(res(steps_per_span=4, xi=xi) for xi in xis)
@@ -125,10 +122,6 @@ def test_native_mc_rejects_filter_bw():
 
 
 # ---------------------------------------------------------------------------------------------------------------- GPU
-def _cols(a):
-    return np.ascontiguousarray(np.asarray(a).T)[None]
-
-
 def _run(ctx, s, xs, ys, bw, precision='f64', launches=None, plates=None, **kw):
     b = xs.shape[0]
     fld = _lib.DeviceField(ctx, s.nfft, s.nfc, b, precision={'f64': _lib.PMX_F64, 'f32': _lib.PMX_F32}[precision])
@@ -170,10 +163,11 @@ def test_two_pol_filtered_dbp_matches_the_oracle(ctx, case):
     gx, gy = _run(ctx, s, xs, ys, bw, launches=1 if onchip else None, gain_db=GAIN_DB if g else None, **kw)
     errs = []
     for b in range(batch):
-        wx, wy = dfo.dbp(xs[b].T, ys[b].T, s.betat, s.gam, s.alphalin, s.nfc, s.length, _man(s), gain=g, bw=bw, **kw)
+        wx, wy = dbp_oracle.dbp(xs[b].T, ys[b].T, s.betat, s.gam, s.alphalin, s.nfc, s.length, _man(s), gain=g, bw=bw,
+                                **kw)
         errs.append(rel_l2(gx[b].T, gy[b].T, wx, wy))
         if b == 0:   # the filter changes the result
-            ux, uy = dfo.dbp(xs[b].T, ys[b].T, s.betat, s.gam, s.alphalin, s.nfc, s.length, _man(s), gain=g, **kw)
+            ux, uy = dbp_oracle.dbp(xs[b].T, ys[b].T, s.betat, s.gam, s.alphalin, s.nfc, s.length, _man(s), gain=g, **kw)
             assert rel_l2(wx, wy, ux, uy) > 1e-6
     print('filtered dbp parity %s: rel_l2 %s' % (case, ['%.3e' % e for e in errs]))
     assert max(errs) <= 1e-10, errs
@@ -198,8 +192,8 @@ def test_pmd_filtered_dbp_matches_the_oracle(ctx, nsymb):
     gx, gy = _run(ctx, s, xs, ys, bw, plates=plates, gain_db=GAIN_DB, **kw)
     db1 = np.asarray(s.db1)
     for b in range(batch):
-        wx, wy = dfo.dbp_pmd(xs[b].T, ys[b].T, s.betat, db1, s.gam, s.alphalin, 1, s.length, _man(s), brfs[b],
-                             gain=G16, bw=bw, **kw)
+        wx, wy = dbp_oracle.dbp_pmd(xs[b].T, ys[b].T, s.betat, db1, s.gam, s.alphalin, 1, s.length, _man(s), brfs[b],
+                                    gain=G16, bw=bw, **kw)
         err = rel_l2(gx[b].T, gy[b].T, wx, wy)
         print('filtered pmd dbp 2^%d b%d: %.3e' % (int(np.log2(s.nfft)), b, err))
         assert err <= 1e-10
@@ -221,7 +215,7 @@ def test_scalar_filtered_dbp_matches_the_oracle(ctx, case):
     u = pmx.GSTATE.FIELDX
     kw = dict(nspan=2, steps_per_span=4)
     gx, _ = _run(ctx, s, _cols(u), np.zeros_like(_cols(u)), bw, launches=1, gain_db=GAIN_DB, **kw)
-    w = dfo.dbp_scalar(u, s.betat, s.gam, s.alphalin, s.nfc, s.length, s.fls[2], s.fls[3], gain=G16, bw=bw, **kw)
+    w = dbp_oracle.dbp_scalar(u, s.betat, s.gam, s.alphalin, s.nfc, s.length, s.fls[2], s.fls[3], gain=G16, bw=bw, **kw)
     err = np.linalg.norm(gx[0].T - w) / np.linalg.norm(w)
     print('filtered scalar dbp %s: %.3e' % (case, err))
     assert err <= 1e-10
@@ -235,14 +229,14 @@ def test_filtered_dbp_fp32(ctx, what):
         s = fiber_setup(base_fiber(length=1e5, dphimax=3e-3, slope=0.057), 'g-sx')
         u = pmx.GSTATE.FIELDX
         gx, _ = _run(ctx, s, _cols(u), np.zeros_like(_cols(u)), 8.0, precision='f32', steps_per_span=4)
-        w = dfo.dbp_scalar(u, s.betat, s.gam, s.alphalin, s.nfc, s.length, 1, 1, steps_per_span=4, bw=8.0)
+        w = dbp_oracle.dbp_scalar(u, s.betat, s.gam, s.alphalin, s.nfc, s.length, 1, 1, steps_per_span=4, bw=8.0)
         err = np.linalg.norm(gx[0].T - w) / np.linalg.norm(w)
     else:
         nsymb = 64 if what.endswith('2e10') else 1024
         gs, s = _setup(nsymb, 16, pavg_mw=4.0)
         gx, gy = _run(ctx, s, _cols(gs.FIELDX), _cols(gs.FIELDY), nsymb / 8.0, precision='f32', steps_per_span=4)
-        err = rel_l2(gx[0].T, gy[0].T, *dfo.dbp(gs.FIELDX, gs.FIELDY, s.betat, s.gam, s.alphalin, 1, s.length, 'no',
-                                                steps_per_span=4, bw=nsymb / 8.0))
+        err = rel_l2(gx[0].T, gy[0].T, *dbp_oracle.dbp(gs.FIELDX, gs.FIELDY, s.betat, s.gam, s.alphalin, 1, s.length, 'no',
+                                                       steps_per_span=4, bw=nsymb / 8.0))
     print('filtered dbp fp32 %s: %.3e' % (what, err))
     assert err <= 1e-5
 
@@ -252,8 +246,8 @@ def test_filtered_dbp_c2_span(ctx):
     """one full C2 span (2^20 samples) on the three passes"""
     gs, s = _setup(65536, 16, pavg_mw=4.0, manakov=True)
     gx, gy = _run(ctx, s, _cols(gs.FIELDX), _cols(gs.FIELDY), 4096.0, steps_per_span=2)
-    err = rel_l2(gx[0].T, gy[0].T, *dfo.dbp(gs.FIELDX, gs.FIELDY, s.betat, s.gam, s.alphalin, 1, s.length, 'yes',
-                                            steps_per_span=2, bw=4096.0))
+    err = rel_l2(gx[0].T, gy[0].T, *dbp_oracle.dbp(gs.FIELDX, gs.FIELDY, s.betat, s.gam, s.alphalin, 1, s.length, 'yes',
+                                                   steps_per_span=2, bw=4096.0))
     print('filtered dbp C2 span: %.3e' % err)
     assert err <= 1e-10
 
@@ -267,8 +261,8 @@ def test_single_channel_filtered_dbp_matches_the_oracle(ctx, nsymb, decim):
     kw = dict(nspan=2, steps_per_span=2)
     gx, gy = _run(ctx, s, _cols(gs.FIELDX), _cols(gs.FIELDY), 0, gain_db=GAIN_DB, decim=decim, shift=0,
                   filter_bw=bw * pmx.GSTATE.SYMBOLRATE / pmx.GSTATE.NSYMB, **kw)
-    wx, wy = dfo.dbp_channel(gs.FIELDX, gs.FIELDY, s.betat, s.gam, s.alphalin, s.length, 'no', 0, decim, gain=G16, bw=bw,
-                             **kw)
+    wx, wy = dbp_oracle.dbp_channel(gs.FIELDX, gs.FIELDY, s.betat, s.gam, s.alphalin, s.length, 'no', 0, decim, gain=G16,
+                                    bw=bw, **kw)
     err = rel_l2(gx[0].T, gy[0].T, wx, wy)
     print('filtered single-channel dbp 2^%d / %d: %.3e' % (int(np.log2(s.nfft)), decim, err))
     assert err <= 1e-10
@@ -334,36 +328,14 @@ def test_pmx_dbp_filter_bw_end_to_end():
     x0, y0 = G.FIELDX.copy(), G.FIELDY.copy()
     pmx.dbp(fib, 'g-s-', nspan=2, gain_db=GAIN_DB, steps_per_span=2, filter_bw=5.0)
     bw = 5.0 * G.NSYMB / G.SYMBOLRATE
-    wx, wy = dfo.dbp(x0, y0, s.betat, s.gam, s.alphalin, 1, s.length, 'no', nspan=2, gain=G16, steps_per_span=2, bw=bw)
+    wx, wy = dbp_oracle.dbp(x0, y0, s.betat, s.gam, s.alphalin, 1, s.length, 'no', nspan=2, gain=G16, steps_per_span=2,
+                            bw=bw)
     err = rel_l2(G.FIELDX, G.FIELDY, wx, wy)
     print('pmx.dbp filter_bw: %.3e' % err)
     assert err <= 1e-10
 
 
 # -------------------------------------------------------------------------------------------------- M front-end (dbp.m)
-def _filtered_gateway(log):
-    """test_matlab_dbp's oracle-backed gateway, with ssfm_mex('dbp', ...) of a 6-element D (two polarizations, full field,
-    no PMD) answered by the filtered oracle"""
-    import test_matlab_dbp as tmd
-    base = tmd.oracle_gateway()
-
-    def call(it, a, nargout):
-        if a[0] != 'dbp' or np.size(a[10]) != 6:
-            return base(it, a, nargout)
-        ux, uy, betat, db1, P, gam = a[1:7]
-        scal, D, fls = a[9], np.asarray(a[10], dtype=np.float64).ravel(), [int(v) for v in np.asarray(a[7]).ravel()]
-        log.append(D)
-        _, _, alphalin, lf, _, manakov = [float(v) for v in np.asarray(P).ravel()]
-        nfft, nfc = np.shape(ux)
-        if np.size(betat) == 0:
-            betat, db1 = tmd._vectors(scal, nfft, nfc, fls[1])
-        out = dfo.dbp(ux, uy, betat, np.asarray(gam, dtype=np.float64).ravel(), alphalin, nfc, lf,
-                      'yes' if manakov else 'no', spm=fls[2], nspan=int(D[0]), gain=D[1] or None,
-                      steps_per_span=int(D[2]), xi=D[3], bw=D[5])
-        return list(out)[:max(nargout, 1)]
-    return call
-
-
 def test_m_front_end_sends_the_bandwidth_in_bins():
     """dbp.m with options.filter_bw: a 6-element D whose sixth entry is filter_bw*NSYMB/SYMBOLRATE, and the field of the
     filtered oracle on pmx.dbp's parameters"""
@@ -374,10 +346,12 @@ def test_m_front_end_sends_the_bandwidth_in_bins():
     tx, ty = np.array(G.FIELDX), np.array(G.FIELDY)
     s = fiber_setup(fib, 'g-s-')
     bw = 7.0 * G.NSYMB / G.SYMBOLRATE
-    want = dfo.dbp(tx, ty, s.betat, s.gam, s.alphalin, 1, s.length, 'no', nspan=2, gain=G16, steps_per_span=2, bw=bw)
-    log = []
-    it = tmd._interp(_filtered_gateway(log))
+    want = dbp_oracle.dbp(tx, ty, s.betat, s.gam, s.alphalin, 1, s.length, 'no', nspan=2, gain=G16, steps_per_span=2,
+                          bw=bw)
+    gw = tmd.oracle_gateway()
+    it = tmd._interp(gw)
     it.call('dbp', [tmd.to_m(fib), 'g-s-', tmd._opts(nspan=2, gain=GAIN_DB, steps=2, filter_bw=7.0)], 0)
+    log = [e['D'] for e in gw.log if e['cmd'] == 'dbp']
     assert len(log) == 1 and log[0].size == 6 and log[0][5] == bw
     ux, uy = tmd._m_field(it)
     assert rel_l2(ux, uy, *want) <= 1e-13
@@ -398,9 +372,8 @@ def test_m_front_end_filtered_on_the_device():
 def test_mc_runner_with_filtered_dbp(ctx):
     """McRunner(compensation='dbp', dbp_params=dict(filter_bw=...)) runs with the 'cohmix' receiver; a very wide filter
     counts what plain DBP counts"""
-    import test_dbp as td
     nsymb, nt, nspan, nreal, batch = 1 << 12, 16, 2, 8, 4
-    G, setup, sym = td._mc_scenario(nsymb, nt, 8.0)
+    G, setup, sym = _mc_scenario(nsymb, nt, 8.0)
     x = {'oftype': 'gauss', 'obw': 1.9, 'eftype': 'bessel5', 'ebw': 0.65, 'lopower': 0.0}
     counts = []
     for dp in (dict(steps_per_span=1), dict(steps_per_span=1, filter_bw=1e9), dict(steps_per_span=1, filter_bw=10.0)):

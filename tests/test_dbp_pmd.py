@@ -1,6 +1,6 @@
 """PMD-aware digital backpropagation (pmx_dbp_desc.pmd, pmx_dbp_set_plates, dbp(brf=...), McRunner(compensation='dbp_pmd')).
 
-The oracle is tests/dbp_pmd_oracle.py, built from the pinned forward oracle's checkstep, matrix_step and matrix_nl_step.
+The oracle is tests/dbp_oracle.dbp_pmd, built from the pinned forward oracle's checkstep, matrix_step and matrix_nl_step.
 It is tied to the forward oracle by the exact-inverse property on 'gps-' links (with the forward run's own steps and
 xi = 1, DBP returns the Tx field) and to the pinned inverse_pmd by the linear limit (xi = 0, one step per span)."""
 import ctypes
@@ -12,12 +12,12 @@ import numpy as np
 import pytest
 
 import oracle.fiber_oracle as orc
-import dbp_pmd_oracle as dpo
+import dbp_oracle
 import polmux_b200 as pmx
-from polmux_b200 import _lib, mc, synth
+from polmux_b200 import _lib, mc
 from polmux_b200.dbp import dbp_plan
 from polmux_b200.fiber import fiber_setup, setup_to_desc
-from common import base_fiber, make_tx, rel_l2
+from common import _cols, _mc_scenario, base_fiber, make_tx, rel_l2
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GAIN_DB = 16.0
@@ -67,8 +67,8 @@ def _forward(ux, uy, s, brfs, gain):
 
 
 def _oracle(ux, uy, s, brfs, real=np.float64, **kw):
-    return dpo.dbp_pmd(ux, uy, s.betat, s.db1, s.gam, s.alphalin, s.nfc, s.length, 'yes' if s.manakov else 'no', brfs,
-                       real=real, **kw)
+    return dbp_oracle.dbp_pmd(ux, uy, s.betat, s.db1, s.gam, s.alphalin, s.nfc, s.length, 'yes' if s.manakov else 'no',
+                              brfs, real=real, **kw)
 
 
 # ---------------------------------------------------------------------------------------------------------------- CPU
@@ -89,7 +89,7 @@ def test_partition_replica_equals_the_forward_schedule(case):
         assert n == 1 and scheds[0][0]['ntrunk'] == 100
     else:
         assert 30 <= n <= 60, n
-    rep = dpo.forward_partition(steps[0], s.length, s.nplates)
+    rep = dbp_oracle.forward_partition(steps[0], s.length, s.nplates)
     assert [(r['ntrunk'], r['nmem'], r['ntot'], r['dzb']) for r in rep] == \
            [(r['ntrunk'], r['nmem'], r['ntot'], r['dzb']) for r in scheds[0]]
 
@@ -115,7 +115,7 @@ def test_oracle_linear_limit_is_inverse_pmd():
     g = 10 ** (GAIN_DB / 10)
     brfs = [r[0] for r in _brfs(s, 2)]
     bx, by = _oracle(gs.FIELDX, gs.FIELDY, s, brfs, nspan=2, gain=g, steps_per_span=1, xi=0.0)
-    wx, wy = dpo.inverse_pmd_chain(gs.FIELDX, gs.FIELDY, brfs, s.betat, s.db1, s.length, s.alphalin, gain=g)
+    wx, wy = dbp_oracle.inverse_pmd_chain(gs.FIELDX, gs.FIELDY, brfs, s.betat, s.db1, s.length, s.alphalin, gain=g)
     err = rel_l2(bx, by, wx, wy)
     assert err <= 1e-12, err
 
@@ -209,10 +209,6 @@ def test_mc_runner_takes_dbp_pmd_with_the_genie_receiver():
 
 
 # ---------------------------------------------------------------------------------------------------------------- GPU
-def _cols(a):
-    return np.ascontiguousarray(np.asarray(a).T)[None]          # GSTATE [nfft, nfc] -> [1][nfc][nfft]
-
-
 def _run_device(ctx, s, xs, ys, plates, precision='f64', **kw):
     """PMD-aware DBP of the fields xs, ys ([batch][nfc][nfft]) on the device -> (x, y) of the same shape"""
     b = xs.shape[0]
@@ -305,7 +301,7 @@ def test_dbp_pmd_inverts_fiber_on_the_device(case):
     brf = pmx.fiber(fib, 'gps-', trace=True, rng=np.random.Generator(np.random.PCG64(11)))
     dz, ntr = np.asarray(pmx.FIBER_LAST['trace_dz']), np.asarray(pmx.FIBER_LAST['trace_ntrunk'])
     assert len(dz) > 1
-    rep = dpo.forward_partition(dz, float(fib['length']), int(fib['nplates']))
+    rep = dbp_oracle.forward_partition(dz, float(fib['length']), int(fib['nplates']))
     assert [r['ntrunk'] for r in rep] == list(ntr)
     pmx.dbp(fib, 'gps-', step_len=dz, brf=brf)
     err = rel_l2(G.FIELDX, G.FIELDY, tx, ty)
@@ -332,7 +328,7 @@ def test_dbp_pmd_inverts_a_two_span_link_on_the_device(ctx):
         b = brfs[k][0]
         plan.set_plates(b['db0'], b['theta'], b['epsilon'])
         dz, ntr = plan.execute(fld, trace_cap=1 << 14).schedule(0)
-        assert [r['ntrunk'] for r in dpo.forward_partition(dz, s.length, s.nplates)] == list(ntr)
+        assert [r['ntrunk'] for r in dbp_oracle.forward_partition(dz, s.length, s.nplates)] == list(ntr)
         steps.append(dz)
         _lib.ampliflat_exec(ctx, fld, gain, [0.0])
     plan.close()
@@ -380,18 +376,6 @@ def test_dbp_pmd_linear_limit_is_the_genie_equaliser(ctx):
         err = rel_l2(gx[b, 0], gy[b, 0], ex[b, 0] * sc, ey[b, 0] * sc)
         print('dbp pmd linear limit vs Link.equalize, realization %d: rel_l2 %.3e' % (b, err))
         assert err <= 1e-12
-
-
-def _mc_scenario(nsymb, nt, pavg_mw):
-    ex, ey, sx, sy = synth.pdm_qpsk(nsymb, nt, 1)
-    pmx.reset_all(nsymb, nt, 1)
-    G = pmx.GSTATE
-    G.SYMBOLRATE, G.LAMBDA, G.POWER = 28.0, np.array([1550.0]), np.array([float(pavg_mw)])
-    pmx.create_field('unique', ex, ey, {'power': 'average'})
-    fib = dict(synth.SMF)
-    fib.update(length=8e4, dgd=0.3, nplates=20, manakov='yes')
-    setup = fiber_setup(fib, 'gps-', rng=np.random.Generator(np.random.PCG64(0)))
-    return G, setup, np.stack([sx[:, 0], sy[:, 0]]).astype(np.uint8)
 
 
 @pytest.mark.gpu

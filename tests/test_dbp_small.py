@@ -4,8 +4,8 @@ and the scalar path from 2^6 to 2^12 samples with and without cross-phase modula
 column sees the power of all backpropagated columns).  The sizes are those of the reference's small scripts, ex06_ber.m
 (32 x 32, one channel, 'g-sx') and ex10_wdm.m (64 x 32, five separate channels, 'g-sx').
 
-Oracles: tests/dbp_oracle.py and tests/dbp_pmd_oracle.py for two polarizations, tests/dbp_scalar_oracle.py for the scalar
-path; the latter is tied to the pinned forward oracle by its exact inverse of scalar_ssfm."""
+Oracle: tests/dbp_oracle.py -- dbp and dbp_pmd for two polarizations, dbp_scalar for the scalar path; the latter is tied
+to the pinned forward oracle by its exact inverse of scalar_ssfm."""
 import ctypes
 import math
 
@@ -14,13 +14,11 @@ import pytest
 
 import oracle.fiber_oracle as orc
 import dbp_oracle
-import dbp_pmd_oracle as dpo
-import dbp_scalar_oracle as dso
 import polmux_b200 as pmx
 from polmux_b200 import _lib, mc
 from polmux_b200.dbp import dbp_plan
 from polmux_b200.fiber import fiber_setup, setup_to_desc
-from common import base_fiber, make_tx, rel_l2, scalar_tx as _scalar_tx
+from common import _cols, _rel, base_fiber, make_tx, rel_l2, scalar_tx as _scalar_tx
 
 GAIN_DB = 16.0
 G16 = 10 ** (GAIN_DB / 10)
@@ -37,7 +35,8 @@ def _scalar_forward(u, s, nspan, gain):
     """noise-free scalar link of the oracle: nspan x [scalar_ssfm ; u*sqrt(gain)] -> (u, steps of every span)"""
     steps = []
     for _ in range(nspan):
-        u, st = dso.scalar_ssfm_steps(u, s.betat, s.dzmaxt, s.dphimaxt, s.gam, s.alphalin, s.nfft, s.nfc, s.length, s.fls)
+        u, st = dbp_oracle.scalar_ssfm_steps(u, s.betat, s.dzmaxt, s.dphimaxt, s.gam, s.alphalin, s.nfft, s.nfc, s.length,
+                                             s.fls)
         steps.append(st)
         if gain is not None:
             u = u * math.sqrt(gain)
@@ -45,11 +44,7 @@ def _scalar_forward(u, s, nspan, gain):
 
 
 def _scalar_oracle(u, s, real=np.float64, **kw):
-    return dso.dbp_scalar(u, s.betat, s.gam, s.alphalin, s.nfc, s.length, spm=s.fls[2], xpm=s.fls[3], real=real, **kw)
-
-
-def _rel(a, b):
-    return float(np.linalg.norm(np.asarray(a) - np.asarray(b)) / np.linalg.norm(np.asarray(b)))
+    return dbp_oracle.dbp_scalar(u, s.betat, s.gam, s.alphalin, s.nfc, s.length, spm=s.fls[2], xpm=s.fls[3], real=real, **kw)
 
 
 # ---------------------------------------------------------------------------------------------------------------- CPU
@@ -60,8 +55,8 @@ def test_scalar_oracle_inverts_the_forward_link(nsymb, nt, nch, flag):
     gs, s = _scalar_setup(nsymb, nt, nch, flag, pavg=8.0)
     fd, nc, ref = orc.scalar_ssfm(gs.FIELDX, s.betat, s.dzmaxt, s.dphimaxt, s.gam, s.alphalin, s.nfft, s.nfc, s.length,
                                   s.fls, 0, None)
-    u1, st1 = dso.scalar_ssfm_steps(gs.FIELDX, s.betat, s.dzmaxt, s.dphimaxt, s.gam, s.alphalin, s.nfft, s.nfc, s.length,
-                                    s.fls)
+    u1, st1 = dbp_oracle.scalar_ssfm_steps(gs.FIELDX, s.betat, s.dzmaxt, s.dphimaxt, s.gam, s.alphalin, s.nfft, s.nfc,
+                                           s.length, s.fls)
     assert np.array_equal(u1, ref) and len(st1) == nc and st1[0] == fd
     u, steps = _scalar_forward(gs.FIELDX, s, 2, G16)
     assert sum(len(x) for x in steps) > 4
@@ -143,10 +138,6 @@ def test_dbp_keeps_the_two_polarization_xpm_error():
 
 
 # ---------------------------------------------------------------------------------------------------------------- GPU
-def _cols(a):
-    return np.ascontiguousarray(np.asarray(a).T)[None]          # GSTATE [nfft, nfc] -> [1][nfc][nfft]
-
-
 def _run_device(ctx, s, xs, ys, precision='f64', plates=None, **kw):
     """DBP of the fields xs, ys ([batch][nfc][nfft]) on the device -> (x, y) of the same shape"""
     b = xs.shape[0]
@@ -242,8 +233,8 @@ def test_pmd_dbp_matches_the_oracle_small(ctx, case):
     gx, gy = _run_device(ctx, s, xs, ys, plates=_pmd_plates(brfs), nspan=nspan, gain_db=GAIN_DB if g else None, **kw)
     errs = []
     for b in range(batch):
-        wx, wy = dpo.dbp_pmd(xs[b].T, ys[b].T, s.betat, s.db1, s.gam, s.alphalin, s.nfc, s.length,
-                             'yes' if manakov else 'no', [row[b] for row in brfs], nspan=nspan, gain=g, **kw)
+        wx, wy = dbp_oracle.dbp_pmd(xs[b].T, ys[b].T, s.betat, s.db1, s.gam, s.alphalin, s.nfc, s.length,
+                                    'yes' if manakov else 'no', [row[b] for row in brfs], nspan=nspan, gain=g, **kw)
         errs.append(rel_l2(gx[b].T, gy[b].T, wx, wy))
     print('small dbp pmd parity %s: rel_l2 %s' % (case, ['%.3e' % e for e in errs]))
     assert max(errs) <= 1e-10, errs

@@ -1,10 +1,9 @@
 """matlab/dbp.m -- the M front-end of digital backpropagation -- and the gateway command ssfm_mex('dbp', ...), executed
 by the mini M interpreter (oracle/mini_m).
 
-CPU: dbp.m with a gateway whose 'dbp' command is served by the DBP oracles (tests/dbp_oracle.py, dbp_pmd_oracle.py,
-dbp_scalar_oracle.py, dbp_channel_oracle.py) equals those oracles run on the parameters the Python mirror pmx.dbp derives
-from the same GSTATE; a PMD-aware DBP inverts two 'gps-' spans that the interpreted fiber.m + ampliflat.m ran; every
-refusal of dbp.m carries pmx.dbp's message.
+CPU: dbp.m with a gateway whose 'dbp' command is served by the DBP oracle (tests/dbp_oracle.py) equals that oracle run
+on the parameters the Python mirror pmx.dbp derives from the same GSTATE; a PMD-aware DBP inverts two 'gps-' spans that
+the interpreted fiber.m + ampliflat.m ran; every refusal of dbp.m carries pmx.dbp's message.
 GPU: the same front-end with the compiled gateway (mexFunction of mex/ssfm_mex.c through the mex.h stand-in) equals
 pmx.dbp on every route, keeps the field resident after fiber.m / ampliflat.m, and inverts a link that fiber.m ran."""
 import math
@@ -15,13 +14,10 @@ import pytest
 
 import oracle.fiber_oracle as orc
 from oracle.mini_m.interp import Interp, MCell, MError, MStruct, to_m
-import dbp_channel_oracle as dco
 import dbp_oracle
-import dbp_pmd_oracle
-import dbp_scalar_oracle
 import mex_bridge
 import polmux_b200 as pmx
-from common import base_fiber, make_tx, rel_l2, scalar_tx
+from common import _rel, base_fiber, make_tx, rel_l2, scalar_tx
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 MDIR = os.path.join(ROOT, 'matlab')
@@ -40,8 +36,10 @@ def _vectors(scal, nfft, nfc, pflag):
 
 
 def oracle_gateway(log=None):
-    """mex_bridge.oracle_gateway() plus ssfm_mex('dbp', ...) answered by the DBP oracles.  Every 'dbp' call is logged
-    (its P, fls, D, band, opt); every two-polarization 'fiber' call logs the oracle's forward steps."""
+    """mex_bridge.oracle_gateway() plus ssfm_mex('dbp', ...) answered by the DBP oracle: every route, with the bandwidth
+    in bins of a 6-entry D (filter_bw) or the trailing taps argument (taps).  Every 'dbp' call is logged (its P, fls, D,
+    band, opt, and its taps or None for the 15-argument call); every two-polarization 'fiber' call logs the oracle's
+    forward steps."""
     base = mex_bridge.oracle_gateway()
     log = [] if log is None else log
 
@@ -64,17 +62,23 @@ def oracle_gateway(log=None):
         if a[0] != 'dbp':
             return base(it, a, nargout)
         ux, uy, betat, db1, P, gam, fls, plates, scal, D, steplen, spansteps, band, opt = a[1:15]
+        taps = np.asarray(a[15], dtype=np.float64) if len(a) > 15 else None
         dzmaxt, dphimaxt, alphalin, lf, nplates, manakov = [float(v) for v in np.asarray(P).ravel()]
         fls = [int(v) for v in np.asarray(fls).ravel()]
-        nspan, gain, steps, xi, pmd = [float(v) for v in np.asarray(D).ravel()]
+        D = np.asarray(D, dtype=np.float64).ravel()
+        nspan, gain, steps, xi, pmd = [float(v) for v in D[:5]]
         opt = np.asarray(opt, dtype=np.float64).ravel()
-        log.append(dict(cmd='dbp', P=np.asarray(P).ravel(), fls=fls, D=np.asarray(D).ravel(), band=np.asarray(band).ravel(),
-                        opt=opt, scal=np.asarray(scal).ravel(), gam=np.asarray(gam).ravel()))
+        log.append(dict(cmd='dbp', P=np.asarray(P).ravel(), fls=fls, D=D, band=np.asarray(band).ravel(), opt=opt,
+                        scal=np.asarray(scal).ravel(), gam=np.asarray(gam).ravel(), taps=taps))
         nfft, nfc = np.shape(ux)
         if np.size(betat) == 0:
             betat, db1 = _vectors(scal, nfft, nfc, fls[1])
         nspan = int(nspan)
         kw = dict(nspan=nspan, gain=gain if gain else None, xi=xi)
+        if D.size > 5 and D[5]:                             # the bandwidth in bins; 0 is no filter
+            kw['bw'] = D[5]
+        if taps is not None and taps.size:
+            kw['taps'] = taps.ravel()
         if steps:
             kw['steps_per_span'] = int(steps)
         else:
@@ -86,9 +90,9 @@ def oracle_gateway(log=None):
         shift, decim = ([int(v) for v in np.asarray(band).ravel()] if ch else (0, 1))
         if opt[0]:                                         # the scalar path
             if ch:
-                out = dco.dbp_channel_scalar(ux, betat, gam, alphalin, lf, shift, decim, spm=fls[2], **kw)
+                out = dbp_oracle.dbp_channel_scalar(ux, betat, gam, alphalin, lf, shift, decim, spm=fls[2], **kw)
             else:
-                out = dbp_scalar_oracle.dbp_scalar(ux, betat, gam, alphalin, nfc, lf, spm=fls[2], xpm=fls[3], **kw)
+                out = dbp_oracle.dbp_scalar(ux, betat, gam, alphalin, nfc, lf, spm=fls[2], xpm=fls[3], **kw)
             return [out, np.zeros((0, 0))][:max(nargout, 1)]
         brfs = None
         if pmd:
@@ -97,11 +101,10 @@ def oracle_gateway(log=None):
             brfs = [{'db0': pl[k * n:(k + 1) * n, 0], 'theta': pl[k * n:(k + 1) * n, 1],
                      'epsilon': pl[k * n:(k + 1) * n, 2]} for k in range(nspan)]
         if ch:
-            ox, oy = dco.dbp_channel(ux, uy, betat, gam, alphalin, lf, mk, shift, decim, db1=db1, brfs=brfs, spm=fls[2], **kw)
-        elif pmd:
-            ox, oy = dbp_pmd_oracle.dbp_pmd(ux, uy, betat, db1, gam, alphalin, nfc, lf, mk, brfs, spm=fls[2], **kw)
+            ox, oy = dbp_oracle.dbp_channel(ux, uy, betat, gam, alphalin, lf, mk, shift, decim, db1=db1, brfs=brfs,
+                                            spm=fls[2], **kw)
         else:
-            ox, oy = dbp_oracle.dbp(ux, uy, betat, gam, alphalin, nfc, lf, mk, spm=fls[2], **kw)
+            ox, oy = dbp_oracle.dbp_pmd(ux, uy, betat, db1, gam, alphalin, nfc, lf, mk, brfs, spm=fls[2], **kw)
         return [ox, oy][:max(nargout, 1)]
     call.log = log
     return call
@@ -137,10 +140,6 @@ def _opts(**kw):
 
 def _brf_m(b):
     return MStruct({k: np.asarray(b[k], dtype=np.float64).reshape(-1, 1) for k in ('db0', 'theta', 'epsilon')})
-
-
-def _rel(a, b):
-    return float(np.linalg.norm(np.asarray(a) - np.asarray(b)) / np.linalg.norm(np.asarray(b)))
 
 
 def _m_field(it):
@@ -202,15 +201,16 @@ def test_explicit_schedule():
 
 
 def test_scalar_xpm_sepfields_ex10_shape():
-    """scalar 'g-sx' on 5 'sepfields' columns of 2^11 samples: XPM-aware DBP == dbp_scalar_oracle; FIELDY stays empty"""
+    """scalar 'g-sx' on 5 'sepfields' columns of 2^11 samples: XPM-aware DBP == dbp_oracle.dbp_scalar; FIELDY stays
+    empty"""
     scalar_tx(64, 32, 5)
     fib = base_fiber(length=5e4)
     G = pmx.GSTATE
     tx = np.array(G.FIELDX)
     s = _setup(fib, 'g-sx')
     assert s.fls[3] == 1 and not s.isv
-    want = dbp_scalar_oracle.dbp_scalar(tx, s.betat, s.gam, s.alphalin, 5, s.length, spm=1, xpm=1, nspan=2,
-                                        gain=10 ** (GAIN_DB / 10), steps_per_span=4)
+    want = dbp_oracle.dbp_scalar(tx, s.betat, s.gam, s.alphalin, 5, s.length, spm=1, xpm=1, nspan=2,
+                                 gain=10 ** (GAIN_DB / 10), steps_per_span=4)
     gw = oracle_gateway()
     it = _interp(gw)
     it.call('dbp', [to_m(fib), 'g-sx', _opts(nspan=2, gain=GAIN_DB, steps=4)], 0)
@@ -224,7 +224,7 @@ def test_scalar_xpm_sepfields_ex10_shape():
 def test_pmd_aware_inverts_two_spans_of_the_interpreted_fiber():
     """two noise-free 'gps-' spans through the interpreted matlab/fiber.m + ampliflat.m (other plates in every span,
     brf returned by fiber.m), then dbp.m with the cell of both brf, xi = 1 and the oracle's forward steps: the Tx field
-    back to <= 1e-12, and == dbp_pmd_oracle"""
+    back to <= 1e-12, and == dbp_oracle.dbp_pmd"""
     make_tx(256, 16, pavg_mw=4.0)
     fib = base_fiber(dgd=0.5, nplates=20, dphimax=0.02)
     G = pmx.GSTATE
@@ -247,16 +247,16 @@ def test_pmd_aware_inverts_two_spans_of_the_interpreted_fiber():
     c = gw.log[-1]
     assert c['fls'][1] == 1 and c['D'][4] == 1
     s = pmx.fiber_setup(fib, 'gps-', rng=np.random.Generator(np.random.PCG64(0)))
-    want = dbp_pmd_oracle.dbp_pmd(rx, ry, s.betat, s.db1, s.gam, s.alphalin, 1, s.length, 'no',
-                                  [{k: np.asarray(b[k]).ravel() for k in ('db0', 'theta', 'epsilon')} for b in brfs],
-                                  nspan=2, gain=10 ** (GAIN_DB / 10), step_len=np.concatenate(steps),
-                                  span_steps=[len(x) for x in steps])
+    want = dbp_oracle.dbp_pmd(rx, ry, s.betat, s.db1, s.gam, s.alphalin, 1, s.length, 'no',
+                              [{k: np.asarray(b[k]).ravel() for k in ('db0', 'theta', 'epsilon')} for b in brfs],
+                              nspan=2, gain=10 ** (GAIN_DB / 10), step_len=np.concatenate(steps),
+                              span_steps=[len(x) for x in steps])
     assert rel_l2(ux, uy, *want) <= 1e-13
 
 
 def test_single_channel():
     """ich = 2, decim = 8 of a 3-channel 'unique' field: the band is [ndfn, 8] with receiver_cohmix's ndfn, and the
-    field == dbp_channel_oracle"""
+    field == dbp_oracle.dbp_channel"""
     make_tx(256, 16, nch=3, pavg_mw=4.0)
     fib = base_fiber(slope=0.057, dphimax=0.02)
     G = pmx.GSTATE
@@ -265,8 +265,8 @@ def test_single_channel():
     from polmux_b200.receiver import channel_ndfn
     for ich in (1, 2):
         m = channel_ndfn(ich)
-        want = dco.dbp_channel(tx, ty, s.betat, s.gam, s.alphalin, s.length, 'no', m, 8, nspan=2,
-                               gain=10 ** (GAIN_DB / 10), steps_per_span=2)
+        want = dbp_oracle.dbp_channel(tx, ty, s.betat, s.gam, s.alphalin, s.length, 'no', m, 8, nspan=2,
+                                      gain=10 ** (GAIN_DB / 10), steps_per_span=2)
         gw = oracle_gateway()
         it = _interp(gw)
         it.call('dbp', [to_m(fib), 'g-s-', _opts(nspan=2, gain=GAIN_DB, steps=2, ich=float(ich), decim=8.0)], 0)
