@@ -402,6 +402,24 @@ int pmx_pb_exec(pmx_pb_plan* plan, pmx_devfield* f);
 int pmx_pb_symbols(pmx_pb_plan* plan, double* A, double* delta);
 void pmx_pb_destroy(pmx_pb_plan* plan);
 
+/* ---- single-channel PB-NLC: one channel of a 'unique' multiplex compensated at a reduced sample rate ------------------
+ * As single-channel DBP (pmx_dbp_channel_create) with the stage in place of the backpropagation.  desc describes the
+ * channel at M = desc->nfft samples (nt and the pulse at that rate, nsymb unchanged); band = {m, r}; the plan runs on
+ * resident one-column FP64 fields of N = M*r samples, per realization, in place:
+ *   down : the band filter at N (H = 1 on the M bins (k - m) mod N of the signed k in [-M/2, M/2)), then the channel at
+ *          baseband, decimated to M samples (pmx_dbp_channel_create's down)
+ *   stage: pmx_pb_exec at M samples (project, triplets, apply)
+ *   up   : stuffed back onto the channel's bins, the band filter at N
+ * Afterwards the field holds channel m alone on its own bins, exactly as single-channel DBP leaves it.  With xi = 0 only
+ * down and up run.  The table is the channel's: its dispersion betat_M[k] = betat_N[(k - m) mod N] less the channel's
+ * phase and group delay, which cancel in the triplets; it differs from the centre channel's only through the dispersion
+ * slope (polmux_b200/pbnlc.py, channel_setup).
+ * Checked before a context is needed: PMX_ERR_INVALID for decim not a power of two >= 2 or M < 2^6; PMX_ERR_UNSUPPORTED
+ * for N > 2^24, nfc != 1 and FP32; and everything pmx_pb_create rejects.  pmx_pb_exec (PMX_ERR_INVALID for a field whose
+ * nfft is not N or whose batch differs), pmx_pb_symbols ([batch][2][nsymb] of the M-sample stage) and pmx_pb_destroy take
+ * the returned plan; it owns the M-sample stage, the band filter and an M x batch work field. */
+int pmx_pb_channel_create(pmx_ctx* ctx, const pmx_pb_desc* desc, const pmx_dbp_band* band, pmx_pb_plan** plan);
+
 /* ---- create_field('unique'): the WDM multiplex on the device (create_field.m:113-149,180-199) ----------------
  * The reference builds the single field as
  *   FIELDX = ifft( sum_ch fastshift( fft(sigx(:,ch)), -ndfn(ch) ) ),   ndfn = round(deltafn/SYMBOLRATE/minfreq)

@@ -35,7 +35,7 @@ EXPORTS = [
     'pmx_ampliflat_exec_at', 'pmx_dsp_count', 'pmx_field_mean_power', 'pmx_pmd_matrix', 'pmx_field_jones', 'pmx_filter_create', 'pmx_field_copy_cols', 'pmx_field_modulate',
     'pmx_cohmix_exec', 'pmx_field_mean_power_xy', 'pmx_cohmix_run', 'pmx_dsp_phases', 'pmx_field_quantize', 'pmx_inverse_pmd_run',
     'pmx_dbp_create', 'pmx_dbp_exec', 'pmx_dbp_set_plates', 'pmx_dbp_channel_create', 'pmx_dbp_set_filter',
-    'pmx_dbp_set_taps', 'pmx_pb_create', 'pmx_pb_exec', 'pmx_pb_symbols', 'pmx_pb_destroy',
+    'pmx_dbp_set_taps', 'pmx_pb_create', 'pmx_pb_exec', 'pmx_pb_symbols', 'pmx_pb_destroy', 'pmx_pb_channel_create',
 ]
 
 
@@ -201,6 +201,7 @@ def load():
     lib.pmx_pb_destroy.argtypes = [vp]
     lib.pmx_pb_destroy.restype = None
     lib.pmx_dbp_channel_create.argtypes = [vp, C.POINTER(FiberDesc), C.POINTER(DbpDesc), C.POINTER(DbpBand), C.POINTER(vp)]
+    lib.pmx_pb_channel_create.argtypes = [vp, C.POINTER(PbDesc), C.POINTER(DbpBand), C.POINTER(vp)]
     _lib = lib
     return lib
 
@@ -656,12 +657,17 @@ def make_pb(nsymb, nt, batch, pulse, weights, gamma, xi, scale, m, n, coef):
 
 
 class PbPlan:
-    """Perturbation-based nonlinearity compensation (pmx_pb_create): execute(field) runs it in place on a resident field."""
+    """Perturbation-based nonlinearity compensation (pmx_pb_create): execute(field) runs it in place on a resident field.
+    With a band (DbpBand: shift, decim) the descriptor is the channel's at nfft/decim samples and the plan is the PB-NLC of
+    that channel of a one-column field of nfft samples (pmx_pb_channel_create)."""
 
-    def __init__(self, ctx: Context, desc_keep):
-        self.ctx, (self.desc, self.keep) = ctx, desc_keep
+    def __init__(self, ctx: Context, desc_keep, band: 'DbpBand' = None):
+        self.ctx, (self.desc, self.keep), self.band = ctx, desc_keep, band
         h = C.c_void_p()
-        ctx.check(ctx.lib.pmx_pb_create(ctx.h, C.byref(self.desc), C.byref(h)))
+        if band is None:
+            ctx.check(ctx.lib.pmx_pb_create(ctx.h, C.byref(self.desc), C.byref(h)))
+        else:
+            ctx.check(ctx.lib.pmx_pb_channel_create(ctx.h, C.byref(self.desc), C.byref(band), C.byref(h)))
         self.h = h
 
     def execute(self, field: DeviceField):

@@ -4024,9 +4024,63 @@ extern "C" int pmx_dbp_exec(pmx_plan* p, pmx_devfield* fld) {
 }
 
 // ---------------------------------------------------------------------------
-// Single-channel DBP (polmux_ssfm.h, pmx_dbp_band): band filter at N, gather to M = N/r, the DBP plan of M samples, stuff
-// back to N, band filter.  The M-sample plan is an ordinary pmx_dbp_create plan on vector tables: the channel's own
-// dispersion, so that nothing in the step kernels knows about the channel's offset.
+// One channel of a one-column multiplex at M = N/r samples (pmx_dbp_band), shared by single-channel DBP and single-channel
+// PB-NLC: down = band filter at N, gather to M; up = stuff back to N, band filter.
+
+// The N-grid bin of M-grid bin j: (k - m) mod N for the signed k of j (m the channel's shift mod N)
+static size_t band_bin(int64_t j, int64_t M, int64_t N, long long m) {
+    return (size_t)((((j < M / 2 ? j : j - M) - m) % N + N) % N);
+}
+
+// The band filter at N samples: H = 1 on the channel's M bins
+static int band_filter_create(pmx_ctx* c, int64_t N, int64_t M, long long m, int batch, int precision, pmx_plan** out) {
+    std::vector<double> H(2 * (size_t)N, 0.0);
+    for (int64_t j = 0; j < M; ++j) H[2 * band_bin(j, M, N, m)] = 1.0;
+    return pmx_filter_create(c, N, 1, batch, precision, H.data(), 1, out);
+}
+
+// fld (N samples) -> w (M samples): the band filter in place on fld, then the channel at baseband, decimated, into w
+static int band_down(pmx_plan* band, pmx_devfield* fld, pmx_devfield* w, int lr, long long m) {
+    pmx_ctx* c = band->ctx;
+    int rc = check_field(band, fld);   // device, precision, nfft, one column, batch
+    if (!rc) rc = pmx_fiber_exec(band, fld, nullptr);
+    if (rc) return rc;
+    CK(c, cudaSetDevice(c->device));
+    const size_t N = (size_t)fld->nfft, M = (size_t)w->nfft;
+    const dim3 gm((unsigned)std::min<size_t>((M + 255) / 256, 148 * 8), fld->batch);
+    if (fld->precision == PMX_F32)
+        pmx_k_band_gather<float2><<<gm, 256, 0, c->stream>>>(reinterpret_cast<const float2*>(fld->data), fld->log2N1, fld->log2N2,
+                                                              reinterpret_cast<float2*>(w->data), w->log2N1, w->log2N2, N, lr, m);
+    else
+        pmx_k_band_gather<double2><<<gm, 256, 0, c->stream>>>(reinterpret_cast<const double2*>(fld->data), fld->log2N1,
+                                                               fld->log2N2, reinterpret_cast<double2*>(w->data), w->log2N1,
+                                                               w->log2N2, N, lr, m);
+    c->launches++;
+    CK(c, cudaGetLastError());
+    return PMX_OK;
+}
+
+// w (M samples) -> fld (N samples): stuffed back onto the channel's bins, then the band filter in place on fld
+static int band_up(pmx_plan* band, pmx_devfield* w, pmx_devfield* fld, int lr, long long m) {
+    pmx_ctx* c = band->ctx;
+    const size_t N = (size_t)fld->nfft;
+    const dim3 gn((unsigned)std::min<size_t>((N + 255) / 256, 148 * 8), fld->batch);
+    if (fld->precision == PMX_F32)
+        pmx_k_band_stuff<float2><<<gn, 256, 0, c->stream>>>(reinterpret_cast<const float2*>(w->data), w->log2N1, w->log2N2,
+                                                             reinterpret_cast<float2*>(fld->data), fld->log2N1, fld->log2N2, N,
+                                                             lr, m);
+    else
+        pmx_k_band_stuff<double2><<<gn, 256, 0, c->stream>>>(reinterpret_cast<const double2*>(w->data), w->log2N1, w->log2N2,
+                                                              reinterpret_cast<double2*>(fld->data), fld->log2N1, fld->log2N2, N,
+                                                              lr, m);
+    c->launches++;
+    CK(c, cudaGetLastError());
+    return pmx_fiber_exec(band, fld, nullptr);
+}
+
+// Single-channel DBP (polmux_ssfm.h, pmx_dbp_band): down, the DBP plan of M samples, up.  The M-sample plan is an ordinary
+// pmx_dbp_create plan on vector tables: the channel's own dispersion, so that nothing in the step kernels knows about the
+// channel's offset.
 extern "C" int pmx_dbp_channel_create(pmx_ctx* c, const pmx_fiber_desc* fd, const pmx_dbp_desc* g, const pmx_dbp_band* band,
                                       pmx_plan** out) {
     // (checked before the context, like pmx_dbp_create)
@@ -4049,7 +4103,7 @@ extern "C" int pmx_dbp_channel_create(pmx_ctx* c, const pmx_fiber_desc* fd, cons
         return set_err(c, PMX_ERR_UNSUPPORTED, "single-channel digital backpropagation on the scalar path: nfft/decim=%lld, "
                        "built for at most 2^12 samples", (long long)M);
     const long long m = ((band->shift % N) + N) % N;
-    auto bin = [&](int64_t j) { return (size_t)((((j < M / 2 ? j : j - M) - m) % N + N) % N); };   // N-grid bin of M-grid bin j
+    auto bin = [&](int64_t j) { return band_bin(j, M, N, m); };
     const bool pmd = g->pmd == 1 && fd->fls[1];
     std::vector<double> bt((size_t)M), d1;
     if (fd->disp_mode == PMX_DISP_SCALAR) {
@@ -4082,8 +4136,6 @@ extern "C" int pmx_dbp_channel_create(pmx_ctx* c, const pmx_fiber_desc* fd, cons
     pmx_plan* inner = nullptr;
     int rc = pmx_dbp_create(c, &e, g, &inner);   // validates the rest before it needs the context
     if (rc) return rc;
-    std::vector<double> H(2 * (size_t)N, 0.0);   // 1 on the channel's M bins
-    for (int64_t j = 0; j < M; ++j) H[2 * bin(j)] = 1.0;
     pmx_plan* p = new (std::nothrow) pmx_plan();
     if (!p) {
         pmx_plan_destroy(inner);
@@ -4096,7 +4148,7 @@ extern "C" int pmx_dbp_channel_create(pmx_ctx* c, const pmx_fiber_desc* fd, cons
     p->ch_dbp = inner;
     p->ch_shift = m;
     p->ch_log2r = lr;
-    rc = pmx_filter_create(c, N, 1, fd->batch, fd->precision, H.data(), 1, &p->ch_band);
+    rc = band_filter_create(c, N, M, m, fd->batch, fd->precision, &p->ch_band);
     if (!rc) rc = pmx_field_create(c, M, 1, fd->batch, fd->precision, &p->ch_work);
     if (rc) {
         pmx_plan_destroy(p);
@@ -4107,38 +4159,10 @@ extern "C" int pmx_dbp_channel_create(pmx_ctx* c, const pmx_fiber_desc* fd, cons
 }
 
 static int dbp_channel_exec(pmx_plan* p, pmx_devfield* fld) {
-    pmx_ctx* c = p->ctx;
-    int rc = check_field(p->ch_band, fld);   // device, precision, nfft, one column, batch
-    if (!rc) rc = pmx_fiber_exec(p->ch_band, fld, nullptr);
-    if (rc) return rc;
-    CK(c, cudaSetDevice(c->device));
-    pmx_devfield* w = p->ch_work;
-    const size_t N = (size_t)fld->nfft, M = (size_t)w->nfft;
-    const dim3 gm((unsigned)std::min<size_t>((M + 255) / 256, 148 * 8), fld->batch);
-    if (fld->precision == PMX_F32)
-        pmx_k_band_gather<float2><<<gm, 256, 0, c->stream>>>(reinterpret_cast<const float2*>(fld->data), fld->log2N1, fld->log2N2,
-                                                              reinterpret_cast<float2*>(w->data), w->log2N1, w->log2N2, N,
-                                                              p->ch_log2r, p->ch_shift);
-    else
-        pmx_k_band_gather<double2><<<gm, 256, 0, c->stream>>>(reinterpret_cast<const double2*>(fld->data), fld->log2N1,
-                                                               fld->log2N2, reinterpret_cast<double2*>(w->data), w->log2N1,
-                                                               w->log2N2, N, p->ch_log2r, p->ch_shift);
-    c->launches++;
-    CK(c, cudaGetLastError());
-    rc = pmx_dbp_exec(p->ch_dbp, w);
-    if (rc) return rc;
-    const dim3 gn((unsigned)std::min<size_t>((N + 255) / 256, 148 * 8), fld->batch);
-    if (fld->precision == PMX_F32)
-        pmx_k_band_stuff<float2><<<gn, 256, 0, c->stream>>>(reinterpret_cast<const float2*>(w->data), w->log2N1, w->log2N2,
-                                                             reinterpret_cast<float2*>(fld->data), fld->log2N1, fld->log2N2, N,
-                                                             p->ch_log2r, p->ch_shift);
-    else
-        pmx_k_band_stuff<double2><<<gn, 256, 0, c->stream>>>(reinterpret_cast<const double2*>(w->data), w->log2N1, w->log2N2,
-                                                              reinterpret_cast<double2*>(fld->data), fld->log2N1, fld->log2N2, N,
-                                                              p->ch_log2r, p->ch_shift);
-    c->launches++;
-    CK(c, cudaGetLastError());
-    return pmx_fiber_exec(p->ch_band, fld, nullptr);
+    int rc = band_down(p->ch_band, fld, p->ch_work, p->ch_log2r, p->ch_shift);
+    if (!rc) rc = pmx_dbp_exec(p->ch_dbp, p->ch_work);
+    if (!rc) rc = band_up(p->ch_band, p->ch_work, fld, p->ch_log2r, p->ch_shift);
+    return rc;
 }
 
 // ---------------------------------------------------------------------------
@@ -4157,6 +4181,13 @@ struct pmx_pb_plan {
     PbCoef* coef = nullptr;   // [ncoef]
     cpx* A = nullptr;         // [batch][2][nsymb] projected symbols
     cpx* D = nullptr;         // [batch][2][nsymb] perturbation
+    // single-channel PB-NLC (pmx_pb_channel_create): the stage at nfft/decim samples, the band filter at nfft, the work field
+    // of the decimated channel, and the channel's shift (mod nfft) and log2(decim)
+    pmx_pb_plan* ch_pb = nullptr;
+    pmx_plan* ch_band = nullptr;
+    pmx_devfield* ch_work = nullptr;
+    long long ch_shift = 0;
+    int ch_log2r = 0;
 };
 
 // A^{x,y}_k = sum_j p[j] u[(k*nt - np/2 + j) mod N] * inorm (j ascending); thread per symbol, grid.y the realization
@@ -4381,6 +4412,12 @@ extern "C" int pmx_pb_exec(pmx_pb_plan* p, pmx_devfield* f) {
                        (long long)p->nfft);
     if (f->batch != p->batch)
         return set_err(c, PMX_ERR_INVALID, "pmx_pb_exec: the field has batch %d, the plan %d", f->batch, p->batch);
+    if (p->ch_pb) {   // single channel: down, the stage at nfft/decim samples, up
+        int rc = band_down(p->ch_band, f, p->ch_work, p->ch_log2r, p->ch_shift);
+        if (!rc) rc = pmx_pb_exec(p->ch_pb, p->ch_work);
+        if (!rc) rc = band_up(p->ch_band, p->ch_work, f, p->ch_log2r, p->ch_shift);
+        return rc;
+    }
     if (p->xi == 0) return PMX_OK;   // nothing to subtract: the field is left as it is
     CK(c, cudaSetDevice(c->device));
     const size_t N = (size_t)p->nfft;
@@ -4400,6 +4437,7 @@ extern "C" int pmx_pb_exec(pmx_pb_plan* p, pmx_devfield* f) {
 
 extern "C" int pmx_pb_symbols(pmx_pb_plan* p, double* A, double* delta) {
     if (!p) return set_err(nullptr, PMX_ERR_INVALID, "pmx_pb_symbols: null plan");
+    if (p->ch_pb) return pmx_pb_symbols(p->ch_pb, A, delta);
     pmx_ctx* c = p->ctx;
     const size_t bytes = (size_t)p->batch * 2 * p->nsymb * sizeof(cpx);
     CK(c, cudaSetDevice(c->device));
@@ -4414,5 +4452,55 @@ extern "C" void pmx_pb_destroy(pmx_pb_plan* p) {
     cudaSetDevice(p->ctx->device);
     for (void* q : {(void*)p->pulse, (void*)p->coef, (void*)p->A, (void*)p->D})
         if (q) cudaFreeAsync(q, p->ctx->stream);
+    pmx_pb_destroy(p->ch_pb);
+    pmx_plan_destroy(p->ch_band);
+    pmx_field_destroy(p->ch_work);
     delete p;
+}
+
+// Single-channel PB-NLC (polmux_ssfm.h): down, the stage of pmx_pb_create at M = nfft/decim samples, up, as single-channel
+// DBP does it.  The descriptor is the stage's at M samples; the plan runs on fields of N = M*decim samples.
+extern "C" int pmx_pb_channel_create(pmx_ctx* c, const pmx_pb_desc* d, const pmx_dbp_band* band, pmx_pb_plan** out) {
+    // (checked before the context, like pmx_pb_create)
+    if (!d || !band || !out) return set_err(c, PMX_ERR_INVALID, "pmx_pb_channel_create: null argument");
+    *out = nullptr;
+    const int lm = ilog2_exact(d->nfft), lr = ilog2_exact(band->decim);
+    if (band->decim < 2 || lr < 1)
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_channel_create: decim=%d, must be a power of two >= 2", band->decim);
+    if (d->nfft < 64)
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_channel_create: nfft/decim = %lld/%d samples, at least 2^6 are needed",
+                       (long long)d->nfft * band->decim, band->decim);
+    if (lm >= 0 && lm + lr > 24)
+        return set_err(c, PMX_ERR_UNSUPPORTED, "single-channel PB-NLC: nfft=%lld, built for powers of two from 2^6 to 2^24",
+                       (long long)d->nfft * band->decim);
+    if (d->nfc != 1)
+        return set_err(c, PMX_ERR_UNSUPPORTED, "single-channel PB-NLC: nfc=%d, built for one column holding every channel "
+                       "(a 'unique' multiplex)", d->nfc);
+    if (d->precision != PMX_F64) return set_err(c, PMX_ERR_UNSUPPORTED, "pmx_pb_channel_create: FP64 fields only");
+    pmx_pb_plan* inner = nullptr;
+    int rc = pmx_pb_create(c, d, &inner);   // validates the rest before it needs the context
+    if (rc) return rc;
+    const int64_t M = d->nfft, N = M << lr;
+    pmx_pb_plan* p = new (std::nothrow) pmx_pb_plan();
+    if (!p) {
+        pmx_pb_destroy(inner);
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_channel_create: out of host memory");
+    }
+    p->ctx = c;
+    p->nfft = N;
+    p->nsymb = d->nsymb;
+    p->nt = d->nt << lr;
+    p->batch = d->batch;
+    p->xi = d->xi;
+    p->ch_pb = inner;
+    p->ch_shift = ((band->shift % N) + N) % N;
+    p->ch_log2r = lr;
+    rc = band_filter_create(c, N, M, p->ch_shift, d->batch, PMX_F64, &p->ch_band);
+    if (!rc) rc = pmx_field_create(c, M, 1, d->batch, PMX_F64, &p->ch_work);
+    if (rc) {
+        pmx_pb_destroy(p);
+        return rc;
+    }
+    *out = p;
+    return PMX_OK;
 }

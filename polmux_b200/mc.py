@@ -230,7 +230,9 @@ class McRunner:
         dbp_params with 'filter_bw' [GHz]: filtered DBP (dbp_plan); with 'nl_taps': enhanced split-step DBP (dbp_plan).
         'pbnlc' ('blind' and 'cohmix', one channel in a one-column field): the all-pass step, then perturbation-based
         nonlinearity compensation (polmux_b200/pbnlc.py, pb_plan) with pb_params (xi, K, prune, pulse, nquad, window;
-        default xi = 1, K = 16) at the launch scale s of the link's loss and gain."""
+        default xi = 1, K = 16) at the launch scale s of the link's loss and gain.  pb_params with 'decim' (a power of two
+        >= 2 dividing nt; a one-column 'unique' field of any number of channels): single-channel PB-NLC on nfft/decim
+        samples -- of channel `ich` for 'cohmix', of the channel at the centre of the grid for 'blind'."""
         import torch
         from . import dsp as _dsp
         self.receiver, self.dsp_params = receiver, dict(dsp_params or {})
@@ -291,7 +293,10 @@ class McRunner:
             self.rx = dict(cd=comp, S=None, pb=None)
             if compensation == 'pbnlc':
                 from .pbnlc import pb_plan
-                self.rx['pb'] = pb_plan(self.rxctx, setup, nspan, gain_db, batch=batch, nt=nt, **dict(pb_params or {}))
+                pp = dict(pb_params or {})
+                if pp.get('decim') is not None:      # single-channel PB-NLC of the receiver's channel
+                    pp['shift'] = S.ndfn if S is not None else 0
+                self.rx['pb'] = pb_plan(self.rxctx, setup, nspan, gain_db, batch=batch, nt=nt, **pp)
             if receiver == 'cohmix':
                 delay = _rx.evaldelay(x['oftype'], x['obw'] * 0.5) + _rx.evaldelay(x['eftype'], x['ebw']) + S.x['post_delay']
                 self.rx.update(S=S, ich=ich, shift=int(round(delay * nt)),

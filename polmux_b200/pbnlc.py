@@ -14,9 +14,16 @@ first-order expansion of -j*gam*[P*u + (s3/3)*J*u] (fiber.m:827-851).
 
 The coefficient table C[m,n] of the whole link (pb_coefficients) is computed once on the host; the stage itself runs on the
 device in one pass at the symbol rate (pmx_pb_create / pmx_pb_exec, include/polmux_ssfm.h).  There is no CPU fallback.
+
+Single-channel PB-NLC (pbnlc(..., ich=, decim=), pb_plan(..., shift=, decim=); pmx_pb_channel_create): a coherent receiver
+sees its own channel only.  As single-channel DBP does it, channel ich of a 'unique' multiplex is cut out by an ideal
+band-pass, brought to baseband and decimated to nfft/decim samples, compensated there with the table of its own dispersion
+(channel_setup) and the pulse it carries at that rate (channel_pulse), then returned to its own bins; the other channels
+are dropped.
 """
 from __future__ import annotations
 
+import dataclasses
 import math
 from typing import Optional
 
@@ -116,6 +123,60 @@ def pb_coefficients(setup: FiberSetup, nspan: int, pulse=None, K: int = 16, prun
     return mm[keep].astype(np.int32), nn[keep].astype(np.int32), C[keep]
 
 
+def _check_decim(decim, nt: Optional[int] = None) -> int:
+    """ValueError with pmx_pb_channel_create's message for a decimation it refuses, and for one that does not divide the
+    samples per symbol nt (the channel keeps every symbol), before any table is computed"""
+    r = int(decim)
+    if r < 2 or r & (r - 1):
+        raise ValueError('pmx_pb_channel_create: decim=%d, must be a power of two >= 2' % r)
+    if nt is not None and int(nt) % r:
+        raise ValueError('decim=%d must divide nt=%d: the channel keeps every symbol at nt/decim samples' % (r, int(nt)))
+    return r
+
+
+def _channel_bins(nfft: int, shift: int, decim: int) -> np.ndarray:
+    """the nfft-grid bins of the M = nfft/decim grid's bins 0..M-1 (FFT order): (k - shift) mod nfft for the signed k"""
+    M = nfft // decim
+    k = np.fft.fftfreq(M, 1.0 / M).round().astype(np.int64)
+    return (k - int(shift)) % nfft
+
+
+def channel_setup(setup: FiberSetup, shift: int, decim: int) -> FiberSetup:
+    """The FiberSetup of the channel that `shift` bins bring to baseband (the receiver's ndfn), on M = nfft/decim samples:
+    the channel's own dispersion, betat_M[k] = betat_N[(k - shift) mod N] for the signed k of the M grid (db1 likewise),
+    the mapping single-channel DBP uses (pmx_dbp_channel_create), less its constant and linear part in k (taken from bins
+    0 and +-1).  That part is the channel's phase and group delay, which cancel in conj(g_0) g_m g_n conj(g_{m+n}) as they
+    would in continuous time.  On the circular grid they would not quite: a group delay of a fraction of a sample moves
+    the table with the aliased part of the products, and a walk-off over the link spreads the pulse over the whole window
+    (default_window).  pb_coefficients on this setup is the channel's table; it differs from the centre channel's only
+    with a dispersion slope."""
+    r = _check_decim(decim)
+    N = int(setup.nfft)
+    M = N // r
+    b = _channel_bins(N, shift, r)
+    bt = np.asarray(setup.betat, dtype=np.float64)[b]
+    k = np.fft.fftfreq(M, 1.0 / M).round().reshape(-1, 1)
+    bt = bt - bt[0] - k * (0.5 * (bt[1] - bt[M - 1]))
+    return dataclasses.replace(setup, nfft=M, betat=np.ascontiguousarray(bt),
+                               db1=np.ascontiguousarray(np.asarray(setup.db1)[b]))
+
+
+def channel_pulse(nt: int, decim: int, nfft: int) -> np.ndarray:
+    """The default pulse of single-channel PB-NLC at nt/decim samples per symbol: the transmit pulse synth.cosroll_pulse(nt,
+    0.2), placed on nfft samples as symbol 0, through the ideal band-pass and decimation of the down step (the real part:
+    the band's one unpaired bin -M/2 is split between -M/2 and +M/2), truncated to the 16*nt/decim samples (at most
+    nfft/decim) pmx_pb_desc allows, symbol 0 at index npulse/2 as the stage places it.  A model choice: the pulse the field
+    carries at that rate, not the pulse a transmitter at that rate would send; pb_plan(pulse=) takes another."""
+    r = _check_decim(decim)
+    N, M, ntm = int(nfft), int(nfft) // r, int(nt) // r
+    p = synth.cosroll_pulse(int(nt), 0.2)
+    u = np.zeros(N, dtype=np.complex128)
+    u[(np.arange(p.size) - p.size // 2) % N] = p
+    v = _sfft.ifft(_sfft.fft(u)[_channel_bins(N, 0, r)] / r).real       # v[n] = (band-passed u)[n*r]
+    L = min(16 * ntm, M)
+    return np.ascontiguousarray(v[(np.arange(L) - L // 2) % M])
+
+
 def scale_factor(setup: FiberSetup, nspan: int, gain_db: Optional[float] = None) -> float:
     """s = (exp(alpha*Ls/2)/sqrt(G))^nspan (G = 1 without an amplifier): the factor that brings the received field to
     launch scale, the net of DBP's per-step and per-span factors"""
@@ -125,35 +186,64 @@ def scale_factor(setup: FiberSetup, nspan: int, gain_db: Optional[float] = None)
 
 def pb_plan(ctx: _lib.Context, setup: FiberSetup, nspan: int, gain_db: Optional[float] = None, xi: float = 1.0,
             K: int = 16, prune: float = 0.0, pulse=None, batch: int = 1, nt: Optional[int] = None, nquad: int = 32,
-            window: Optional[int] = None, coefs=None) -> _lib.PbPlan:
+            window: Optional[int] = None, coefs=None, shift: Optional[int] = None,
+            decim: Optional[int] = None) -> _lib.PbPlan:
     """The PB-NLC stage of nspan spans of the fiber `setup` describes (amplifier of gain_db [dB] after each; None: none), for
     resident one-column FP64 fields of `batch` realizations: pmx_pb_create with the table of pb_coefficients (or `coefs`,
-    a (m, n, C) table), the model and gamma of the fiber, and s = scale_factor(setup, nspan, gain_db)."""
+    a (m, n, C) table), the model and gamma of the fiber, and s = scale_factor(setup, nspan, gain_db).
+    decim: single-channel PB-NLC of a one-column field (pmx_pb_channel_create) -- the channel that `shift` bins bring to
+    baseband (the receiver's ndfn; default 0), compensated on nfft/decim samples with the table of channel_setup at
+    nt/decim samples per symbol; the pulse (and a `coefs` table) then belong to that rate, the default pulse is
+    channel_pulse."""
     nt = int(nt or GSTATE.NT)
-    p = np.asarray(synth.cosroll_pulse(nt, 0.2) if pulse is None else pulse, dtype=np.float64).ravel()
+    if decim is None and shift is not None:
+        raise ValueError('pb_plan: shift selects a channel for single-channel PB-NLC and needs decim')
     if setup.nfc != 1:
         raise ValueError('pmx_pb_create: nfc=%d, PB-NLC takes one-column fields holding one channel' % setup.nfc)
     _lib.check_pb_k(K)
+    band = None
+    if decim is not None:
+        r = _check_decim(decim, nt)
+        if pulse is None:
+            pulse = channel_pulse(nt, r, setup.nfft)
+        band = _lib.make_band(shift or 0, r)
+        setup, nt = channel_setup(setup, shift or 0, r), nt // r
+    p = np.asarray(synth.cosroll_pulse(nt, 0.2) if pulse is None else pulse, dtype=np.float64).ravel()
     m, n, C = pb_coefficients(setup, nspan, p, K, prune, nt, nquad, window) if coefs is None else coefs
     w, gam = model_weights(setup)
     return _lib.PbPlan(ctx, _lib.make_pb(setup.nfft // nt, nt, batch, p, w, gam, xi, scale_factor(setup, nspan, gain_db),
-                                         m, n, C))
+                                         m, n, C), band)
 
 
 def pbnlc(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, xi: float = 1.0, K: int = 16, prune: float = 0.0,
-          pulse=None, ctx: Optional[_lib.Context] = None, nquad: int = 32, window: Optional[int] = None):
+          pulse=None, ctx: Optional[_lib.Context] = None, nquad: int = 32, window: Optional[int] = None,
+          ich: Optional[int] = None, decim: Optional[int] = None):
     """Compensates GSTATE.FIELDX / FIELDY in place for nspan spans of the fiber x, the amplifier of gain_db [dB] after each
     (None: no amplifier): the all-pass step that undoes the link's chromatic dispersion (as Link.cd_plan), then the PB-NLC
     stage with the triplet table of K (pb_coefficients) at s = scale_factor(...), the fraction xi of the perturbation
     subtracted.  The nonlinear model is the one fiber() used: Manakov when x.manakov is 'yes' and the flag has 'p', else the
-    CNLSE.  One channel (GSTATE.NCH == 1), two polarizations, FP64.  The field stays resident on the device like dbp()
-    leaves it."""
+    CNLSE.  One channel (GSTATE.NCH == 1), two polarizations, FP64.  ich, decim: single-channel PB-NLC of channel ich
+    (1-based) of a 'unique' multiplex of any NCH on nfft/decim samples (pb_plan; a given pulse is at that rate); afterwards
+    the field holds that channel alone, on its own bins.  The field stays resident on the device like dbp() leaves it."""
     from .mc import cd_plan_of
     G = GSTATE
     f = str(flag).lower()
     if len(f) != 4:
         raise ValueError("wrong flag. E.g. flag can be 'g---','gp--','-s--', etc")
-    if G.NCH != 1:
+    shift = None
+    if decim is not None:
+        if ich is None:
+            raise ValueError('pbnlc: single-channel PB-NLC (decim) needs the channel ich')
+        if ich < 1 or ich > G.NCH:
+            raise ValueError('The channel does not exist')
+        if G.field_shape()[1] != 1:
+            raise ValueError("pbnlc: single-channel PB-NLC takes a field holding every channel in one column ('unique')")
+        _check_decim(decim, G.NT)
+        from .receiver import channel_ndfn
+        shift = int(channel_ndfn(ich, G)) if G.NCH > 1 else 0
+    elif ich is not None:
+        raise ValueError('pbnlc: ich selects a channel for single-channel PB-NLC and needs decim')
+    elif G.NCH != 1:
         raise ValueError('pbnlc: PB-NLC takes a field holding one channel (GSTATE.NCH == 1), got %d' % G.NCH)
     if not G.has_y():
         raise ValueError('pbnlc: PB-NLC takes two-polarization fields (FIELDY is empty)')
@@ -167,7 +257,7 @@ def pbnlc(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, xi: flo
     ctx = ctx or _lib.default_context()
     cd = cd_plan_of(ctx, s, int(nspan), 1, precision='f64')
     try:
-        plan = pb_plan(ctx, s, nspan, gain_db, xi, K, prune, pulse, nquad=nquad, window=window)
+        plan = pb_plan(ctx, s, nspan, gain_db, xi, K, prune, pulse, nquad=nquad, window=window, shift=shift, decim=decim)
     except Exception:
         cd.close()
         raise

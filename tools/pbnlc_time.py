@@ -1,6 +1,8 @@
-"""Times perturbation-based nonlinearity compensation (pmx_pb_create / pmx_pb_exec) on the C2 shape.
+"""Times perturbation-based nonlinearity compensation (pmx_pb_create / pmx_pb_exec) on the C2 shape, or with --decim
+single-channel PB-NLC (pmx_pb_channel_create) on the C4 and C2 shapes.
 
     python tools/pbnlc_time.py [--nspan 10] [--reps 20] [--ks 4,8,16,32,64] [--out DIR]
+    python tools/pbnlc_time.py --decim 16,32,64 [--nch 9] [--reps 5] [--out DIR]
 
 C2 (BASELINE.md): one 28-GBaud PDM-QPSK channel, 2^16 symbols x 16 samples = 2^20 samples, 80 km spans with 16 dB
 amplifiers, Manakov.  In one process:
@@ -11,7 +13,16 @@ amplifiers, Manakov.  In one process:
   2. per group of 16 realizations: the CD all-pass step + PB-NLC (K = 32, the table of the link) against DBP at one step per
      span on the whole field (single-channel DBP of the one channel, decim 2) and full DBP, each the median wall time of
      a call that ends synchronised (the PB-NLC plan with xi = 1e-9, so that the repeated runs on one field stay bounded).
-The card's name, power limit and maximum SM clock are read in the same run and printed with the numbers."""
+The card's name, power limit and maximum SM clock are read in the same run and printed with the numbers.
+
+With --decim: C4 (BASELINE.md: --nch 28-GBaud channels at 50 GHz in one 'unique' field of 2^16 symbols x 64 samples =
+2^22 samples, 20 x 80 km Manakov spans with 16 dB amplifiers, 1 mW per channel, one realization) and C2 (one channel,
+2^16 x 16 = 2^20 samples, 10 spans, batch 16).  For every decim r of the list that divides the shape's samples per
+symbol, the centre channel: the CD all-pass step + single-channel PB-NLC (xi = 1, the channel's tables of K = 16 and 32
+at nt/r samples per symbol) and single-channel DBP at 1 and 4 steps per span.  All plans are made first and then run in
+turn, round after round, so that they are alternated in one process; each is reported as the median over --reps rounds of
+the wall time of one call on a field refreshed from the Tx (a call returns synchronised), in ms per link (per group of
+the batch).  The card's name, power limit and SM clocks are read in the same run."""
 import argparse
 import json
 import os
@@ -30,14 +41,15 @@ import polmux_b200 as pmx  # noqa: E402
 from polmux_b200 import _lib, mc, synth  # noqa: E402
 from polmux_b200.dbp import dbp_plan  # noqa: E402
 from polmux_b200.fiber import fiber_setup  # noqa: E402
-from polmux_b200.pbnlc import pb_coefficients, pb_plan, model_weights  # noqa: E402
+from polmux_b200.pbnlc import channel_pulse, channel_setup, pb_coefficients, pb_plan, model_weights  # noqa: E402
+from polmux_b200.receiver import channel_ndfn  # noqa: E402
 
 FP64_INSTR = 52
 
 
 def card():
     try:
-        return subprocess.run(['nvidia-smi', '-i', '0', '--query-gpu=name,power.limit,clocks.max.sm',
+        return subprocess.run(['nvidia-smi', '-i', '0', '--query-gpu=name,power.limit,clocks.sm,clocks.max.sm',
                                '--format=csv,noheader'], capture_output=True, text=True, timeout=30).stdout.strip()
     except Exception as e:  # noqa: BLE001
         return 'nvidia-smi unavailable (%s)' % e
@@ -77,6 +89,81 @@ def wall_ms(fn, reps):
     return 1000.0 * float(np.median(ts))
 
 
+def channel_shape(name, nsymb, nt, nch, nspan, batch, decims, reps):
+    """the rows of one shape: CD + single-channel PB-NLC (K 16, 32) and single-channel DBP (1, 4 steps/span) per decim"""
+    ex, ey, _, _ = synth.pdm_qpsk(nsymb, nt, nch)
+    pmx.reset_all(nsymb, nt, nch)
+    G = pmx.GSTATE
+    G.SYMBOLRATE, G.LAMBDA, G.POWER = 28.0, synth.wdm_lambdas(nch, 1550.0, 0.4), np.full(nch, 1.0)
+    pmx.create_field('unique', ex, ey, {'power': 'average'})
+    fib = dict(synth.SMF)
+    fib.update(length=8e4, manakov='yes')
+    s = fiber_setup(fib, 'g-s-')
+    s.manakov = True
+    shift = int(channel_ndfn((nch + 1) // 2)) if nch > 1 else 0
+    ctx = _lib.default_context(0)
+    N = s.nfft
+    tx = _lib.DeviceField(ctx, N, 1, 1)
+    tx.upload(G.FIELDX_TX, G.FIELDY_TX)
+    fld = _lib.DeviceField(ctx, N, 1, batch)
+    cd = mc.cd_plan_of(ctx, s, nspan, batch, precision='f64')
+    runs = []                                            # (info, callable on fld)
+    for r in decims:
+        if nt % r:
+            print('%s: decim %d does not divide nt = %d, skipped' % (name, r, nt))
+            continue
+        t0 = time.perf_counter()
+        p = channel_pulse(nt, r, N)
+        m, n, C = pb_coefficients(channel_setup(s, shift, r), nspan, p, 32, nt=nt // r)
+        print('%s r=%d: channel table of K = 32 (%d x 80 km) in %.1f s on one host thread'
+              % (name, r, nspan, time.perf_counter() - t0))
+        for K in (16, 32):
+            sel = (np.abs(m) <= K) & (np.abs(n) <= K)
+            pb = pb_plan(ctx, s, nspan, 16.0, K=K, batch=batch, nt=nt, coefs=(m[sel], n[sel], C[sel]), shift=shift,
+                         decim=r)
+            runs.append((dict(run='cd+pbnlc', decim=r, K=K, ncoef=int(sel.sum())),
+                         lambda f, pb=pb: (cd.execute(f), pb.execute(f), ctx.sync()), pb))
+        for k in (1, 4):
+            plan = dbp_plan(ctx, s, nspan, 16.0, steps_per_span=k, batch=batch, precision='f64', shift=shift, decim=r)
+            runs.append((dict(run='dbp', decim=r, steps_per_span=k), lambda f, plan=plan: (plan.execute(f), ctx.sync()),
+                         plan))
+    times = [[] for _ in runs]
+    for rep in range(reps + 1):                          # round 0 warms every plan up
+        for i, (_, fn, _) in enumerate(runs):
+            fld.broadcast_from(tx)
+            ctx.sync()
+            t0 = time.perf_counter()
+            fn(fld)
+            if rep:
+                times[i].append(time.perf_counter() - t0)
+    rows = []
+    for (info, _, plan), t in zip(runs, times):
+        plan.close()
+        row = dict(shape=name, nfft=N, batch=batch, nspan=nspan, shift=shift, ms_per_link=1e3 * float(np.median(t)),
+                   spread_ms=[1e3 * min(t), 1e3 * max(t)], **info)
+        rows.append(row)
+        what = ('CD + PB-NLC K=%-2d' % info['K']) if info['run'] == 'cd+pbnlc' else ('DBP %d step/span ' % info['steps_per_span'])
+        print('%s batch %2d r=%-2d (2^%d)  %s %9.2f ms per link  [%.2f .. %.2f]'
+              % (name, batch, info['decim'], (N // info['decim']).bit_length() - 1, what, row['ms_per_link'], *row['spread_ms']))
+    cd.close()
+    fld.close()
+    tx.close()
+    return rows
+
+
+def channel_main(a):
+    decims = [int(v) for v in a.decim.split(',')]
+    info = card()
+    print('card:', info)
+    rows = channel_shape('C4', 1 << 16, 64, a.nch, 20, 1, decims, a.reps)
+    rows += channel_shape('C2', 1 << 16, 16, 1, 10, 16, decims, a.reps)
+    print('card (after the runs):', card())
+    if a.out:
+        os.makedirs(a.out, exist_ok=True)
+        with open(os.path.join(a.out, 'pbnlc_channel_time.json'), 'w') as f:
+            json.dump(dict(card=info, runs=rows), f, indent=1)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--nsymb', type=int, default=1 << 16)
@@ -84,8 +171,12 @@ def main():
     ap.add_argument('--nspan', type=int, default=10)
     ap.add_argument('--reps', type=int, default=20)
     ap.add_argument('--ks', default='4,8,16,32,64')
-    ap.add_argument('--out', default=None, help='directory for pbnlc_time.json')
+    ap.add_argument('--decim', default=None, help='single-channel PB-NLC at these decimations (comma list) on C4 and C2')
+    ap.add_argument('--nch', type=int, default=9, help='channels of the C4 multiplex (with --decim)')
+    ap.add_argument('--out', default=None, help='directory for pbnlc_time.json (pbnlc_channel_time.json with --decim)')
     a = ap.parse_args()
+    if a.decim:
+        return channel_main(a)
     import torch
     torch.cuda.init()
     info = card()
