@@ -420,6 +420,47 @@ void pmx_pb_destroy(pmx_pb_plan* plan);
  * the returned plan; it owns the M-sample stage, the band filter and an M x batch work field. */
 int pmx_pb_channel_create(pmx_ctx* ctx, const pmx_pb_desc* desc, const pmx_dbp_band* band, pmx_pb_plan** plan);
 
+/* ---- the PB-NLC triplet table on the device: what polmux_b200/pbnlc.py, pb_coefficients, computes on the host ----------
+ * For a link of nspan spans of `length` [m], loss alphalin [1/m] and dispersion betat (per metre, FFT order, on the grid
+ * of nfft = nsymb*nt samples the stage runs on; for single-channel PB-NLC the channel's M samples, pbnlc.channel_setup):
+ *   window : W symbols; 0 takes the default rule: the pulse placed on nfft samples and dispersed over nspan*length, the
+ *            samples holding all but 1e-9 of its energy (centred, 0.5e-9 cut from either end), plus 2K+8 symbols, rounded
+ *            up to a power of two, at most nsymb.  W must divide nsymb; Ws = W*nt samples.  The rule is evaluated on the
+ *            device's transform and a sequential host sum where pbnlc.default_window uses numpy's FFT and pairwise sum:
+ *            when a 1e-9 energy boundary falls within rounding of a sample, or the count lands within rounding of a
+ *            power of two, the two may pick neighbouring windows (window_used tells which was taken).
+ *   nodes  : nquad Gauss-Legendre nodes (x, w) per span s: zeta = s*length + length/2*(x+1), weight length/2*w*exp(-alphalin*
+ *            length/2*(x+1))
+ *   pulses : g_q = ifft(fft(p0) .* exp(-i*bt*zeta_q)) on Ws samples, p0[(j - npulse/2) mod Ws] = pulse[j], bt[k] =
+ *            betat[k*nfft/Ws] (the link's bins on the window's grid)
+ *   rows   : R[m][n] = sum_q w_q sum_t b(t) conj(b(t - n*nt)) / sum p^2, b(t) = conj(g_q(t)) g_q(t - m*nt), indices mod Ws,
+ *            0 <= m, n <= K (R[m][-n] = conj(R[m][n]))
+ *   table  : C[m][n] = R[m][n] for m >= 0, conj(R[-m][n]) for m < 0, then C <- (C + C^T)/2 (exactly symmetric); the entries
+ *            with |C| >= prune*|C[0][0]| (every entry for prune = 0), m-major with n ascending, -K <= m, n <= K.
+ * The outputs hold (2K+1)^2 entries; coef is (re, im) interleaved, so (m, n, coef, ncoef) go into pmx_pb_desc as they are.
+ * window_used (may be NULL) receives W.  The lag sums run on the device in a fixed order without atomics: two calls give
+ * the same bits.  Checked before a context is needed: PMX_ERR_INVALID for nfft not a power of two from 2^6 to 2^24, nt < 1
+ * or not dividing nfft, a bad pulse (as pmx_pb_create), K outside 0..PMX_PB_MAX_K, nquad < 1, nspan < 1, more than 2^20
+ * nodes, a non-finite or non-positive length, a negative or non-finite alphalin, a NULL or non-finite betat, a non-finite
+ * prune, a window that is negative or does not divide nsymb, and NULL outputs; PMX_ERR_UNSUPPORTED for a window of fewer
+ * than 2^6 samples, given or by the default rule. */
+typedef struct pmx_pb_table_desc {
+    int64_t nfft;           /* samples of the grid the stage runs on                                                    */
+    int32_t nt;             /* samples per symbol                                                                       */
+    int32_t npulse;         /* pulse samples, as in pmx_pb_desc                                                         */
+    const double* betat;    /* [nfft] phase per metre, FFT order                                                         */
+    const double* pulse;    /* [npulse] real pulse table, as in pmx_pb_desc                                              */
+    int32_t nspan;          /* spans                                                                                    */
+    int32_t K;              /* |m|, |n| <= K, 0 .. PMX_PB_MAX_K                                                          */
+    double length;          /* span length [m]                                                                          */
+    double alphalin;        /* loss [1/m]                                                                               */
+    int32_t nquad;          /* Gauss-Legendre nodes per span                                                            */
+    int32_t window;         /* symbols of the window; 0: the default rule                                               */
+    double prune;           /* keep |C| >= prune*|C[0][0]|                                                              */
+} pmx_pb_table_desc;
+int pmx_pb_table(pmx_ctx* ctx, const pmx_pb_table_desc* desc, int32_t* m, int32_t* n, double* coef, int32_t* ncoef,
+                 int32_t* window_used);
+
 /* ---- create_field('unique'): the WDM multiplex on the device (create_field.m:113-149,180-199) ----------------
  * The reference builds the single field as
  *   FIELDX = ifft( sum_ch fastshift( fft(sigx(:,ch)), -ndfn(ch) ) ),   ndfn = round(deltafn/SYMBOLRATE/minfreq)

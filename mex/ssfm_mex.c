@@ -60,6 +60,20 @@
  *       band   [] or [shift decim]: single-channel DBP of the channel shift bins bring to baseband, on Nfft/decim samples
  *       taps   absent or [], or enhanced split-step DBP: the real FIR c(1..2K+1) on the intensity of every nonlinear step,
  *              c(K+1) at lag 0 (pmx_dbp_set_taps)
+ *   [ux,uy] = ssfm_mex('pbnlc', ux, uy, betat, scal, tbetat, L, W, pulse, band, opt)
+ *       perturbation-based nonlinearity compensation of a link (matlab/pbnlc.m; pmx_pb_table, pmx_pb_create /
+ *       pmx_pb_channel_create, pmx_pb_exec) on a one-column two-polarization FP64 field, in one call: the all-pass step
+ *       that undoes the dispersion of all spans (one linear step of nspan*Lf with betat negated, no loss; with scal the
+ *       library rebuilds it from the negated beta1, beta2, b30, dgdrms = 0), then the triplet table the library computes
+ *       and the stage; the field is released as for 'dbp'
+ *       betat  Nfft x 1 (the all-pass step in the vector dispersion mode); scal [] or as for 'fiber' (the scalar mode)
+ *       tbetat the dispersion the table is computed on: betat, or for single-channel PB-NLC the channel's Nfft/decim bins
+ *              less its phase and group delay (pbnlc.channel_setup)
+ *       L      [nspan Lf alphalin nt K nquad window prune]: nt samples per symbol on tbetat's grid, window 0 = the default
+ *       W      [a b c gamma xi scale]: model weights, gamma of the triplet sum (Manakov with the 8/9), fraction subtracted,
+ *              the factor s = (exp(alphalin*Lf/2)/sqrt(G))^nspan that brings the received field to launch scale
+ *       pulse  the real pulse table at tbetat's rate; band [] or [shift decim] (pmx_pb_channel_create)
+ *       opt    [precision resident gflag]: precision must be 0 (FP64), gflag 0 = no dispersion in the flag (no all-pass)
  *   ssfm_mex('reset')                    drops the resident field
  *   c = ssfm_mex('stats')                [uploads downloads resident_hits] since the MEX file was loaded
  *
@@ -778,6 +792,167 @@ static void cmd_dbp(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[])
     release(f, nfft, nfc, precision, !scalar_field, resident, nlhs, plhs);
 }
 
+static void cmd_pbnlc(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[])
+{
+    /* prhs: 'pbnlc', ux, uy, betat, scal, tbetat, L, W, pulse, band, opt */
+    pmx_fiber_desc d;
+    pmx_pb_table_desc td;
+    pmx_pb_desc pd;
+    pmx_dbp_band b;
+    pmx_plan *cd = NULL;
+    pmx_pb_plan *pb = NULL;
+    pmx_devfield *f;
+    double zero1 = 0.0, gam0 = 0.0, beta_buf[2];
+    const double *L, *W;
+    mxArray *nbt = NULL, *tab = NULL;
+    size_t nfft, k, cap;
+    int32_t ncoef = 0, win = 0, *tm, *tn;
+    double *coef;
+    int resident, rc, channel, K;
+    const mxArray *opt = prhs[10];
+
+    if (nrhs != 11 || nlhs > 2)
+        mexErrMsgTxt("[ux,uy] = ssfm_mex('pbnlc',ux,uy,betat,scal,tbetat,L,W,pulse,band,opt): wrong number of arguments.");
+    nfft = mxGetM(prhs[1]);
+    if (nfft == 0)
+        mexErrMsgTxt("ssfm_mex: empty x field.");
+    if (mxGetN(prhs[1]) != 1)
+        mexErrMsgTxt("pmx_pb_create: PB-NLC takes one-column fields");
+    if (mxGetM(prhs[2]) != nfft || mxGetN(prhs[2]) != 1)
+        mexErrMsgTxt("pmx_pb_create: PB-NLC takes two-polarization fields of one column (ux and uy the same size)");
+    if (opt_at(opt, 0, 0.0) != 0.0)
+        mexErrMsgTxt("pmx_pb_create: FP64 fields only");
+    if (mxGetNumberOfElements(prhs[6]) != 8)
+        mexErrMsgTxt("ssfm_mex: L must be [nspan Lf alphalin nt K nquad window prune].");
+    if (mxGetNumberOfElements(prhs[7]) != 6)
+        mexErrMsgTxt("ssfm_mex: W must be [a b c gamma xi scale].");
+    if (mxGetNumberOfElements(prhs[5]) == 0 || mxGetNumberOfElements(prhs[8]) == 0)
+        mexErrMsgTxt("ssfm_mex: tbetat and pulse must not be empty.");
+    resident = opt_at(opt, 1, 0.0) != 0.0;
+    L = mxGetPr(prhs[6]);
+    W = mxGetPr(prhs[7]);
+    if (!(L[0] >= 1.0))
+        mexErrMsgTxt("pbnlc: nspan must be >= 1");
+
+    /* the all-pass step: mc.cd_plan_of -- one linear step of the whole link, dispersion negated, no loss */
+    memset(&d, 0, sizeof d);
+    d.nfft = (int64_t)nfft;
+    d.nfc = 1;
+    d.batch = 1;
+    d.precision = PMX_F64;
+    d.length = d.dzmaxt = L[1] * L[0];
+    d.dphimaxt = INFINITY;
+    d.alphalin = 0.0;
+    d.gam = &gam0;
+    d.fls[0] = opt_at(opt, 2, 1.0) != 0.0;
+    d.nplates = d.plate_sets = 1;
+    d.db0 = d.theta = d.epsilon = &zero1;
+    if (mxGetNumberOfElements(prhs[4]) != 0) {
+        const double *sc = mxGetPr(prhs[4]);
+        if (mxGetNumberOfElements(prhs[4]) != 7)
+            mexErrMsgTxt("ssfm_mex: scal must be [symbolrate nsymb nt b30 dgdrms beta1 beta2].");
+        d.disp_mode = PMX_DISP_SCALAR;
+        d.symbolrate = sc[0];
+        d.nsymb = (int32_t)sc[1];
+        d.nt = (int32_t)sc[2];
+        d.b30 = -sc[3];
+        d.dgdrms = 0.0;
+        beta_buf[0] = -sc[5];
+        beta_buf[1] = -sc[6];
+        d.beta1 = beta_buf;
+        d.beta2 = beta_buf + 1;
+    } else {
+        if (mxGetM(prhs[3]) != nfft || mxGetN(prhs[3]) != 1)
+            mexErrMsgTxt("ssfm_mex: betat must be Nfft x 1.");
+        nbt = mxCreateDoubleMatrix(nfft, 1, mxREAL);
+        for (k = 0; k < nfft; k++)
+            mxGetPr(nbt)[k] = -mxGetPr(prhs[3])[k];
+        d.disp_mode = PMX_DISP_VECTOR;
+        d.betat = mxGetPr(nbt);
+    }
+
+    /* the table on the device */
+    memset(&td, 0, sizeof td);
+    td.nfft = (int64_t)mxGetNumberOfElements(prhs[5]);
+    td.nt = (int32_t)L[3];
+    td.betat = mxGetPr(prhs[5]);
+    td.npulse = (int32_t)mxGetNumberOfElements(prhs[8]);
+    td.pulse = mxGetPr(prhs[8]);
+    td.nspan = (int32_t)L[0];
+    td.length = L[1];
+    td.alphalin = L[2];
+    td.K = (int32_t)L[4];
+    td.nquad = (int32_t)L[5];
+    td.window = (int32_t)L[6];
+    td.prune = L[7];
+    K = td.K >= 0 && td.K <= PMX_PB_MAX_K ? td.K : 0;
+    cap = (size_t)(2 * K + 1) * (size_t)(2 * K + 1);
+    tab = mxCreateDoubleMatrix(4 * cap, 1, mxREAL);   /* coef [cap][2], then m and n as int32 */
+    coef = mxGetPr(tab);
+    tm = (int32_t *)(coef + 2 * cap);
+    tn = tm + cap;
+    channel = mxGetNumberOfElements(prhs[9]) != 0;
+    if (channel) {
+        if (mxGetNumberOfElements(prhs[9]) != 2)
+            mexErrMsgTxt("ssfm_mex: band must be [shift decim].");
+        memset(&b, 0, sizeof b);
+        b.shift = (int64_t)mxGetPr(prhs[9])[0];
+        b.decim = (int32_t)mxGetPr(prhs[9])[1];
+    }
+
+    ensure_ctx();
+    rc = pmx_pb_table(g_ctx, &td, tm, tn, coef, &ncoef, &win);
+    if (rc != PMX_OK) {
+        if (nbt)
+            mxDestroyArray(nbt);
+        mxDestroyArray(tab);
+        fail("ssfm_mex: PB-NLC table failed");
+    }
+    memset(&pd, 0, sizeof pd);
+    pd.nfft = td.nfft;
+    pd.nt = td.nt;
+    pd.nsymb = (int32_t)(td.nfft / td.nt);
+    pd.batch = 1;
+    pd.nfc = 1;
+    pd.precision = PMX_F64;
+    pd.npulse = td.npulse;
+    pd.pulse = td.pulse;
+    for (k = 0; k < 3; k++)
+        pd.weights[k] = W[k];
+    pd.gamma = W[3];
+    pd.xi = W[4];
+    pd.scale = W[5];
+    pd.ncoef = ncoef;
+    pd.m = tm;
+    pd.n = tn;
+    pd.coef = coef;
+    rc = channel ? pmx_pb_channel_create(g_ctx, &pd, &b, &pb) : pmx_pb_create(g_ctx, &pd, &pb);
+    mxDestroyArray(tab); /* the plan has taken the table */
+    if (rc != PMX_OK) {
+        if (nbt)
+            mxDestroyArray(nbt);
+        fail("ssfm_mex: PB-NLC plan creation failed");
+    }
+    rc = pmx_plan_create(g_ctx, &d, &cd);
+    if (nbt)
+        mxDestroyArray(nbt);
+    if (rc != PMX_OK) {
+        pmx_pb_destroy(pb);
+        fail("ssfm_mex: all-pass plan creation failed");
+    }
+    f = acquire(prhs[1], prhs[2], PMX_F64);
+    rc = pmx_fiber_exec(cd, f, NULL);
+    if (rc == PMX_OK)
+        rc = pmx_pb_exec(pb, f);
+    pmx_plan_destroy(cd);
+    pmx_pb_destroy(pb);
+    if (rc != PMX_OK) {
+        pmx_field_destroy(f);
+        fail("ssfm_mex: PB-NLC failed");
+    }
+    release(f, nfft, 1, PMX_F64, 1, resident, nlhs, plhs);
+}
+
 /* complex mxArray (split storage) -> interleaved re,im in a fresh mxArray-owned buffer of 2*n doubles */
 static double *interleave(const mxArray *a, size_t n, mxArray **owner)
 {
@@ -964,12 +1139,14 @@ static void command(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[])
         cmd_invpmd(nlhs, plhs, nrhs, prhs);
     } else if (!strcmp(cmd, "dbp")) {
         cmd_dbp(nlhs, plhs, nrhs, prhs);
+    } else if (!strcmp(cmd, "pbnlc")) {
+        cmd_pbnlc(nlhs, plhs, nrhs, prhs);
     } else if (!strcmp(cmd, "reset")) {
         drop_resident();
     } else if (!strcmp(cmd, "stats")) {
         plhs[0] = mxCreateDoubleMatrix(1, 3, mxREAL);
         memcpy(mxGetPr(plhs[0]), g_stats, sizeof g_stats);
     } else {
-        mexErrMsgTxt("ssfm_mex: unknown command (fiber, ampliflat, cohmix, invpmd, dbp, reset, stats).");
+        mexErrMsgTxt("ssfm_mex: unknown command (fiber, ampliflat, cohmix, invpmd, dbp, pbnlc, reset, stats).");
     }
 }

@@ -36,6 +36,7 @@ EXPORTS = [
     'pmx_cohmix_exec', 'pmx_field_mean_power_xy', 'pmx_cohmix_run', 'pmx_dsp_phases', 'pmx_field_quantize', 'pmx_inverse_pmd_run',
     'pmx_dbp_create', 'pmx_dbp_exec', 'pmx_dbp_set_plates', 'pmx_dbp_channel_create', 'pmx_dbp_set_filter',
     'pmx_dbp_set_taps', 'pmx_pb_create', 'pmx_pb_exec', 'pmx_pb_symbols', 'pmx_pb_destroy', 'pmx_pb_channel_create',
+    'pmx_pb_table',
 ]
 
 
@@ -94,6 +95,12 @@ class PbDesc(C.Structure):
                 ('precision', C.c_int32), ('npulse', C.c_int32), ('pulse', _dp), ('weights', C.c_double * 3),
                 ('gamma', C.c_double), ('xi', C.c_double), ('scale', C.c_double), ('ncoef', C.c_int32),
                 ('reserved', C.c_int32), ('m', _ip), ('n', _ip), ('coef', _dp)]
+
+
+class PbTableDesc(C.Structure):
+    _fields_ = [('nfft', C.c_int64), ('nt', C.c_int32), ('npulse', C.c_int32), ('betat', _dp), ('pulse', _dp),
+                ('nspan', C.c_int32), ('K', C.c_int32), ('length', C.c_double), ('alphalin', C.c_double),
+                ('nquad', C.c_int32), ('window', C.c_int32), ('prune', C.c_double)]
 
 
 class McReceiver(C.Structure):
@@ -202,6 +209,7 @@ def load():
     lib.pmx_pb_destroy.restype = None
     lib.pmx_dbp_channel_create.argtypes = [vp, C.POINTER(FiberDesc), C.POINTER(DbpDesc), C.POINTER(DbpBand), C.POINTER(vp)]
     lib.pmx_pb_channel_create.argtypes = [vp, C.POINTER(PbDesc), C.POINTER(DbpBand), C.POINTER(vp)]
+    lib.pmx_pb_table.argtypes = [vp, C.POINTER(PbTableDesc), _ip, _ip, _dp, _ip, _ip]
     _lib = lib
     return lib
 
@@ -654,6 +662,36 @@ def make_pb(nsymb, nt, batch, pulse, weights, gamma, xi, scale, m, n, coef):
     d.ncoef = keep['m'].size
     d.m, d.n, d.coef = keep['m'].ctypes.data_as(_ip), keep['n'].ctypes.data_as(_ip), _ptr(keep['coef'])
     return d, keep
+
+
+def make_pb_table(nfft, nt, betat, pulse, nspan, length, alphalin, K, nquad, window, prune):
+    """-> (PbTableDesc, keep-alive dict): the triplet table of pmx_pb_table; window None or 0 takes the default rule"""
+    keep = {'betat': _f64(np.asarray(betat, dtype=np.float64).ravel()),
+            'pulse': _f64(np.asarray(pulse, dtype=np.float64).ravel())}
+    d = PbTableDesc()
+    d.nfft, d.nt, d.npulse = int(nfft), int(nt), keep['pulse'].size
+    d.betat, d.pulse = _ptr(keep['betat']), _ptr(keep['pulse'])
+    d.nspan, d.K, d.length, d.alphalin = int(nspan), int(K), float(length), float(alphalin)
+    d.nquad, d.window, d.prune = int(nquad), int(window or 0), float(prune)
+    return d, keep
+
+
+def pb_table(ctx, desc_keep):
+    """pmx_pb_table: -> (m, n, C, window): int32 [ncoef], int32 [ncoef], complex128 [ncoef], the window in symbols.  ctx
+    None checks the descriptor only (the library refuses a bad one before it needs a context)."""
+    d, _ = desc_keep
+    cap = (2 * max(int(d.K), 0) + 1) ** 2
+    m = np.zeros(cap, dtype=np.int32)
+    n = np.zeros(cap, dtype=np.int32)
+    coef = np.zeros(cap, dtype=np.complex128)
+    cnt, win = C.c_int32(0), C.c_int32(0)
+    lib = load() if ctx is None else ctx.lib
+    rc = lib.pmx_pb_table(None if ctx is None else ctx.h, C.byref(d), m.ctypes.data_as(_ip), n.ctypes.data_as(_ip),
+                          coef.ctypes.data_as(_dp), C.byref(cnt), C.byref(win))
+    if rc != PMX_OK:
+        raise PolmuxError(rc, lib.pmx_last_error(None if ctx is None else ctx.h).decode())
+    k = cnt.value
+    return m[:k].copy(), n[:k].copy(), coef[:k].copy(), int(win.value)
 
 
 class PbPlan:

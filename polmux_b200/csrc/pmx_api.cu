@@ -1011,9 +1011,18 @@ __global__ void __launch_bounds__(256) pmx_k_permute_c(const double2* __restrict
     }
 }
 
-extern "C" int pmx_filter_create(pmx_ctx* c, int64_t nfft, int32_t nfc, int32_t batch, int32_t precision, const double* H,
-                                 int32_t hcols, pmx_plan** out) {
-    if (!c || !H || !out) return set_err(c, PMX_ERR_INVALID, "pmx_filter_create: null argument");
+// The filter plan of pmx_filter_create with H taken from `raw`, a [hcols][nfft] table in FFT order that is already on the
+// device (host_raw = 0) or on the host (host_raw = 1).  pmx_pb_table writes its per-node tables on the device and calls
+// filter_set_raw again for every chunk of nodes.
+static int filter_set_raw(pmx_plan* p, const double2* raw, int32_t hcols) {
+    pmx_k_permute_c<<<(unsigned)std::min<size_t>(((size_t)p->d.nfft * hcols + 255) / 256, 148 * 16), 256, 0,
+                      p->ctx->stream>>>(raw, p->hfilt, p->log2N1, p->log2N2, hcols);
+    p->ctx->launches++;
+    return cudaGetLastError() == cudaSuccess ? PMX_OK : PMX_ERR_CUDA;
+}
+
+static int filter_create(pmx_ctx* c, int64_t nfft, int32_t nfc, int32_t batch, int32_t precision, const double* H,
+                         int host_raw, int32_t hcols, pmx_plan** out) {
     *out = nullptr;
     if (nfc < 1 || (hcols != 1 && hcols != nfc))
         return set_err(c, PMX_ERR_INVALID, "pmx_filter_create: H must have one column, or one per field column");
@@ -1043,11 +1052,13 @@ extern "C" int pmx_filter_create(pmx_ctx* c, int64_t nfft, int32_t nfc, int32_t 
     const size_t n = (size_t)nfft * hcols;
     double2* raw = nullptr;
     cudaError_t e = cudaMallocAsync(&p->hfilt, n * sizeof(double2), c->stream);
-    if (e == cudaSuccess) e = cudaMallocAsync(&raw, n * sizeof(double2), c->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(raw, H, n * sizeof(double2), cudaMemcpyHostToDevice, c->stream);
+    if (host_raw) {
+        if (e == cudaSuccess) e = cudaMallocAsync(&raw, n * sizeof(double2), c->stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(raw, H, n * sizeof(double2), cudaMemcpyHostToDevice, c->stream);
+    }
     if (e == cudaSuccess) {
-        pmx_k_permute_c<<<(unsigned)std::min<size_t>((n + 255) / 256, 148 * 16), 256, 0, c->stream>>>(raw, p->hfilt, p->log2N1,
-                                                                                                   p->log2N2, hcols);
+        pmx_k_permute_c<<<(unsigned)std::min<size_t>((n + 255) / 256, 148 * 16), 256, 0, c->stream>>>(
+            host_raw ? raw : reinterpret_cast<const double2*>(H), p->hfilt, p->log2N1, p->log2N2, hcols);
         c->launches++;
         e = cudaGetLastError();
     }
@@ -1060,6 +1071,12 @@ extern "C" int pmx_filter_create(pmx_ctx* c, int64_t nfft, int32_t nfc, int32_t 
     p->hfilt_stride = hcols > 1 ? (long long)nfft : 0;
     *out = p;
     return PMX_OK;
+}
+
+extern "C" int pmx_filter_create(pmx_ctx* c, int64_t nfft, int32_t nfc, int32_t batch, int32_t precision, const double* H,
+                                 int32_t hcols, pmx_plan** out) {
+    if (!c || !H || !out) return set_err(c, PMX_ERR_INVALID, "pmx_filter_create: null argument");
+    return filter_create(c, nfft, nfc, batch, precision, H, 1, hcols, out);
 }
 
 // ---------------------------------------------------------------------------
@@ -4502,5 +4519,408 @@ extern "C" int pmx_pb_channel_create(pmx_ctx* c, const pmx_pb_desc* d, const pmx
         return rc;
     }
     *out = p;
+    return PMX_OK;
+}
+
+// ---------------------------------------------------------------------------
+// The PB-NLC triplet table on the device (pmx_pb_table, see the header).  The dispersed pulses g_q of a chunk of nodes are
+// one filter plan of Ws samples with a column per node (H = exp(-i*bt*zeta_q), written on the device); the lag sums
+// R[m][n] = sum_q w_q sum_t b(t) conj(b(t - n*nt)), b(t) = conj(g_q(t)) g_q(t - m*nt), are taken directly.  A CTA of
+// pmx_k_pb_lagsum owns one (node, m) and a group of tiles of the window: per step it lands b for RC phases r and TJ + K
+// symbols j (t = j*nt + r, K symbols of halo before the tile) in shared memory, phase-major, so that the threads of the lags
+// n, n+1, ... of one phase read consecutive samples b_r[j - n] and share b_r[j] as a broadcast.  A thread owns up to
+// PMX_PBT_IT (phase, lag) items; the phases are summed in shared memory and the tile groups and nodes by
+// pmx_k_pb_lagreduce, every sum in a fixed order without atomics.  The rows n < 0 are conj(R[m][-n]) (the correlation of a
+// circular sequence), so only 0 <= n <= K are summed.
+#define PMX_PBT_THREADS 256
+#define PMX_PBT_IT 4          // (phase, lag) items per thread: RC*(K+1) <= PMX_PBT_THREADS*PMX_PBT_IT
+#define PMX_PBT_SAMPLES 1024  // samples of b per step: RC phases x TJ symbols
+#define PMX_PBT_GROUPS 4      // tile groups of a window, each a CTA of its own
+
+// the real pulse p0 (time order) into the x polarization of every column of a resident field; y = 0
+__global__ void __launch_bounds__(256) pmx_k_pb_fill(cpx* __restrict__ field, int lg, int l1, int l2, int ncol,
+                                                     const double* __restrict__ p0) {
+    const size_t N = (size_t)1 << lg, total = N * ncol;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const size_t col = i >> lg, t = i & (N - 1);
+        st_sa(field + 2 * (col * N + pmx_mem_index(t, l1, l2)), make_double2(p0[t], 0.0), make_double2(0.0, 0.0));
+    }
+}
+
+// raw[col][k] = exp(-i*bt[k]*zeta[col]) = (cos, -sin) of the product, FFT order, as pbnlc._lin_step forms it
+__global__ void __launch_bounds__(256) pmx_k_pb_disp(double2* __restrict__ raw, const double* __restrict__ bt, int lg,
+                                                     const double* __restrict__ zeta, int ncol) {
+    const size_t N = (size_t)1 << lg, total = N * ncol;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        double s, c;
+        sincos(bt[i & (N - 1)] * zeta[i >> lg], &s, &c);
+        raw[i] = make_double2(c, -s);
+    }
+}
+
+// e[i] = |x[(i + N/2) mod N]|^2 of column 0: the energy of the pulse in fftshift order (the default window's rule)
+__global__ void __launch_bounds__(256) pmx_k_pb_energy(const cpx* __restrict__ field, int lg, int l1, int l2,
+                                                       double* __restrict__ e) {
+    const size_t N = (size_t)1 << lg;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (size_t)gridDim.x * blockDim.x) {
+        const cpx x = field[2 * pmx_mem_index((i + N / 2) & (N - 1), l1, l2)];
+        e[i] = x.x * x.x + x.y * x.y;
+    }
+}
+
+// part[q][m][group][n] = sum over the group's tiles and every phase of b(t) conj(b(t - n*nt)) for node q (the column q of
+// field), 0 <= n <= K; grid (groups, K+1, nodes)
+__global__ void __launch_bounds__(PMX_PBT_THREADS) pmx_k_pb_lagsum(const cpx* __restrict__ field, int lg, int l1, int l2,
+                                                                   int nt, int K, int RC, int TJ, int tiles_per_group,
+                                                                   cpx* __restrict__ part) {
+    extern __shared__ __align__(16) unsigned char smp[];
+    cpx* sb = reinterpret_cast<cpx*>(smp);   // [RC][TJ + K]: b at symbol J0 - K + jj, phase r0 + rr
+    const size_t N = (size_t)1 << lg;
+    const int q = blockIdx.z, m = blockIdx.y, grp = blockIdx.x;
+    const int K1 = K + 1, row = TJ + K, items = RC * K1, nu = (items + PMX_PBT_THREADS - 1) / PMX_PBT_THREADS;
+    const cpx* g = field + (size_t)q * N * 2;
+    const long long shift = (long long)m * nt;
+    int off[PMX_PBT_IT], lag[PMX_PBT_IT];
+    double2 acc[PMX_PBT_IT];
+#pragma unroll
+    for (int u = 0; u < PMX_PBT_IT; ++u) {
+        const int it = threadIdx.x + u * PMX_PBT_THREADS;
+        const int rr = it < items ? it / K1 : 0;
+        lag[u] = it < items ? it - rr * K1 : 0;
+        off[u] = rr * row;
+        acc[u] = make_double2(0.0, 0.0);
+    }
+    for (int tile = 0; tile < tiles_per_group; ++tile) {
+        const long long J0 = (long long)(grp * tiles_per_group + tile) * TJ;
+        for (int r0 = 0; r0 < nt; r0 += RC) {
+            __syncthreads();   // the previous step's reads are done
+            for (int i = threadIdx.x; i < RC * row; i += PMX_PBT_THREADS) {
+                const int jj = i / RC, rr = i - jj * RC;
+                const long long t = (J0 - K + jj) * nt + r0 + rr;
+                const cpx a = g[2 * pmx_mem_index((size_t)t & (N - 1), l1, l2)];
+                const cpx b = g[2 * pmx_mem_index((size_t)(t - shift) & (N - 1), l1, l2)];
+                sb[rr * row + jj] = pb_mul_conj(b, a);   // conj(g(t)) g(t - m*nt)
+            }
+            __syncthreads();
+            for (int jj = K; jj < row; ++jj) {
+#pragma unroll
+                for (int u = 0; u < PMX_PBT_IT; ++u)
+                    if (u < nu) acc[u] = pb_mac_conj(acc[u], sb[off[u] + jj], sb[off[u] + jj - lag[u]]);
+            }
+        }
+    }
+    __syncthreads();
+#pragma unroll
+    for (int u = 0; u < PMX_PBT_IT; ++u) {
+        const int it = threadIdx.x + u * PMX_PBT_THREADS;
+        if (it < items) sb[it] = acc[u];   // [rr][n]: items <= RC*row
+    }
+    __syncthreads();
+    for (int n = threadIdx.x; n < K1; n += PMX_PBT_THREADS) {
+        double2 s = make_double2(0.0, 0.0);
+        for (int rr = 0; rr < RC; ++rr) s = make_double2(s.x + sb[rr * K1 + n].x, s.y + sb[rr * K1 + n].y);
+        part[(((size_t)q * K1 + m) * gridDim.x + grp) * K1 + n] = s;
+    }
+}
+
+// R[m][n] (+)= sum_q w[q] * sum_group part[q][m][group][n], nodes ascending; first = 1 starts from zero
+__global__ void __launch_bounds__(256) pmx_k_pb_lagreduce(const cpx* __restrict__ part, int nq, int K1, int ngrp,
+                                                          const double* __restrict__ w, cpx* __restrict__ R, int first) {
+    const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= K1 * K1) return;
+    const int m = idx / K1, n = idx - m * K1;
+    double2 acc = first ? make_double2(0.0, 0.0) : R[idx];
+    for (int q = 0; q < nq; ++q) {
+        double2 s = make_double2(0.0, 0.0);
+        for (int gi = 0; gi < ngrp; ++gi) {
+            const cpx v = part[(((size_t)q * K1 + m) * ngrp + gi) * K1 + n];
+            s = make_double2(s.x + v.x, s.y + v.y);
+        }
+        acc = make_double2(fma(w[q], s.x, acc.x), fma(w[q], s.y, acc.y));
+    }
+    R[idx] = acc;
+}
+
+// Gauss-Legendre nodes and weights on [-1, 1], ascending (Newton on P_n from the usual first guesses; the odd order's
+// middle node exactly 0)
+static void gauss_legendre(int nq, std::vector<double>& x, std::vector<double>& w) {
+    x.assign(nq, 0.0);
+    w.assign(nq, 0.0);
+    auto legendre = [nq](double z, double& pp) {   // P_n(z), and P_n'(z) into pp
+        double p1 = 1.0, p2 = 0.0;
+        for (int j = 1; j <= nq; ++j) {
+            const double p3 = p2;
+            p2 = p1;
+            p1 = ((2.0 * j - 1.0) * z * p2 - (j - 1.0) * p3) / j;
+        }
+        pp = nq * (z * p1 - p2) / (z * z - 1.0);
+        return p1;
+    };
+    for (int i = 0; i < (nq + 1) / 2; ++i) {
+        double z = std::cos(M_PI * (i + 0.75) / (nq + 0.5)), pp = 0.0;
+        if (2 * i + 1 == nq) z = 0.0;
+        for (int it = 0; it < 100; ++it) {
+            const double dz = legendre(z, pp) / pp;
+            z -= dz;
+            if (std::fabs(dz) <= 1e-16) break;
+        }
+        legendre(z, pp);
+        const double wi = 2.0 / ((1.0 - z * z) * pp * pp);
+        x[i] = -z;
+        x[nq - 1 - i] = z;
+        w[i] = w[nq - 1 - i] = wi;
+    }
+}
+
+static int pb_table_check(pmx_ctx* c, const pmx_pb_table_desc* d) {
+    const int lg = ilog2_exact(d->nfft);
+    if (lg < 6 || lg > 24)
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_table: nfft=%lld, built for powers of two from 2^6 to 2^24",
+                       (long long)d->nfft);
+    if (d->nt < 1 || d->nfft % d->nt)
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_table: nt=%d must divide nfft = %lld (nsymb*nt = nfft)", d->nt,
+                       (long long)d->nfft);
+    if (!d->pulse || d->npulse < 2 || d->npulse % 2 || d->npulse > 16 * d->nt || d->npulse > d->nfft)
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_table: npulse=%d, the pulse must have an even count of 2 to min(16*nt, "
+                       "nfft) = %lld samples", d->npulse, (long long)std::min<int64_t>(16 * (int64_t)d->nt, d->nfft));
+    double e = 0;
+    for (int j = 0; j < d->npulse; ++j) {
+        if (!std::isfinite(d->pulse[j])) return set_err(c, PMX_ERR_INVALID, "pmx_pb_table: pulse sample %d is not finite", j);
+        e += d->pulse[j] * d->pulse[j];
+    }
+    if (!(e > 0) || !std::isfinite(e)) return set_err(c, PMX_ERR_INVALID, "pmx_pb_table: the pulse has no energy");
+    if (d->K < 0 || d->K > PMX_PB_MAX_K)
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_table: K=%d, |m| and |n| at most %d", d->K, PMX_PB_MAX_K);
+    if (d->nquad < 1) return set_err(c, PMX_ERR_INVALID, "pmx_pb_table: nquad=%d, at least one node per span", d->nquad);
+    if (d->nspan < 1) return set_err(c, PMX_ERR_INVALID, "pmx_pb_table: nspan=%d, at least one span", d->nspan);
+    if ((int64_t)d->nspan * d->nquad > (1 << 20))
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_table: nspan*nquad = %d x %d nodes, at most 2^20", d->nspan, d->nquad);
+    if (!std::isfinite(d->length) || !(d->length > 0))
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_table: the span length must be finite and positive");
+    if (!std::isfinite(d->alphalin) || d->alphalin < 0)
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_table: alphalin must be finite and non-negative");
+    if (!std::isfinite(d->prune)) return set_err(c, PMX_ERR_INVALID, "pmx_pb_table: prune must be finite");
+    if (!d->betat) return set_err(c, PMX_ERR_INVALID, "pmx_pb_table: null betat");
+    for (int64_t k = 0; k < d->nfft; ++k)
+        if (!std::isfinite(d->betat[k]))
+            return set_err(c, PMX_ERR_INVALID, "pmx_pb_table: betat[%lld] is not finite", (long long)k);
+    const int64_t nsymb = d->nfft / d->nt;
+    if (d->window < 0 || (d->window > 0 && nsymb % d->window))
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_table: the window (%d symbols) must divide the block (%lld symbols)",
+                       d->window, (long long)nsymb);
+    if (d->window > 0 && (int64_t)d->window * d->nt < 64)
+        return set_err(c, PMX_ERR_UNSUPPORTED, "pmx_pb_table: a window of %lld samples, at least 2^6 are needed",
+                       (long long)d->window * d->nt);
+    return PMX_OK;
+}
+
+// Disperses p0 (time order, Ws = 2^lg samples) by exp(-i*bt*zeta) for each of the ncol zeta into the columns of f with the
+// filter plan fp (created on the first call: *fp == nullptr); raw: [ncol][Ws] device scratch.
+static int pb_disperse(pmx_ctx* c, int lg, int ncol, const double* d_bt, const double* d_zeta, const double* d_p0,
+                       double2* raw, pmx_devfield* f, pmx_plan** fp) {
+    const size_t total = ((size_t)1 << lg) * ncol;
+    const unsigned grid = (unsigned)std::min<size_t>((total + 255) / 256, 148 * 16);
+    pmx_k_pb_disp<<<grid, 256, 0, c->stream>>>(raw, d_bt, lg, d_zeta, ncol);
+    pmx_k_pb_fill<<<grid, 256, 0, c->stream>>>(f->data, lg, f->log2N1, f->log2N2, ncol, d_p0);
+    c->launches += 2;
+    CK(c, cudaGetLastError());
+    int rc = PMX_OK;
+    if (!*fp) rc = filter_create(c, (int64_t)1 << lg, ncol, 1, PMX_F64, reinterpret_cast<const double*>(raw), 0, ncol, fp);
+    else if (filter_set_raw(*fp, raw, ncol)) rc = set_err(c, PMX_ERR_CUDA, "pmx_pb_table: the filter table launch failed");
+    if (!rc) rc = pmx_fiber_exec(*fp, f, nullptr);
+    return rc;
+}
+
+// device buffers of one pmx_pb_table call, released whatever happens
+struct PbTableScratch {
+    pmx_ctx* c;
+    std::vector<void*> bufs;
+    pmx_devfield* f = nullptr;
+    pmx_plan* fp = nullptr;
+    explicit PbTableScratch(pmx_ctx* ctx) : c(ctx) {}
+    template <typename T>
+    cudaError_t alloc(T** p, size_t count) {
+        *p = nullptr;
+        cudaError_t e = cudaMallocAsync(p, std::max<size_t>(count, 1) * sizeof(T), c->stream);
+        if (e == cudaSuccess) bufs.push_back(*p);
+        return e;
+    }
+    void release_field() {
+        pmx_plan_destroy(fp);
+        pmx_field_destroy(f);
+        fp = nullptr;
+        f = nullptr;
+    }
+    ~PbTableScratch() {
+        release_field();
+        for (void* p : bufs) cudaFreeAsync(p, c->stream);
+        cudaStreamSynchronize(c->stream);
+    }
+};
+
+#define PBT_CK(call)                                                                                     \
+    do {                                                                                                 \
+        cudaError_t e__ = (call);                                                                        \
+        if (e__ != cudaSuccess) return set_err(c, PMX_ERR_CUDA, "pmx_pb_table: %s", cudaGetErrorString(e__)); \
+    } while (0)
+
+// the default window (pbnlc.default_window): the pulse on nfft samples dispersed over nspan*length on the device, its
+// energy in fftshift order on the host
+static int pb_default_window(pmx_ctx* c, const pmx_pb_table_desc* d, int* W) {
+    const int lg = ilog2_exact(d->nfft);
+    const size_t N = (size_t)d->nfft;
+    const int64_t nsymb = d->nfft / d->nt;
+    std::vector<double> p0(N, 0.0);
+    for (int j = 0; j < d->npulse; ++j) p0[(size_t)((j - d->npulse / 2) % (int64_t)N + (int64_t)N) % N] = d->pulse[j];
+    const double zeta = d->length * d->nspan;
+    PbTableScratch s(c);
+    double *d_bt = nullptr, *d_zeta = nullptr, *d_p0 = nullptr, *d_e = nullptr;
+    double2* raw = nullptr;
+    PBT_CK(s.alloc(&d_bt, N));
+    PBT_CK(s.alloc(&d_zeta, 1));
+    PBT_CK(s.alloc(&d_p0, N));
+    PBT_CK(s.alloc(&d_e, N));
+    PBT_CK(s.alloc(&raw, N));
+    PBT_CK(cudaMemcpyAsync(d_bt, d->betat, N * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    PBT_CK(cudaMemcpyAsync(d_zeta, &zeta, sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    PBT_CK(cudaMemcpyAsync(d_p0, p0.data(), N * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    int rc = pmx_field_create(c, d->nfft, 1, 1, PMX_F64, &s.f);
+    if (!rc) rc = pb_disperse(c, lg, 1, d_bt, d_zeta, d_p0, raw, s.f, &s.fp);
+    if (rc) return rc;
+    pmx_k_pb_energy<<<(unsigned)std::min<size_t>((N + 255) / 256, 148 * 16), 256, 0, c->stream>>>(s.f->data, lg, s.f->log2N1,
+                                                                                                s.f->log2N2, d_e);
+    c->launches++;
+    PBT_CK(cudaGetLastError());
+    std::vector<double> e(N);
+    PBT_CK(cudaMemcpyAsync(e.data(), d_e, N * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    PBT_CK(cudaStreamSynchronize(c->stream));
+    double tot = 0;
+    for (double v : e) tot += v;
+    const double tol = 1e-9, vlo = 0.5 * tol, vhi = 1 - 0.5 * tol;
+    size_t lo = N, hi = N;
+    double cum = 0;
+    for (size_t i = 0; i < N; ++i) {   // searchsorted(c, v): the first i with c[i] >= v
+        cum += e[i];
+        const double ci = cum / tot;
+        if (lo == N && ci >= vlo) lo = i;
+        if (hi == N && ci >= vhi) {
+            hi = i;
+            break;
+        }
+    }
+    const double need = (double)(hi - lo + 1) / d->nt + 2 * d->K + 8;
+    int64_t w = 1;
+    while (w < need) w *= 2;
+    *W = (int)std::min<int64_t>(w, nsymb);
+    return PMX_OK;
+}
+
+extern "C" int pmx_pb_table(pmx_ctx* c, const pmx_pb_table_desc* d, int32_t* m_out, int32_t* n_out, double* coef_out,
+                            int32_t* ncoef, int32_t* window_used) {
+    // (the descriptor is checked before the context, so that the checks run without a device)
+    if (!d || !m_out || !n_out || !coef_out || !ncoef) return set_err(c, PMX_ERR_INVALID, "pmx_pb_table: null argument");
+    if (int rc = pb_table_check(c, d)) return rc;
+    if (!c) return set_err(c, PMX_ERR_INVALID, "pmx_pb_table: null ctx");
+    CK(c, cudaSetDevice(c->device));
+    const int K = d->K, K1 = K + 1, nt = d->nt;
+    int W = d->window;
+    if (W == 0) {
+        if (int rc = pb_default_window(c, d, &W)) return rc;
+        if ((int64_t)W * nt < 64)
+            return set_err(c, PMX_ERR_UNSUPPORTED, "pmx_pb_table: a window of %lld samples, at least 2^6 are needed",
+                           (long long)W * nt);
+    }
+    const int64_t Ws = (int64_t)W * nt;
+    const int lg = ilog2_exact(Ws);
+    // the nodes, the window's bins and pulse
+    std::vector<double> gx, gw;
+    gauss_legendre(d->nquad, gx, gw);
+    const int nq = d->nspan * d->nquad;
+    const int chunk = std::min(nq, Ws >= 4096 ? 64 : 8);   // columns per filter plan (on-chip kernels below 2^12: 8)
+    const int nchunk = (nq + chunk - 1) / chunk;
+    std::vector<double> zeta((size_t)nchunk * chunk), wq(nq), bt(Ws), p0(Ws, 0.0);
+    for (int s = 0; s < d->nspan; ++s)
+        for (int i = 0; i < d->nquad; ++i) {
+            const double z = 0.5 * d->length * (gx[i] + 1.0);
+            zeta[(size_t)s * d->nquad + i] = s * d->length + z;
+            wq[(size_t)s * d->nquad + i] = 0.5 * d->length * gw[i] * std::exp(-d->alphalin * z);
+        }
+    for (size_t i = nq; i < zeta.size(); ++i) zeta[i] = zeta[nq - 1];   // the last chunk's spare columns (not summed)
+    const int64_t stride = d->nfft / Ws;
+    for (int64_t k = 0; k < Ws; ++k) bt[k] = d->betat[k * stride];
+    for (int j = 0; j < d->npulse; ++j) p0[(size_t)(((j - d->npulse / 2) % Ws + Ws) % Ws)] = d->pulse[j];
+    double norm = 0;
+    for (int j = 0; j < d->npulse; ++j) norm += d->pulse[j] * d->pulse[j];
+    // the lag-sum geometry: RC phases x TJ symbols per step, groups of tiles
+    int RC = 1;
+    while (RC * 2 <= nt && RC * 2 * K1 <= PMX_PBT_THREADS * PMX_PBT_IT) RC *= 2;
+    const int TJ = (int)std::min<int64_t>(W, std::max(1, PMX_PBT_SAMPLES / RC));
+    const int tiles = W / TJ, ngrp = std::min(tiles, PMX_PBT_GROUPS), tpg = tiles / ngrp;
+    const int smem = RC * (TJ + K) * (int)sizeof(cpx);
+    if (smem > 48 * 1024) CK(c, cudaFuncSetAttribute(pmx_k_pb_lagsum, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    std::vector<double2> R((size_t)K1 * K1);
+    {
+        PbTableScratch s(c);
+        double *d_bt = nullptr, *d_zeta = nullptr, *d_w = nullptr, *d_p0 = nullptr;
+        double2 *raw = nullptr, *part = nullptr, *d_R = nullptr;
+        PBT_CK(s.alloc(&d_bt, Ws));
+        PBT_CK(s.alloc(&d_zeta, zeta.size()));
+        PBT_CK(s.alloc(&d_w, nq));
+        PBT_CK(s.alloc(&d_p0, Ws));
+        PBT_CK(s.alloc(&raw, (size_t)Ws * chunk));
+        PBT_CK(s.alloc(&part, (size_t)chunk * K1 * ngrp * K1));
+        PBT_CK(s.alloc(&d_R, (size_t)K1 * K1));
+        PBT_CK(cudaMemcpyAsync(d_bt, bt.data(), Ws * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+        PBT_CK(cudaMemcpyAsync(d_zeta, zeta.data(), zeta.size() * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+        PBT_CK(cudaMemcpyAsync(d_w, wq.data(), nq * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+        PBT_CK(cudaMemcpyAsync(d_p0, p0.data(), Ws * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+        int rc = pmx_field_create(c, Ws, chunk, 1, PMX_F64, &s.f);
+        if (rc) return rc;
+        for (int ch = 0; ch < nchunk; ++ch) {
+            const int q0 = ch * chunk, nc = std::min(chunk, nq - q0);
+            rc = pb_disperse(c, lg, chunk, d_bt, d_zeta + q0, d_p0, raw, s.f, &s.fp);
+            if (rc) return rc;
+            pmx_k_pb_lagsum<<<dim3((unsigned)ngrp, (unsigned)K1, (unsigned)nc), PMX_PBT_THREADS, smem, c->stream>>>(
+                s.f->data, lg, s.f->log2N1, s.f->log2N2, nt, K, RC, TJ, tpg, part);
+            pmx_k_pb_lagreduce<<<(unsigned)((K1 * K1 + 255) / 256), 256, 0, c->stream>>>(part, nc, K1, ngrp, d_w + q0, d_R,
+                                                                                       ch == 0);
+            c->launches += 2;
+            PBT_CK(cudaGetLastError());
+        }
+        PBT_CK(cudaMemcpyAsync(R.data(), d_R, R.size() * sizeof(double2), cudaMemcpyDeviceToHost, c->stream));
+        PBT_CK(cudaStreamSynchronize(c->stream));
+    }
+    // the table: rows m >= 0 from R (lags n < 0 conjugate), rows m < 0 conjugate, then exactly symmetric, pruned
+    const int D = 2 * K + 1;
+    std::vector<double2> C((size_t)D * D);
+    auto row = [&](int m, int n) {   // R[m][n] / sum p^2 for m >= 0, any |n| <= K
+        const double2 v = R[(size_t)m * K1 + std::abs(n)];
+        return make_double2(v.x / norm, n < 0 ? -v.y / norm : v.y / norm);
+    };
+    for (int m = -K; m <= K; ++m)
+        for (int n = -K; n <= K; ++n) {
+            const double2 v = row(std::abs(m), n);
+            C[(size_t)(m + K) * D + (n + K)] = m < 0 ? make_double2(v.x, -v.y) : v;
+        }
+    std::vector<double2> S(C.size());
+    for (int i = 0; i < D; ++i)
+        for (int j = 0; j < D; ++j) {
+            const double2 a = C[(size_t)i * D + j], b = C[(size_t)j * D + i];
+            S[(size_t)i * D + j] = make_double2(0.5 * (a.x + b.x), 0.5 * (a.y + b.y));
+        }
+    const double thr = d->prune * std::hypot(S[(size_t)K * D + K].x, S[(size_t)K * D + K].y);
+    int cnt = 0;
+    for (int i = 0; i < D; ++i)
+        for (int j = 0; j < D; ++j) {
+            const double2 v = S[(size_t)i * D + j];
+            if (d->prune != 0 && !(std::hypot(v.x, v.y) >= thr)) continue;
+            m_out[cnt] = i - K;
+            n_out[cnt] = j - K;
+            coef_out[2 * cnt] = v.x;
+            coef_out[2 * cnt + 1] = v.y;
+            ++cnt;
+        }
+    *ncoef = cnt;
+    if (window_used) *window_used = W;
     return PMX_OK;
 }

@@ -229,10 +229,11 @@ class McRunner:
         on nfft/decim samples -- of channel `ich` for 'cohmix', of the channel at the centre of the grid for 'blind'.
         dbp_params with 'filter_bw' [GHz]: filtered DBP (dbp_plan); with 'nl_taps': enhanced split-step DBP (dbp_plan).
         'pbnlc' ('blind' and 'cohmix', one channel in a one-column field): the all-pass step, then perturbation-based
-        nonlinearity compensation (polmux_b200/pbnlc.py, pb_plan) with pb_params (xi, K, prune, pulse, nquad, window;
-        default xi = 1, K = 16) at the launch scale s of the link's loss and gain.  pb_params with 'decim' (a power of two
-        >= 2 dividing nt; a one-column 'unique' field of any number of channels): single-channel PB-NLC on nfft/decim
-        samples -- of channel `ich` for 'cohmix', of the channel at the centre of the grid for 'blind'."""
+        nonlinearity compensation (polmux_b200/pbnlc.py, pb_plan) with pb_params (xi, K, prune, pulse, nquad, window, table;
+        default xi = 1, K = 16, table 'host': numpy; 'device': pmx_pb_table) at the launch scale s of the link's loss and
+        gain.  pb_params with 'decim' (a power of two >= 2 dividing nt; a one-column 'unique' field of any number of
+        channels): single-channel PB-NLC on nfft/decim samples -- of channel `ich` for 'cohmix', of the channel at the
+        centre of the grid for 'blind'."""
         import torch
         from . import dsp as _dsp
         self.receiver, self.dsp_params = receiver, dict(dsp_params or {})

@@ -12,8 +12,9 @@ the field projected onto the pulse of symbol k (centred at time index k*nt, circ
 those of the library's nonlinear step: Manakov (1, 1, 0) with gam carrying the 8/9, the CNLSE (1, 2/3, 1/3) -- the
 first-order expansion of -j*gam*[P*u + (s3/3)*J*u] (fiber.m:827-851).
 
-The coefficient table C[m,n] of the whole link (pb_coefficients) is computed once on the host; the stage itself runs on the
-device in one pass at the symbol rate (pmx_pb_create / pmx_pb_exec, include/polmux_ssfm.h).  There is no CPU fallback.
+The coefficient table C[m,n] of the whole link (pb_coefficients) is computed once, on the host (numpy, the reference) or,
+with table='device', by the library (pmx_pb_table: the same table, the lag sums on the device); the stage itself runs on
+the device in one pass at the symbol rate (pmx_pb_create / pmx_pb_exec, include/polmux_ssfm.h).  There is no CPU fallback.
 
 Single-channel PB-NLC (pbnlc(..., ich=, decim=), pb_plan(..., shift=, decim=); pmx_pb_channel_create): a coherent receiver
 sees its own channel only.  As single-channel DBP does it, channel ich of a 'unique' multiplex is cut out by an ideal
@@ -79,7 +80,7 @@ def default_window(setup: FiberSetup, nspan: int, pulse, nt: int, K: int, tol: f
 
 
 def pb_coefficients(setup: FiberSetup, nspan: int, pulse=None, K: int = 16, prune: float = 0.0, nt: Optional[int] = None,
-                    nquad: int = 32, window: Optional[int] = None):
+                    nquad: int = 32, window: Optional[int] = None, ctx: Optional[_lib.Context] = None):
     """The triplet coefficients of nspan spans of the fiber `setup` describes:
         C[m,n] = sum_s int_0^Ls exp(-alpha*z) <g_0, g_m g_n conj(g_{m+n})>(s*Ls + z) dz,   |m|, |n| <= K,
     g_m(zeta) the pulse of symbol m (centred at m*nt) after lin_step(betat*zeta) (no loss), <u, v> = sum conj(u) v / sum p^2.
@@ -89,12 +90,15 @@ def pb_coefficients(setup: FiberSetup, nspan: int, pulse=None, K: int = 16, prun
     By translation invariance the row m is the autocorrelation of a_m = conj(g_0) g_m at symbol-spaced lags,
     C[m,n] = sum_t a_m(t) conj(a_m(t - n*nt)): one FFT per row and node.  Only the rows m >= 0 are transformed: the
     autocorrelation gives C[m,-n] = conj(C[m,n]), and with C[m,n] = C[n,m], C[-m,n] = conj(C[m,n]).
+    ctx: the library computes the same table on that context's device (pmx_pb_table), orders of magnitude faster.
     -> (m, n, C): int32 [ncoef], int32 [ncoef], complex128 [ncoef], m-major with n ascending."""
     nt = int(nt or GSTATE.NT)
     K = int(K)
     if K < 0:
         raise ValueError('pb_coefficients: K must be >= 0')
     p = np.asarray(synth.cosroll_pulse(nt, 0.2) if pulse is None else pulse, dtype=np.float64).ravel()
+    if ctx is not None:
+        return pb_table(ctx, setup, nspan, p, K, prune, nt, nquad, window)[:3]
     N = int(setup.nfft)
     nsymb = N // nt
     W = int(window or default_window(setup, nspan, p, nt, K))
@@ -121,6 +125,28 @@ def pb_coefficients(setup: FiberSetup, nspan: int, pulse=None, K: int = 16, prun
     mm, nn = np.meshgrid(lags, lags, indexing='ij')
     keep = np.abs(C) >= float(prune) * abs(C[K, K]) if prune else np.ones(C.shape, dtype=bool)
     return mm[keep].astype(np.int32), nn[keep].astype(np.int32), C[keep]
+
+
+def pb_table(ctx: Optional[_lib.Context], setup: FiberSetup, nspan: int, pulse, K: int = 16, prune: float = 0.0,
+             nt: Optional[int] = None, nquad: int = 32, window: Optional[int] = None):
+    """pb_coefficients computed by the library (pmx_pb_table) -> (m, n, C, window): the table and the window it used, in
+    symbols (default_window's for window None).  ctx None only checks the arguments, as the library does before it needs a
+    device.  A bad argument raises ValueError with the library's message, as the host path raises ValueError for its own."""
+    nt = int(nt or GSTATE.NT)
+    bt = np.asarray(setup.betat, dtype=np.float64)[:, 0] if np.ndim(setup.betat) == 2 else setup.betat
+    try:
+        return _lib.pb_table(ctx, _lib.make_pb_table(setup.nfft, nt, bt, pulse, nspan, setup.length, setup.alphalin, K,
+                                                     nquad, window, prune))
+    except _lib.PolmuxError as e:
+        if e.code == _lib.PMX_ERR_INVALID:
+            raise ValueError(str(e)) from e
+        raise
+
+
+def _check_table(table: str) -> str:
+    if table not in ('host', 'device'):
+        raise ValueError("pb_plan: table must be 'host' (numpy) or 'device' (pmx_pb_table), got %r" % (table,))
+    return table
 
 
 def _check_decim(decim, nt: Optional[int] = None) -> int:
@@ -187,15 +213,17 @@ def scale_factor(setup: FiberSetup, nspan: int, gain_db: Optional[float] = None)
 def pb_plan(ctx: _lib.Context, setup: FiberSetup, nspan: int, gain_db: Optional[float] = None, xi: float = 1.0,
             K: int = 16, prune: float = 0.0, pulse=None, batch: int = 1, nt: Optional[int] = None, nquad: int = 32,
             window: Optional[int] = None, coefs=None, shift: Optional[int] = None,
-            decim: Optional[int] = None) -> _lib.PbPlan:
+            decim: Optional[int] = None, table: str = 'host') -> _lib.PbPlan:
     """The PB-NLC stage of nspan spans of the fiber `setup` describes (amplifier of gain_db [dB] after each; None: none), for
     resident one-column FP64 fields of `batch` realizations: pmx_pb_create with the table of pb_coefficients (or `coefs`,
     a (m, n, C) table), the model and gamma of the fiber, and s = scale_factor(setup, nspan, gain_db).
     decim: single-channel PB-NLC of a one-column field (pmx_pb_channel_create) -- the channel that `shift` bins bring to
     baseband (the receiver's ndfn; default 0), compensated on nfft/decim samples with the table of channel_setup at
     nt/decim samples per symbol; the pulse (and a `coefs` table) then belong to that rate, the default pulse is
-    channel_pulse."""
+    channel_pulse.  table: 'host' computes the table with numpy (pb_coefficients), 'device' with the library on ctx's device
+    (pmx_pb_table); the two agree to rounding."""
     nt = int(nt or GSTATE.NT)
+    _check_table(table)
     if decim is None and shift is not None:
         raise ValueError('pb_plan: shift selects a channel for single-channel PB-NLC and needs decim')
     if setup.nfc != 1:
@@ -209,7 +237,9 @@ def pb_plan(ctx: _lib.Context, setup: FiberSetup, nspan: int, gain_db: Optional[
         band = _lib.make_band(shift or 0, r)
         setup, nt = channel_setup(setup, shift or 0, r), nt // r
     p = np.asarray(synth.cosroll_pulse(nt, 0.2) if pulse is None else pulse, dtype=np.float64).ravel()
-    m, n, C = pb_coefficients(setup, nspan, p, K, prune, nt, nquad, window) if coefs is None else coefs
+    if coefs is None:
+        coefs = pb_coefficients(setup, nspan, p, K, prune, nt, nquad, window, ctx=ctx if table == 'device' else None)
+    m, n, C = coefs
     w, gam = model_weights(setup)
     return _lib.PbPlan(ctx, _lib.make_pb(setup.nfft // nt, nt, batch, p, w, gam, xi, scale_factor(setup, nspan, gain_db),
                                          m, n, C), band)
@@ -217,16 +247,18 @@ def pb_plan(ctx: _lib.Context, setup: FiberSetup, nspan: int, gain_db: Optional[
 
 def pbnlc(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, xi: float = 1.0, K: int = 16, prune: float = 0.0,
           pulse=None, ctx: Optional[_lib.Context] = None, nquad: int = 32, window: Optional[int] = None,
-          ich: Optional[int] = None, decim: Optional[int] = None):
+          ich: Optional[int] = None, decim: Optional[int] = None, table: str = 'host'):
     """Compensates GSTATE.FIELDX / FIELDY in place for nspan spans of the fiber x, the amplifier of gain_db [dB] after each
     (None: no amplifier): the all-pass step that undoes the link's chromatic dispersion (as Link.cd_plan), then the PB-NLC
     stage with the triplet table of K (pb_coefficients) at s = scale_factor(...), the fraction xi of the perturbation
     subtracted.  The nonlinear model is the one fiber() used: Manakov when x.manakov is 'yes' and the flag has 'p', else the
     CNLSE.  One channel (GSTATE.NCH == 1), two polarizations, FP64.  ich, decim: single-channel PB-NLC of channel ich
     (1-based) of a 'unique' multiplex of any NCH on nfft/decim samples (pb_plan; a given pulse is at that rate); afterwards
-    the field holds that channel alone, on its own bins.  The field stays resident on the device like dbp() leaves it."""
+    the field holds that channel alone, on its own bins.  table: 'host' (numpy) or 'device' (pmx_pb_table) computes the
+    triplet table (pb_plan).  The field stays resident on the device like dbp() leaves it."""
     from .mc import cd_plan_of
     G = GSTATE
+    _check_table(table)
     f = str(flag).lower()
     if len(f) != 4:
         raise ValueError("wrong flag. E.g. flag can be 'g---','gp--','-s--', etc")
@@ -257,7 +289,8 @@ def pbnlc(x, flag: str, nspan: int = 1, gain_db: Optional[float] = None, xi: flo
     ctx = ctx or _lib.default_context()
     cd = cd_plan_of(ctx, s, int(nspan), 1, precision='f64')
     try:
-        plan = pb_plan(ctx, s, nspan, gain_db, xi, K, prune, pulse, nquad=nquad, window=window, shift=shift, decim=decim)
+        plan = pb_plan(ctx, s, nspan, gain_db, xi, K, prune, pulse, nquad=nquad, window=window, shift=shift, decim=decim,
+                       table=table)
     except Exception:
         cd.close()
         raise

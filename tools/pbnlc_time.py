@@ -3,6 +3,7 @@ single-channel PB-NLC (pmx_pb_channel_create) on the C4 and C2 shapes.
 
     python tools/pbnlc_time.py [--nspan 10] [--reps 20] [--ks 4,8,16,32,64] [--out DIR]
     python tools/pbnlc_time.py --decim 16,32,64 [--nch 9] [--reps 5] [--out DIR]
+    python tools/pbnlc_time.py --table [--nch 9] [--reps 3] [--out DIR]
 
 C2 (BASELINE.md): one 28-GBaud PDM-QPSK channel, 2^16 symbols x 16 samples = 2^20 samples, 80 km spans with 16 dB
 amplifiers, Manakov.  In one process:
@@ -22,7 +23,14 @@ symbol, the centre channel: the CD all-pass step + single-channel PB-NLC (xi = 1
 at nt/r samples per symbol) and single-channel DBP at 1 and 4 steps per span.  All plans are made first and then run in
 turn, round after round, so that they are alternated in one process; each is reported as the median over --reps rounds of
 the wall time of one call on a field refreshed from the Tx (a call returns synchronised), in ms per link (per group of
-the batch).  The card's name, power limit and SM clocks are read in the same run."""
+the batch).  The card's name, power limit and SM clocks are read in the same run.
+
+With --table: the triplet table on the host (pb_coefficients, numpy) against the device (pmx_pb_table) for C2 (10 spans,
+nquad 32, default window) at K = 16, 32 and 64, and for the centre channel of C4 at decim 16 (channel_setup /
+channel_pulse, 20 spans, K = 16).  The two are alternated in one process, round after round, after a first device call
+that warms up; each is the median wall time over --reps rounds of a call that returns the table on the host.  The
+device's lag sums are (K+1)^2 * Ws * nodes complex multiply-adds (Ws the window in samples), 4 DFMA each; their rate is
+printed as a share of the FP64 pipe tools/ubench/fp64_rate.cu measures in the same call.  The tables are compared."""
 import argparse
 import json
 import os
@@ -41,7 +49,7 @@ import polmux_b200 as pmx  # noqa: E402
 from polmux_b200 import _lib, mc, synth  # noqa: E402
 from polmux_b200.dbp import dbp_plan  # noqa: E402
 from polmux_b200.fiber import fiber_setup  # noqa: E402
-from polmux_b200.pbnlc import channel_pulse, channel_setup, pb_coefficients, pb_plan, model_weights  # noqa: E402
+from polmux_b200.pbnlc import channel_pulse, channel_setup, pb_coefficients, pb_plan, pb_table, model_weights  # noqa: E402
 from polmux_b200.receiver import channel_ndfn  # noqa: E402
 
 FP64_INSTR = 52
@@ -164,6 +172,64 @@ def channel_main(a):
             json.dump(dict(card=info, runs=rows), f, indent=1)
 
 
+def table_main(a):
+    import torch
+    torch.cuda.init()
+    info = card()
+    print('card:', info)
+    dfma = fp64_pipe()
+    mhz = float(re.findall(r'([0-9.]+) MHz', info)[-1]) if 'MHz' in info else float('nan')
+    pipe = dfma * 148 * mhz * 1e6
+    print('FP64 pipe: %.1f DFMA/clk/SM (fp64_rate.cu) x 148 SMs x %.0f MHz = %.3g DFMA/s' % (dfma, mhz, pipe))
+    ctx = _lib.default_context(0)
+    cases = []                                           # (name, setup, nspan, pulse, K, nt)
+    for name, nsymb, nt, nch, nspan, decim in (('C2', 1 << 16, 16, 1, 10, None), ('C4', 1 << 16, 64, a.nch, 20, 16)):
+        ex, ey, _, _ = synth.pdm_qpsk(nsymb, nt, nch)
+        pmx.reset_all(nsymb, nt, nch)
+        G = pmx.GSTATE
+        G.SYMBOLRATE, G.LAMBDA, G.POWER = 28.0, synth.wdm_lambdas(nch, 1550.0, 0.4), np.full(nch, 1.0)
+        pmx.create_field('unique', ex, ey, {'power': 'average'})
+        fib = dict(synth.SMF)
+        fib.update(length=8e4, manakov='yes')
+        s = fiber_setup(fib, 'g-s-')
+        s.manakov = True
+        if decim is None:
+            for K in (16, 32, 64):
+                cases.append(('%s K=%d' % (name, K), s, nspan, synth.cosroll_pulse(nt, 0.2), K, nt))
+        else:
+            shift = int(channel_ndfn((nch + 1) // 2)) if nch > 1 else 0
+            cases.append(('%s r=%d K=16' % (name, decim), channel_setup(s, shift, decim), nspan,
+                          channel_pulse(nt, decim, s.nfft), 16, nt // decim))
+    rows = []
+    for name, s, nspan, p, K, nt in cases:
+        _, _, _, W = pb_table(ctx, s, nspan, p, K, nt=nt)                 # warm-up; the window it takes
+        th, td = [], []
+        for _ in range(a.reps):
+            t0 = time.perf_counter()
+            host = pb_coefficients(s, nspan, p, K, nt=nt)
+            th.append(time.perf_counter() - t0)
+            t0 = time.perf_counter()
+            dev = pb_table(ctx, s, nspan, p, K, nt=nt)
+            td.append(time.perf_counter() - t0)
+        c00 = abs(host[2][host[2].size // 2])
+        err = float(np.abs(dev[2] - host[2]).max() / c00) if np.array_equal(dev[0], host[0]) else float('inf')
+        nodes, Ws = nspan * 32, W * nt
+        macs = (K + 1) ** 2 * Ws * nodes
+        dms = 1e3 * float(np.median(td))
+        row = dict(case=name, nfft=s.nfft, nt=nt, nspan=nspan, K=K, window=W, window_samples=Ws, nodes=nodes,
+                   host_s=float(np.median(th)), device_ms=dms, device_spread_ms=[1e3 * min(td), 1e3 * max(td)],
+                   lag_macs=macs, dfma_share=4 * macs / (dms * 1e-3) / pipe, max_dC_rel=err)
+        rows.append(row)
+        print('%-12s window %5d symbols (%6d samples), %3d nodes: host %6.2f s, device %8.2f ms [%.2f .. %.2f], '
+              'lag sums at %.1f %% of the FP64 pipe, max |dC|/|C00| %.1e'
+              % (name, W, Ws, nodes, row['host_s'], dms, *row['device_spread_ms'], 100 * row['dfma_share'], err))
+    print('card (after the runs):', card())
+    if a.out:
+        os.makedirs(a.out, exist_ok=True)
+        with open(os.path.join(a.out, 'pbnlc_table_time.json'), 'w') as f:
+            json.dump(dict(card=info, dfma_per_clk_sm=dfma, runs=rows), f, indent=1)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--nsymb', type=int, default=1 << 16)
@@ -172,11 +238,14 @@ def main():
     ap.add_argument('--reps', type=int, default=20)
     ap.add_argument('--ks', default='4,8,16,32,64')
     ap.add_argument('--decim', default=None, help='single-channel PB-NLC at these decimations (comma list) on C4 and C2')
-    ap.add_argument('--nch', type=int, default=9, help='channels of the C4 multiplex (with --decim)')
+    ap.add_argument('--table', action='store_true', help='the triplet table on the host against the device')
+    ap.add_argument('--nch', type=int, default=9, help='channels of the C4 multiplex (with --decim or --table)')
     ap.add_argument('--out', default=None, help='directory for pbnlc_time.json (pbnlc_channel_time.json with --decim)')
     a = ap.parse_args()
     if a.decim:
         return channel_main(a)
+    if a.table:
+        return table_main(a)
     import torch
     torch.cuda.init()
     info = card()
