@@ -420,6 +420,48 @@ void pmx_pb_destroy(pmx_pb_plan* plan);
  * the returned plan; it owns the M-sample stage, the band filter and an M x batch work field. */
 int pmx_pb_channel_create(pmx_ctx* ctx, const pmx_pb_desc* desc, const pmx_dbp_band* band, pmx_pb_plan** plan);
 
+/* ---- XPM-aware single-channel PB-NLC: the neighbours' symbols compensate the channel's cross-phase modulation ---------
+ * Single-channel PB-NLC (pmx_pb_channel_create: the channel of interest, COI, at shift m0) plus the first-order
+ * inter-channel triplets of nint interferers, the channels that shift[c] bins bring to baseband (a joint multi-channel
+ * receiver has their symbols).  Per realization, in place, with xi != 0:
+ *   interferers: for c = 0 .. nint-1 in list order, a copy of the field, the band filter of channel c at N, the channel at
+ *                baseband decimated to M (as down), projected as the COI is (the COI's pulse, nt and norm): B_c [2][nsymb]
+ *   COI        : down, project (A), the SPM triplets (Delta), as pmx_pb_channel_create
+ *   XPM        : Delta^x_k += sum_c sum_i C'_ci * ( w1*A^x_{k+m} B^x_{k+n} conj(B^x_{k+m+n}) + w2*A^x_{k+m} B^y_{k+n}
+ *                conj(B^y_{k+m+n}) + w3*A^y_{k+m} B^x_{k+n} conj(B^y_{k+m+n}) + w4*A^y_{k+m} B^y_{k+n} conj(B^x_{k+m+n}) ),
+ *                x <-> y for Delta^y, B = B_c, (m, n, C) = entry i of interferer c's table, C' = -j*gamma*s^2*C with the
+ *                COI's gamma and s; interferers in list order, each table in list order, no atomics
+ *   apply, up  : as pmx_pb_channel_create
+ * (w1, w2, w3, w4) = (2, 1, 1, 0) is Manakov (gamma with the 8/9), (2, 2/3, 2/3, 2/3) the CNLSE: the first-order terms of
+ * the nonlinear step at the COI's frequency linear in A and in B*conj(B).  Four-wave mixing between two interferers and
+ * the triplets whose indices do not satisfy i + j - l = k are left out.  The tables come from polmux_b200/pbnlc.py,
+ * xpm_coefficients: the overlap conj(g_0) g_m h_n conj(h_{m+n}) of the COI's pulse g and the interferer's h, each dispersed
+ * with its own dispersion in the COI's frame (the walk-off kept).  With xi = 0 only the COI's down and up run, as for
+ * pmx_pb_channel_create; no interferer is extracted.
+ * Checked before a context is needed: PMX_ERR_INVALID for nint outside 1 .. PMX_PB_XPM_MAX_INT, an interferer shift equal
+ * (mod N) to the COI's or to another interferer's, an ncoef below 1 or a total above PMX_PB_MAX_COEF, |m| >
+ * PMX_PB_MAX_K, |n| > PMX_PB_XPM_MAX_N, NULL lists and non-finite weights or coefficients; and everything
+ * pmx_pb_channel_create refuses (PMX_ERR_UNSUPPORTED for FP32 and nfc != 1).  pmx_pb_exec, pmx_pb_symbols (the COI's A
+ * and the total Delta) and pmx_pb_destroy take the plan; pmx_pb_xpm_symbols reads an interferer's B.  Besides the channel
+ * plan it owns a band filter per interferer, an N x batch copy of the field and the B buffers. */
+#define PMX_PB_XPM_MAX_INT 8       /* interferers per plan                                                               */
+#define PMX_PB_XPM_MAX_N 1024      /* |n| <= PMX_PB_XPM_MAX_N in an interferer's table (the walk-off of the link)          */
+typedef struct pmx_pb_xpm_desc {
+    int32_t nint;           /* interferers, 1 .. PMX_PB_XPM_MAX_INT                                                     */
+    int32_t reserved;
+    const int64_t* shift;   /* [nint] bins that bring interferer c to baseband (the receiver's ndfn)                    */
+    const int32_t* ncoef;   /* [nint] entries of each interferer's table, >= 1, PMX_PB_MAX_COEF in all                  */
+    const int32_t* m;       /* [sum ncoef] the tables concatenated in interferer order                                  */
+    const int32_t* n;       /* [sum ncoef] */
+    const double* coef;     /* [sum ncoef][2] C = (re, im), finite                                                      */
+    double weights[4];      /* (w1, w2, w3, w4)                                                                          */
+} pmx_pb_xpm_desc;
+int pmx_pb_xpm_create(pmx_ctx* ctx, const pmx_pb_desc* desc, const pmx_dbp_band* band, const pmx_pb_xpm_desc* xpm,
+                      pmx_pb_plan** plan);
+/* The projected symbols B of interferer c (list order) of the last pmx_pb_exec with xi != 0, [batch][2][nsymb] complex
+ * (re, im interleaved) into a host buffer.  PMX_ERR_INVALID for a plan without interferers or c out of range. */
+int pmx_pb_xpm_symbols(pmx_pb_plan* plan, int32_t c, double* B);
+
 /* ---- the PB-NLC triplet table on the device: what polmux_b200/pbnlc.py, pb_coefficients, computes on the host ----------
  * For a link of nspan spans of `length` [m], loss alphalin [1/m] and dispersion betat (per metre, FFT order, on the grid
  * of nfft = nsymb*nt samples the stage runs on; for single-channel PB-NLC the channel's M samples, pbnlc.channel_setup):

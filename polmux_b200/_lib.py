@@ -36,7 +36,7 @@ EXPORTS = [
     'pmx_cohmix_exec', 'pmx_field_mean_power_xy', 'pmx_cohmix_run', 'pmx_dsp_phases', 'pmx_field_quantize', 'pmx_inverse_pmd_run',
     'pmx_dbp_create', 'pmx_dbp_exec', 'pmx_dbp_set_plates', 'pmx_dbp_channel_create', 'pmx_dbp_set_filter',
     'pmx_dbp_set_taps', 'pmx_pb_create', 'pmx_pb_exec', 'pmx_pb_symbols', 'pmx_pb_destroy', 'pmx_pb_channel_create',
-    'pmx_pb_table',
+    'pmx_pb_table', 'pmx_pb_xpm_create', 'pmx_pb_xpm_symbols',
 ]
 
 
@@ -101,6 +101,11 @@ class PbTableDesc(C.Structure):
     _fields_ = [('nfft', C.c_int64), ('nt', C.c_int32), ('npulse', C.c_int32), ('betat', _dp), ('pulse', _dp),
                 ('nspan', C.c_int32), ('K', C.c_int32), ('length', C.c_double), ('alphalin', C.c_double),
                 ('nquad', C.c_int32), ('window', C.c_int32), ('prune', C.c_double)]
+
+
+class PbXpmDesc(C.Structure):
+    _fields_ = [('nint', C.c_int32), ('reserved', C.c_int32), ('shift', C.POINTER(C.c_int64)), ('ncoef', _ip), ('m', _ip),
+                ('n', _ip), ('coef', _dp), ('weights', C.c_double * 4)]
 
 
 class McReceiver(C.Structure):
@@ -210,6 +215,8 @@ def load():
     lib.pmx_dbp_channel_create.argtypes = [vp, C.POINTER(FiberDesc), C.POINTER(DbpDesc), C.POINTER(DbpBand), C.POINTER(vp)]
     lib.pmx_pb_channel_create.argtypes = [vp, C.POINTER(PbDesc), C.POINTER(DbpBand), C.POINTER(vp)]
     lib.pmx_pb_table.argtypes = [vp, C.POINTER(PbTableDesc), _ip, _ip, _dp, _ip, _ip]
+    lib.pmx_pb_xpm_create.argtypes = [vp, C.POINTER(PbDesc), C.POINTER(DbpBand), C.POINTER(PbXpmDesc), C.POINTER(vp)]
+    lib.pmx_pb_xpm_symbols.argtypes = [vp, C.c_int32, _dp]
     _lib = lib
     return lib
 
@@ -638,6 +645,8 @@ def make_dbp(nspan, gain=0.0, steps_per_span=None, step_len=None, span_steps=Non
 
 
 PB_MAX_K = 128             # PMX_PB_MAX_K
+PB_XPM_MAX_INT = 8         # PMX_PB_XPM_MAX_INT
+PB_XPM_MAX_N = 1024        # PMX_PB_XPM_MAX_N
 
 
 def check_pb_k(K):
@@ -694,19 +703,62 @@ def pb_table(ctx, desc_keep):
     return m[:k].copy(), n[:k].copy(), coef[:k].copy(), int(win.value)
 
 
+def make_pb_xpm(shifts, tables, weights):
+    """-> (PbXpmDesc, keep-alive dict): the interferers brought to baseband by `shifts` bins, tables[c] = (m, n, coef) the
+    XPM table of interferer c, weights (w1, w2, w3, w4)"""
+    tables = [tuple(t) for t in tables]
+    if len(tables) != len(shifts):
+        raise ValueError('make_pb_xpm: one table per interferer')
+    ms = [np.asarray(t[0]).ravel() for t in tables]
+    ns = [np.asarray(t[1]).ravel() for t in tables]
+    cs = [np.asarray(t[2], dtype=np.complex128).ravel() for t in tables]
+    if any(not (a.size == b.size == c.size) for a, b, c in zip(ms, ns, cs)):
+        raise ValueError('make_pb_xpm: m, n and coef must have one value per entry')
+    cat = lambda xs, dt: np.ascontiguousarray(np.concatenate(xs) if xs else np.zeros(0), dtype=dt)
+    keep = {'shift': np.ascontiguousarray(np.asarray(shifts).ravel(), dtype=np.int64),
+            'ncoef': np.ascontiguousarray([a.size for a in ms], dtype=np.int32),
+            'm': cat(ms, np.int32), 'n': cat(ns, np.int32), 'coef': cat(cs, np.complex128).view(np.float64)}
+    d = PbXpmDesc()
+    d.nint = keep['shift'].size
+    d.shift = keep['shift'].ctypes.data_as(C.POINTER(C.c_int64))
+    d.ncoef, d.m, d.n = (keep[k].ctypes.data_as(_ip) for k in ('ncoef', 'm', 'n'))
+    d.coef = _ptr(keep['coef'])
+    d.weights = (C.c_double * 4)(*[float(w) for w in weights])
+    return d, keep
+
+
+def check_pb_xpm(desc_keep, band, xpm_keep):
+    """ValueError with the library's message if pmx_pb_xpm_create refuses the request (checked without a context)"""
+    lib = load()
+    h = C.c_void_p()
+    rc = lib.pmx_pb_xpm_create(None, C.byref(desc_keep[0]), C.byref(band), C.byref(xpm_keep[0]), C.byref(h))
+    msg = lib.pmx_last_error(None).decode()
+    if rc != PMX_OK and 'null ctx' not in msg:
+        raise ValueError(msg)
+
+
 class PbPlan:
     """Perturbation-based nonlinearity compensation (pmx_pb_create): execute(field) runs it in place on a resident field.
     With a band (DbpBand: shift, decim) the descriptor is the channel's at nfft/decim samples and the plan is the PB-NLC of
-    that channel of a one-column field of nfft samples (pmx_pb_channel_create)."""
+    that channel of a one-column field of nfft samples (pmx_pb_channel_create); with xpm (make_pb_xpm) as well, the
+    XPM-aware PB-NLC of that channel (pmx_pb_xpm_create)."""
 
-    def __init__(self, ctx: Context, desc_keep, band: 'DbpBand' = None):
-        self.ctx, (self.desc, self.keep), self.band = ctx, desc_keep, band
+    def __init__(self, ctx: Context, desc_keep, band: 'DbpBand' = None, xpm=None):
+        self.ctx, (self.desc, self.keep), self.band, self.xpm = ctx, desc_keep, band, xpm
         h = C.c_void_p()
         if band is None:
             ctx.check(ctx.lib.pmx_pb_create(ctx.h, C.byref(self.desc), C.byref(h)))
-        else:
+        elif xpm is None:
             ctx.check(ctx.lib.pmx_pb_channel_create(ctx.h, C.byref(self.desc), C.byref(band), C.byref(h)))
+        else:
+            ctx.check(ctx.lib.pmx_pb_xpm_create(ctx.h, C.byref(self.desc), C.byref(band), C.byref(xpm[0]), C.byref(h)))
         self.h = h
+
+    def xpm_symbols(self, c):
+        """-> B of interferer c of the last execute, [batch][2][nsymb] complex128 (pmx_pb_xpm_symbols)"""
+        b = np.zeros((self.desc.batch, 2, self.desc.nsymb), dtype=np.complex128)
+        self.ctx.check(self.ctx.lib.pmx_pb_xpm_symbols(self.h, int(c), b.ctypes.data_as(_dp)))
+        return b
 
     def execute(self, field: DeviceField):
         self.ctx.check(self.ctx.lib.pmx_pb_exec(self.h, field.h))

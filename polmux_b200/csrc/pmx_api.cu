@@ -4205,6 +4205,17 @@ struct pmx_pb_plan {
     pmx_devfield* ch_work = nullptr;
     long long ch_shift = 0;
     int ch_log2r = 0;
+    // XPM-aware single-channel PB-NLC (pmx_pb_xpm_create), on the channel plan: the interferers' shifts (mod nfft) and band
+    // filters, the copy of the field each is cut from, their symbols B [nint][batch][2][nsymb], their folded tables
+    // concatenated with offsets [nint+1], the halos of the XPM kernel (max |m|; max of |n| and |m+n|) and the weights
+    int xpm_n = 0, xpm_ha = 0, xpm_hb = 0;
+    long long xpm_shift[PMX_PB_XPM_MAX_INT] = {};
+    pmx_plan* xpm_band[PMX_PB_XPM_MAX_INT] = {};
+    pmx_devfield* xpm_copy = nullptr;
+    cpx* xpm_B = nullptr;
+    PbCoef* xpm_coef = nullptr;
+    int* xpm_off = nullptr;
+    double xpm_w[4] = {};
 };
 
 // A^{x,y}_k = sum_j p[j] u[(k*nt - np/2 + j) mod N] * inorm (j ascending); thread per symbol, grid.y the realization
@@ -4333,6 +4344,137 @@ __global__ void __launch_bounds__(256) pmx_k_pb_apply(cpx* __restrict__ field, s
     }
 }
 
+// The XPM triplet sum (pmx_pb_xpm_create): Delta += the inter-channel triplets of every interferer, on the COI's symbols A
+// and the interferer's B.  Shaped like pmx_k_pb_triplet: a CTA takes PMX_PB_TILE symbols of one realization, lands A with
+// a halo of ha = max |m| and, per interferer in turn, B with a halo of hb = max(|n|, |m+n|), both polarizations, in shared
+// memory; a thread owns PMX_PB_RB symbols PMX_PB_THREADS apart and reads each coefficient as a broadcast.  The sums start
+// from the SPM Delta and take the interferers in list order, each table in list order: a fixed order, no atomics.  Per entry
+// and symbol the loop runs the 4 products B*conj(B) P = Bx_n conj(Bx_s), Q = By_n conj(By_s), R = Bx_n conj(By_s),
+// S = By_n conj(Bx_s) (8 FMA + 8 MUL), the 4 weighted sums w1*P + w2*Q, w3*R + w4*S, w1*Q + w2*P, w3*S + w4*R (8 FMA +
+// 8 MUL), T^x = A^x_m u + A^y_m v and T^y likewise (8 FMA + 4 MUL + 8 FMA) and the two accumulations C'*T (8 FMA): 56 FP64
+// instructions, 36 FMA and 20 MUL, 92 flops per entry and symbol (an FMA counted as two), from 6 shared-memory loads of 16
+// bytes.
+__device__ __forceinline__ double2 pb_mac(double2 acc, double2 a, double2 b) {   // acc + a*b
+    return make_double2(fma(-a.y, b.y, fma(a.x, b.x, acc.x)), fma(a.y, b.x, fma(a.x, b.y, acc.y)));
+}
+__global__ void __launch_bounds__(PMX_PB_THREADS) pmx_k_pb_xpm(const cpx* __restrict__ A, const cpx* __restrict__ B,
+                                                               int nsymb, int batch, int nint, const PbCoef* __restrict__ coef,
+                                                               const int* __restrict__ off, int ha, int hb, double w1,
+                                                               double w2, double w3, double w4, cpx* __restrict__ D) {
+    extern __shared__ __align__(16) unsigned char smp[];
+    const int sa = PMX_PB_TILE + 2 * ha, sb = PMX_PB_TILE + 2 * hb;
+    cpx* ax = reinterpret_cast<cpx*>(smp);   // [sa]: symbol k0 - ha + i at i
+    cpx* ay = ax + sa;
+    cpx* bx = ay + sa;                        // [sb]: symbol k0 - hb + i at i
+    cpx* by = bx + sb;
+    const int b = blockIdx.y, k0 = blockIdx.x * PMX_PB_TILE;
+    const cpx* gax = A + (size_t)(2 * b) * nsymb;
+    for (int i = threadIdx.x; i < sa; i += PMX_PB_THREADS) {
+        int k = (k0 - ha + i) % nsymb;
+        if (k < 0) k += nsymb;
+        ax[i] = gax[k];
+        ay[i] = gax[nsymb + k];
+    }
+    double2 dx[PMX_PB_RB], dy[PMX_PB_RB];
+#pragma unroll
+    for (int r = 0; r < PMX_PB_RB; ++r) {
+        const int k = k0 + threadIdx.x + r * PMX_PB_THREADS;
+        dx[r] = k < nsymb ? D[(size_t)(2 * b) * nsymb + k] : make_double2(0.0, 0.0);
+        dy[r] = k < nsymb ? D[(size_t)(2 * b + 1) * nsymb + k] : make_double2(0.0, 0.0);
+    }
+    for (int c = 0; c < nint; ++c) {
+        __syncthreads();   // the previous interferer's tile is read
+        const cpx* gbx = B + ((size_t)c * batch + b) * 2 * nsymb;
+        for (int i = threadIdx.x; i < sb; i += PMX_PB_THREADS) {
+            int k = (k0 - hb + i) % nsymb;
+            if (k < 0) k += nsymb;
+            bx[i] = gbx[k];
+            by[i] = gbx[nsymb + k];
+        }
+        __syncthreads();
+        const int e = __ldg(&off[c + 1]);
+        for (int i = __ldg(&off[c]); i < e; ++i) {
+            const double cr = __ldg(&coef[i].cr), ci = __ldg(&coef[i].ci);
+            const int m = __ldg(&coef[i].m), n = __ldg(&coef[i].n);
+#pragma unroll
+            for (int r = 0; r < PMX_PB_RB; ++r) {
+                const int o = threadIdx.x + r * PMX_PB_THREADS;
+                const double2 xm = ax[ha + o + m], ym = ay[ha + o + m];
+                const double2 xn = bx[hb + o + n], yn = by[hb + o + n], xs = bx[hb + o + m + n], ys = by[hb + o + m + n];
+                const double2 P = pb_mul_conj(xn, xs), Q = pb_mul_conj(yn, ys), R = pb_mul_conj(xn, ys), S = pb_mul_conj(yn, xs);
+                const double2 u = make_double2(fma(w1, P.x, w2 * Q.x), fma(w1, P.y, w2 * Q.y));
+                const double2 v = make_double2(fma(w3, R.x, w4 * S.x), fma(w3, R.y, w4 * S.y));
+                const double2 u2 = make_double2(fma(w1, Q.x, w2 * P.x), fma(w1, Q.y, w2 * P.y));
+                const double2 v2 = make_double2(fma(w3, S.x, w4 * R.x), fma(w3, S.y, w4 * R.y));
+                const double2 tx = pb_mac(pb_mul(xm, u), ym, v);
+                const double2 ty = pb_mac(pb_mul(ym, u2), xm, v2);
+                dx[r] = make_double2(fma(cr, tx.x, fma(-ci, tx.y, dx[r].x)), fma(cr, tx.y, fma(ci, tx.x, dx[r].y)));
+                dy[r] = make_double2(fma(cr, ty.x, fma(-ci, ty.y, dy[r].x)), fma(cr, ty.y, fma(ci, ty.x, dy[r].y)));
+            }
+        }
+    }
+#pragma unroll
+    for (int r = 0; r < PMX_PB_RB; ++r) {
+        const int k = k0 + threadIdx.x + r * PMX_PB_THREADS;
+        if (k < nsymb) {
+            D[(size_t)(2 * b) * nsymb + k] = dx[r];
+            D[(size_t)(2 * b + 1) * nsymb + k] = dy[r];
+        }
+    }
+}
+
+// The three launches of the stage on a field of the plan's nfft and batch (checked by the caller)
+static void pb_project(pmx_pb_plan* p, const pmx_devfield* f, cpx* out) {
+    pmx_ctx* c = p->ctx;
+    pmx_k_pb_project<<<dim3((unsigned)((p->nsymb + 255) / 256), p->batch), 256, 0, c->stream>>>(
+        f->data, (size_t)p->nfft, f->log2N1, f->log2N2, p->nsymb, p->nt, p->pulse, p->npulse, p->inorm, out);
+    c->launches++;
+}
+static int pb_triplet(pmx_pb_plan* p) {
+    pmx_ctx* c = p->ctx;
+    const int smem = (PMX_PB_TILE + 4 * p->K) * 2 * (int)sizeof(cpx);
+    if (smem > 48 * 1024) CK(c, cudaFuncSetAttribute(pmx_k_pb_triplet, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    pmx_k_pb_triplet<<<dim3((unsigned)((p->nsymb + PMX_PB_TILE - 1) / PMX_PB_TILE), p->batch), PMX_PB_THREADS, smem,
+                       c->stream>>>(p->A, p->nsymb, p->coef, p->ncoef, p->K, p->wa, p->wb, p->wc, p->D);
+    c->launches++;
+    return PMX_OK;
+}
+static void pb_apply(pmx_pb_plan* p, pmx_devfield* f) {
+    pmx_ctx* c = p->ctx;
+    const size_t N = (size_t)p->nfft;
+    pmx_k_pb_apply<<<dim3((unsigned)std::min<size_t>((N + 255) / 256, 148 * 8), p->batch), 256, 0, c->stream>>>(
+        f->data, N, f->log2N1, f->log2N2, p->nsymb, p->nt, p->pulse, p->npulse, p->D, p->xi);
+    c->launches++;
+}
+
+// XPM-aware single channel (xi != 0): every interferer cut from a copy of the field and projected, then the COI's down,
+// projection and SPM triplets, the XPM triplets added to Delta, apply and up
+static int pb_xpm_exec(pmx_pb_plan* p, pmx_devfield* f) {
+    pmx_ctx* c = p->ctx;
+    pmx_pb_plan* s = p->ch_pb;
+    const size_t per = (size_t)p->batch * 2 * s->nsymb;
+    int rc = PMX_OK;
+    for (int i = 0; i < p->xpm_n && !rc; ++i) {
+        rc = pmx_field_copy_cols(p->xpm_copy, 0, f, 0, p->batch);
+        if (!rc) rc = band_down(p->xpm_band[i], p->xpm_copy, p->ch_work, p->ch_log2r, p->xpm_shift[i]);
+        if (!rc) pb_project(s, p->ch_work, p->xpm_B + i * per);
+    }
+    if (!rc) rc = band_down(p->ch_band, f, p->ch_work, p->ch_log2r, p->ch_shift);
+    if (rc) return rc;
+    CK(c, cudaSetDevice(c->device));
+    pb_project(s, p->ch_work, s->A);
+    if (int e = pb_triplet(s)) return e;
+    const int smem = (2 * (PMX_PB_TILE + 2 * p->xpm_ha) + 2 * (PMX_PB_TILE + 2 * p->xpm_hb)) * (int)sizeof(cpx);
+    if (smem > 48 * 1024) CK(c, cudaFuncSetAttribute(pmx_k_pb_xpm, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    pmx_k_pb_xpm<<<dim3((unsigned)((s->nsymb + PMX_PB_TILE - 1) / PMX_PB_TILE), p->batch), PMX_PB_THREADS, smem, c->stream>>>(
+        s->A, p->xpm_B, s->nsymb, p->batch, p->xpm_n, p->xpm_coef, p->xpm_off, p->xpm_ha, p->xpm_hb, p->xpm_w[0], p->xpm_w[1],
+        p->xpm_w[2], p->xpm_w[3], s->D);
+    c->launches++;
+    pb_apply(s, p->ch_work);
+    CK(c, cudaGetLastError());
+    return band_up(p->ch_band, p->ch_work, f, p->ch_log2r, p->ch_shift);
+}
+
 extern "C" int pmx_pb_create(pmx_ctx* c, const pmx_pb_desc* d, pmx_pb_plan** out) {
     // (the descriptor is checked before the context, so that the checks run without a device)
     if (!d || !out) return set_err(c, PMX_ERR_INVALID, "pmx_pb_create: null argument");
@@ -4430,6 +4572,7 @@ extern "C" int pmx_pb_exec(pmx_pb_plan* p, pmx_devfield* f) {
     if (f->batch != p->batch)
         return set_err(c, PMX_ERR_INVALID, "pmx_pb_exec: the field has batch %d, the plan %d", f->batch, p->batch);
     if (p->ch_pb) {   // single channel: down, the stage at nfft/decim samples, up
+        if (p->xpm_n && p->xi != 0) return pb_xpm_exec(p, f);
         int rc = band_down(p->ch_band, f, p->ch_work, p->ch_log2r, p->ch_shift);
         if (!rc) rc = pmx_pb_exec(p->ch_pb, p->ch_work);
         if (!rc) rc = band_up(p->ch_band, p->ch_work, f, p->ch_log2r, p->ch_shift);
@@ -4437,17 +4580,9 @@ extern "C" int pmx_pb_exec(pmx_pb_plan* p, pmx_devfield* f) {
     }
     if (p->xi == 0) return PMX_OK;   // nothing to subtract: the field is left as it is
     CK(c, cudaSetDevice(c->device));
-    const size_t N = (size_t)p->nfft;
-    const int l1 = f->log2N1, l2 = f->log2N2;
-    pmx_k_pb_project<<<dim3((unsigned)((p->nsymb + 255) / 256), p->batch), 256, 0, c->stream>>>(
-        f->data, N, l1, l2, p->nsymb, p->nt, p->pulse, p->npulse, p->inorm, p->A);
-    const int smem = (PMX_PB_TILE + 4 * p->K) * 2 * (int)sizeof(cpx);
-    if (smem > 48 * 1024) CK(c, cudaFuncSetAttribute(pmx_k_pb_triplet, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    pmx_k_pb_triplet<<<dim3((unsigned)((p->nsymb + PMX_PB_TILE - 1) / PMX_PB_TILE), p->batch), PMX_PB_THREADS, smem,
-                       c->stream>>>(p->A, p->nsymb, p->coef, p->ncoef, p->K, p->wa, p->wb, p->wc, p->D);
-    pmx_k_pb_apply<<<dim3((unsigned)std::min<size_t>((N + 255) / 256, 148 * 8), p->batch), 256, 0, c->stream>>>(
-        f->data, N, l1, l2, p->nsymb, p->nt, p->pulse, p->npulse, p->D, p->xi);
-    c->launches += 3;
+    pb_project(p, f, p->A);
+    if (int rc = pb_triplet(p)) return rc;
+    pb_apply(p, f);
     CK(c, cudaGetLastError());
     return PMX_OK;
 }
@@ -4467,11 +4602,14 @@ extern "C" int pmx_pb_symbols(pmx_pb_plan* p, double* A, double* delta) {
 extern "C" void pmx_pb_destroy(pmx_pb_plan* p) {
     if (!p) return;
     cudaSetDevice(p->ctx->device);
-    for (void* q : {(void*)p->pulse, (void*)p->coef, (void*)p->A, (void*)p->D})
+    for (void* q : {(void*)p->pulse, (void*)p->coef, (void*)p->A, (void*)p->D, (void*)p->xpm_B, (void*)p->xpm_coef,
+                    (void*)p->xpm_off})
         if (q) cudaFreeAsync(q, p->ctx->stream);
     pmx_pb_destroy(p->ch_pb);
     pmx_plan_destroy(p->ch_band);
     pmx_field_destroy(p->ch_work);
+    for (pmx_plan* q : p->xpm_band) pmx_plan_destroy(q);
+    pmx_field_destroy(p->xpm_copy);
     delete p;
 }
 
@@ -4519,6 +4657,108 @@ extern "C" int pmx_pb_channel_create(pmx_ctx* c, const pmx_pb_desc* d, const pmx
         return rc;
     }
     *out = p;
+    return PMX_OK;
+}
+
+// XPM-aware single-channel PB-NLC (polmux_ssfm.h): the channel plan, plus per interferer a band filter at N, and the
+// interferers' symbols and tables for pmx_k_pb_xpm
+extern "C" int pmx_pb_xpm_create(pmx_ctx* c, const pmx_pb_desc* d, const pmx_dbp_band* band, const pmx_pb_xpm_desc* x,
+                                 pmx_pb_plan** out) {
+    // (checked before the context, like pmx_pb_channel_create)
+    if (!d || !band || !x || !out) return set_err(c, PMX_ERR_INVALID, "pmx_pb_xpm_create: null argument");
+    *out = nullptr;
+    if (x->nint < 1 || x->nint > PMX_PB_XPM_MAX_INT)
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_xpm_create: nint=%d, 1 to %d interferers", x->nint, PMX_PB_XPM_MAX_INT);
+    if (!x->shift || !x->ncoef || !x->m || !x->n || !x->coef)
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_xpm_create: null interferer list");
+    for (int i = 0; i < 4; ++i)
+        if (!std::isfinite(x->weights[i])) return set_err(c, PMX_ERR_INVALID, "pmx_pb_xpm_create: weight %d is not finite", i);
+    int64_t total = 0;
+    std::vector<int> off(x->nint + 1, 0);   // [nint+1] where each interferer's table starts
+    for (int i = 0; i < x->nint; ++i) {
+        if (x->ncoef[i] < 1)
+            return set_err(c, PMX_ERR_INVALID, "pmx_pb_xpm_create: interferer %d has ncoef=%d, at least 1", i, x->ncoef[i]);
+        total += x->ncoef[i];
+        off[i + 1] = (int)std::min<int64_t>(total, INT32_MAX);
+    }
+    if (total > PMX_PB_MAX_COEF)
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_xpm_create: %lld entries in all, at most %d", (long long)total,
+                       PMX_PB_MAX_COEF);
+    // the shifts mod N, when the band and the descriptor give N (otherwise pmx_pb_channel_create refuses them below)
+    const int lr = ilog2_exact(band->decim);
+    if (band->decim >= 2 && lr >= 1 && d->nfft >= 1 && d->nfft <= ((int64_t)1 << 30)) {
+        const int64_t N = d->nfft << lr;
+        auto mod = [N](int64_t v) { return ((v % N) + N) % N; };
+        for (int i = 0; i < x->nint; ++i) {
+            if (mod(x->shift[i]) == mod(band->shift))
+                return set_err(c, PMX_ERR_INVALID, "pmx_pb_xpm_create: interferer %d has the channel's own shift %lld", i,
+                               (long long)x->shift[i]);
+            for (int j = 0; j < i; ++j)
+                if (mod(x->shift[i]) == mod(x->shift[j]))
+                    return set_err(c, PMX_ERR_INVALID, "pmx_pb_xpm_create: interferers %d and %d have the same shift %lld", j,
+                                   i, (long long)x->shift[i]);
+        }
+    }
+    const double g = d->gamma * d->scale * d->scale;
+    std::vector<PbCoef> list((size_t)total);
+    int ha = 0, hb = 0;
+    for (int64_t i = 0; i < total; ++i) {
+        const int m = x->m[i], n = x->n[i];
+        if (std::abs(m) > PMX_PB_MAX_K || std::abs(n) > PMX_PB_XPM_MAX_N)
+            return set_err(c, PMX_ERR_INVALID, "pmx_pb_xpm_create: entry %lld has (m, n) = (%d, %d), |m| at most %d and |n| "
+                           "at most %d", (long long)i, m, n, PMX_PB_MAX_K, PMX_PB_XPM_MAX_N);
+        const double cr = x->coef[2 * i], ci = x->coef[2 * i + 1];
+        if (!std::isfinite(cr) || !std::isfinite(ci))
+            return set_err(c, PMX_ERR_INVALID, "pmx_pb_xpm_create: coefficient %lld is not finite", (long long)i);
+        list[i] = PbCoef{g * ci, -(g * cr), m, n};   // -j*gamma*s^2*C
+        ha = std::max(ha, std::abs(m));
+        hb = std::max(hb, std::max(std::abs(n), std::abs(m + n)));
+    }
+    pmx_pb_plan* p = nullptr;
+    int rc = pmx_pb_channel_create(c, d, band, &p);   // validates the rest before it needs the context
+    if (rc) return rc;
+    const int64_t N = p->nfft;
+    p->xpm_n = x->nint;
+    p->xpm_ha = ha;
+    p->xpm_hb = hb;
+    for (int i = 0; i < 4; ++i) p->xpm_w[i] = x->weights[i];
+    for (int i = 0; i < x->nint && !rc; ++i) {
+        p->xpm_shift[i] = ((x->shift[i] % N) + N) % N;
+        rc = band_filter_create(c, N, d->nfft, p->xpm_shift[i], d->batch, PMX_F64, &p->xpm_band[i]);
+    }
+    if (!rc) rc = pmx_field_create(c, N, 1, d->batch, PMX_F64, &p->xpm_copy);
+    if (rc) {
+        pmx_pb_destroy(p);
+        return rc;
+    }
+    const size_t bbytes = (size_t)x->nint * d->batch * 2 * d->nsymb * sizeof(cpx);
+    cudaError_t err = cudaSetDevice(c->device);
+    if (err == cudaSuccess) err = cudaMallocAsync(&p->xpm_B, bbytes, c->stream);
+    if (err == cudaSuccess) err = cudaMallocAsync(&p->xpm_coef, sizeof(PbCoef) * total, c->stream);
+    if (err == cudaSuccess) err = cudaMallocAsync(&p->xpm_off, sizeof(int) * off.size(), c->stream);
+    if (err == cudaSuccess) err = cudaMemsetAsync(p->xpm_B, 0, bbytes, c->stream);
+    if (err == cudaSuccess)
+        err = cudaMemcpyAsync(p->xpm_coef, list.data(), sizeof(PbCoef) * total, cudaMemcpyHostToDevice, c->stream);
+    if (err == cudaSuccess)
+        err = cudaMemcpyAsync(p->xpm_off, off.data(), sizeof(int) * off.size(), cudaMemcpyHostToDevice, c->stream);
+    if (err == cudaSuccess) err = cudaStreamSynchronize(c->stream);   // the host tables are this frame's
+    if (err != cudaSuccess) {
+        pmx_pb_destroy(p);
+        return set_err(c, PMX_ERR_CUDA, "pmx_pb_xpm_create: %s", cudaGetErrorString(err));
+    }
+    *out = p;
+    return PMX_OK;
+}
+
+extern "C" int pmx_pb_xpm_symbols(pmx_pb_plan* p, int32_t i, double* B) {
+    if (!p || !B) return set_err(p ? p->ctx : nullptr, PMX_ERR_INVALID, "pmx_pb_xpm_symbols: null argument");
+    pmx_ctx* c = p->ctx;
+    if (i < 0 || i >= p->xpm_n)
+        return set_err(c, PMX_ERR_INVALID, "pmx_pb_xpm_symbols: interferer %d, the plan has %d", i, p->xpm_n);
+    const size_t per = (size_t)p->batch * 2 * p->ch_pb->nsymb;
+    CK(c, cudaSetDevice(c->device));
+    CK(c, cudaMemcpyAsync(B, p->xpm_B + i * per, per * sizeof(cpx), cudaMemcpyDeviceToHost, c->stream));
+    CK(c, cudaStreamSynchronize(c->stream));
     return PMX_OK;
 }
 

@@ -233,7 +233,8 @@ class McRunner:
         default xi = 1, K = 16, table 'host': numpy; 'device': pmx_pb_table) at the launch scale s of the link's loss and
         gain.  pb_params with 'decim' (a power of two >= 2 dividing nt; a one-column 'unique' field of any number of
         channels): single-channel PB-NLC on nfft/decim samples -- of channel `ich` for 'cohmix', of the channel at the
-        centre of the grid for 'blind'."""
+        centre of the grid for 'blind'; with 'xpm' as well (a list of channels, 'adjacent' or 'all'), XPM-aware with the
+        symbols of those channels (pbnlc.pb_plan's xpm)."""
         import torch
         from . import dsp as _dsp
         self.receiver, self.dsp_params = receiver, dict(dsp_params or {})
@@ -297,6 +298,10 @@ class McRunner:
                 pp = dict(pb_params or {})
                 if pp.get('decim') is not None:      # single-channel PB-NLC of the receiver's channel
                     pp['shift'] = S.ndfn if S is not None else 0
+                if pp.get('xpm') is not None:        # its interferers, by channel number
+                    from .pbnlc import xpm_shifts
+                    from .gstate import GSTATE
+                    pp['xpm'] = xpm_shifts(pp['xpm'], ich if S is not None else (GSTATE.NCH + 1) // 2)
                 self.rx['pb'] = pb_plan(self.rxctx, setup, nspan, gain_db, batch=batch, nt=nt, **pp)
             if receiver == 'cohmix':
                 delay = _rx.evaldelay(x['oftype'], x['obw'] * 0.5) + _rx.evaldelay(x['eftype'], x['ebw']) + S.x['post_delay']

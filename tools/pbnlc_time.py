@@ -4,6 +4,7 @@ single-channel PB-NLC (pmx_pb_channel_create) on the C4 and C2 shapes.
     python tools/pbnlc_time.py [--nspan 10] [--reps 20] [--ks 4,8,16,32,64] [--out DIR]
     python tools/pbnlc_time.py --decim 16,32,64 [--nch 9] [--reps 5] [--out DIR]
     python tools/pbnlc_time.py --table [--nch 9] [--reps 3] [--out DIR]
+    python tools/pbnlc_time.py --xpm [--nch 9] [--reps 5] [--out DIR]
 
 C2 (BASELINE.md): one 28-GBaud PDM-QPSK channel, 2^16 symbols x 16 samples = 2^20 samples, 80 km spans with 16 dB
 amplifiers, Manakov.  In one process:
@@ -30,7 +31,17 @@ nquad 32, default window) at K = 16, 32 and 64, and for the centre channel of C4
 channel_pulse, 20 spans, K = 16).  The two are alternated in one process, round after round, after a first device call
 that warms up; each is the median wall time over --reps rounds of a call that returns the table on the host.  The
 device's lag sums are (K+1)^2 * Ws * nodes complex multiply-adds (Ws the window in samples), 4 DFMA each; their rate is
-printed as a share of the FP64 pipe tools/ubench/fp64_rate.cu measures in the same call.  The tables are compared."""
+printed as a share of the FP64 pipe tools/ubench/fp64_rate.cu measures in the same call.  The tables are compared.
+
+With --xpm: XPM-aware single-channel PB-NLC (pmx_pb_xpm_create) of the centre channel of C4 at decim 16 and K = 16, with
+the 2 adjacent and with all 8 other channels as interferers (their tables from xpm_coefficients, default Kn -- capped at
+PMX_PB_XPM_MAX_N -- pruned at 1e-4 of the largest entry; nquad 2: the timing depends on the entry count only).  In one
+process: (1) the XPM kernel (pmx_k_pb_xpm) alone: its device time from torch.profiler over --reps executions and its FP64
+rate -- 56 FP64 instructions (36 DFMA, 20 DMUL) per entry and symbol, counted from the code -- as a share of the FP64 pipe
+fp64_rate.cu measures in the same call; (2) per link, alternated round after round as with --decim: CD + XPM-aware PB-NLC
+(2 and 8 interferers), CD + single-channel PB-NLC, single-channel DBP and full-field DBP at one step per span.  The
+extraction of the interferers (copy, band filter at N, gather, projection) is the XPM plan's time less the single-channel
+plan's and the XPM kernel's."""
 import argparse
 import json
 import os
@@ -53,6 +64,7 @@ from polmux_b200.pbnlc import channel_pulse, channel_setup, pb_coefficients, pb_
 from polmux_b200.receiver import channel_ndfn  # noqa: E402
 
 FP64_INSTR = 52
+XPM_FP64_INSTR = 56
 
 
 def card():
@@ -230,6 +242,94 @@ def table_main(a):
             json.dump(dict(card=info, dfma_per_clk_sm=dfma, runs=rows), f, indent=1)
 
 
+def xpm_main(a):
+    import torch
+    from polmux_b200.pbnlc import xpm_coefficients, xpm_channels
+    torch.cuda.init()
+    info = card()
+    print('card:', info)
+    dfma = fp64_pipe()
+    mhz = float(re.findall(r'([0-9.]+) MHz', info)[-1]) if 'MHz' in info else float('nan')
+    pipe = dfma * 148 * mhz * 1e6
+    print('FP64 pipe: %.1f DFMA/clk/SM (fp64_rate.cu) x 148 SMs x %.0f MHz = %.3g FP64 instr/s' % (dfma, mhz, pipe))
+    nsymb, nt, nch, nspan, r, K = 1 << 16, 64, a.nch, 20, 16, 16
+    ex, ey, _, _ = synth.pdm_qpsk(nsymb, nt, nch)
+    pmx.reset_all(nsymb, nt, nch)
+    G = pmx.GSTATE
+    G.SYMBOLRATE, G.LAMBDA, G.POWER = 28.0, synth.wdm_lambdas(nch, 1550.0, 0.4), np.full(nch, 1.0)
+    pmx.create_field('unique', ex, ey, {'power': 'average'})
+    fib = dict(synth.SMF)
+    fib.update(length=8e4, manakov='yes')
+    s = fiber_setup(fib, 'g-s-')
+    s.manakov = True
+    ich = (nch + 1) // 2
+    shift = int(channel_ndfn(ich))
+    ctx = _lib.default_context(0)
+    N = s.nfft
+    p = channel_pulse(nt, r, N)
+    t0 = time.perf_counter()
+    spm = pb_coefficients(channel_setup(s, shift, r), nspan, p, K, nt=nt // r)
+    tabs = {}
+    for c in xpm_channels('all', ich, nch):
+        tabs[c] = xpm_coefficients(s, nspan, shift, int(channel_ndfn(c)), r, p, K, prune=1e-4, nt=nt, nquad=2)
+    print('C4 r=%d: tables in %.1f s on one host thread; XPM entries per interferer %s'
+          % (r, time.perf_counter() - t0, {c: len(t[2]) for c, t in tabs.items()}))
+    tx = _lib.DeviceField(ctx, N, 1, 1)
+    tx.upload(G.FIELDX_TX, G.FIELDY_TX)
+    fld = _lib.DeviceField(ctx, N, 1, 1)
+    cd = mc.cd_plan_of(ctx, s, nspan, 1, precision='f64')
+    res = {'card': info, 'dfma_per_clk_sm': dfma, 'kernel': [], 'runs': []}
+    runs = []
+    for name, chans in (('2 adjacent', xpm_channels('adjacent', ich, nch)), ('all %d' % (nch - 1), list(tabs))):
+        pb = pb_plan(ctx, s, nspan, 16.0, K=K, nt=nt, coefs=spm, shift=shift, decim=r,
+                     xpm=[int(channel_ndfn(c)) for c in chans], xpm_coefs=[tabs[c] for c in chans])
+        ncoef = sum(len(tabs[c][2]) for c in chans)
+        fld.broadcast_from(tx)
+        ms = kernel_ms(lambda: (pb.execute(fld), ctx.sync()), a.reps, 'pmx_k_pb_xpm')
+        rate = XPM_FP64_INSTR * ncoef * nsymb / (ms * 1e-3)
+        row = dict(interferers=len(chans), ncoef=ncoef, xpm_kernel_ms=ms, fp64_instr_per_s=rate, pipe_share=rate / pipe)
+        res['kernel'].append(row)
+        print('XPM kernel, %s interferers, %6d entries: %8.3f ms  %.3g FP64 instr/s  %.1f %% of the pipe'
+              % (name, ncoef, ms, rate, 100 * rate / pipe))
+        runs.append((dict(run='cd+pbnlc_xpm', interferers=len(chans), ncoef=ncoef),
+                     lambda f, pb=pb: (cd.execute(f), pb.execute(f), ctx.sync()), pb))
+    pb = pb_plan(ctx, s, nspan, 16.0, K=K, nt=nt, coefs=spm, shift=shift, decim=r)
+    runs.append((dict(run='cd+pbnlc', ncoef=len(spm[2])), lambda f, pb=pb: (cd.execute(f), pb.execute(f), ctx.sync()), pb))
+    for name, kw in (('dbp_channel', dict(shift=shift, decim=r)), ('dbp_full', {})):
+        plan = dbp_plan(ctx, s, nspan, 16.0, steps_per_span=1, batch=1, precision='f64', **kw)
+        runs.append((dict(run=name, steps_per_span=1), lambda f, plan=plan: (plan.execute(f), ctx.sync()), plan))
+    times = [[] for _ in runs]
+    for rep in range(a.reps + 1):                        # round 0 warms every plan up
+        for i, (_, fn, _) in enumerate(runs):
+            fld.broadcast_from(tx)
+            ctx.sync()
+            t0 = time.perf_counter()
+            fn(fld)
+            if rep:
+                times[i].append(time.perf_counter() - t0)
+    for (info_run, _, plan), t in zip(runs, times):
+        plan.close()
+        row = dict(ms_per_link=1e3 * float(np.median(t)), spread_ms=[1e3 * min(t), 1e3 * max(t)], **info_run)
+        res['runs'].append(row)
+        print('C4 r=%d K=%d %-28s %9.2f ms per link  [%.2f .. %.2f]'
+              % (r, K, json.dumps(info_run), row['ms_per_link'], *row['spread_ms']))
+    single = next(x['ms_per_link'] for x in res['runs'] if x['run'] == 'cd+pbnlc')
+    for x, k in zip(res['runs'][:2], res['kernel']):
+        ext = (x['ms_per_link'] - single - k['xpm_kernel_ms']) / x['interferers']
+        x['extraction_ms_per_interferer'] = ext
+        print('extraction (copy, band filter at N, gather, projection): %.2f ms per interferer (%d interferers)'
+              % (ext, x['interferers']))
+    cd.close()
+    fld.close()
+    tx.close()
+    res['card_after'] = card()
+    print('card (after the runs):', res['card_after'])
+    if a.out:
+        os.makedirs(a.out, exist_ok=True)
+        with open(os.path.join(a.out, 'pbnlc_xpm_time.json'), 'w') as f:
+            json.dump(res, f, indent=1)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--nsymb', type=int, default=1 << 16)
@@ -239,13 +339,16 @@ def main():
     ap.add_argument('--ks', default='4,8,16,32,64')
     ap.add_argument('--decim', default=None, help='single-channel PB-NLC at these decimations (comma list) on C4 and C2')
     ap.add_argument('--table', action='store_true', help='the triplet table on the host against the device')
-    ap.add_argument('--nch', type=int, default=9, help='channels of the C4 multiplex (with --decim or --table)')
+    ap.add_argument('--xpm', action='store_true', help='XPM-aware single-channel PB-NLC on C4 (2 and all interferers)')
+    ap.add_argument('--nch', type=int, default=9, help='channels of the C4 multiplex (with --decim, --table or --xpm)')
     ap.add_argument('--out', default=None, help='directory for pbnlc_time.json (pbnlc_channel_time.json with --decim)')
     a = ap.parse_args()
     if a.decim:
         return channel_main(a)
     if a.table:
         return table_main(a)
+    if a.xpm:
+        return xpm_main(a)
     import torch
     torch.cuda.init()
     info = card()
